@@ -2,7 +2,7 @@
 """bench.py -- BASELINE.json's headline metric on B200: encode Mpix/s of one synthetic 8320x40000 BGR image,
 quality 95, 4:2:2, optimized Huffman (config 2), bit-exact with libjpeg-turbo.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 N=1 : the whole image on one GPU.  N>1 (torchrun, one rank per GPU): the image is cut into MCU-row strips, one per
       GPU, stitched through a 4 KB per-strip record exchanged over peer memory (NCCL all_gather as the fallback).
@@ -12,9 +12,12 @@ pinned HOST buffers (H2D of the pixels and D2H of the JPEG inside the timed regi
 
 --impl reference: the reference's nvJPEG path (baseline/ref_nvjpeg.cu = its exact call sequence, see that file) on
       the same GPU, else -- if nvJPEG cannot run -- libjpeg-turbo (cv2.imencode) on the host cores.
+--dump-outputs DIR: the JPEG of the last timed step as .npy arrays (see dump_outputs), so that two builds can be
+      compared output for output; the input image is the same on every run.
 """
 import argparse
 import ctypes as C
+import hashlib
 import json
 import os
 import subprocess
@@ -26,6 +29,7 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the tree may be read-only: leave no __pycache__ in it
 
 W, H, QUALITY, CSS, OPT = 8320, 40000, 95, "422", 1
 WORKLOAD = "8320x40000 BGR synth(seed=0,amp=8), q95, 4:2:2, optimized Huffman (BASELINE.json configs[1])"
@@ -51,6 +55,22 @@ def measured_peak():
             return float(json.load(f)["hbm_gbs"]), "measured"
     except Exception:
         return PEAKS_FALLBACK_GBS, "fallback"
+
+
+DUMP_SAMPLE = 1 << 22
+
+
+def dump_outputs(d, jpg):
+    """Writes the JPEG bytes `jpg` as float arrays: jpeg_length.npy, jpeg_sha256.npy (the 32 digest bytes of the whole
+    stream), jpeg_index.npy and jpeg_bytes.npy (the bytes at those positions: all of them up to DUMP_SAMPLE bytes, else
+    a sorted sample of positions drawn with seed 0, so that the directory stays below 64 MB)."""
+    os.makedirs(d, exist_ok=True)
+    n = int(jpg.size)
+    idx = np.arange(n) if n <= DUMP_SAMPLE else np.unique(np.random.default_rng(0).integers(0, n, DUMP_SAMPLE))
+    np.save(os.path.join(d, "jpeg_length.npy"), np.array([n], np.float64))
+    np.save(os.path.join(d, "jpeg_sha256.npy"), np.frombuffer(hashlib.sha256(jpg.tobytes()).digest(), np.uint8).astype(np.float32))
+    np.save(os.path.join(d, "jpeg_index.npy"), idx.astype(np.float64))
+    np.save(os.path.join(d, "jpeg_bytes.npy"), jpg[idx].astype(np.float32))
 
 
 class ClockSampler(threading.Thread):
@@ -255,7 +275,7 @@ def run_b200(args, rank, world, local_rank):
     import torch
     import torch.distributed as dist
     import nvjpeg_imagecompressor_b200 as P
-    from nvjpeg_imagecompressor_b200.strips import StripEncoder, strip_rows
+    from nvjpeg_imagecompressor_b200.strips import StripEncoder, _view, strip_rows
     from nvjpeg_imagecompressor_b200.synth import synth_rows
     if not torch.cuda.is_available():
         raise SystemExit("bench.py needs a CUDA device: there is no CPU path")
@@ -285,8 +305,7 @@ def run_b200(args, rank, world, local_rank):
         eng.set_stream(stream.cuda_stream)
 
         def step():   # asynchronous, like the strip step: the length word stays in HBM next to the bytes
-            eng.encode_device(img.data_ptr(), W * 3, W, H)
-            return 0
+            return eng.encode_device(img.data_ptr(), W * 3, W, H)[0]
     else:
         enc = StripEncoder(W, H, QUALITY, bool(OPT), CSS, device=local_rank)
         exchange = {"peer memory": "NVLink stores into the peers' memory + flags (no collective)",
@@ -296,13 +315,12 @@ def run_b200(args, rank, world, local_rank):
 
         def step():
             enc.encode_strip(img.data_ptr(), W * 3)
-            return 0
 
     if sampler:
         sampler.start()
     with torch.cuda.stream(stream):
         for _ in range(args.warmup):
-            nbytes = step()
+            step()
         barrier()
         if sampler:
             sampler.t_lo = time.time()
@@ -312,12 +330,19 @@ def run_b200(args, rank, world, local_rank):
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
         for _ in range(args.steps):
-            nbytes = step()
+            out_ptr = step()
         e1.record(stream)
         barrier()
         ms_total = e0.elapsed_time(e1)
         launches = eng.launch_count() - launches0
         nbytes = eng.encode_finish()   # device-side checks of the last encode + its length (N>1: this rank's strip)
+        last_jpeg = None   # host copy of the last timed step's JPEG, taken before any later step overwrites it
+        if args.dump_outputs:
+            if world == 1:
+                last_jpeg = _view(out_ptr, (nbytes,), "|u1", dev).cpu().numpy()
+            else:
+                whole = enc.gather_jpeg(0)
+                last_jpeg = whole.cpu().numpy() if rank == 0 else None
         eng.enable_timing(True)
         ks = args.steps if world == 1 else max(1, min(args.steps, 5))
         for _ in range(ks):
@@ -542,6 +567,8 @@ def run_b200(args, rank, world, local_rank):
         digest = hashlib.sha256(whole.cpu().numpy().tobytes()).hexdigest() if rank == 0 else None
     if rank != 0:
         return None
+    if last_jpeg is not None:
+        dump_outputs(args.dump_outputs, last_jpeg)
     bit_exact = None
     try:   # libjpeg-turbo's digest of this very encode (tests/golden/make_golden.py, cv2.imencode in the build container)
         with open(os.path.join(os.path.dirname(os.path.abspath(__file__)), "tests", "golden", "golden.json")) as f:
@@ -648,7 +675,13 @@ def main():
     ap.add_argument("--ref-progressive", type=int, default=0,
                     help="1 = nvJPEG progressive encoding as the reference ships it (ImageCompressorImpl.cu:28); default is "
                          "baseline sequential, the stream type this engine and the north-star target")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="write the JPEG of the last timed step to DIR as .npy arrays (--impl b200)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of --impl b200")
     args.warmup = max(3, args.warmup) if args.impl == "b200" else max(1, args.warmup)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))

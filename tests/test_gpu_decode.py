@@ -233,36 +233,33 @@ def test_headline_full_image_decode_digest(P, golden, oracle):
         eng.close()
 
 
+def _nvjpeg_golden():
+    """What the reference's nvJPEG path wrote (tests/golden/make_golden_nvjpeg.py, which runs the nvJPEG harness
+    baseline/ref_nvjpeg.cu = the reference's call sequence): small streams with libjpeg-turbo's pixel digests, and
+    nvJPEG's size and PSNR at 4096x3072."""
+    import json
+    with open(os.path.join(HERE, "golden", "golden_nvjpeg.json")) as f:
+        return json.load(f)
+
+
+def _decode_nvjpeg_files(P, progressive):
+    files = [c for c in _nvjpeg_golden()["files"] if c["progressive"] == progressive]
+    assert len(files) == 3
+    eng = P.Engine(max(c["W"] for c in files), max(c["H"] for c in files), 95, True, "444")
+    for c in files:
+        jpg = np.fromfile(os.path.join(HERE, "golden", c["file"]), np.uint8)
+        assert sha(jpg) == c["jpeg_sha256"], c
+        if progressive:
+            assert 0xC2 in jpg[:1024].tolist()   # a progressive frame header
+        got = eng.decode(jpg)
+        assert got.shape == (c["H"], c["W"], 3) and sha(got) == c["decoded_sha256"], c
+    eng.close()
+
+
 def test_decode_nvjpeg_streams(P):
     """BASELINE.json config 5: JPEGs written by the reference's nvJPEG path (baseline sequential, optimised Huffman, no
-    restart markers) decode to exactly the pixels libjpeg-turbo produces from the same bytes. Uses the nvJPEG harness
-    (baseline/_ref/libref_nvjpeg.so = the reference's call sequence); skipped where it was not built."""
-    import ctypes as C
-    cv2 = pytest.importorskip("cv2")
-    lib = os.path.join(os.path.dirname(HERE), "baseline", "_ref", "libref_nvjpeg.so")
-    if not os.path.exists(lib):
-        pytest.skip("nvJPEG harness not built")
-    L = C.CDLL(lib)
-    from nvjpeg_imagecompressor_b200.synth import synth
-    W, H = 2048, 1536
-    img = synth(W, H, 3).cpu().numpy()
-    eng = P.Engine(W, H, 95, True, "444")
-    for css in (1, 0, 3):   # the harness' css numbering = this library's (444, 422, 440, 420, 411)
-        h = C.c_void_p()
-        assert L.ref_create(W, H, 90, 1, css, 0, C.byref(h)) == 0
-        if L.ref_build_compress_env(h) != 0:
-            pytest.skip("nvJPEG cannot run here")
-        out = np.empty(W * H * 3, np.uint8)
-        n = C.c_size_t(0)
-        rc = L.ref_compress(h, C.c_void_p(img.ctypes.data), C.c_size_t(W * 3), C.c_void_p(out.ctypes.data), C.c_size_t(out.size), C.byref(n))
-        assert rc == 0
-        jpg = out[: n.value].copy()
-        L.ref_destroy(h)
-        want = cv2.imdecode(jpg, cv2.IMREAD_COLOR)
-        assert want is not None and want.shape == (H, W, 3)
-        got = eng.decode(jpg)
-        assert np.array_equal(got, want), f"css {css}: {np.count_nonzero(got != want)} values differ"
-    eng.close()
+    restart markers; 4:2:2, 4:4:4 and 4:2:0) decode to exactly the pixels libjpeg-turbo produces from the same bytes."""
+    _decode_nvjpeg_files(P, 0)
 
 
 def test_against_reference_nvjpeg_output(P):
@@ -270,32 +267,18 @@ def test_against_reference_nvjpeg_output(P):
     (4:2:2, q95, optimised Huffman): file size within 2 %, PSNR of the reconstruction not below nvJPEG's by more than
     0.05 dB. (Measured: +1.5 % bytes and +0.39 dB -- the bit-exact libjpeg-turbo arithmetic reconstructs better than
     nvJPEG's, so "within 0.05 dB" can only hold one-sided while the stream is pinned to libjpeg-turbo.)"""
-    import ctypes as C
-    lib = os.path.join(os.path.dirname(HERE), "baseline", "_ref", "libref_nvjpeg.so")
-    if not os.path.exists(lib):
-        pytest.skip("nvJPEG harness not built")
-    L = C.CDLL(lib)
+    ref = _nvjpeg_golden()["size_psnr"]
     from nvjpeg_imagecompressor_b200.synth import synth
-    W, H = 4096, 3072
-    img = synth(W, H, 0).cpu().numpy()
-    h = C.c_void_p()
-    assert L.ref_create(W, H, 95, 1, 1, 0, C.byref(h)) == 0
-    if L.ref_build_compress_env(h) != 0:
-        pytest.skip("nvJPEG cannot run here")
-    out = np.empty(W * H * 3, np.uint8)
-    n = C.c_size_t(0)
-    assert L.ref_compress(h, C.c_void_p(img.ctypes.data), C.c_size_t(W * 3), C.c_void_p(out.ctypes.data), C.c_size_t(out.size), C.byref(n)) == 0
-    ref_jpg = out[: n.value].copy()
-    L.ref_destroy(h)
-    eng = P.Engine(W, H, 95, True, "422")
+    W, H = ref["W"], ref["H"]
+    img = synth(W, H, ref["seed"], ref["amp"]).cpu().numpy()
+    eng = P.Engine(W, H, ref["quality"], bool(ref["optimize"]), ref["css"])
     mine = eng.encode(img)
-    psnr_ref = eng.psnr(img, eng.decode(ref_jpg))[0]
     psnr_mine = eng.psnr(img, eng.decode(mine))[0]
     eng.close()
-    assert abs(mine.size - ref_jpg.size) <= 0.02 * ref_jpg.size, (mine.size, ref_jpg.size)
-    assert psnr_mine >= psnr_ref - 0.05, (psnr_mine, psnr_ref)
-    print(f"size {mine.size} vs nvJPEG {ref_jpg.size} ({100.0 * (mine.size - ref_jpg.size) / ref_jpg.size:+.2f} %), "
-          f"PSNR {psnr_mine:.3f} vs {psnr_ref:.3f} dB")
+    assert abs(mine.size - ref["jpeg_len"]) <= 0.02 * ref["jpeg_len"], (mine.size, ref["jpeg_len"])
+    assert psnr_mine >= ref["psnr"] - 0.05, (psnr_mine, ref["psnr"])
+    print(f"size {mine.size} vs nvJPEG {ref['jpeg_len']} ({100.0 * (mine.size - ref['jpeg_len']) / ref['jpeg_len']:+.2f} %), "
+          f"PSNR {psnr_mine:.3f} vs {ref['psnr']:.3f} dB")
 
 
 def test_restart_interval_streams(P, oracle, golden_rst):
@@ -361,31 +344,5 @@ def test_progressive_streams(P, oracle):
 
 def test_decode_reference_progressive_nvjpeg_streams(P):
     """The unmodified reference encodes PROGRESSIVE 4:4:4 (ImageCompressorImpl.cu:28,31): the streams its nvJPEG call
-    sequence writes with that setting decode to cv2.imdecode's pixels."""
-    import ctypes as C
-    cv2 = pytest.importorskip("cv2")
-    lib = os.path.join(os.path.dirname(HERE), "baseline", "_ref", "libref_nvjpeg.so")
-    if not os.path.exists(lib):
-        pytest.skip("nvJPEG harness not built")
-    L = C.CDLL(lib)
-    from nvjpeg_imagecompressor_b200.synth import synth
-    W, H = 1024, 768
-    img = synth(W, H, 3).cpu().numpy()
-    eng = P.Engine(W, H, 95, True, "444")
-    for css in (0, 1, 3):
-        h = C.c_void_p()
-        assert L.ref_create(W, H, 95, 1, css, 1, C.byref(h)) == 0   # progressive = 1
-        if L.ref_build_compress_env(h) != 0:
-            pytest.skip("nvJPEG cannot run here")
-        out = np.empty(W * H * 3, np.uint8)
-        n = C.c_size_t(0)
-        rc = L.ref_compress(h, C.c_void_p(img.ctypes.data), C.c_size_t(W * 3), C.c_void_p(out.ctypes.data), C.c_size_t(out.size), C.byref(n))
-        assert rc == 0
-        jpg = out[: n.value].copy()
-        L.ref_destroy(h)
-        assert 0xC2 in jpg[:1024].tolist()   # a progressive frame header
-        want = cv2.imdecode(jpg, cv2.IMREAD_COLOR)
-        assert want is not None and want.shape == (H, W, 3)
-        got = eng.decode(jpg)
-        assert np.array_equal(got, want), f"css {css}: {np.count_nonzero(got != want)} values differ"
-    eng.close()
+    sequence writes with that setting (4:4:4, 4:2:2 and 4:2:0) decode to cv2.imdecode's pixels."""
+    _decode_nvjpeg_files(P, 1)
