@@ -254,10 +254,8 @@ B2J_API int b2j_debug_read(b2j_ctx *ctx, int what, void *dst, size_t cap, size_t
  * two-pass recovery path); output is unchanged */
 /* bit2 (B2J_DEBUG_SHORT_DECODE_SCHEDULE): the decoder's unchecked synchronisation schedule is cut to one launch, so
  * every multi-chunk image takes the validated retry; output is unchanged */
-/* bit3 (B2J_DEBUG_FUSED): whole-image encodes without restart markers run entropy coding, tile scan and byte stuffing
- * as ONE kernel (k_pack_stuff) instead of k_pack + k_scan_tiles + k_stuff: same bytes, slower on B200 (DESIGN.md 7);
- * the per-tile bit buffers (B2J_DBG_SLOTS) and B2J_DBG_TILE_BITS are not filled on that path */
-enum { B2J_DEBUG_COEF = 1, B2J_DEBUG_SMALL_PACK_BUFFERS = 2, B2J_DEBUG_SHORT_DECODE_SCHEDULE = 4, B2J_DEBUG_FUSED = 8 };
+/* bit3: unused and ignored; older callers may still set it, so it must not be given a new meaning */
+enum { B2J_DEBUG_COEF = 1, B2J_DEBUG_SMALL_PACK_BUFFERS = 2, B2J_DEBUG_SHORT_DECODE_SCHEDULE = 4 };
 B2J_API int b2j_set_debug(b2j_ctx *ctx, int flags);
 
 /* per-stage device times (ms) of the last encode/decode, measured with CUDA events on the context stream */

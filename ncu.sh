@@ -1,11 +1,10 @@
 #!/bin/bash
 # ncu.sh -- the committed Nsight Compute captures behind profiles/ (the reference's ncu.sh:1 profiles its own binary the
-# same way). Run on a B200 box (gpurun -- './ncu.sh <tag> [encode|decode|metrics|fused|launches]'); read the reports on the
+# same way). Run on a B200 box (./ncu.sh <tag> [encode|decode|metrics|launches]); read the reports on the
 # CPU box with scripts/ncu_export.py. Every profiled command first runs plain and must exit 0.
 #   encode   : --set full of one launch of every encode kernel, headline config (8320x40000 4:2:2 q95 optimised)
 #   decode   : --set full of one decode of the headline JPEG
 #   metrics  : --set full of k_diff_psnr (difference map + SSD), k_idct and k_upcolor on the secondary-compression path
-#   fused    : --set full of k_pack_stuff (the single-kernel entropy coder behind B2J_DEBUG_FUSED), headline config
 #   launches : per-launch device times of bench.py (gpu__time_duration only)
 set -e
 TAG=${1:-r02}
@@ -29,16 +28,11 @@ metrics)
     $NCU --set full --import-source on -k regex:"k_diff_psnr|k_idct|k_upcolor" -s 3 -c 3 \
         -f -o $OUT/prof_${TAG}_metrics python scripts/secondary_multi.py --iters 1 > $OUT/${TAG}_metrics_ncu.log 2>&1
     ;;
-fused)
-    python scripts/stage_times.py --iters 3 --debug 8 > $OUT/${TAG}_fused_stage_times.jsonl
-    $NCU --set full --import-source on -k regex:"k_pack_stuff" -s 1 -c 1 \
-        -f -o $OUT/prof_${TAG}_fused python scripts/stage_times.py --iters 3 --debug 8 > $OUT/${TAG}_fused_ncu.log 2>&1
-    ;;
 launches)
     python bench.py --steps 2 --warmup 3 > $OUT/${TAG}_bench_plain.json
     $NCU --metrics gpu__time_duration.sum -k regex:"^k_|b2j" -c 400 --csv --log-file $OUT/launches_${TAG}.csv \
         python bench.py --steps 2 --warmup 3 > $OUT/${TAG}_launches.log 2>&1
     ;;
-*) echo "usage: $0 <tag> [encode|decode|metrics|fused|launches]"; exit 2;;
+*) echo "usage: $0 <tag> [encode|decode|metrics|launches]"; exit 2;;
 esac
 echo "ncu.sh $TAG $WHAT done"

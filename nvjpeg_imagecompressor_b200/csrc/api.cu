@@ -68,7 +68,6 @@ struct b2j_ctx {
     size_t slot_words_cap;
     int debug;
     uint32_t *d_slots, *d_tile_bits;
-    uint8_t *d_fuse;                            // k_pack_stuff's per-item look-back state (40 bytes per tile)
     uint64_t *d_tile_off, *d_desc, *d_sdesc;   // look-back descriptors: byte stuffing, tile scan
     uint32_t *d_chunk_tile;                    // [ndesc] tile holding the first bit of every k_stuff chunk (written by the scan)
     size_t ndesc, nsdesc;
@@ -184,8 +183,8 @@ const char *b2j_last_error(const b2j_ctx *ctx) { return ctx ? ctx->err : "null c
 
 static int ensure_tiles(b2j_ctx *ctx, const Geom &g) {
     if (g.ntiles <= ctx->tiles_cap) return B2J_OK;
-    cudaFree(ctx->d_slots); cudaFree(ctx->d_tile_bits); cudaFree(ctx->d_tile_off); cudaFree(ctx->d_recs); cudaFree(ctx->d_fuse);
-    ctx->d_slots = nullptr; ctx->d_tile_bits = nullptr; ctx->d_tile_off = nullptr; ctx->d_recs = nullptr; ctx->d_fuse = nullptr; ctx->tiles_cap = 0;
+    cudaFree(ctx->d_slots); cudaFree(ctx->d_tile_bits); cudaFree(ctx->d_tile_off); cudaFree(ctx->d_recs);
+    ctx->d_slots = nullptr; ctx->d_tile_bits = nullptr; ctx->d_tile_off = nullptr; ctx->d_recs = nullptr; ctx->tiles_cap = 0;
     const int n = g.ntiles + g.ntiles / 8 + 16;
     const bool was_ready = ctx->enc_ready;
     ctx->enc_ready = false;   // stays false if an allocation below fails: no phase launches with null tile buffers
@@ -193,7 +192,6 @@ static int ensure_tiles(b2j_ctx *ctx, const Geom &g) {
     CK(cudaMalloc(&ctx->d_tile_bits, (size_t)(n + 1) * 4));
     CK(cudaMalloc(&ctx->d_tile_off, (size_t)(n + 2) * 8));
     CK(cudaMalloc(&ctx->d_recs, (size_t)(n + 1) * sizeof(TileRec)));
-    CK(cudaMalloc(&ctx->d_fuse, (size_t)(n + 1) * 40));   // k_pack_stuff: two look-back descriptors + the tail word per item, two items per tile
     ctx->tiles_cap = n;
     ctx->enc_ready = was_ready;
     return B2J_OK;
@@ -278,7 +276,7 @@ void b2j_destroy(b2j_ctx *ctx) {
     cudaFree(ctx->d_img); cudaFree(ctx->d_coef); cudaFree(ctx->d_pool); cudaFree(ctx->d_recs); cudaFree(ctx->d_slots); cudaFree(ctx->d_tile_bits);
     for (int i = 0; i < ctx->n_opened; i++) cudaIpcCloseMemHandle(ctx->peer_opened[i]);
     cudaFree(ctx->d_arena); cudaFree(ctx->d_peers);
-    cudaFree(ctx->d_chunk_tile); cudaFree(ctx->d_fuse);
+    cudaFree(ctx->d_chunk_tile);
     cudaFree(ctx->d_tile_off); cudaFree(ctx->d_ctrl);   // d_pred_in, d_sdesc, d_desc live in d_ctrl's allocation
     cudaFree(ctx->d_huff); cudaFree(ctx->d_quant); cudaFree(ctx->d_out); cudaFree(ctx->d_recon); cudaFree(ctx->d_diff);
     cudaFree(ctx->d_rplanes); cudaFree(ctx->d_rtb);
@@ -514,30 +512,11 @@ int b2j_strip_state_get(b2j_ctx *ctx, b2j_strip_state *st) {
 }
 
 // ------------------------------------------------------------------------------------------ whole-image encode
-// Entropy coding of a whole image: k_pack -> k_scan_tiles -> k_stuff (the strips' kernels). B2J_DEBUG_FUSED selects the
-// single-kernel variant k_pack_stuff instead (no restart markers): bit-exact, measured SLOWER on B200 (1.03 ms against
-// 0.52 + 0.01 + 0.29 ms for the headline image, profiles/r02h_fused_summary.txt) because every item has to wait for
-// the slowest of the few thousand items in flight before it learns its bit offset, and again for its byte offset;
-// kept for that measurement and as a second implementation the tests compare.
+// Entropy coding of a whole image: k_pack -> k_scan_tiles -> k_stuff (the strips' kernels).
 static int enc_tail(b2j_ctx *ctx, int width, int height) {
-    if (ctx->rst_rows || !(ctx->debug & B2J_DEBUG_FUSED)) {
-        int rc = b2j_strip_phase1b(ctx); if (rc) return rc;
-        rc = b2j_strip_phase2(ctx, width, height); if (rc) return rc;
-        return b2j_strip_phase3(ctx, 0, 0xFF, 3);
-    }
-    const int n = fuse_items(ctx->g.ntiles);
-    uint64_t *desc_bits = reinterpret_cast<uint64_t *>(ctx->d_fuse), *desc_bytes = desc_bits + n;
-    uint32_t *tail = reinterpret_cast<uint32_t *>(desc_bytes + n);
-    CK(launch_dc_edge_hist(ctx->d_recs, ctx->g, ctx->d_pred_in, ctx->d_ctrl->hist, ctx->d_ctrl->rec.last_dc, ctx->p.optimize, ctx->d_pool, 1, nullptr, 0, ctx->stream,
-                           reinterpret_cast<uint32_t *>(ctx->d_fuse)));
-    tick(ctx, 3);
-    CK(launch_tables(ctx->d_ctrl->hist, ctx->p.optimize, ctx->d_huff, ctx->d_quant, width, height, ctx->g.hs, ctx->g.vs, ctx->d_out, 1, 0, &ctx->d_ctrl->huff_err, ctx->stream));
-    tick(ctx, 4);
-    CK(launch_pack_stuff(ctx->d_pool, ctx->d_recs, ctx->g, ctx->d_huff, ctx->d_slots, ctx->debug & 2, desc_bits, desc_bytes, tail,
-                         &ctx->d_ctrl->ticket, ctx->d_out, ctx->out_cap, &ctx->d_ctrl->out_len, &ctx->d_ctrl->err, ctx->stream));
-    tick(ctx, 5); tick(ctx, 6); tick(ctx, 7);   // the pack interval is the fused kernel; scan and stuff read 0
-    ctx->launches += 3;
-    return B2J_OK;
+    int rc = b2j_strip_phase1b(ctx); if (rc) return rc;
+    rc = b2j_strip_phase2(ctx, width, height); if (rc) return rc;
+    return b2j_strip_phase3(ctx, 0, 0xFF, 3);
 }
 
 int b2j_encode_device(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width, int height, const uint8_t **d_out,

@@ -190,7 +190,6 @@ __device__ __forceinline__ void st_volatile_u64(uint64_t *p, uint64_t v) {
 
 // Decoupled look-back over 64-bit descriptors; executed by ONE full warp. Chunk ids must be handed out in
 // launch order (atomic ticket) so every predecessor is resident or finished. Returns the exclusive prefix.
-template <bool BACKOFF = false>   // BACKOFF: waits double from 64 ns to ~1 us (many independent waiters that should not steal issue slots)
 __device__ __forceinline__ uint64_t lookback_exclusive(uint64_t *desc, int id, uint64_t local, uint32_t *err) {
     const int lane = threadIdx.x & 31;
     if (id == 0) {
@@ -204,13 +203,12 @@ __device__ __forceinline__ uint64_t lookback_exclusive(uint64_t *desc, int id, u
         int idx = j - lane;
         uint64_t d = LB_INC;
         if (idx >= 0) {
-            unsigned spins = 0, ns = 64;
+            unsigned spins = 0;
             d = ld_volatile_u64(&desc[idx]);
             while ((d >> 62) == 0) {
-                if (BACKOFF) { __nanosleep(ns); ns = min(ns * 2u, 1024u); }
-                else __nanosleep(20);
+                __nanosleep(20);
                 d = ld_volatile_u64(&desc[idx]);
-                if (++spins > (BACKOFF ? (1u << 18) : (1u << 22))) { *err = 1; d = LB_INC; break; }  // never hang the GPU
+                if (++spins > (1u << 22)) { *err = 1; d = LB_INC; break; }  // never hang the GPU
             }
         }
         unsigned inc = __ballot_sync(0xffffffffu, (d >> 62) == 2);

@@ -529,19 +529,12 @@ k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__r
 __global__ void __launch_bounds__(256)
 k_dc_edge_hist(const TileRec *__restrict__ recs, Geom g, const int16_t *__restrict__ pred_in,
                uint32_t *__restrict__ ghist, int16_t *__restrict__ last_dc, int do_hist,
-               uint32_t *__restrict__ pool, int resolve, StripRecord *__restrict__ xr, int rst_tiles,
-               uint32_t *__restrict__ fuse_zero) {
+               uint32_t *__restrict__ pool, int resolve, StripRecord *__restrict__ xr, int rst_tiles) {
     __shared__ uint32_t s_h[2][16];   // DC categories 0..11 of the two DC tables, aggregated per CTA
     pdl_trigger();
     pdl_wait();
     const int t = blockIdx.x * blockDim.x + threadIdx.x;
     const int ntile = g.tiles_x * g.mcuy;
-    // k_pack_stuff's look-back state (two items per tile: two descriptors + the tail word each), cleared on the way
-    if (fuse_zero && t < ntile * 3) {
-#pragma unroll
-        for (int k = 0; k < 4; k++)
-            if (4 * t + k < 10 * ntile) fuse_zero[4 * t + k] = 0;
-    }
     if (threadIdx.x < 32) s_h[threadIdx.x >> 4][threadIdx.x & 15] = 0;
     __syncthreads();
     if (t < ntile * 3 && (do_hist || resolve) && !(xr && t < 3)) {
@@ -626,10 +619,9 @@ cudaError_t launch_fdct(const uint8_t *img, size_t step, const Geom &g, const Qu
 }
 
 cudaError_t launch_dc_edge_hist(const TileRec *recs, const Geom &g, const int16_t *pred_in, uint32_t *hist,
-                                int16_t *last_dc, int do_hist, uint32_t *pool, int resolve, StripRecord *xr, int rst_tiles, cudaStream_t s,
-                                uint32_t *fuse_zero) {
+                                int16_t *last_dc, int do_hist, uint32_t *pool, int resolve, StripRecord *xr, int rst_tiles, cudaStream_t s) {
     const int n = max(64, g.tiles_x * g.mcuy * 3);
-    return launch_pdl(k_dc_edge_hist, dim3((n + 255) / 256), dim3(256), 0, s, recs, g, pred_in, hist, last_dc, do_hist, pool, resolve, xr, rst_tiles, fuse_zero);
+    return launch_pdl(k_dc_edge_hist, dim3((n + 255) / 256), dim3(256), 0, s, recs, g, pred_in, hist, last_dc, do_hist, pool, resolve, xr, rst_tiles);
 }
 
 }  // namespace b2j

@@ -405,8 +405,8 @@ __device__ __forceinline__ void load_tokens(const uint4 *tk4, uint32_t v0, uint3
 }
 
 // The warp's share [lo, hi) of the walk, coded into `buf` starting at bit `run`; returns the bit position after it.
-template <bool WINDOWED, class SH>
-__device__ __forceinline__ int pack_scatter(const SH &sh, uint32_t *buf, uint32_t nwords, const uint4 *tk4, uint32_t a,
+template <bool WINDOWED>
+__device__ __forceinline__ int pack_scatter(const PackShared &sh, uint32_t *buf, uint32_t nwords, const uint4 *tk4, uint32_t a,
                                             uint32_t lo, uint32_t hi, int run, int lane, uint32_t zr_y, uint32_t zr_c) {
     for (uint32_t s0 = lo; s0 < hi; s0 += PACK_STEP) {
         const uint32_t v0 = s0 + lane * PACK_K;
@@ -467,8 +467,7 @@ __device__ __forceinline__ int pack_scatter(const SH &sh, uint32_t *buf, uint32_
 }
 
 // bits of the warp's share without coding them (two-pass path)
-template <class SH>
-__device__ __forceinline__ uint32_t pack_length(const SH &sh, const uint4 *tk4, uint32_t a, uint32_t lo, uint32_t hi, int lane) {
+__device__ __forceinline__ uint32_t pack_length(const PackShared &sh, const uint4 *tk4, uint32_t a, uint32_t lo, uint32_t hi, int lane) {
     uint32_t len = 0;
     for (uint32_t v0 = lo + lane * PACK_K; v0 < hi; v0 += PACK_STEP) {
         uint32_t w[PACK_K];
@@ -506,8 +505,7 @@ __device__ __forceinline__ void pack_flush_shared_words(uint32_t *bnd, const uin
 // Code tables in token-bin order (common.cuh tok_bin): code << size, and the full length per (ZRL count, bin); -> the
 // ZRL (0xF0) codes of the two AC tables as code << 8 | length. The tables are k_tables' output: every load of them must
 // stay behind pdl_wait() (volatile: a load through a const __restrict__ pointer may be hoisted above the wait).
-template <class SH>
-__device__ __forceinline__ void pack_build_tables(SH &sh, const HuffDev *huff, int tid, uint32_t &zr_y, uint32_t &zr_c) {
+__device__ __forceinline__ void pack_build_tables(PackShared &sh, const HuffDev *huff, int tid, uint32_t &zr_y, uint32_t &zr_c) {
     const volatile HuffDev *vh = huff;
     for (int i = tid; i < 1024; i += PACK_THREADS) {
         const uint32_t bin = (uint32_t)i, t = bin_table(bin), nb = (bin >> 2) & 15u;
@@ -1024,318 +1022,6 @@ k_stuff(StuffArgs a) {
 }
 
 // ------------------------------------------------------------------------------------------------------
-// k_pack_stuff: k_pack, the tile scan and k_stuff in ONE kernel for whole-image encodes without restart markers: the
-// coded bits never travel through HBM and there is no second kernel with its own latency chain. The unit of work is
-// an ITEM = one of FUSE_PARTS consecutive parts of an fdct tile's token run, and one WARP does everything for its
-// item on its own -- the CTA only shares the code tables, so the item loop has no CTA barrier at all and the
-// latencies of the look-backs are covered by the other warps of the SM. Items are handed out by a ticket (every
-// predecessor of an item is running or done):
-//   1. k_pack's coding of the item's tokens into the warp's bit buffer, from bit 32 (word 0 is the lead word)
-//   2. the stream's last 8 bits up to the item's end are published (`tail`); decoupled look-back #1 over the items'
-//      BIT counts -> G = the item's bit offset in the entropy-coded segment. The item owns the stream bytes that END
-//      inside it: the first one starts with the G & 7 last bits before the item (the predecessor's tail -> lead
-//      word), the bits after its last whole byte go to the next item; the image's last item pads with 1-bits.
-//   3. 16-byte pieces of that byte string (one per lane and round, straight from the bit buffer with a funnel shift
-//      by the phase): 0xFF count -> warp scan -> the item's stuffed size -> decoupled look-back #2 over the BYTE
-//      counts -> the item's place in the output
-//   4. round by round: the pieces' bytes staged with their 0x00s (k_stuff's PRMT expansion), copied out as 16-byte
-//      vectors
-// Items whose bits do not fit the warp's buffer (q ~ 100) are coded window by window into global memory (the slot
-// area of the unfused path) and stuffed from there after a counting pass.
-constexpr int FUSE_PARTS = 2;                           // items per fdct tile
-constexpr int FUSE_BITS_WORDS = 1024;                   // bit buffer per warp: 32 kbit (a typical item is ~13 kbit)
-constexpr int FUSE_BUF_WORDS = FUSE_BITS_WORDS + 16;    // + lead word and zero words behind
-constexpr int FUSE_ROUND = 32 * 16;                     // unstuffed bytes per round: one 16-byte piece per lane
-constexpr int FUSE_STAGE_WORDS = (2 * FUSE_ROUND + 64) / 4;
-constexpr int FUSE_CTAS = 7;                            // resident CTAs per SM (shared memory)
-constexpr uint32_t FUSE_DENSE_TOKENS = 3500;            // above this the item may not fit the buffer: coded through global memory
-constexpr int FUSE_SLOT_WORDS = SLOT_WORDS / FUSE_PARTS;
-
-struct FusedShared {
-    uint32_t code[1024];
-    uint8_t len[4096];
-    uint32_t lut[16];
-    uint32_t buf[PACK_WARPS][FUSE_BUF_WORDS];
-    uint32_t stage[PACK_WARPS][FUSE_STAGE_WORDS];
-};
-
-__device__ __forceinline__ uint32_t ld_volatile_u32(const uint32_t *p) {
-    uint32_t v;
-    asm volatile("ld.volatile.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-    return v;
-}
-__device__ __forceinline__ void st_volatile_u32(uint32_t *p, uint32_t v) {
-    asm volatile("st.volatile.global.u32 [%0], %1;" ::"l"(p), "r"(v) : "memory");
-}
-
-// the last 8 bits of the stream up to the end of item t (published by the item's warp as soon as it has coded them)
-__device__ __forceinline__ uint32_t fuse_wait_tail(const uint32_t *tail, int t, uint32_t *err) {
-    uint32_t v = ld_volatile_u32(&tail[t]);
-    unsigned spins = 0;
-    while (!(v >> 31)) {
-        __nanosleep(100);
-        v = ld_volatile_u32(&tail[t]);
-        if (++spins > (1u << 20)) { *err = 1; break; }   // never hang the GPU
-    }
-    return v & 0xFFu;
-}
-
-// 16 bytes of the byte string whose bytes are the bits of src from bit 32 * w0 + ((32 - s) & 31) on: piece j, MSB first
-__device__ __forceinline__ void fuse_load_piece(const uint32_t *src, uint32_t w0, uint32_t s, uint32_t j, uint32_t (&w)[4]) {
-    const uint32_t *p = src + w0 + 4u * j;
-    uint32_t x[5];
-#pragma unroll
-    for (int q = 0; q < 5; q++) x[q] = p[q];
-#pragma unroll
-    for (int q = 0; q < 4; q++) w[q] = __funnelshift_l(x[q + 1], x[q], s);
-}
-// 0xFF bytes among the first nvalid bytes of a piece
-__device__ __forceinline__ uint32_t fuse_count_ff(const uint32_t (&w)[4], int nvalid) {
-    uint32_t nff = 0;
-#pragma unroll
-    for (int q = 0; q < 4; q++) {
-        uint32_t m = w[q] & (w[q] >> 4) & 0x0F0F0F0Fu;
-        m &= m >> 2;
-        m &= m >> 1;
-        m &= 0x01010101u;
-        if (nvalid < 16) {
-#pragma unroll
-            for (int bb = 0; bb < 4; bb++)
-                if (4 * q + bb >= nvalid) m &= ~(1u << (24 - 8 * bb));
-        }
-        nff += __popc(m);
-    }
-    return nff;
-}
-
-struct FuseArgs {
-    const uint32_t *pool;
-    const TileRec *recs;
-    int ntiles;
-    const HuffDev *huff;
-    uint32_t *slots;
-    uint32_t buf_words;                 // bit buffer words the coder may fill (tests: small -> the global-memory path)
-    uint64_t *desc_bits, *desc_bytes;   // look-back descriptors, one per item (zeroed)
-    uint32_t *tail;                     // per item: 1 << 31 | the stream's last 8 bits up to its end (zeroed)
-    uint32_t *ticket;                   // zeroed
-    uint8_t *out;
-    size_t cap;
-    uint64_t *out_len;
-    uint32_t *err;
-};
-
-// stuffed size of bytes [0, nb) of the byte string at (src, w0, s); one warp, result in every lane
-__device__ __forceinline__ uint32_t fuse_count_span(const uint32_t *src, uint32_t w0, uint32_t s, uint64_t nb) {
-    const int lane = threadIdx.x & 31;
-    uint32_t c = 0;
-#pragma unroll 1
-    for (uint64_t jb = (uint64_t)lane * 16u; jb < nb; jb += FUSE_ROUND) {
-        const int nvalid = (int)min((uint64_t)16, nb - jb);
-        uint32_t w[4];
-        fuse_load_piece(src, w0, s, (uint32_t)(jb >> 4), w);
-        c += (uint32_t)nvalid + fuse_count_ff(w, nvalid);
-    }
-#pragma unroll
-    for (int o = 16; o; o >>= 1) c += __shfl_xor_sync(0xffffffffu, c, o);
-    return c;
-}
-
-// Bytes [0, nb) of the byte string at (src, w0, s) -> stuffed -> a.out + hdr + goff, round by round (32 pieces of 16
-// bytes: offsets from a warp scan, bytes staged with their 0x00s, copied out as 16-byte vectors). One warp; `stage`
-// must be zero and is zero afterwards. Returns the stuffed size.
-__device__ __forceinline__ uint32_t fuse_stuff_span(uint32_t *stage, const uint32_t *lut, const FuseArgs &a, const uint32_t *src, uint32_t w0,
-                                                    uint32_t s, uint64_t nb, uint64_t goff, uint32_t hdr, bool last_span) {
-    const int lane = threadIdx.x & 31;
-    const uint32_t sbase = smem_u32(stage);
-    uint32_t done = 0;
-#pragma unroll 1
-    for (uint64_t r0 = 0; r0 < nb; r0 += FUSE_ROUND) {
-        const uint64_t jb = r0 + (uint64_t)lane * 16u;
-        const int nvalid = jb < nb ? (int)min((uint64_t)16, nb - jb) : 0;
-        uint32_t w[4] = {0, 0, 0, 0};
-        uint32_t cnt = 0;
-        if (nvalid) {
-            fuse_load_piece(src, w0, s, (uint32_t)(jb >> 4), w);
-            cnt = (uint32_t)nvalid + fuse_count_ff(w, nvalid);
-        }
-        uint32_t inc = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const uint32_t y = __shfl_up_sync(0xffffffffu, inc, o);
-            if (lane >= o) inc += y;
-        }
-        const uint32_t rt = __shfl_sync(0xffffffffu, inc, 31);
-        uint32_t o = inc - cnt;
-        if (nvalid == 16) {
-#pragma unroll
-            for (int q = 0; q < 4; q++) o += stuff_place_word(w[q], o, sbase, lut);
-        } else {
-            for (int k = 0; k < nvalid; k++) {
-                const uint32_t wq = (k >> 2) == 0 ? w[0] : ((k >> 2) == 1 ? w[1] : ((k >> 2) == 2 ? w[2] : w[3]));
-                const uint32_t byte = (wq >> (24 - 8 * (k & 3))) & 0xFFu;
-                atomicOr(&stage[o >> 2], byte << ((o & 3u) * 8u));
-                o += byte == 0xFFu ? 2u : 1u;
-            }
-        }
-        __syncwarp();
-        const uint64_t g0 = (uint64_t)hdr + goff + done;
-        if (g0 + rt + (last_span ? 2u : 0u) > a.cap) {
-            if (lane == 0) *a.err = 3;
-        } else {
-            uint8_t *dst = a.out + g0;
-            const uint8_t *s_out = reinterpret_cast<const uint8_t *>(stage);
-            // bytes up to the first 16-byte boundary of the output and behind the last one: one byte per lane
-            const uint32_t head = min(rt, (16u - (uint32_t)(reinterpret_cast<uintptr_t>(dst) & 15u)) & 15u);
-            const uint32_t nvec = (rt - head) >> 4, tail0 = head + 16u * nvec;
-            if ((uint32_t)lane < head) dst[lane] = s_out[lane];
-            if (tail0 + (uint32_t)lane < rt) dst[tail0 + lane] = s_out[tail0 + lane];
-            for (uint32_t v = lane; v < nvec; v += 32) {
-                const uint32_t k0 = head + 16u * v;
-                const uint32_t wi = k0 >> 2, bs = (k0 & 3u) * 8u;
-                const uint32_t x0 = stage[wi], x1 = stage[wi + 1], x2 = stage[wi + 2], x3 = stage[wi + 3], x4 = stage[wi + 4];
-                uint4 o4;
-                o4.x = __funnelshift_r(x0, x1, bs); o4.y = __funnelshift_r(x1, x2, bs);
-                o4.z = __funnelshift_r(x2, x3, bs); o4.w = __funnelshift_r(x3, x4, bs);
-                *reinterpret_cast<uint4 *>(dst + k0) = o4;
-            }
-        }
-        __syncwarp();
-        for (uint32_t v = lane; v * 16 < rt + 20; v += 32) reinterpret_cast<uint4 *>(stage)[v] = make_uint4(0, 0, 0, 0);
-        __syncwarp();
-        done += rt;
-    }
-    return done;
-}
-
-__global__ void __launch_bounds__(PACK_THREADS, FUSE_CTAS)
-k_pack_stuff(FuseArgs a) {
-    __shared__ __align__(16) FusedShared sh;
-    const int tid = threadIdx.x, lane = tid & 31, wid = tid >> 5;
-    for (int i = tid; i < PACK_WARPS * FUSE_BUF_WORDS; i += PACK_THREADS) sh.buf[0][i] = 0;
-    for (int i = tid; i < PACK_WARPS * FUSE_STAGE_WORDS; i += PACK_THREADS) sh.stage[0][i] = 0;
-    if (tid < 16) {   // PRMT selectors of stuff_place_word
-        uint32_t sel = 0;
-        int n = 0;
-        for (int i = 0; i < 4; i++) {
-            sel |= (uint32_t)i << (4 * n++);
-            if (tid & (1 << i)) sel |= 4u << (4 * n++);
-        }
-        for (; n < 8; n++) sel |= 4u << (4 * n);
-        sh.lut[tid] = sel;
-    }
-    pdl_wait();   // everything above ran under k_tables
-    uint32_t zr_y, zr_c;
-    pack_build_tables(sh, a.huff, tid, zr_y, zr_c);   // ends with a CTA barrier: the last one of this kernel
-    const uint32_t hdr = reinterpret_cast<const volatile HuffDev *>(a.huff)->hdr_len;
-    uint32_t *buf = sh.buf[wid], *stage = sh.stage[wid];
-    const int nitems = a.ntiles * FUSE_PARTS;
-    const int nwarps = (int)gridDim.x * PACK_WARPS;
-
-    for (;;) {
-        int it = 0;
-        if (lane == 0) it = (int)atomicAdd(a.ticket, 1u);
-        it = __shfl_sync(0xffffffffu, it, 0);
-        if (it >= nitems) break;
-        const bool last_item = it == nitems - 1;
-        const int t = it / FUSE_PARTS, part = it - t * FUSE_PARTS;
-        const TileRec rec = a.recs[t];
-        const uint32_t al = rec.base & 3u;
-        const uint4 *tk4 = reinterpret_cast<const uint4 *>(a.pool + (rec.base - al));
-        const uint32_t c0 = (uint32_t)(((uint64_t)rec.count * part) / FUSE_PARTS), c1 = (uint32_t)(((uint64_t)rec.count * (part + 1)) / FUSE_PARTS);
-        const uint32_t first = al + c0, hi = al + c1, lo = first & ~(uint32_t)(PACK_K - 1);
-        if (part == 0 && it + nwarps < nitems) {   // the tile some warp takes about one item time from now: on its way into L2
-            const TileRec nx = a.recs[(it + nwarps) / FUSE_PARTS];
-            const char *p0 = reinterpret_cast<const char *>(a.pool + (nx.base & ~31u));
-            const uint32_t nbytes = ((nx.base & 31u) + nx.count) * 4u;
-            for (uint32_t o = lane * 128u; o < nbytes; o += 32u * 128u) asm volatile("prefetch.global.L2 [%0];" ::"l"(p0 + o));
-        }
-
-        // ---- 1. code the item into the warp's buffer from bit 32 (or only measure it: dense items)
-        const bool dense = c1 - c0 > FUSE_DENSE_TOKENS;
-        uint32_t len;
-        if (!dense) len = (uint32_t)pack_scatter<false>(sh, buf, 1u + a.buf_words, tk4, first, lo, hi, 32, lane, zr_y, zr_c) - 32u;
-        else len = pack_length(sh, tk4, first, lo, hi, lane);
-        const bool two_pass = dense || len > a.buf_words * 32u - 64u;
-
-        // ---- 2. the stream's last 8 bits up to the end of this item; look-back #1
-        uint32_t pred_tail = 0xFFFFFFFFu;   // lane 0: the stream's last 8 bits before this item, once they were needed
-        if (!two_pass && lane == 0) {
-            const uint32_t take = min(8u, len), pos = 32u + len - take;
-            uint32_t acc = take ? __funnelshift_l(buf[(pos >> 5) + 1], buf[pos >> 5], pos & 31u) >> (32u - take) : 0u;
-            if (take < 8u) {   // an item of fewer than 8 bits (flat image, one MCU): the rest comes from before
-                pred_tail = it ? fuse_wait_tail(a.tail, it - 1, a.err) : 0u;
-                acc = ((pred_tail << take) | acc) & 0xFFu;
-            }
-            st_volatile_u32(&a.tail[it], 0x80000000u | acc);
-        }
-        const uint64_t G = lookback_exclusive<true>(a.desc_bits, it, len, a.err);
-        uint32_t *slot = a.slots + (size_t)it * FUSE_SLOT_WORDS;
-        if (two_pass) {
-            if (!dense) {   // the buffer holds a prefix of the item
-                for (uint32_t i = lane; i < (uint32_t)FUSE_BUF_WORDS; i += 32) buf[i] = 0;
-                __syncwarp();
-            }
-            const uint32_t nwords = (len + 31u) >> 5;
-            if (nwords + 4u > (uint32_t)FUSE_SLOT_WORDS) { if (lane == 0) *a.err = 4; continue; }   // beyond any real code table
-            for (uint32_t wbase = 0; wbase < nwords; wbase += FUSE_BITS_WORDS) {
-                pack_scatter<true>(sh, buf, FUSE_BITS_WORDS, tk4, first, lo, hi, -(int)(wbase * 32u), lane, zr_y, zr_c);
-                __syncwarp();
-                const uint32_t wn = min((uint32_t)FUSE_BITS_WORDS, nwords - wbase);
-                for (uint32_t i = lane; i < wn; i += 32) { slot[1u + wbase + i] = buf[i]; buf[i] = 0; }
-                __syncwarp();
-            }
-            if (lane == 0) {
-                slot[1u + nwords] = 0; slot[2u + nwords] = 0;   // the pieces read a little past the end
-                const uint32_t pos = len - 8u;                  // a dense item has thousands of bits
-                const uint32_t v = __funnelshift_l(slot[1u + (pos >> 5) + 1u], slot[1u + (pos >> 5)], pos & 31u) >> 24;
-                st_volatile_u32(&a.tail[it], 0x80000000u | v);
-            }
-        }
-        const uint32_t phi = (uint32_t)G & 7u;
-        const uint64_t nbytes64 = ((G + len + (last_item ? 7u : 0u)) >> 3) - (G >> 3);
-        if (lane == 0) {
-            uint32_t *wsrc = two_pass ? slot : buf;
-            uint32_t lead = 0;
-            if (phi) {   // the first byte starts with the last phi bits of the stream before this item (phi != 0: it > 0)
-                if (pred_tail == 0xFFFFFFFFu) pred_tail = fuse_wait_tail(a.tail, it - 1, a.err);
-                lead = pred_tail & ((1u << phi) - 1u);
-            }
-            wsrc[0] = lead;
-            if (last_item) {   // jchuff.c flush_bits: the last byte is filled with 1-bits
-                const uint32_t pad = (8u - ((phi + len) & 7u)) & 7u;
-                if (pad) {
-                    const uint32_t pos = 32u + len, wi = pos >> 5, sb = pos & 31u;
-                    const uint64_t v = ((uint64_t)((1u << pad) - 1u) << (64u - pad)) >> sb;
-                    wsrc[wi] |= (uint32_t)(v >> 32);
-                    if ((uint32_t)v) wsrc[wi + 1] |= (uint32_t)v;
-                }
-            }
-        }
-        __syncwarp();
-        const uint32_t w0 = phi ? 0u : 1u, s = (32u - phi) & 31u;
-        // ---- 3. + 4. (the same code for both homes of the bit string; separate calls keep the address spaces apart)
-        uint64_t end;
-        if (!two_pass) {
-            const uint32_t st = fuse_count_span(buf, w0, s, nbytes64);
-            const uint64_t goff = lookback_exclusive<true>(a.desc_bytes, it, st, a.err);
-            fuse_stuff_span(stage, sh.lut, a, buf, w0, s, nbytes64, goff, hdr, last_item);
-            end = (uint64_t)hdr + goff + st;
-            for (uint32_t i = lane; i < ((32u + len + 31u) >> 5) + 2u; i += 32) buf[i] = 0;
-            __syncwarp();
-        } else {
-            const uint32_t st = fuse_count_span(slot, w0, s, nbytes64);
-            const uint64_t goff = lookback_exclusive<true>(a.desc_bytes, it, st, a.err);
-            fuse_stuff_span(stage, sh.lut, a, slot, w0, s, nbytes64, goff, hdr, last_item);
-            end = (uint64_t)hdr + goff + st;
-        }
-        if (last_item && lane == 0) {
-            if (end + 2 <= a.cap) { a.out[end] = 0xFF; a.out[end + 1] = 0xD9; }
-            *a.out_len = end + 2;
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------------------
 cudaError_t launch_tables(const uint32_t *hist, int optimize, HuffDev *huff, const QuantDev *qd, int full_w, int full_h,
                           int hs, int vs, uint8_t *out, int emit_header, int restart_interval, uint32_t *err_out, cudaStream_t s) {
     return launch_pdl(k_tables, dim3(1), dim3(128), 0, s, hist, optimize, huff, qd, full_w, full_h, hs, vs, out, emit_header, restart_interval, err_out);
@@ -1520,18 +1206,6 @@ cudaError_t launch_set_seam(int *seam, int skip, int ext, cudaStream_t s) {
 cudaError_t launch_seam_from_bits(int *seam, const int64_t *bits_all, int rank, int world, cudaStream_t s) {
     k_seam_from_bits<<<1, 1, 0, s>>>(seam, bits_all, rank, world);
     return cudaGetLastError();
-}
-int fuse_items(int ntiles) { return ntiles * FUSE_PARTS; }
-cudaError_t launch_pack_stuff(const uint32_t *pool, const TileRec *recs, const Geom &g, const HuffDev *huff, uint32_t *slots,
-                              int small_buffers, uint64_t *desc_bits, uint64_t *desc_bytes, uint32_t *tail,
-                              uint32_t *ticket, uint8_t *out, size_t cap, uint64_t *out_len, uint32_t *err, cudaStream_t s) {
-    FuseArgs a;
-    a.pool = pool; a.recs = recs; a.ntiles = g.ntiles; a.huff = huff; a.slots = slots;
-    a.buf_words = small_buffers ? 48u : (uint32_t)FUSE_BITS_WORDS;
-    a.desc_bits = desc_bits; a.desc_bytes = desc_bytes; a.tail = tail; a.ticket = ticket; a.out = out; a.cap = cap;
-    a.out_len = out_len; a.err = err;
-    const int grid = std::min((g.ntiles * FUSE_PARTS + PACK_WARPS - 1) / PACK_WARPS, 148 * FUSE_CTAS);
-    return launch_pdl(k_pack_stuff, dim3(grid), dim3(PACK_THREADS), 0, s, a);
 }
 
 cudaError_t launch_stuff(const StuffArgs &a, int grid, cudaStream_t s) {

@@ -14,8 +14,7 @@ cudaError_t launch_fdct(const uint8_t *img, size_t step, const Geom &g, const Qu
 // resolve != 0: also rewrite each tile's three raw-DC tokens in `pool` as final DC-difference tokens
 cudaError_t launch_dc_edge_hist(const TileRec *recs, const Geom &g, const int16_t *pred_in, uint32_t *hist,
                                 int16_t *last_dc, int do_hist, uint32_t *pool, int resolve, StripRecord *xr, int rst_tiles,
-                                cudaStream_t s, uint32_t *fuse_zero = nullptr);
-// fuse_zero != NULL: also clears the 10 * ntiles words of k_pack_stuff's per-item look-back state
+                                cudaStream_t s);
 // restart_interval != 0: DRI marker (MCUs per interval) between the DHTs and SOS
 cudaError_t launch_tables(const uint32_t *hist, int optimize, HuffDev *huff, const QuantDev *qd, int full_w, int full_h,
                           int hs, int vs, uint8_t *out, int emit_header, int restart_interval, uint32_t *err_out, cudaStream_t s);
@@ -25,13 +24,6 @@ cudaError_t launch_rst_pad(uint32_t *slots, uint32_t *tile_bits, int ntiles, int
 // small_buffers != 0 (tests): the per-warp bit buffers pretend to hold 24 words, forcing the overflow path
 cudaError_t launch_pack(const uint32_t *pool, const TileRec *recs, const Geom &g, const HuffDev *huff,
                         uint32_t *slots, uint32_t *tile_bits, int small_buffers, cudaStream_t s);
-// k_pack + tile scan + k_stuff in one kernel (whole-image encodes without restart markers): out = header (written by
-// k_tables) + stuffed entropy-coded segment + EOI. Per item (fuse_items(ntiles) of them): desc_bits, desc_bytes, tail;
-// they and the ticket must be zero. small_buffers != 0 (tests): every item takes the global-memory path.
-int fuse_items(int ntiles);
-cudaError_t launch_pack_stuff(const uint32_t *pool, const TileRec *recs, const Geom &g, const HuffDev *huff, uint32_t *slots,
-                              int small_buffers, uint64_t *desc_bits, uint64_t *desc_bytes, uint32_t *tail,
-                              uint32_t *ticket, uint8_t *out, size_t cap, uint64_t *out_len, uint32_t *err, cudaStream_t s);
 // desc: scan_desc_count(ntiles) zeroed look-back descriptors; ticket: zeroed. Also writes, for every k_stuff chunk
 // c < nchunk_cap that starts inside the strip, the tile that holds its first bit (k_stuff starts there: no search)
 int scan_desc_count(int ntiles);

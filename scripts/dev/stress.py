@@ -1,6 +1,6 @@
 """Randomised parity run against the checker (development aid, needs a B200): random sizes up to 2000 x 1500, all
-samplings, qualities, both Huffman modes; every encode also through the fused entropy kernel (debug flag 8), with
-restart rows now and then, and every stream decoded back and compared with the checker's decode.
+samplings, qualities, both Huffman modes; every encode also with the entropy coder's small-buffer recovery path
+(debug flag 2), with restart rows now and then, and every stream decoded back and compared with the checker's decode.
     python scripts/dev/stress.py [cases] [seed]"""
 import sys, os, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.dirname(os.path.abspath(__file__)))))
@@ -27,7 +27,7 @@ for case in range(ncase):
     g = O.geometry(W, H, css)
     rows = int(rng.integers(1, 4)) if rng.random() < 0.25 and rng.integers(1, 4) * g.mcux <= 65535 else 0
     want = O.encode(img, css, q, opt, rows * g.mcux) if rows else O.encode(img, css, q, opt)
-    for dbg in ((0,) if rows else (0, 8, 2, 10)):
+    for dbg in ((0,) if rows else (0, 2)):
         eng.set_debug(dbg); eng.set_restart_rows(rows)
         jpg = eng.encode(img)
         ntot += 1

@@ -13,7 +13,7 @@ ap.add_argument("--css", default="422")
 ap.add_argument("--quality", type=int, default=95)
 ap.add_argument("--optimize", type=int, default=1)
 ap.add_argument("--iters", type=int, default=5)
-ap.add_argument("--debug", type=int, default=0, help="b2j_set_debug flags, e.g. 8 = the fused k_pack_stuff entropy kernel")
+ap.add_argument("--debug", type=int, default=0, help="b2j_set_debug flags (include/b2jpeg.h)")
 a = ap.parse_args()
 img = synth(a.width, a.height)
 torch.cuda.synchronize()

@@ -87,9 +87,8 @@ def test_pack_buffer_regimes(P, oracle):
                 eng = P.Engine(W, H, q, bool(opt), css)
                 for name, img in (("noise", noise), ("soft", soft)):
                     want = oracle.encode(img, css, q, opt)
-                    # 2 = B2J_DEBUG_SMALL_PACK_BUFFERS: every warp buffer overflows -> recovery path; 8 = B2J_DEBUG_FUSED:
-                    # the single-kernel k_pack_stuff instead of k_pack + k_scan_tiles + k_stuff
-                    for dbg in (0, 2, 8, 10):
+                    # 2 = B2J_DEBUG_SMALL_PACK_BUFFERS: every warp buffer overflows -> recovery path
+                    for dbg in (0, 2):
                         eng.set_debug(dbg)
                         jpg = eng.encode(img)
                         assert jpg.size == want.size and np.array_equal(jpg, want), f"{name} css{css} q{q} opt{opt} dbg{dbg}"
@@ -97,8 +96,8 @@ def test_pack_buffer_regimes(P, oracle):
 
 
 def test_tiny_tiles(P, oracle):
-    """Flat and narrow images: tiles of one MCU whose codes are 1-2 bits each (a tile shorter than a byte: the fused
-    entropy kernel, debug flag 8, chains the tail bits through several items), and single-tile images."""
+    """Flat and narrow images: tiles of one MCU whose codes are 1-2 bits each (a tile shorter than a byte), and
+    single-tile images."""
     rng = np.random.default_rng(5)
     for css in range(5):
         for W, H in ((8, 8), (8, 200), (16, 64), (24, 40), (40, 16), (2000, 8)):
@@ -106,11 +105,9 @@ def test_tiny_tiles(P, oracle):
                 img = np.full((H, W, 3), 131, np.uint8) if kind == "flat" else rng.integers(0, 256, (H, W, 3), dtype=np.uint8)
                 for q, opt in ((95, 1), (50, 0)):
                     eng = P.Engine(W, H, q, bool(opt), css)
-                    for dbg in (0, 8):
-                        eng.set_debug(dbg)
-                        jpg = eng.encode(img)
-                        want = oracle.encode(img, css, q, opt)
-                        assert jpg.size == want.size and np.array_equal(jpg, want), (css, W, H, kind, q, opt, dbg)
+                    jpg = eng.encode(img)
+                    want = oracle.encode(img, css, q, opt)
+                    assert jpg.size == want.size and np.array_equal(jpg, want), (css, W, H, kind, q, opt)
                     eng.close()
 
 
@@ -197,11 +194,9 @@ def test_headline_full_image_digest(P, golden, oracle):
     assert sha(img) == h["image"]["raw_sha256"]
     for e in h["encodes"][:2]:
         eng = P.Engine(W, H, e["quality"], bool(e["optimize"]), e["css"])
-        for dbg in (0, 8):   # 8 = B2J_DEBUG_FUSED: the single-kernel entropy coder gives the same bytes
-            eng.set_debug(dbg)
-            jpg = eng.encode(img)
-            assert jpg.size == e["jpeg_len"], (e, dbg)
-            assert sha(jpg)[:32] == e["jpeg_sha256_128"], (e, dbg)
+        jpg = eng.encode(img)
+        assert jpg.size == e["jpeg_len"], e
+        assert sha(jpg)[:32] == e["jpeg_sha256_128"], e
         eng.close()
 
 
