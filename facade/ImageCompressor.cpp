@@ -27,6 +27,8 @@ public:
         *c = nullptr;
     }
     b2j_ctx *any() { return enc ? enc : dec; }
+    bool gray() const { return p.css == B2J_CSS_GRAY; }
+    int mat_type() const { return gray() ? CV_8UC1 : CV_8UC3; }   // what compress() takes and decode() returns
 };
 
 static int css_of(int sampling) {
@@ -35,6 +37,7 @@ static int css_of(int sampling) {
     case 440: return B2J_CSS_440;
     case 420: return B2J_CSS_420;
     case 411: return B2J_CSS_411;
+    case 400: return B2J_CSS_GRAY;
     default: return B2J_CSS_422;
     }
 }
@@ -57,6 +60,11 @@ NvjpegCompressRunner::~NvjpegCompressRunner() {
 void NvjpegCompressRunner::buildCompressEnv() {
     if (compressor->ensure(&compressor->enc) != 0) std::cerr << "[ERROR] buildCompressEnv: no CUDA device / out of memory" << std::endl;
     else b2j_set_restart_rows(compressor->enc, compressor->restart_rows);
+    if (compressor->ngpus > 1 && compressor->gray()) {   // the strips assume three components: compress() fails instead
+        std::cerr << "[ERROR] buildCompressEnv: gray (400) images are not encoded over several GPUs" << std::endl;
+        compressor->drop(&compressor->enc, compressor->dec);
+        return;
+    }
     if (compressor->ngpus > 1 && !compressor->multi) {
         int ids[16], n = 0;
         if (const char *e = getenv("B2J_MULTI_DEVICES")) {   // e.g. "0,1,2,3" (tests: "0,0" = two contexts on one GPU)
@@ -87,7 +95,7 @@ std::vector<unsigned char> NvjpegCompressRunner::compress(cv::Mat image, int *ru
     auto t0 = std::chrono::steady_clock::now();
     std::vector<unsigned char> obuffer;
     b2j_ctx *c = compressor->enc;
-    if (c && !image.empty() && image.type() == CV_8UC3) {
+    if (c && !image.empty() && image.type() == compressor->mat_type()) {
         size_t n = 0;
         int rc;
         if (compressor->multi && compressor->restart_rows == 0) {
@@ -114,7 +122,7 @@ cv::Mat NvjpegCompressRunner::reconstruct(const std::vector<unsigned char> &jpg,
     b2j_ctx *c = compressor->dec ? compressor->dec : compressor->enc;
     int w = 0, h = 0;
     if (c && !jpg.empty() && b2j_decode(c, jpg.data(), jpg.size(), nullptr, 0, &w, &h) == B2J_OK) {
-        result.create(h, w, CV_8UC3);
+        result.create(h, w, compressor->mat_type());
         if (b2j_decode(c, jpg.data(), jpg.size(), result.data, result.step, &w, &h) != B2J_OK) {
             std::cerr << "[ERROR] decode: " << b2j_last_error(c) << std::endl;
             result = cv::Mat();
@@ -183,7 +191,7 @@ double NvjpegCompressRunner::psnr(cv::Mat a, cv::Mat b, int *run_state) {
 std::vector<unsigned char> NvjpegCompressRunner::secondaryCompress(cv::Mat image, std::vector<unsigned char> *diff_jpeg, cv::Mat *reconstruction,
                                                                    double *psnr_db, bool offset128, int *run_state) {
     std::vector<unsigned char> j1, j2;
-    b2j_ctx *c = compressor->enc;
+    b2j_ctx *c = compressor->gray() ? nullptr : compressor->enc;   // not on gray contexts (b2j_secondary refuses them)
     if (c && !image.empty() && image.type() == CV_8UC3) {
         // device resident: upload once, both encodes and the reconstruction stay in HBM; the host vectors are sized to
         // the two streams after the fact (b2j_secondary_device / _finish), the pixels come down only if asked for

@@ -39,7 +39,9 @@ private:
     NvjpegCompressRunnerImpl *compressor;
 
 public:
-    // sampling: 444, 422, 440, 420 or 411. ngpus > 1: compress() cuts the image into MCU-row strips over that many GPUs of
+    // sampling: 444, 422, 440, 420, 411, or 400 (gray: compress() takes CV_8UC1, decode() / reconstruct() return CV_8UC1
+    // -- the one-component file, or the Y plane of a colour file; secondaryCompress() and ngpus > 1 are not available
+    // and give the failure signal). ngpus > 1: compress() cuts the image into MCU-row strips over that many GPUs of
     // this node (devices 0 .. ngpus-1, or the comma-separated list in B2J_MULTI_DEVICES) from this one process
     // (b2j_multi_*); the bytes are the single-GPU bytes.
     NvjpegCompressRunner(int width = 8320, int height = 40000, int quality = 95, bool optimize = true, int sampling = 422,
@@ -49,8 +51,8 @@ public:
     NvjpegCompressRunner(const NvjpegCompressRunner &) = delete;
     NvjpegCompressRunner &operator=(const NvjpegCompressRunner &) = delete;
 
-    // CV_8UC3 BGR pixels (any row step) -> complete JFIF bytes. Empty vector and *run_state = 0 on failure (empty or
-    // oversized image, CUDA error), 1 on success; run_state may be null. Replaces ImageCompressor.cpp:45-61 /
+    // CV_8UC3 BGR pixels (CV_8UC1 with sampling 400; any row step) -> complete JFIF bytes. Empty vector and
+    // *run_state = 0 on failure (empty, oversized or wrongly typed image, CUDA error), 1 on success; run_state may be null. Replaces ImageCompressor.cpp:45-61 /
     // ImageCompressorImpl.cu:269-294 (cv::split + 3 x cudaMemcpy + nvjpegEncodeImage + retrieve): b2j_encode, pageable
     // pixels are staged by the engine's copy threads. Prints the reference's "[INFO] ... Cost Time" line unless B2J_QUIET=1.
     std::vector<unsigned char> compress(cv::Mat image, int *run_state);

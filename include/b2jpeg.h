@@ -19,7 +19,8 @@
  *                                 defined in SURVEY.md section 8 row a-12
  *
  * Conventions: plain pointers and sizes only (no cv::Mat, no torch types); pixels are 8-bit BGR interleaved
- * (cv::Mat CV_8UC3) with a row pitch `step` in bytes; every function returns 0 on success or a negative
+ * (cv::Mat CV_8UC3) with a row pitch `step >= 3 * width` in bytes -- on a context created with css = B2J_CSS_GRAY they
+ * are 8-bit single-channel rows (cv::Mat CV_8UC1) with `step >= width`, wherever this header says "bgr"; every function returns 0 on success or a negative
  * B2J_E* code and never calls exit() (the reference's CHECK_CUDA/CHECK_NVJPEG exit(1),
  * ImageCompressorImpl.cuh:16-34, is deliberately not reproduced). One context = one encoder/decoder state on
  * one GPU, not thread-safe, synchronous at return unless stated otherwise (as the reference,
@@ -41,8 +42,15 @@ extern "C" {
 #define B2J_API __attribute__((visibility("default")))
 #endif
 
-/* nvjpegChromaSubsampling_t values the reference's README sweeps (README.md:44-51) */
-enum { B2J_CSS_444 = 0, B2J_CSS_422 = 1, B2J_CSS_440 = 2, B2J_CSS_420 = 3, B2J_CSS_411 = 4 };
+/* nvjpegChromaSubsampling_t values the reference's README sweeps (README.md:44-51), and NVJPEG_CSS_GRAY (5 is not valid).
+ * A B2J_CSS_GRAY context works on one byte per pixel:
+ *   encode: the one-component stream libjpeg-turbo writes for a grayscale image (one DQT, SOF0 with one component,
+ *           DC0/AC0 only; restart intervals of b2j_set_restart_rows rows of blocks);
+ *   decode: a one-component file (baseline, restart markers, progressive; any sampling factor in its SOF) as libjpeg
+ *           decodes it, and the Y plane of a three-component file (libjpeg's JCS_GRAYSCALE output);
+ *   the strip / peer / multi-GPU encoders, b2j_reconstruct_* and b2j_secondary* refuse it with B2J_EINVAL.
+ * Every other context refuses one-component files with B2J_EFORMAT; b2j_peek reports them as B2J_CSS_GRAY. */
+enum { B2J_CSS_444 = 0, B2J_CSS_422 = 1, B2J_CSS_440 = 2, B2J_CSS_420 = 3, B2J_CSS_411 = 4, B2J_CSS_GRAY = 6 };
 
 enum {
     B2J_OK = 0,
@@ -50,7 +58,7 @@ enum {
     B2J_ECUDA = -2,      /* CUDA runtime error (b2j_last_error has the text) */
     B2J_ENOMEM = -3,
     B2J_ECAPACITY = -4,  /* output buffer too small */
-    B2J_EFORMAT = -5,    /* not a baseline 3-component JPEG this decoder handles */
+    B2J_EFORMAT = -5,    /* not a JPEG this decoder handles (or a one-component file on a colour context) */
     B2J_EINTERNAL = -6,  /* a device-side consistency check failed */
     B2J_ESIZE = -7       /* image does not match the context's width/height */
 };

@@ -8,7 +8,8 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(_HERE)
 LIB_PATH = os.environ.get("B2J_LIB") or os.path.join(_HERE, "libb2jpeg.so")   # B2J_LIB: development builds of the same library
 
-CSS = {"444": 0, "422": 1, "440": 2, "420": 3, "411": 4}
+CSS = {"444": 0, "422": 1, "440": 2, "420": 3, "411": 4, "gray": 6, "400": 6}   # 6: B2J_CSS_GRAY (NVJPEG_CSS_GRAY)
+CSS_GRAY = 6
 ERRORS = {0: "OK", -1: "EINVAL", -2: "ECUDA", -3: "ENOMEM", -4: "ECAPACITY", -5: "EFORMAT", -6: "EINTERNAL", -7: "ESIZE"}
 
 FLAG_NO_PINNED, FLAG_ENCODE, FLAG_DECODE = 1, 2, 4

@@ -119,15 +119,18 @@ extern "C" { static int upload_linear(void *user, uint8_t *d_dst, const uint8_t 
         }                                                                                               \
     } while (0)
 
+// B2J_CSS_GRAY: one component, one block per MCU (nc = 1, bpm = 1, hs = vs = 1); component 0 only in wib/hib/dw/dh
 static int make_geom(int W, int H, int css, Geom *g) {
     static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
-    if (W <= 0 || H <= 0 || W > 65535 || H > 65535 || css < 0 || css > 4) return B2J_EINVAL;
+    const bool gray = css == B2J_CSS_GRAY;
+    if (W <= 0 || H <= 0 || W > 65535 || H > 65535 || css < 0 || (css > 4 && !gray)) return B2J_EINVAL;
     memset(g, 0, sizeof(*g));
-    g->W = W; g->H = H; g->hs = HS[css]; g->vs = VS[css];
+    g->W = W; g->H = H; g->hs = gray ? 1 : HS[css]; g->vs = gray ? 1 : VS[css];
+    g->nc = gray ? 1 : 3;
     g->mcux = (W + 8 * g->hs - 1) / (8 * g->hs);
     g->mcuy = (H + 8 * g->vs - 1) / (8 * g->vs);
-    g->bpm = g->hs * g->vs + 2;
-    for (int c = 0; c < 3; c++) {
+    g->bpm = gray ? 1 : g->hs * g->vs + 2;
+    for (int c = 0; c < g->nc; c++) {
         const int h = c ? 1 : g->hs, v = c ? 1 : g->vs;
         g->dw[c] = (W * h + g->hs - 1) / g->hs;
         g->dh[c] = (H * v + g->vs - 1) / g->vs;
@@ -138,7 +141,7 @@ static int make_geom(int W, int H, int css, Geom *g) {
     if (nb > 0x7fffffffLL / 64) return B2J_EINVAL;
     g->nblocks = (int)nb;
     // fdct tiles: as even as possible, an even MCU count per tile (16-byte alignment of the bulk copies)
-    const int tmax = fdct_tm_max(g->hs, g->vs);
+    const int tmax = fdct_tm_max(g->hs, g->vs, g->nc);
     g->tiles_x = (g->mcux + tmax - 1) / tmax;
     int tm = (g->mcux + g->tiles_x - 1) / g->tiles_x;
     tm = (tm + 1) & ~1;
@@ -170,6 +173,17 @@ static void make_quant(int quality, QuantDev *q) {
             q->finv[t][i] = (float)((1.0 / (double)d) * (1.0 + 1.0 / 1048576.0)) * 4096.0f;   // see k_fdct: exact for |c| <= 2^18
         }
 }
+
+// bytes per pixel of the context's images: 1 (8-bit gray) or 3 (BGR)
+static inline int chans(const b2j_ctx *ctx) { return ctx->p.css == B2J_CSS_GRAY ? 1 : 3; }
+
+// the entry points that assume three components (strips, peers, reconstruction, secondary compression) refuse gray
+static int refuse_gray(b2j_ctx *ctx, const char *what) {
+    if (ctx->p.css != B2J_CSS_GRAY) return B2J_OK;
+    snprintf(ctx->err, sizeof(ctx->err), "%s: not supported on a gray (B2J_CSS_GRAY) context", what);
+    return B2J_EINVAL;
+}
+#define REFUSE_GRAY(ctx, what) do { const int _r = refuse_gray((ctx), (what)); if (_r) return _r; } while (0)
 
 extern "C" {
 
@@ -337,6 +351,7 @@ static inline void tick(b2j_ctx *ctx, int i) { if (ctx->timing) cudaEventRecord(
 
 int b2j_strip_phase1(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width, int rows) {
     if (!ctx || !d_bgr) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_strip_phase1");
     CK(cudaSetDevice(ctx->device));
     int rc = enc_alloc(ctx); if (rc) return rc;
     rc = set_strip_geom(ctx, width, rows); if (rc) return rc;
@@ -349,7 +364,9 @@ int b2j_strip_phase1(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width,
     return B2J_OK;
 }
 
-int b2j_strip_phase1b(b2j_ctx *ctx) {
+// phase1b / phase2 / phase3: the whole-image encode's back half on every context; the exported strip entry points
+// below wrap them and refuse gray contexts
+static int strip_phase1b(b2j_ctx *ctx) {
     if (!ctx || !ctx->enc_ready) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     CK(launch_dc_edge_hist(ctx->d_recs, ctx->g, ctx->d_pred_in, ctx->d_ctrl->hist, ctx->d_ctrl->rec.last_dc, ctx->p.optimize, ctx->d_pool, 1, nullptr, ctx->rst_rows * ctx->g.tiles_x, ctx->stream));
@@ -358,11 +375,11 @@ int b2j_strip_phase1b(b2j_ctx *ctx) {
     return B2J_OK;
 }
 
-int b2j_strip_phase2(b2j_ctx *ctx, int full_w, int full_h) {
+static int strip_phase2(b2j_ctx *ctx, int full_w, int full_h) {
     if (!ctx || !ctx->enc_ready) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     // header is always composed; phase3 decides whether it is part of this strip's output (hdr_len is re-set there)
-    CK(launch_tables(ctx->d_ctrl->hist, ctx->p.optimize, ctx->d_huff, ctx->d_quant, full_w, full_h, ctx->g.hs, ctx->g.vs, ctx->d_out, 1, ctx->rst_rows * ctx->g.mcux, &ctx->d_ctrl->huff_err, ctx->stream));
+    CK(launch_tables(ctx->d_ctrl->hist, ctx->p.optimize, ctx->d_huff, ctx->d_quant, full_w, full_h, ctx->g.hs, ctx->g.vs, ctx->g.nc, ctx->d_out, 1, ctx->rst_rows * ctx->g.mcux, &ctx->d_ctrl->huff_err, ctx->stream));
     tick(ctx, 4);
     CK(launch_pack(ctx->d_pool, ctx->d_recs, ctx->g, ctx->d_huff, ctx->d_slots, ctx->d_tile_bits, ctx->debug & 2, ctx->stream));
     if (ctx->rst_rows) {   // pad every interval to a byte boundary and append its RSTn marker, before the tile scan
@@ -394,7 +411,7 @@ static int phase3_launch(b2j_ctx *ctx, int flags, bool hdr_done = false) {
     return B2J_OK;
 }
 
-int b2j_strip_phase3(b2j_ctx *ctx, int skip_bits, int ext_byte, int flags) {
+static int strip_phase3(b2j_ctx *ctx, int skip_bits, int ext_byte, int flags) {
     if (!ctx || !ctx->enc_ready || skip_bits < 0 || skip_bits > 7) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     if (skip_bits != 0 || (ext_byte & 0xFF) != 0xFF) {   // the zeroed control block already says "skip 0, pad with ones"
@@ -404,8 +421,22 @@ int b2j_strip_phase3(b2j_ctx *ctx, int skip_bits, int ext_byte, int flags) {
     return phase3_launch(ctx, flags);
 }
 
+int b2j_strip_phase1b(b2j_ctx *ctx) {
+    if (ctx) REFUSE_GRAY(ctx, "b2j_strip_phase1b");
+    return strip_phase1b(ctx);
+}
+int b2j_strip_phase2(b2j_ctx *ctx, int full_w, int full_h) {
+    if (ctx) REFUSE_GRAY(ctx, "b2j_strip_phase2");
+    return strip_phase2(ctx, full_w, full_h);
+}
+int b2j_strip_phase3(b2j_ctx *ctx, int skip_bits, int ext_byte, int flags) {
+    if (ctx) REFUSE_GRAY(ctx, "b2j_strip_phase3");
+    return strip_phase3(ctx, skip_bits, ext_byte, flags);
+}
+
 int b2j_strip_phase3_dev(b2j_ctx *ctx, const int64_t *d_bits_all, int rank, int world, int flags) {
     if (!ctx || !ctx->enc_ready || !d_bits_all || rank < 0 || rank >= world) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_strip_phase3_dev");
     CK(cudaSetDevice(ctx->device));
     CK(launch_seam_from_bits(ctx->d_ctrl->seam, d_bits_all, rank, world, ctx->stream));
     ctx->launches += 1;
@@ -415,6 +446,7 @@ int b2j_strip_phase3_dev(b2j_ctx *ctx, const int64_t *d_bits_all, int rank, int 
 // One-collective schedule: phase1x -> all-gather of d_record -> phase2x (everything else, no further exchange).
 int b2j_strip_phase1x(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width, int rows) {
     if (!ctx || !d_bgr) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_strip_phase1x");
     CK(cudaSetDevice(ctx->device));
     int rc = enc_alloc(ctx); if (rc) return rc;
     rc = set_strip_geom(ctx, width, rows); if (rc) return rc;
@@ -436,6 +468,7 @@ int b2j_strip_phase1x(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width
 
 int b2j_strip_phase2x(b2j_ctx *ctx, const void *d_records_all, int rank, int world, int full_w, int full_h, int flags) {
     if (!ctx || !ctx->enc_ready || rank < 0 || rank >= world || world > 256) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_strip_phase2x");
     CK(cudaSetDevice(ctx->device));
     const StripRecord *rec = static_cast<const StripRecord *>(d_records_all);
     const uint32_t *xflags = nullptr;
@@ -447,7 +480,7 @@ int b2j_strip_phase2x(b2j_ctx *ctx, const void *d_records_all, int rank, int wor
     }
     CK(launch_strip_merge(rec, rank, world, ctx->d_ctrl->hist, ctx->d_pool, ctx->d_recs, xflags, ctx->xseq, ctx->peer_timeout_ns, &ctx->d_ctrl->err, ctx->stream));
     ctx->launches += 1;
-    int rc = b2j_strip_phase2(ctx, full_w, full_h); if (rc) return rc;
+    int rc = strip_phase2(ctx, full_w, full_h); if (rc) return rc;
     CK(launch_strip_seam(rec, rank, world, ctx->d_huff, !(flags & 1), ctx->d_ctrl->seam, ctx->d_ctrl->strip_bits, &ctx->d_ctrl->err, ctx->stream));
     ctx->launches += 1;
     return phase3_launch(ctx, flags, true);
@@ -456,6 +489,7 @@ int b2j_strip_phase2x(b2j_ctx *ctx, const void *d_records_all, int rank, int wor
 // ---- peer-memory exchange set-up (GPUs of one node, one process per GPU) ----------------------------------------
 int b2j_peer_export(b2j_ctx *ctx, void *ipc_handle_64, void **d_arena) {
     if (!ctx) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_peer_export");
     CK(cudaSetDevice(ctx->device));
     if (!ctx->d_arena) {
         CK(cudaMalloc(&ctx->d_arena, sizeof(XchgArena)));
@@ -473,6 +507,7 @@ int b2j_peer_export(b2j_ctx *ctx, void *ipc_handle_64, void **d_arena) {
 
 int b2j_peer_open(b2j_ctx *ctx, const void *ipc_handle_64, void **d_ptr) {
     if (!ctx || !ipc_handle_64 || !d_ptr || ctx->n_opened >= XCHG_MAX_WORLD) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_peer_open");
     CK(cudaSetDevice(ctx->device));
     cudaIpcMemHandle_t h;
     memcpy(&h, ipc_handle_64, 64);
@@ -485,6 +520,7 @@ int b2j_peer_open(b2j_ctx *ctx, const void *ipc_handle_64, void **d_ptr) {
 
 int b2j_peer_connect(b2j_ctx *ctx, int rank, int world, void *const *d_arenas) {
     if (!ctx || !d_arenas || world < 1 || world > XCHG_MAX_WORLD || rank < 0 || rank >= world || !ctx->d_arena) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_peer_connect");
     CK(cudaSetDevice(ctx->device));
     XchgArena *host[XCHG_MAX_WORLD];
     for (int r = 0; r < world; r++) {
@@ -503,6 +539,7 @@ int b2j_peer_connect(b2j_ctx *ctx, int rank, int world, void *const *d_arenas) {
 
 int b2j_strip_state_get(b2j_ctx *ctx, b2j_strip_state *st) {
     if (!ctx || !st) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_strip_state_get");
     CK(cudaSetDevice(ctx->device));
     int rc = enc_alloc(ctx); if (rc) return rc;
     st->d_hist = ctx->d_ctrl->hist; st->d_last_dc = ctx->d_ctrl->rec.last_dc; st->d_pred_in = ctx->d_pred_in;
@@ -514,14 +551,14 @@ int b2j_strip_state_get(b2j_ctx *ctx, b2j_strip_state *st) {
 // ------------------------------------------------------------------------------------------ whole-image encode
 // Entropy coding of a whole image: k_pack -> k_scan_tiles -> k_stuff (the strips' kernels).
 static int enc_tail(b2j_ctx *ctx, int width, int height) {
-    int rc = b2j_strip_phase1b(ctx); if (rc) return rc;
-    rc = b2j_strip_phase2(ctx, width, height); if (rc) return rc;
-    return b2j_strip_phase3(ctx, 0, 0xFF, 3);
+    int rc = strip_phase1b(ctx); if (rc) return rc;
+    rc = strip_phase2(ctx, width, height); if (rc) return rc;
+    return strip_phase3(ctx, 0, 0xFF, 3);
 }
 
 int b2j_encode_device(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width, int height, const uint8_t **d_out,
                       const uint64_t **d_len) {
-    if (!ctx || !d_bgr || step < (size_t)width * 3) return B2J_EINVAL;
+    if (!ctx || !d_bgr || step < (size_t)width * chans(ctx)) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     int rc = enc_alloc(ctx); if (rc) return rc;
     rc = set_strip_geom(ctx, width, height); if (rc) return rc;
@@ -671,6 +708,7 @@ static int upload_fdct_group(b2j_ctx *ctx, const uint8_t *bgr, size_t step, size
     const int my0 = gi * rows_per;
     if (my0 >= g.mcuy) return B2J_OK;
     const int mcu_h = 8 * g.vs, width = g.W, height = g.H;
+    const size_t row_bytes = (size_t)width * chans(ctx);
     const int nr = std::min(rows_per, g.mcuy - my0);
     const int y0 = my0 * mcu_h, y1 = std::min(height, (my0 + nr) * mcu_h);
     if (gi == 0) {
@@ -681,13 +719,13 @@ static int upload_fdct_group(b2j_ctx *ctx, const uint8_t *bgr, size_t step, size
         StageRing &r = ctx->ring;
         const int slot = gi % StageRing::N;
         if (r.busy[slot]) CK(cudaEventSynchronize(r.ev[slot]));
-        ctx->pool->copy2d(r.buf[slot], (size_t)width * 3, bgr + (size_t)y0 * step, step, (size_t)width * 3, y1 - y0);
-        CK(cudaMemcpy2DAsync(ctx->d_img + (size_t)y0 * dstep, dstep, r.buf[slot], (size_t)width * 3, (size_t)width * 3, y1 - y0,
+        ctx->pool->copy2d(r.buf[slot], row_bytes, bgr + (size_t)y0 * step, step, row_bytes, y1 - y0);
+        CK(cudaMemcpy2DAsync(ctx->d_img + (size_t)y0 * dstep, dstep, r.buf[slot], row_bytes, row_bytes, y1 - y0,
                              cudaMemcpyHostToDevice, ctx->copy_stream));
         CK(cudaEventRecord(r.ev[slot], ctx->copy_stream));
         r.busy[slot] = true;
     } else {
-        CK(cudaMemcpy2DAsync(ctx->d_img + (size_t)y0 * dstep, dstep, bgr + (size_t)y0 * step, step, (size_t)width * 3, y1 - y0,
+        CK(cudaMemcpy2DAsync(ctx->d_img + (size_t)y0 * dstep, dstep, bgr + (size_t)y0 * step, step, row_bytes, y1 - y0,
                              cudaMemcpyHostToDevice, ctx->copy_stream));
     }
     CK(cudaEventRecord(ctx->ev_copy[gi], ctx->copy_stream));
@@ -701,19 +739,20 @@ static int upload_groups_of(const Geom &g) { return std::max(1, std::min(32, g.m
 
 // host pixels -> complete JPEG in the context's device buffer; *len = its size (waits for the encode)
 int b2j_encode_begin(b2j_ctx *ctx, const uint8_t *bgr, size_t step, int width, int height, size_t *len) {
-    if (!ctx || !bgr || !len || step < (size_t)width * 3) return B2J_EINVAL;
+    if (!ctx || !bgr || !len || step < (size_t)width * chans(ctx)) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     int rc = enc_alloc(ctx); if (rc) return rc;
     rc = set_strip_geom(ctx, width, height); if (rc) return rc;
     const Geom &g = ctx->g;
-    const size_t dstep = ((size_t)width * 3 + 15) & ~(size_t)15;  // 16-byte pitch keeps the TMA path for any width
+    const size_t row_bytes = (size_t)width * chans(ctx);
+    const size_t dstep = (row_bytes + 15) & ~(size_t)15;  // 16-byte pitch keeps the TMA path for any width
     rc = ensure_img(ctx, dstep * height); if (rc) return rc;
     tick(ctx, 0);
     rc = enc_reset(ctx); if (rc) return rc;
     // upload in MCU-row groups on the copy stream; the fdct of a group starts as soon as its rows have landed
     const int ngroups = upload_groups_of(g);
     const bool pageable_in = is_pageable_host(bgr);
-    if (pageable_in) { rc = ensure_hostpipe(ctx, (size_t)((g.mcuy + ngroups - 1) / ngroups) * 8 * g.vs * (size_t)width * 3); if (rc) return rc; }
+    if (pageable_in) { rc = ensure_hostpipe(ctx, (size_t)((g.mcuy + ngroups - 1) / ngroups) * 8 * g.vs * row_bytes); if (rc) return rc; }
     tick(ctx, 1);
     for (int gi = 0; gi < ngroups; gi++) { rc = upload_fdct_group(ctx, bgr, step, dstep, gi, ngroups, ctx->p.optimize, pageable_in); if (rc) return rc; }
     tick(ctx, 2);
@@ -769,6 +808,10 @@ const char *b2j_multi_last_error(const b2j_multi *m) { return m ? m->err : "null
 
 int b2j_multi_create(const b2j_params *p, int ngpus, const int *device_ids, b2j_multi **out) {
     if (!p || !out || ngpus < 1 || ngpus > XCHG_MAX_WORLD) return B2J_EINVAL;
+    if (p->css == B2J_CSS_GRAY) {   // the strips' records and seams assume three components
+        fprintf(stderr, "[b2jpeg] b2j_multi_create: not supported for gray (B2J_CSS_GRAY) images\n");
+        return B2J_EINVAL;
+    }
     b2j_multi *m = new (std::nothrow) b2j_multi();
     if (!m) return B2J_ENOMEM;
     memset(m, 0, sizeof(*m));
@@ -923,7 +966,12 @@ int b2j_last_timings(b2j_ctx *ctx, b2j_timings *t) { if (!ctx || !t) return B2J_
 // ------------------------------------------------------------------------------------------ decode
 static int dec_ensure(b2j_ctx *ctx) {
     if (ctx->dec) return B2J_OK;
-    ctx->dec = dec_create(ctx->cap_g.nblocks, ctx->err, sizeof(ctx->err));
+    // a gray context also decodes the Y plane of colour files of its configured size: room for their blocks (4:4:4 has
+    // the most per pixel)
+    int nb = ctx->cap_g.nblocks;
+    Geom g444;
+    if (ctx->p.css == B2J_CSS_GRAY && make_geom(ctx->cap_g.W, ctx->cap_g.H, B2J_CSS_444, &g444) == B2J_OK) nb = g444.nblocks;
+    ctx->dec = dec_create(nb, ctx->err, sizeof(ctx->err));
     if (ctx->dec) dec_set_uploader(ctx->dec, upload_linear, ctx);   // pageable JPEG bytes go up through the staging ring
     return ctx->dec ? B2J_OK : B2J_ECUDA;
 }
@@ -946,12 +994,23 @@ int b2j_peek(const uint8_t *jpg, size_t len, int *width, int *height, int *css) 
     return B2J_OK;
 }
 
+// A colour context takes three-component files only; a gray context takes one-component files and the Y plane of
+// three-component ones (libjpeg's JCS_GRAYSCALE output)
+static int check_components(b2j_ctx *ctx, int file_css) {
+    if (file_css != B2J_CSS_GRAY || chans(ctx) == 1) return B2J_OK;
+    snprintf(ctx->err, sizeof(ctx->err), "one-component (gray) JPEG: decode it on a B2J_CSS_GRAY context");
+    return B2J_EFORMAT;
+}
+
 // progressive (SOF2) files: parsed and decoded scan by scan (dec_prog.cu); returns B2J_EFORMAT if it is not one
 static int decode_progressive_to(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *d_bgr, size_t step, bool alloc_recon,
                                  int *width, int *height) {
     ProgInfo pi;
     int rc = parse_progressive(jpg, len, &pi);
     if (rc) return rc;
+    rc = check_components(ctx, pi.css);
+    if (rc) { prog_free(&pi); return rc; }
+    const int ch = chans(ctx);
     if (width) *width = pi.W;
     if (height) *height = pi.H;
     Geom g;
@@ -959,7 +1018,7 @@ static int decode_progressive_to(b2j_ctx *ctx, const uint8_t *jpg, size_t len, u
     if (!rc && (d_bgr || alloc_recon)) {
         size_t dstep = step;
         if (alloc_recon) {
-            dstep = ((size_t)pi.W * 3 + 15) & ~(size_t)15;
+            dstep = ((size_t)pi.W * ch + 15) & ~(size_t)15;
             if (ctx->d_recon_bytes < dstep * pi.H) {
                 cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0;
                 if (cudaMalloc(&ctx->d_recon, dstep * pi.H) != cudaSuccess) { prog_free(&pi); return B2J_ECUDA; }
@@ -967,9 +1026,9 @@ static int decode_progressive_to(b2j_ctx *ctx, const uint8_t *jpg, size_t len, u
             }
             d_bgr = ctx->d_recon;
         }
-        if (dstep < (size_t)pi.W * 3) rc = B2J_EINVAL;
+        if (dstep < (size_t)pi.W * ch) rc = B2J_EINVAL;
         if (!rc) rc = dec_ensure(ctx);
-        if (!rc) rc = dec_run_progressive(ctx->dec, jpg, len, pi, g, d_bgr, dstep, ctx->stream, &ctx->launches);
+        if (!rc) rc = dec_run_progressive(ctx->dec, jpg, len, pi, g, d_bgr, dstep, ch == 1, ctx->stream, &ctx->launches);
     }
     prog_free(&pi);
     return rc;
@@ -977,16 +1036,18 @@ static int decode_progressive_to(b2j_ctx *ctx, const uint8_t *jpg, size_t len, u
 
 static int decode_parsed(b2j_ctx *ctx, const uint8_t *jpg, size_t len, const JpegInfo &info, uint8_t *d_bgr, size_t step, bool careful,
                          const uint8_t *d_scan_src = nullptr) {
-    if (step < (size_t)info.W * 3) return B2J_EINVAL;
+    if (step < (size_t)info.W * chans(ctx)) return B2J_EINVAL;
     int rc = dec_ensure(ctx); if (rc) return rc;
     Geom g; rc = make_geom(info.W, info.H, info.css, &g); if (rc) return rc;
     dec_set_spec_launches(ctx->dec, (ctx->debug & 4) ? 1 : 3);
-    return dec_run(ctx->dec, jpg, len, info, g, d_bgr, step, ctx->stream, ctx->timing ? &ctx->tm : nullptr, &ctx->launches, careful, d_scan_src);
+    return dec_run(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, ctx->timing ? &ctx->tm : nullptr,
+                   &ctx->launches, careful, d_scan_src);
 }
 
 static int parse_for(b2j_ctx *ctx, const uint8_t *jpg, size_t len, JpegInfo *info, int *width, int *height) {
     int rc = parse_jpeg(jpg, len, info);
     if (rc) { snprintf(ctx->err, sizeof(ctx->err), "unsupported or corrupt JPEG (parse rc=%d)", rc); return B2J_EFORMAT; }
+    rc = check_components(ctx, info->css); if (rc) return rc;
     if (width) *width = info->W;
     if (height) *height = info->H;
     return B2J_OK;
@@ -997,7 +1058,7 @@ int b2j_decode_device(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *d_b
     CK(cudaSetDevice(ctx->device));
     JpegInfo info;
     int rc = parse_for(ctx, jpg, len, &info, width, height);
-    if (rc == B2J_EFORMAT) {   // not a baseline file: progressive? (decoded synchronously, nothing left for b2j_decode_finish)
+    if (rc == B2J_EFORMAT && info.css != B2J_CSS_GRAY) {   // not a baseline file: progressive? (decoded synchronously, nothing left for b2j_decode_finish)
         if (ctx->last_jpg) { const int rf = b2j_decode_finish(ctx); if (rf) return rf; }
         const int rp = decode_progressive_to(ctx, jpg, len, d_bgr, step, false, width, height);
         if (rp != B2J_EFORMAT) return rp;
@@ -1057,22 +1118,23 @@ int b2j_decode(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *bgr, size_
     CK(cudaSetDevice(ctx->device));
     JpegInfo info;
     int rc = parse_for(ctx, jpg, len, &info, width, height);
-    if (rc == B2J_EFORMAT) {   // not a baseline file: progressive?
+    const int ch = chans(ctx);
+    if (rc == B2J_EFORMAT && info.css != B2J_CSS_GRAY) {   // not a baseline file: progressive?
         int pw = 0, ph = 0;
         const int rp = decode_progressive_to(ctx, jpg, len, nullptr, 0, bgr != nullptr, &pw, &ph);
         if (rp != B2J_EFORMAT) {
             if (width) *width = pw;
             if (height) *height = ph;
             if (rp || !bgr) return rp;
-            if (step < (size_t)pw * 3) return B2J_EINVAL;
-            const size_t dstep = ((size_t)pw * 3 + 15) & ~(size_t)15;
-            return download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)pw * 3, ph, ctx->stream);
+            if (step < (size_t)pw * ch) return B2J_EINVAL;
+            const size_t dstep = ((size_t)pw * ch + 15) & ~(size_t)15;
+            return download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)pw * ch, ph, ctx->stream);
         }
     }
     if (rc) return rc;
     if (!bgr) return B2J_OK;
-    if (step < (size_t)info.W * 3) return B2J_EINVAL;
-    const size_t dstep = ((size_t)info.W * 3 + 15) & ~(size_t)15;
+    if (step < (size_t)info.W * ch) return B2J_EINVAL;
+    const size_t dstep = ((size_t)info.W * ch + 15) & ~(size_t)15;
     if (ctx->d_recon_bytes < dstep * info.H) {
         cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0;
         CK(cudaMalloc(&ctx->d_recon, dstep * info.H));
@@ -1081,7 +1143,7 @@ int b2j_decode(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *bgr, size_
     for (int attempt = 0; attempt < 2; attempt++) {
         rc = decode_parsed(ctx, jpg, len, info, ctx->d_recon, dstep, attempt == 1);
         if (rc) return rc;
-        rc = download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)info.W * 3, info.H, ctx->stream); if (rc) return rc;
+        rc = download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)info.W * ch, info.H, ctx->stream); if (rc) return rc;
         rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
         if (rc != DEC_RETRY) break;   // else: the speculative synchronisation schedule was too short: once more, checked
     }
@@ -1159,6 +1221,7 @@ static int recon_layout(b2j_ctx *ctx, uint8_t **py, uint8_t **pcb, uint8_t **pcr
 // before b2j_reconstruct_color: the vertical chroma filter of 4:2:0 / 4:4:0 looks one row across the border.
 int b2j_reconstruct_planes(b2j_ctx *ctx, b2j_recon_planes *out) {
     if (!ctx) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_reconstruct_planes");
     if (!ctx->enc_ready || !(ctx->debug & 1) || !ctx->d_coef) { snprintf(ctx->err, sizeof(ctx->err), "b2j_reconstruct_* needs an encode with B2J_DEBUG_COEF set"); return B2J_EINVAL; }
     const Geom &g = ctx->g;
     CK(cudaSetDevice(ctx->device));
@@ -1187,7 +1250,9 @@ int b2j_reconstruct_planes(b2j_ctx *ctx, b2j_recon_planes *out) {
 
 // Second half: upsampling + colour conversion of the planes. halo_top / halo_bottom != 0: the halo rows are filled.
 int b2j_reconstruct_color(b2j_ctx *ctx, uint8_t *d_bgr, size_t step, int halo_top, int halo_bottom) {
-    if (!ctx || !d_bgr || !ctx->d_rplanes) return B2J_EINVAL;
+    if (!ctx || !d_bgr) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_reconstruct_color");
+    if (!ctx->d_rplanes) return B2J_EINVAL;
     const Geom &g = ctx->g;
     if (step < (size_t)g.W * 3) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
@@ -1200,6 +1265,7 @@ int b2j_reconstruct_color(b2j_ctx *ctx, uint8_t *d_bgr, size_t step, int halo_to
 
 int b2j_reconstruct_device(b2j_ctx *ctx, uint8_t *d_bgr, size_t step) {
     if (!ctx || !d_bgr) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_reconstruct_device");
     int rc = b2j_reconstruct_planes(ctx, nullptr); if (rc) return rc;
     return b2j_reconstruct_color(ctx, d_bgr, step, 0, 0);
 }
@@ -1209,7 +1275,9 @@ int b2j_reconstruct_device(b2j_ctx *ctx, uint8_t *d_bgr, size_t step) {
 // not waited for; b2j_secondary_finish returns the two lengths and the PSNR.
 int b2j_secondary_device(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width, int height, int diff_mode,
                          const uint8_t **d_jpg1, const uint8_t **d_jpg2, const uint8_t **d_recon, const uint8_t **d_diff) {
-    if (!ctx || !d_bgr || step != (size_t)width * 3 || (diff_mode != 0 && diff_mode != 1)) return B2J_EINVAL;   // contiguous rows
+    if (!ctx) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_secondary_device");
+    if (!d_bgr || step != (size_t)width * 3 || (diff_mode != 0 && diff_mode != 1)) return B2J_EINVAL;   // contiguous rows
     CK(cudaSetDevice(ctx->device));
     const size_t bytes = (size_t)width * 3 * height;
     if (ctx->d_recon_bytes < bytes) { cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0; CK(cudaMalloc(&ctx->d_recon, bytes)); ctx->d_recon_bytes = bytes; }
@@ -1239,7 +1307,9 @@ int b2j_secondary_device(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int wi
 }
 
 int b2j_secondary_finish(b2j_ctx *ctx, size_t *len1, size_t *len2, double *psnr, uint64_t *ssd) {
-    if (!ctx || !ctx->second) return B2J_EINVAL;
+    if (!ctx) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_secondary_finish");
+    if (!ctx->second) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     // the SSD lives in the first encoder's control block: b2j_diff_psnr_device ran after its encode was queued, and
     // fetch_ret copies the block (length, checks, SSD) in one go
@@ -1257,7 +1327,9 @@ int b2j_secondary_finish(b2j_ctx *ctx, size_t *len1, size_t *len2, double *psnr,
 int b2j_secondary(b2j_ctx *ctx, const uint8_t *bgr, size_t step, int width, int height, int diff_mode, uint8_t *jpg1,
                   size_t cap1, size_t *len1, uint8_t *jpg2, size_t cap2, size_t *len2, uint8_t *recon, size_t recon_step,
                   double *psnr) {
-    if (!ctx || !bgr || step < (size_t)width * 3 || (diff_mode != 0 && diff_mode != 1)) return B2J_EINVAL;
+    if (!ctx) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_secondary");
+    if (!bgr || step < (size_t)width * 3 || (diff_mode != 0 && diff_mode != 1)) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     int rc = enc_alloc(ctx); if (rc) return rc;
     // host pixels -> device (contiguous rows), then everything stays there: b2j_secondary_device
@@ -1279,7 +1351,9 @@ int b2j_secondary(b2j_ctx *ctx, const uint8_t *bgr, size_t step, int width, int 
 
 // the results of the last b2j_secondary / b2j_secondary_device (+ _finish) -> host memory; any pointer may be NULL
 int b2j_secondary_fetch(b2j_ctx *ctx, uint8_t *jpg1, size_t cap1, uint8_t *jpg2, size_t cap2, uint8_t *recon, size_t recon_step) {
-    if (!ctx || !ctx->second || !ctx->enc_ready) return B2J_EINVAL;
+    if (!ctx) return B2J_EINVAL;
+    REFUSE_GRAY(ctx, "b2j_secondary_fetch");
+    if (!ctx->second || !ctx->enc_ready) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     const size_t n1 = (size_t)ctx->h_ret->out_len, n2 = (size_t)ctx->second->h_ret->out_len;
     int rc = B2J_OK;

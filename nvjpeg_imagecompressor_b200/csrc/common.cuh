@@ -8,9 +8,9 @@ namespace b2j {
 // ---- geometry of one image / MCU-row strip (libjpeg jcmaster.c per_scan_setup) -------------------------
 struct Geom {
     int W, H;          // pixels
-    int hs, vs;        // luma sampling factors; chroma is 1x1
+    int hs, vs;        // luma sampling factors; chroma is 1x1 (gray: 1x1)
     int mcux, mcuy;    // MCU grid
-    int bpm;           // blocks per MCU = hs*vs + 2
+    int bpm;           // blocks per MCU = hs*vs + 2 (gray: 1)
     int wib[3], hib[3];// real blocks per component (width/height in blocks)
     int dh[3];         // true downsampled height in samples
     int dw[3];         // true downsampled width in samples
@@ -18,6 +18,7 @@ struct Geom {
     int tiles_x;       // fdct tiles per MCU row
     int nblocks;       // mcux*mcuy*bpm, scan order
     int ntiles;        // fdct/pack tiles = tiles_x * mcuy
+    int nc;            // components per image: 3 (Y, Cb, Cr) or 1 (gray: one non-interleaved scan, an MCU is one block)
 };
 
 // One token per coded coefficient / EOB / DC difference:
@@ -47,7 +48,7 @@ __host__ __device__ constexpr uint32_t bin_symbol(uint32_t bin) {   // JPEG symb
 __host__ __device__ constexpr uint32_t tok_dc(uint32_t table, uint32_t size, uint32_t vbits) { return (tcode_of(table) << 16) | (size << 18) | vbits; }
 struct TileRec {                               // one per fdct tile (<= 256 blocks, one MCU-row segment)
     uint32_t base, count;                      // token run in the pool
-    int16_t first_dc[3], last_dc[3];           // DCs of the tile's first / last MCU (last Y block, Cb, Cr)
+    int16_t first_dc[3], last_dc[3];           // DCs of the tile's first / last MCU (last Y block, Cb, Cr; gray: [0] only)
     uint16_t pos_cb, pos_cr;                   // run offsets of the first MCU's Cb / Cr DC tokens (Y: offset 0)
 };
 

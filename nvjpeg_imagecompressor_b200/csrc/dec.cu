@@ -156,7 +156,7 @@ static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interv
 }
 
 int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr, size_t step,
-            cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src) {
+            bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src) {
     const int rst = info.restart_interval;   // MCUs per restart interval (0: none)
     if (rst && info.scan_len >= 0xFFFFFFF0ull) { snprintf(d->err, d->errlen, "restart-marker scans of 4 GB and more are not supported"); return B2J_EFORMAT; }
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
@@ -165,7 +165,7 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
     if (rc) return rc;
     const size_t n = info.scan_len;
     const size_t nsub_max = (n * 8 + DEC_SUB_BITS - 1) / DEC_SUB_BITS;
-    const int hv = g.bpm - 2;
+    const int hv = g.hs * g.vs;   // luma blocks per MCU (gray: 1 of 1)
     if (tm) cudaEventRecord(d->ev[0], s);
     // h_tb / h_flag are rewritten by the host below: a previous decode on this decoder must have drained first
     if (d->in_flight) { DCK(cudaStreamSynchronize(d->last_stream)); d->in_flight = false; }
@@ -266,16 +266,23 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
     DCK(launch_scan_u32(d->d_nblk, d->d_blk_start, nsub_max, d->d_desc + d->desc_cap, &d->d_ctrl->ticket[1], &d->d_ctrl->err, s));
     DCK(launch_dec_write(d->d_u, &d->d_ctrl->u_len, d->d_tb, d->d_st_out, d->d_blk_start, g.bpm, hv, d->d_coef, d->d_dc, (uint32_t)g.nblocks,
                          &d->d_ctrl->err, nsub_max, bnd, nmark, s));
-    DCK(launch_dc_scan(d->d_dc, g, d->d_desc + 2 * d->desc_cap, &d->d_ctrl->ticket[2], d->desc_cap, &d->d_ctrl->err, s));
+    DCK(launch_dc_scan(d->d_dc, g, gray_out ? 1 : g.nc, d->d_desc + 2 * d->desc_cap, &d->d_ctrl->ticket[2], d->desc_cap,
+                       &d->d_ctrl->err, s));
     if (tm) cudaEventRecord(d->ev[3], s);
-    uint8_t *py = d->d_planes;
-    uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
-    uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
-    DCK(launch_idct(d->d_coef, d->d_dc, g, d->d_tb, py, pcb, pcr, rst, s));
-    if (tm) cudaEventRecord(d->ev[4], s);
-    DCK(launch_upcolor(py, pcb, pcr, g, d_bgr, step, s));
-    if (tm) cudaEventRecord(d->ev[5], s);
-    if (launches) (*launches) += 5;
+    if (gray_out) {   // Y straight from the IDCT into the caller's image: no planes, no colour pass (dec_color stays 0)
+        DCK(launch_idct_gray(d->d_coef, d->d_dc, g, d->d_tb, d_bgr, step, rst, s));
+        if (tm) { cudaEventRecord(d->ev[4], s); cudaEventRecord(d->ev[5], s); }
+        if (launches) (*launches) += 4;
+    } else {
+        uint8_t *py = d->d_planes;
+        uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
+        uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
+        DCK(launch_idct(d->d_coef, d->d_dc, g, d->d_tb, py, pcb, pcr, rst, s));
+        if (tm) cudaEventRecord(d->ev[4], s);
+        DCK(launch_upcolor(py, pcb, pcr, g, d_bgr, step, s));
+        if (tm) cudaEventRecord(d->ev[5], s);
+        if (launches) (*launches) += 5;
+    }
     if (tm) {
         DCK(cudaStreamSynchronize(s));
         cudaEventElapsedTime(&tm->dec_parse, d->ev[0], d->ev[1]);
@@ -289,7 +296,7 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
 }
 
 int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, uint8_t *d_bgr,
-                        size_t step, cudaStream_t s, uint64_t *launches) {
+                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches) {
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
     int rc = ensure(d, 4096, g, 0);
     if (rc) return rc;
@@ -297,7 +304,7 @@ int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const ProgIn
     d->speculated = false;
     d->last_stream = s;
     DCK(cudaMemsetAsync(&d->d_ctrl->err, 0, 4, s));
-    return dec_progressive(jpg, len, info, g, d->d_coef, d->d_tb, d->d_planes, d_bgr, step, s, launches, d->err, d->errlen);
+    return dec_progressive(jpg, len, info, g, d->d_coef, d->d_tb, d->d_planes, d_bgr, step, gray_out, s, launches, d->err, d->errlen);
 }
 
 int dec_check(Decoder *d, char *err, size_t errlen) {

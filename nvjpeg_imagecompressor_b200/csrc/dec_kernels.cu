@@ -934,9 +934,13 @@ __device__ __forceinline__ void cp_async_commit() { asm volatile("cp.async.commi
 template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
+// GRAY: only the luma blocks are transformed and their samples go straight to the caller's 8-bit image (py, pitch
+// out_step), cut at the image's right and bottom edges: no Y plane in between (it would cost two more passes over W * H
+// bytes) and no colour kernel behind it.
+template <bool GRAY>
 __global__ void __launch_bounds__(256, 2)
 k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom g, const DecTables *__restrict__ tb,
-       uint8_t *__restrict__ py, uint8_t *__restrict__ pcb, uint8_t *__restrict__ pcr, int rst_mcus) {
+       uint8_t *__restrict__ py, uint8_t *__restrict__ pcb, uint8_t *__restrict__ pcr, int rst_mcus, size_t out_step) {
     extern __shared__ __align__(16) uint4 s_c[];   // [2][IDCT_TILE * 8], chunk c of block b at b * 8 + (c ^ (b & 7))
     __shared__ __align__(16) int s_q[2][64];       // zig-zag order
     const int tid = threadIdx.x;
@@ -954,14 +958,14 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
     int t = blockIdx.x;
     if (t < ntile) issue(t, 0);
     if (tid < 128) s_q[tid >> 6][tid & 63] = (int)tb->q[tid >> 6][zigzag_nat_rt(tid & 63)];
-    const int hv = g.bpm - 2;
+    const int hv = GRAY ? g.hs * g.vs : g.bpm - 2;   // luma blocks per MCU (a colour file on a gray context keeps its chroma)
     for (int k = 0; t < ntile; t += gridDim.x, k++) {
         const int tn = t + gridDim.x;
         if (tn < ntile) { issue(tn, (k + 1) & 1); cp_async_wait<1>(); }
         else cp_async_wait<0>();
         __syncthreads();   // tile t has landed (every thread waited for its own requests)
         const int b0 = t * IDCT_TILE, nb = min(IDCT_TILE, g.nblocks - b0);
-        if (tid < nb) {
+        if (tid < nb && (!GRAY || (b0 + tid) % g.bpm < hv)) {
             const uint4 *sc = s_c + (k & 1) * (IDCT_TILE * 8);
             const int b = b0 + tid;
             const int m = b / g.bpm, bn = b - m * g.bpm;
@@ -997,7 +1001,15 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
             for (int c = 0; c < 8; c++) idct8<11>(v[c], v[8 + c], v[16 + c], v[24 + c], v[32 + c], v[40 + c], v[48 + c], v[56 + c]);
             uint8_t *dst;
             size_t stride;
-            if (isY) {
+            int gx0 = 0, nrow = 8;   // GRAY: the block's first column and its rows inside the image
+            if (GRAY) {
+                const int by = bn / g.hs, bx = bn - by * g.hs;
+                const int gy0 = (my * g.vs + by) * 8;
+                gx0 = (mx * g.hs + bx) * 8;
+                nrow = min(8, g.H - gy0);
+                stride = out_step;
+                dst = py + (size_t)gy0 * stride + (size_t)gx0;
+            } else if (isY) {
                 const int by = bn / g.hs, bx = bn - by * g.hs;
                 stride = (size_t)g.mcux * 8 * g.hs;
                 dst = py + ((size_t)(my * g.vs + by) * 8) * stride + (size_t)(mx * g.hs + bx) * 8;
@@ -1013,7 +1025,13 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
                 for (int c = 0; c < 8; c++) x[c] = (uint32_t)min(255, max(0, v[r * 8 + c] + 128));
                 const uint32_t lo = __byte_perm(__byte_perm(x[0], x[1], 0x0040), __byte_perm(x[2], x[3], 0x0040), 0x5410);
                 const uint32_t hi = __byte_perm(__byte_perm(x[4], x[5], 0x0040), __byte_perm(x[6], x[7], 0x0040), 0x5410);
-                *reinterpret_cast<uint2 *>(dst + r * stride) = make_uint2(lo, hi);
+                if (!GRAY) {
+                    *reinterpret_cast<uint2 *>(dst + r * stride) = make_uint2(lo, hi);
+                } else if (r < nrow) {
+                    uint8_t *d = dst + r * stride;
+                    if (gx0 + 8 <= g.W && ((reinterpret_cast<uintptr_t>(d) & 7) == 0)) *reinterpret_cast<uint2 *>(d) = make_uint2(lo, hi);
+                    else for (int c = 0; c < min(8, g.W - gx0); c++) d[c] = (uint8_t)x[c];
+                }
             }
         }
         __syncthreads();   // buffer k & 1 is free for the tile after next
@@ -1244,15 +1262,16 @@ cudaError_t launch_scan_u32(const uint32_t *in, uint32_t *out, size_t n, uint64_
     return cudaGetLastError();
 }
 
-cudaError_t launch_dc_scan(int16_t *coef, const Geom &g, uint64_t *desc, uint32_t *ticket, size_t desc_stride, uint32_t *err,
-                           cudaStream_t s) {
-    dim3 grid(148 * 2, 3);
-    k_dc_scan<<<grid, 256, 0, s>>>(coef, g.bpm, g.bpm - 2, (size_t)g.mcux * g.mcuy, desc, ticket, desc_stride, err);
+cudaError_t launch_dc_scan(int16_t *coef, const Geom &g, int ncomp, uint64_t *desc, uint32_t *ticket, size_t desc_stride,
+                           uint32_t *err, cudaStream_t s) {
+    dim3 grid(148 * 2, ncomp);
+    k_dc_scan<<<grid, 256, 0, s>>>(coef, g.bpm, g.hs * g.vs, (size_t)g.mcux * g.mcuy, desc, ticket, desc_stride, err);
     return cudaGetLastError();
 }
 
-cudaError_t launch_idct(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *py, uint8_t *pcb,
-                        uint8_t *pcr, int rst_mcus, cudaStream_t s) {
+template <bool GRAY>
+static cudaError_t idct_launch(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *py, uint8_t *pcb,
+                               uint8_t *pcr, int rst_mcus, size_t out_step, cudaStream_t s) {
     // the dynamic shared-memory attribute is per device: one bit per device ordinal
     static std::atomic<uint64_t> attr_done{0};
     int dev = 0;
@@ -1260,13 +1279,24 @@ cudaError_t launch_idct(const int16_t *coef, const int16_t *dcarr, const Geom &g
     if (e != cudaSuccess) return e;
     const uint64_t bit = 1ull << (dev & 63);
     if (!(attr_done.load(std::memory_order_acquire) & bit)) {
-        e = cudaFuncSetAttribute(k_idct, cudaFuncAttributeMaxDynamicSharedMemorySize, IDCT_SMEM);
+        e = cudaFuncSetAttribute(k_idct<GRAY>, cudaFuncAttributeMaxDynamicSharedMemorySize, IDCT_SMEM);
         if (e != cudaSuccess) return e;
         attr_done.fetch_or(bit, std::memory_order_release);
     }
     const int ntile = (g.nblocks + IDCT_TILE - 1) / IDCT_TILE;
-    k_idct<<<std::max(1, std::min(ntile, 148 * 2)), 256, IDCT_SMEM, s>>>(coef, dcarr, g, (const DecTables *)tb, py, pcb, pcr, rst_mcus);
+    k_idct<GRAY><<<std::max(1, std::min(ntile, 148 * 2)), 256, IDCT_SMEM, s>>>(coef, dcarr, g, (const DecTables *)tb, py, pcb, pcr,
+                                                                               rst_mcus, out_step);
     return cudaGetLastError();
+}
+
+cudaError_t launch_idct(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *py, uint8_t *pcb,
+                        uint8_t *pcr, int rst_mcus, cudaStream_t s) {
+    return idct_launch<false>(coef, dcarr, g, tb, py, pcb, pcr, rst_mcus, 0, s);
+}
+
+cudaError_t launch_idct_gray(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *gray, size_t step,
+                             int rst_mcus, cudaStream_t s) {
+    return idct_launch<true>(coef, dcarr, g, tb, gray, nullptr, nullptr, rst_mcus, step, s);
 }
 
 template <int HS, int VS>

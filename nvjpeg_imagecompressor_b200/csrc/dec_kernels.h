@@ -43,19 +43,25 @@ cudaError_t launch_dec_write(const uint8_t *u, const uint64_t *u_len, const void
                              uint32_t *err, size_t nsub_max, const uint32_t *bnd, const uint32_t *nmark, cudaStream_t s);
 cudaError_t launch_scan_u32(const uint32_t *in, uint32_t *out, size_t n, uint64_t *desc, uint32_t *ticket, uint32_t *err,
                             cudaStream_t s);
-// coef here = the compact DC array (one int16 per block)
-cudaError_t launch_dc_scan(int16_t *coef, const Geom &g, uint64_t *desc, uint32_t *ticket, size_t desc_stride, uint32_t *err,
-                           cudaStream_t s);
+// coef here = the compact DC array (one int16 per block); ncomp: the first ncomp components (1: luma only)
+cudaError_t launch_dc_scan(int16_t *coef, const Geom &g, int ncomp, uint64_t *desc, uint32_t *ticket, size_t desc_stride,
+                           uint32_t *err, cudaStream_t s);
 // rst_mcus: restart interval in MCUs (0: none): DC predictors return to 0 at every interval start
 cudaError_t launch_idct(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *py, uint8_t *pcb,
                         uint8_t *pcr, int rst_mcus, cudaStream_t s);
+// the luma blocks only, their samples stored straight into the caller's 8-bit image (gray output: libjpeg's
+// JCS_GRAYSCALE, no upsampling or colour conversion); chroma blocks of a three-component file are skipped
+cudaError_t launch_idct_gray(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *gray, size_t step,
+                             int rst_mcus, cudaStream_t s);
 // halo_top / halo_bottom: the chroma planes hold one valid row above row 0 / below the last row (a strip of a larger
 // image: the vertical filter of 4:2:0 / 4:4:0 then reads the neighbour strip's row instead of replicating the edge)
 cudaError_t launch_upcolor(const uint8_t *py, const uint8_t *pcb, const uint8_t *pcr, const Geom &g, uint8_t *bgr, size_t step,
                            cudaStream_t s, int halo_top = 0, int halo_bottom = 0);
 
 // progressive files (dec_prog.cu): all scans into d_coef, then IDCT + upsampling; synchronises the stream before returning
+// gray_out: 8-bit Y samples into d_bgr (launch_idct_gray) instead of IDCT + upsampling + colour conversion
 int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
-                    uint8_t *d_planes, uint8_t *d_bgr, size_t step, cudaStream_t s, uint64_t *launches, char *err, size_t errlen);
+                    uint8_t *d_planes, uint8_t *d_bgr, size_t step, bool gray_out, cudaStream_t s, uint64_t *launches,
+                    char *err, size_t errlen);
 
 }  // namespace b2j

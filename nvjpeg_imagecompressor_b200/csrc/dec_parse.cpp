@@ -47,9 +47,9 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
             }
             break;
         case 0xC0: case 0xC1:
-            if (n < 15 || s[0] != 8 || s[5] != 3) return B2J_EFORMAT;
-            info->H = be16(s + 1); info->W = be16(s + 3); ncomp = 3;
-            for (int c = 0; c < 3; c++) { cid[c] = s[6 + 3 * c]; chv[c] = s[7 + 3 * c]; ctq[c] = s[8 + 3 * c] & 3; }
+            if (n < 9 || s[0] != 8 || (s[5] != 3 && s[5] != 1) || n < 6 + 3 * s[5]) return B2J_EFORMAT;
+            info->H = be16(s + 1); info->W = be16(s + 3); ncomp = s[5];
+            for (int c = 0; c < ncomp; c++) { cid[c] = s[6 + 3 * c]; chv[c] = s[7 + 3 * c]; ctq[c] = s[8 + 3 * c] & 3; }
             break;
         case 0xC2: case 0xC3: case 0xC5: case 0xC6: case 0xC7: case 0xC9: case 0xCA: case 0xCB: case 0xCD: case 0xCE: case 0xCF:
             return B2J_EFORMAT;  // progressive / lossless / arithmetic (SURVEY.md 8f N4)
@@ -78,25 +78,40 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
             info->restart_interval = be16(s);
             break;
         case 0xDA: {
-            if (ncomp != 3 || n < 10 || s[0] != 3) return B2J_EFORMAT;
+            if (ncomp == 1) {   // one component (gray): one non-interleaved scan, laid out 1x1 whatever the SOF says
+                if (n < 6 || s[0] != 1 || s[1] != cid[0]) return B2J_EFORMAT;
+                const int td = s[2] >> 4, ta = s[2] & 15;
+                if (td > 3 || ta > 3 || !have_h[0][td] || !have_h[1][ta] || !have_q[ctq[0]]) return B2J_EFORMAT;
+                if (info->W <= 0 || info->H <= 0) return B2J_EFORMAT;
+                info->css = B2J_CSS_GRAY; info->hs = info->vs = 1;
+                for (int t = 0; t < 2; t++) memcpy(info->qt[t], q[ctq[0]], 128);
+                for (int t = 0; t < 4; t += 2) {
+                    memcpy(info->bits[t], hb[0][td], 17); memcpy(info->vals[t], hv[0][td], 256);
+                    memcpy(info->bits[t + 1], hb[1][ta], 17); memcpy(info->vals[t + 1], hv[1][ta], 256);
+                }
+            }
+            if (ncomp != 3 && ncomp != 1) return B2J_EFORMAT;
+            if (ncomp == 3 && (n < 10 || s[0] != 3)) return B2J_EFORMAT;
             int td[3], ta[3];
-            for (int c = 0; c < 3; c++) {
+            for (int c = 0; c < 3 && ncomp == 3; c++) {
                 if (s[1 + 2 * c] != cid[c]) return B2J_EFORMAT;
                 td[c] = s[2 + 2 * c] >> 4; ta[c] = s[2 + 2 * c] & 15;
                 if (td[c] > 3 || ta[c] > 3 || !have_h[0][td[c]] || !have_h[1][ta[c]]) return B2J_EFORMAT;
             }
-            if (chv[1] != 0x11 || chv[2] != 0x11 || td[1] != td[2] || ta[1] != ta[2] || ctq[1] != ctq[2]) return B2J_EFORMAT;
-            if (!have_q[ctq[0]] || !have_q[ctq[1]]) return B2J_EFORMAT;
-            info->hs = chv[0] >> 4; info->vs = chv[0] & 15;
-            static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
-            info->css = -1;
-            for (int i = 0; i < 5; i++) if (HS[i] == info->hs && VS[i] == info->vs) info->css = i;
-            if (info->css < 0 || info->W <= 0 || info->H <= 0) return B2J_EFORMAT;
-            memcpy(info->qt[0], q[ctq[0]], 128); memcpy(info->qt[1], q[ctq[1]], 128);
-            memcpy(info->bits[0], hb[0][td[0]], 17); memcpy(info->vals[0], hv[0][td[0]], 256);
-            memcpy(info->bits[1], hb[1][ta[0]], 17); memcpy(info->vals[1], hv[1][ta[0]], 256);
-            memcpy(info->bits[2], hb[0][td[1]], 17); memcpy(info->vals[2], hv[0][td[1]], 256);
-            memcpy(info->bits[3], hb[1][ta[1]], 17); memcpy(info->vals[3], hv[1][ta[1]], 256);
+            if (ncomp == 3) {
+                if (chv[1] != 0x11 || chv[2] != 0x11 || td[1] != td[2] || ta[1] != ta[2] || ctq[1] != ctq[2]) return B2J_EFORMAT;
+                if (!have_q[ctq[0]] || !have_q[ctq[1]]) return B2J_EFORMAT;
+                info->hs = chv[0] >> 4; info->vs = chv[0] & 15;
+                static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
+                info->css = -1;
+                for (int i = 0; i < 5; i++) if (HS[i] == info->hs && VS[i] == info->vs) info->css = i;
+                if (info->css < 0 || info->W <= 0 || info->H <= 0) return B2J_EFORMAT;
+                memcpy(info->qt[0], q[ctq[0]], 128); memcpy(info->qt[1], q[ctq[1]], 128);
+                memcpy(info->bits[0], hb[0][td[0]], 17); memcpy(info->vals[0], hv[0][td[0]], 256);
+                memcpy(info->bits[1], hb[1][ta[0]], 17); memcpy(info->vals[1], hv[1][ta[0]], 256);
+                memcpy(info->bits[2], hb[0][td[1]], 17); memcpy(info->vals[2], hv[0][td[1]], 256);
+                memcpy(info->bits[3], hb[1][ta[1]], 17); memcpy(info->vals[3], hv[1][ta[1]], 256);
+            }
             info->scan_offset = p + L;
             // the entropy-coded segment ends at the first marker that is neither a stuffed zero nor RSTn. Fast path for
             // the files this engine and libjpeg write (one scan, EOI as the last two bytes): no 0xFF search at all.
@@ -169,8 +184,15 @@ int parse_progressive(const uint8_t *jpg, size_t len, ProgInfo *info) {
                 s += 1 + sz; n -= 1 + sz;
             }
         } else if (m == 0xC2) {
-            if (have_sof || n < 15 || s[0] != 8 || s[5] != 3) { bad = true; }
-            else {
+            if (have_sof || n < 9 || s[0] != 8 || (s[5] != 3 && s[5] != 1) || n < 6 + 3 * s[5]) { bad = true; }
+            else if (s[5] == 1) {   // one component (gray): any sampling factor, laid out 1x1
+                info->H = be16(s + 1); info->W = be16(s + 3);
+                cid[0] = s[6]; ctq[0] = ctq[1] = ctq[2] = s[8] & 3;
+                cid[1] = cid[2] = -1;   // no scan can name them
+                info->hs = info->vs = 1; info->css = B2J_CSS_GRAY;
+                if (info->W <= 0 || info->H <= 0) bad = true;
+                have_sof = !bad;
+            } else {
                 info->H = be16(s + 1); info->W = be16(s + 3);
                 for (int c = 0; c < 3; c++) { cid[c] = s[6 + 3 * c]; chv[c] = s[7 + 3 * c]; ctq[c] = s[8 + 3 * c] & 3; }
                 if (chv[1] != 0x11 || chv[2] != 0x11 || ctq[1] != ctq[2]) bad = true;

@@ -328,7 +328,8 @@ k_prog_apply(const uint64_t *__restrict__ cm, const uint64_t *__restrict__ corr,
     } while (0)
 
 int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
-                    uint8_t *d_planes, uint8_t *d_bgr, size_t step, cudaStream_t s, uint64_t *launches, char *err, size_t errlen) {
+                    uint8_t *d_planes, uint8_t *d_bgr, size_t step, bool gray_out, cudaStream_t s, uint64_t *launches,
+                    char *err, size_t errlen) {
     int rc = B2J_OK;
     uint8_t *d_all = nullptr, *d_file = nullptr, *d_u = nullptr;
     ProgScanDev *d_sc = nullptr;
@@ -405,12 +406,17 @@ int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const 
         if (!htb) { rc = B2J_ENOMEM; goto done; }
         memcpy(htb->q, info.qt, sizeof(htb->q));
         PCK(cudaMemcpyAsync(d_tb, htb, dec_tables_size(), cudaMemcpyHostToDevice, s));
-        uint8_t *py = d_planes;
-        uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
-        uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
-        PCK(launch_idct(d_coef, nullptr, g, d_tb, py, pcb, pcr, 0, s));
-        PCK(launch_upcolor(py, pcb, pcr, g, d_bgr, step, s));
-        if (launches) (*launches) += 2;
+        if (gray_out) {
+            PCK(launch_idct_gray(d_coef, nullptr, g, d_tb, d_bgr, step, 0, s));
+            if (launches) (*launches) += 1;
+        } else {
+            uint8_t *py = d_planes;
+            uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
+            uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
+            PCK(launch_idct(d_coef, nullptr, g, d_tb, py, pcb, pcr, 0, s));
+            PCK(launch_upcolor(py, pcb, pcr, g, d_bgr, step, s));
+            if (launches) (*launches) += 2;
+        }
     }
     PCK(cudaStreamSynchronize(s));   // the host vectors and the temporary buffers go away below
 done:

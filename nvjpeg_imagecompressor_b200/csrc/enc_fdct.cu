@@ -9,6 +9,8 @@
 // One CTA = one tile of up to TM_MAX MCUs inside one MCU row:
 //   TMA bulk copies (cp.async.bulk, one per pixel row) stage the raw BGR rows in shared memory   [interior tiles]
 //   stage A: every thread converts 8 pixels x VS rows -> Y / Cb / Cr sample planes in shared memory
+//            (gray, NC = 1: the staged rows ARE the Y plane -- jccolor.c grayscale_convert is a copy -- and an MCU is
+//            one block, so a tile holds PACK_BLOCKS MCUs: 2048 pixels x 8 rows, the 16 KB of a 4:4:4 tile's rows)
 //   stage B: one thread per 8x8 block: 64 samples in registers, both FDCT passes, reciprocal quantisation in place,
 //            branch-free count of the non-zero coefficients; a CTA scan of the counts gives every block its place
 //            in the tile's token run, then the jchuff.c run-length walk stores one (run | value) entry per non-zero
@@ -26,23 +28,24 @@
 
 namespace b2j {
 
-template <int HS, int VS>
+template <int HS, int VS, int NC = 3>
 struct K1 {
+    static_assert(NC == 3 || (NC == 1 && HS == 1 && VS == 1), "gray is one 1x1 component");
     static constexpr int HV = HS * VS;
-    static constexpr int BPM = HV + 2;
-    static constexpr int TM_MAX = (256 / BPM) & ~1;  // 444: 84, 422/440: 64, 420/411: 42
+    static constexpr int BPM = NC == 1 ? 1 : HV + 2;
+    static constexpr int TM_MAX = (256 / BPM) & ~1;  // 444: 84, 422/440: 64, 420/411: 42, gray: 256
     static constexpr int MCU_W = 8 * HS, MCU_H = 8 * VS;
     static constexpr int TILE_PX = TM_MAX * MCU_W;
-    static constexpr int RAW_STRIDE = TILE_PX * 3;  // multiple of 16 for all five modes
+    static constexpr int RAW_STRIDE = TILE_PX * NC;  // multiple of 16 for all six modes
     static constexpr int RAW_BYTES = RAW_STRIDE * MCU_H;
     static constexpr int TOK_BYTES = 64 * 256 * 4 + 256;    // the tile's token run: <= 64 tokens per block
-    static constexpr int Y_STRIDE = TILE_PX;
+    static constexpr int Y_STRIDE = NC == 1 ? RAW_STRIDE : TILE_PX;
     static constexpr int Y_BYTES = Y_STRIDE * MCU_H;
     static constexpr int C_STRIDE = TM_MAX * 8;
     static constexpr int C_BYTES = C_STRIDE * 8;
     // the raw pixel tile and the sample planes both live inside the token area: they are dead before the first token
-    // is stored (a barrier separates the sample loads of stage B from its token stores)
-    static constexpr int OFF_Y = (RAW_BYTES + 15) & ~15;
+    // is stored (a barrier separates the sample loads of stage B from its token stores). Gray: the raw tile is the Y plane.
+    static constexpr int OFF_Y = NC == 1 ? 0 : (RAW_BYTES + 15) & ~15;
     static constexpr int OFF_CB = OFF_Y + Y_BYTES;
     static constexpr int OFF_CR = OFF_CB + C_BYTES;
     static constexpr int OFF_Q = TOK_BYTES;              // float[3][64] (+ pad): luma, chroma, all-zero (dummy blocks)
@@ -174,7 +177,7 @@ __device__ __forceinline__ int nbits_of(int v) { return 32 - __clz(v < 0 ? -v : 
 // the value bits are jchuff.c's (value, or value - 1 if negative, masked). Raw-DC tokens (first MCU of the tile) pass
 // through. Every token counts one symbol in the bin given by its bits [25:16]; the three raw-DC tokens land in bins
 // 2 / 7 / 11 and are taken out again by thread 0 (k_dc_edge_hist counts their real symbols).
-template <bool HIST>
+template <bool HIST, int NC>
 __device__ __forceinline__ void stage_c(const uint32_t *tok, uint32_t *__restrict__ dst, uint32_t total, uint32_t *hs, int tid) {
 #pragma unroll 4
     for (uint32_t i = tid; i < total; i += 256) {
@@ -194,15 +197,18 @@ __device__ __forceinline__ void stage_c(const uint32_t *tok, uint32_t *__restric
             if (nz) atomicAdd(&hs[(15u << 6) | (((tk >> 16) - (tk >> 22) - 1u) & 3u)], nz);
         }
     }
-    if (HIST && tid == 0) { atomicSub(&hs[2], 1u); atomicSub(&hs[7], 1u); atomicSub(&hs[11], 1u); }   // tcode 2 / 3 | component << 2
+    if (HIST && tid == 0) {   // tcode 2 / 3 | component << 2
+        atomicSub(&hs[2], 1u);
+        if (NC == 3) { atomicSub(&hs[7], 1u); atomicSub(&hs[11], 1u); }
+    }
 }
 
-template <int HS, int VS, bool DUMP>
+template <int HS, int VS, bool DUMP, int NC = 3>
 __global__ void __launch_bounds__(256, 3)
 k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__restrict__ qd,
        uint32_t *__restrict__ pool, uint32_t *__restrict__ pool_count, TileRec *__restrict__ recs,
        uint32_t *__restrict__ ghist, int do_hist, int bulk_ok, int my0, int16_t *__restrict__ coef) {
-    using C = K1<HS, VS>;
+    using C = K1<HS, VS, NC>;
     extern __shared__ __align__(128) uint8_t smem[];
     uint8_t *raw = smem;
     uint32_t *tok = reinterpret_cast<uint32_t *>(smem);
@@ -230,8 +236,8 @@ k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__r
         for (int i = tid; i < 1024; i += 256) hs[i] = 0;
 
     if (interior) {
-        const unsigned row_bytes = (unsigned)tile_px * 3;
-        const uint8_t *src = img + (size_t)y0 * step + (size_t)x0 * 3;
+        const unsigned row_bytes = (unsigned)tile_px * NC;
+        const uint8_t *src = img + (size_t)y0 * step + (size_t)x0 * NC;
         if (bulk_ok) {
             if (tid == 0) {
                 mbar_init(bar, 1);
@@ -249,8 +255,8 @@ k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__r
                 for (int i = tid; i < (int)row_bytes; i += 256) raw[r * C::RAW_STRIDE + i] = src[(size_t)r * step + i];
             __syncthreads();
         }
-        // ---- stage A (fast): one warp per row group (VS pixel rows), 8 pixels per lane and step
-        const int ngx = nmcu * HS;
+        // ---- stage A (fast): one warp per row group (VS pixel rows), 8 pixels per lane and step (gray: nothing to do)
+        const int ngx = NC == 1 ? 0 : nmcu * HS;
         const int rg = wid;
         for (int gx = lane; gx < ngx; gx += 32) {
             // jccolor.c rgb_ycc_convert on packed pixels: every component is two 2-way dot products (IDP.2A, 16-bit
@@ -311,6 +317,13 @@ k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__r
                 *reinterpret_cast<uint16_t *>(dcb) = (uint16_t)ob[0];
                 *reinterpret_cast<uint16_t *>(dcr) = (uint16_t)orr[0];
             }
+        }
+    } else if (NC == 1) {
+        // ---- edge tiles, gray: the last column / row replicated (jcsample.c expand_right_edge, jcprepct.c)
+        for (int i = tid; i < C::MCU_H * tile_px; i += 256) {
+            const int r = i / tile_px, x = i - r * tile_px;
+            const int yy = min(y0 + r, g.H - 1), xx = min(x0 + x, g.W - 1);
+            Yp[r * C::Y_STRIDE + x] = img[(size_t)yy * step + (size_t)xx];
         }
     } else {
         // ---- stage A (edge tiles): per-sample with libjpeg's padding rules (jcprepct.c / jcsample.c expand_right_edge)
@@ -469,8 +482,8 @@ k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__r
     uint32_t off = inc - (uint32_t)ntok, total = 0;
 #pragma unroll
     for (int w = 0; w < 8; w++) { const uint32_t x = misc[w]; if (w < wid) off += x; total += x; }
-    if (tid == C::HV) misc[9] = off;        // run offsets of the first MCU's chroma DC tokens
-    if (tid == C::HV + 1) misc[10] = off;
+    if (NC == 3 && tid == C::HV) misc[9] = off;        // run offsets of the first MCU's chroma DC tokens
+    if (NC == 3 && tid == C::HV + 1) misc[10] = off;
 
     // ---- run-length walk (jchuff.c encode_one_block): one entry per non-zero AC coefficient, straight to its slot:
     //      the token's run / ZRL-count and table fields | coefficient: the run counter advances by TOK_RUN_STEP, which
@@ -501,16 +514,23 @@ k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__r
         const uint32_t base = atomicAdd(pool_count, total);
         misc[8] = base;
         TileRec r;
-        r.base = base; r.count = total; r.pos_cb = (uint16_t)misc[9]; r.pos_cr = (uint16_t)misc[10];
-        r.first_dc[0] = dcs[0]; r.first_dc[1] = dcs[C::HV]; r.first_dc[2] = dcs[C::HV + 1];
-        r.last_dc[0] = dcs[nblk - 3]; r.last_dc[1] = dcs[nblk - 2]; r.last_dc[2] = dcs[nblk - 1];
+        r.base = base; r.count = total;
+        if (NC == 1) {
+            r.pos_cb = r.pos_cr = 0;
+            r.first_dc[0] = dcs[0]; r.first_dc[1] = r.first_dc[2] = 0;
+            r.last_dc[0] = dcs[nblk - 1]; r.last_dc[1] = r.last_dc[2] = 0;
+        } else {
+            r.pos_cb = (uint16_t)misc[9]; r.pos_cr = (uint16_t)misc[10];
+            r.first_dc[0] = dcs[0]; r.first_dc[1] = dcs[C::HV]; r.first_dc[2] = dcs[C::HV + 1];
+            r.last_dc[0] = dcs[nblk - 3]; r.last_dc[1] = dcs[nblk - 2]; r.last_dc[2] = dcs[nblk - 1];
+        }
         recs[tile] = r;
     }
     __syncthreads();
 
     // ---- stage C: the run in output order -> final tokens, symbol statistics, coalesced stores
-    if (do_hist) stage_c<true>(tok, pool + (size_t)misc[8], total, hs, tid);
-    else stage_c<false>(tok, pool + (size_t)misc[8], total, hs, tid);
+    if (do_hist) stage_c<true, NC>(tok, pool + (size_t)misc[8], total, hs, tid);
+    else stage_c<false, NC>(tok, pool + (size_t)misc[8], total, hs, tid);
 
     if (do_hist) {
         __syncthreads();
@@ -526,6 +546,8 @@ k_fdct(const uint8_t *__restrict__ img, size_t step, Geom g, const QuantDev *__r
 // raw-DC tokens of every tile are rewritten in the pool as final difference tokens, so the entropy coder sees one
 // uniform token format. With `xr` (one-collective strip exchange) the strip's first MCU is left alone -- its
 // predictors arrive with the exchange, k_strip_merge finishes it -- and the record's DC / first-token fields are filled.
+// NC: DCs per tile edge (components per image; gray has one raw-DC token per tile).
+template <int NC>
 __global__ void __launch_bounds__(256)
 k_dc_edge_hist(const TileRec *__restrict__ recs, Geom g, const int16_t *__restrict__ pred_in,
                uint32_t *__restrict__ ghist, int16_t *__restrict__ last_dc, int do_hist,
@@ -537,8 +559,8 @@ k_dc_edge_hist(const TileRec *__restrict__ recs, Geom g, const int16_t *__restri
     const int ntile = g.tiles_x * g.mcuy;
     if (threadIdx.x < 32) s_h[threadIdx.x >> 4][threadIdx.x & 15] = 0;
     __syncthreads();
-    if (t < ntile * 3 && (do_hist || resolve) && !(xr && t < 3)) {
-        const int tile = t / 3, c = t - tile * 3;
+    if (t < ntile * NC && (do_hist || resolve) && !(xr && t < NC)) {
+        const int tile = t / NC, c = t - tile * NC;
         const TileRec r = recs[tile];
         const int dc = r.first_dc[c];
         // restart intervals (rst_tiles = tiles per interval, whole MCU rows): predictors return to 0 at an interval start
@@ -551,9 +573,9 @@ k_dc_edge_hist(const TileRec *__restrict__ recs, Geom g, const int16_t *__restri
             pool[r.base + p] = tok_dc(c ? 2u : 0u, (uint32_t)nb, (uint32_t)(diff + (diff >> 31)) & ((1u << nb) - 1u));
         }
     }
-    if (t < 3) last_dc[t] = recs[ntile - 1].last_dc[t];
+    if (t < NC) last_dc[t] = recs[ntile - 1].last_dc[t];
     if (xr) {
-        if (t < 3) xr->first_dc[t] = recs[0].first_dc[t];
+        if (t < NC) xr->first_dc[t] = recs[0].first_dc[t];
         if (t >= 32 && t < 40) {   // tile 0 only: the other tiles' first tokens are being rewritten by this launch
             const uint32_t n = min(recs[0].count, 8u), j = (uint32_t)t - 32u;
             xr->tok[j] = j < n ? pool[recs[0].base + j] : 0u;
@@ -567,11 +589,11 @@ k_dc_edge_hist(const TileRec *__restrict__ recs, Geom g, const int16_t *__restri
     }
 }
 
-template <int HS, int VS, bool DUMP>
+template <int HS, int VS, bool DUMP, int NC>
 static cudaError_t launch_one2(const uint8_t *img, size_t step, const Geom &g, const QuantDev *qd, uint32_t *pool,
                                uint32_t *pool_count, TileRec *recs, uint32_t *hist, int do_hist, int my0, int nrows,
                                int16_t *coef, cudaStream_t s) {
-    using C = K1<HS, VS>;
+    using C = K1<HS, VS, NC>;
     constexpr int SM = C::SMEM;
     // the attribute is per device: one bit per device ordinal (a process may hold contexts on several GPUs)
     static std::atomic<uint64_t> attr_done{0};
@@ -580,35 +602,36 @@ static cudaError_t launch_one2(const uint8_t *img, size_t step, const Geom &g, c
     if (e != cudaSuccess) return e;
     const uint64_t bit = 1ull << (dev & 63);
     if (!(attr_done.load(std::memory_order_acquire) & bit)) {
-        e = cudaFuncSetAttribute(k_fdct<HS, VS, DUMP>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM);
+        e = cudaFuncSetAttribute(k_fdct<HS, VS, DUMP, NC>, cudaFuncAttributeMaxDynamicSharedMemorySize, SM);
         if (e != cudaSuccess) return e;
         attr_done.fetch_or(bit, std::memory_order_release);
     }
     // TMA bulk copies need 16-byte aligned global addresses and sizes for every row of every interior tile
-    const int row_unit = g.tm * C::MCU_W * 3;  // byte offset between tiles in a row
+    const int row_unit = g.tm * C::MCU_W * NC;  // byte offset between tiles in a row
     int bulk_ok = ((reinterpret_cast<uintptr_t>(img) & 15) == 0) && (step % 16 == 0) && (row_unit % 16 == 0);
     // the last tile of a row may hold fewer MCUs: its byte count must be a multiple of 16 as well
     const int last_n = g.mcux - (g.tiles_x - 1) * g.tm;
-    if ((last_n * C::MCU_W * 3) % 16 != 0 && (long long)g.mcux * C::MCU_W <= g.W) bulk_ok = 0;
+    if ((last_n * C::MCU_W * NC) % 16 != 0 && (long long)g.mcux * C::MCU_W <= g.W) bulk_ok = 0;
     dim3 grid(g.tiles_x, nrows);
-    k_fdct<HS, VS, DUMP><<<grid, 256, SM, s>>>(img, step, g, qd, pool, pool_count, recs, hist, do_hist, bulk_ok, my0, coef);
+    k_fdct<HS, VS, DUMP, NC><<<grid, 256, SM, s>>>(img, step, g, qd, pool, pool_count, recs, hist, do_hist, bulk_ok, my0, coef);
     return cudaGetLastError();
 }
 
-template <int HS, int VS>
+template <int HS, int VS, int NC = 3>
 static cudaError_t launch_one(const uint8_t *img, size_t step, const Geom &g, const QuantDev *qd, uint32_t *pool,
                               uint32_t *pool_count, TileRec *recs, uint32_t *hist, int do_hist, int my0, int nrows,
                               int16_t *coef, cudaStream_t s) {
-    return coef ? launch_one2<HS, VS, true>(img, step, g, qd, pool, pool_count, recs, hist, do_hist, my0, nrows, coef, s)
-                : launch_one2<HS, VS, false>(img, step, g, qd, pool, pool_count, recs, hist, do_hist, my0, nrows, coef, s);
+    return coef ? launch_one2<HS, VS, true, NC>(img, step, g, qd, pool, pool_count, recs, hist, do_hist, my0, nrows, coef, s)
+                : launch_one2<HS, VS, false, NC>(img, step, g, qd, pool, pool_count, recs, hist, do_hist, my0, nrows, coef, s);
 }
 
-int fdct_tm_max(int hs, int vs) { return (256 / (hs * vs + 2)) & ~1; }
+int fdct_tm_max(int hs, int vs, int nc) { return (256 / (nc == 1 ? 1 : hs * vs + 2)) & ~1; }
 
 cudaError_t launch_fdct(const uint8_t *img, size_t step, const Geom &g, const QuantDev *qd, uint32_t *pool,
                         uint32_t *pool_count, TileRec *recs, uint32_t *hist, int do_hist, int my0, int nrows,
                         int16_t *coef_dump, cudaStream_t s) {
 #define B2J_ARGS img, step, g, qd, pool, pool_count, recs, hist, do_hist, my0, nrows, coef_dump, s
+    if (g.nc == 1) return launch_one<1, 1, 1>(B2J_ARGS);
     if (g.hs == 1 && g.vs == 1) return launch_one<1, 1>(B2J_ARGS);
     if (g.hs == 2 && g.vs == 1) return launch_one<2, 1>(B2J_ARGS);
     if (g.hs == 1 && g.vs == 2) return launch_one<1, 2>(B2J_ARGS);
@@ -620,8 +643,10 @@ cudaError_t launch_fdct(const uint8_t *img, size_t step, const Geom &g, const Qu
 
 cudaError_t launch_dc_edge_hist(const TileRec *recs, const Geom &g, const int16_t *pred_in, uint32_t *hist,
                                 int16_t *last_dc, int do_hist, uint32_t *pool, int resolve, StripRecord *xr, int rst_tiles, cudaStream_t s) {
-    const int n = max(64, g.tiles_x * g.mcuy * 3);
-    return launch_pdl(k_dc_edge_hist, dim3((n + 255) / 256), dim3(256), 0, s, recs, g, pred_in, hist, last_dc, do_hist, pool, resolve, xr, rst_tiles);
+    const int n = max(64, g.tiles_x * g.mcuy * g.nc);
+    if (g.nc == 1)
+        return launch_pdl(k_dc_edge_hist<1>, dim3((n + 255) / 256), dim3(256), 0, s, recs, g, pred_in, hist, last_dc, do_hist, pool, resolve, xr, rst_tiles);
+    return launch_pdl(k_dc_edge_hist<3>, dim3((n + 255) / 256), dim3(256), 0, s, recs, g, pred_in, hist, last_dc, do_hist, pool, resolve, xr, rst_tiles);
 }
 
 }  // namespace b2j

@@ -39,12 +39,15 @@ __constant__ uint8_t c_std_ac_val[2][162] = {
      0xe2, 0xe3, 0xe4, 0xe5, 0xe6, 0xe7, 0xe8, 0xe9, 0xea, 0xf2, 0xf3, 0xf4, 0xf5, 0xf6, 0xf7, 0xf8, 0xf9, 0xfa}};
 
 // ------------------------------------------------------------------------------------------------------
-// k_tables: one CTA, warp t builds table t (DC0, AC0, DC1, AC1), then the JFIF headers are written.
+// k_tables: one CTA, warp t builds table t (DC0, AC0, DC1, AC1), then the JFIF headers are written. NC = 1 (gray):
+// only DC0 / AC0 are coded; warps 2 and 3 load the standard chroma tables (never emitted, never looked up) instead of
+// building codes from the all-zero DC1 / AC1 histograms, and the headers have one DQT, two DHTs and one component.
 //
 // jpeg_gen_optimal_table, warp-parallel: lane l owns symbols l, l+32, ... (9 per lane, symbol 256 = the reserved
 // all-ones code point). Each merge step finds c1 = least non-zero frequency with ties to the LARGER index, c2 = next
 // least, by two warp reductions each (min of frequency, then max of index among the minima); tree membership is a
 // group id per symbol so "increment codesize along the others chain" becomes "increment every member".
+template <int NC>
 __global__ void __launch_bounds__(128)
 k_tables(const uint32_t *hist /* the predecessor's output: no __restrict__, loads must stay behind pdl_wait() */, int optimize,
          HuffDev *__restrict__ huff, const QuantDev *__restrict__ qd,
@@ -68,7 +71,7 @@ k_tables(const uint32_t *hist /* the predecessor's output: no __restrict__, load
     __syncthreads();
     pdl_wait();
 
-    if (!optimize) {
+    if (!optimize || (NC == 1 && t >= 2)) {
         if (lane < 17) s_bits[t][lane] = c_std_bits[t][lane];
         const int ns = (t & 1) ? 162 : 12;
         for (int i = lane; i < ns; i += 32) s_vals[t][i] = (t & 1) ? c_std_ac_val[t >> 1][i] : c_std_dc_val[i];
@@ -243,15 +246,18 @@ k_tables(const uint32_t *hist /* the predecessor's output: no __restrict__, load
     }
     __syncthreads();
 
-    // ---- headers (jcmarker.c): SOI, JFIF APP0, 2 x DQT, SOF0, 4 x DHT, SOS -- section offsets by thread 0, bytes by
+    // ---- headers (jcmarker.c): SOI, JFIF APP0, 2 x DQT, SOF0, 4 x DHT, SOS (gray: 1 x DQT, 2 x DHT) -- section offsets by thread 0, bytes by
     //      all threads
     __shared__ uint32_t s_off[9];   // DQT0, DQT1, SOF0, DHT0..3, SOS, DRI (jcmarker.c: after the scan's DHTs, before SOS)
+    constexpr int NH = NC == 1 ? 2 : 4;   // DHTs
     if (threadIdx.x == 0) {
         uint32_t n = 20;
-        s_off[0] = n; n += 69; s_off[1] = n; n += 69; s_off[2] = n; n += 19;
-        for (int q = 0; q < 4; q++) { s_off[3 + q] = n; n += 21 + s_nsym[q]; }
+        s_off[0] = n; n += 69;
+        if (NC == 3) { s_off[1] = n; n += 69; }
+        s_off[2] = n; n += 10 + 3 * NC;
+        for (int q = 0; q < NH; q++) { s_off[3 + q] = n; n += 21 + s_nsym[q]; }
         s_off[8] = n; if (restart_interval) n += 6;
-        s_off[7] = n; n += 14;
+        s_off[7] = n; n += 8 + 2 * NC;
         if (!emit_header) n = 0;
         s_hdr_len = n;
         huff->hdr_len = n;
@@ -266,7 +272,7 @@ k_tables(const uint32_t *hist /* the predecessor's output: no __restrict__, load
             const uint8_t app0[20] = {0xFF, 0xD8, 0xFF, 0xE0, 0, 16, 'J', 'F', 'I', 'F', 0, 1, 1, 0, 0, 1, 0, 1, 0, 0};
             h[x] = app0[x];
         }
-        {   // DQT: thread x -> table x >> 6, coefficient x & 63 (zig-zag order)
+        if (NC == 3 || x < 64) {   // DQT: thread x -> table x >> 6, coefficient x & 63 (zig-zag order)
             const int q = x >> 6, k = x & 63;
             uint8_t *d = h + s_off[q];
             if (k == 0) { d[0] = 0xFF; d[1] = 0xDB; d[2] = 0; d[3] = 67; d[4] = (uint8_t)q; }
@@ -274,9 +280,15 @@ k_tables(const uint32_t *hist /* the predecessor's output: no __restrict__, load
         }
         if (x == 32) {
             uint8_t *d = h + s_off[2];
-            const uint8_t sof[19] = {0xFF, 0xC0, 0, 17, 8, (uint8_t)(full_h >> 8), (uint8_t)full_h, (uint8_t)(full_w >> 8), (uint8_t)full_w,
-                                     3, 1, (uint8_t)((hs << 4) | vs), 0, 2, 0x11, 1, 3, 0x11, 1};
-            for (int i = 0; i < 19; i++) d[i] = sof[i];
+            if constexpr (NC == 1) {
+                const uint8_t sof[13] = {0xFF, 0xC0, 0, 11, 8, (uint8_t)(full_h >> 8), (uint8_t)full_h, (uint8_t)(full_w >> 8), (uint8_t)full_w,
+                                         1, 1, 0x11, 0};
+                for (int i = 0; i < 13; i++) d[i] = sof[i];
+            } else {
+                const uint8_t sof[19] = {0xFF, 0xC0, 0, 17, 8, (uint8_t)(full_h >> 8), (uint8_t)full_h, (uint8_t)(full_w >> 8), (uint8_t)full_w,
+                                         3, 1, (uint8_t)((hs << 4) | vs), 0, 2, 0x11, 1, 3, 0x11, 1};
+                for (int i = 0; i < 19; i++) d[i] = sof[i];
+            }
         }
         if (x == 96 && restart_interval) {
             uint8_t *d = h + s_off[8];
@@ -284,10 +296,15 @@ k_tables(const uint32_t *hist /* the predecessor's output: no __restrict__, load
         }
         if (x == 64) {
             uint8_t *d = h + s_off[7];
-            const uint8_t sos[14] = {0xFF, 0xDA, 0, 12, 3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0};
-            for (int i = 0; i < 14; i++) d[i] = sos[i];
+            if constexpr (NC == 1) {
+                const uint8_t sos[10] = {0xFF, 0xDA, 0, 8, 1, 1, 0x00, 0, 63, 0};
+                for (int i = 0; i < 10; i++) d[i] = sos[i];
+            } else {
+                const uint8_t sos[14] = {0xFF, 0xDA, 0, 12, 3, 1, 0x00, 2, 0x11, 3, 0x11, 0, 63, 0};
+                for (int i = 0; i < 14; i++) d[i] = sos[i];
+            }
         }
-        {   // DHT q by warp q
+        if (NC == 3 || x < 64) {   // DHT q by warp q
             const int q = x >> 5;
             const int ns = (int)s_nsym[q];
             uint8_t *d = h + s_off[3 + q];
@@ -1023,8 +1040,10 @@ k_stuff(StuffArgs a) {
 
 // ------------------------------------------------------------------------------------------------------
 cudaError_t launch_tables(const uint32_t *hist, int optimize, HuffDev *huff, const QuantDev *qd, int full_w, int full_h,
-                          int hs, int vs, uint8_t *out, int emit_header, int restart_interval, uint32_t *err_out, cudaStream_t s) {
-    return launch_pdl(k_tables, dim3(1), dim3(128), 0, s, hist, optimize, huff, qd, full_w, full_h, hs, vs, out, emit_header, restart_interval, err_out);
+                          int hs, int vs, int nc, uint8_t *out, int emit_header, int restart_interval, uint32_t *err_out, cudaStream_t s) {
+    if (nc == 1)
+        return launch_pdl(k_tables<1>, dim3(1), dim3(128), 0, s, hist, optimize, huff, qd, full_w, full_h, hs, vs, out, emit_header, restart_interval, err_out);
+    return launch_pdl(k_tables<3>, dim3(1), dim3(128), 0, s, hist, optimize, huff, qd, full_w, full_h, hs, vs, out, emit_header, restart_interval, err_out);
 }
 cudaError_t launch_pack(const uint32_t *pool, const TileRec *recs, const Geom &g, const HuffDev *huff,
                         uint32_t *slots, uint32_t *tile_bits, int small_buffers, cudaStream_t s) {

@@ -5,7 +5,7 @@
 namespace b2j {
 
 // encode
-int fdct_tm_max(int hs, int vs);
+int fdct_tm_max(int hs, int vs, int nc);   // MCUs per fdct tile (even); nc = components per image
 // MCU rows [my0, my0+nrows) of the image `img` (img points at pixel row 0); coef_dump != NULL also writes coefficients
 cudaError_t launch_fdct(const uint8_t *img, size_t step, const Geom &g, const QuantDev *qd, uint32_t *pool,
                         uint32_t *pool_count, TileRec *recs, uint32_t *hist, int do_hist, int my0, int nrows,
@@ -16,8 +16,9 @@ cudaError_t launch_dc_edge_hist(const TileRec *recs, const Geom &g, const int16_
                                 int16_t *last_dc, int do_hist, uint32_t *pool, int resolve, StripRecord *xr, int rst_tiles,
                                 cudaStream_t s);
 // restart_interval != 0: DRI marker (MCUs per interval) between the DHTs and SOS
+// nc == 1 (gray): only DC0/AC0 are built and emitted, with the one-component DQT / SOF0 / SOS
 cudaError_t launch_tables(const uint32_t *hist, int optimize, HuffDev *huff, const QuantDev *qd, int full_w, int full_h,
-                          int hs, int vs, uint8_t *out, int emit_header, int restart_interval, uint32_t *err_out, cudaStream_t s);
+                          int hs, int vs, int nc, uint8_t *out, int emit_header, int restart_interval, uint32_t *err_out, cudaStream_t s);
 // restart intervals of rst_tiles tiles (whole MCU rows): every interval but the last gets 1-padding to a byte boundary
 // and its RSTn marker appended to its last tile's bits (run between k_pack and the tile scan)
 cudaError_t launch_rst_pad(uint32_t *slots, uint32_t *tile_bits, int ntiles, int rst_tiles, cudaStream_t s);

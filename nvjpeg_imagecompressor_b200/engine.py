@@ -16,15 +16,21 @@ def _ptr(a):
     return C.c_void_p(a.ctypes.data)
 
 
+def css_id(css):
+    return N.CSS[css] if isinstance(css, str) else int(css)
+
+
 class Engine:
     """width/height: the largest image this context will see (buffers are sized once, like the reference's
-    initCompressEnv, ImageCompressorImpl.cu:33-37)."""
+    initCompressEnv, ImageCompressorImpl.cu:33-37). css "gray" (or "400", 6): images are (H, W) uint8, one byte per
+    pixel -- encode takes (H, W) or (H, W, 1), decode returns (H, W) for one-component files and the Y plane of colour
+    ones; the strip, reconstruction and secondary-compression entry points refuse such a context."""
 
     def __init__(self, width=8320, height=40000, quality=95, optimize=True, css="422", device=-1, flags=0):
         self._L = N.lib()
-        p = N.Params(int(width), int(height), int(quality), int(bool(optimize)),
-                     N.CSS[css] if isinstance(css, str) else int(css), int(device), int(flags))
+        p = N.Params(int(width), int(height), int(quality), int(bool(optimize)), css_id(css), int(device), int(flags))
         self.params = p
+        self.channels = 1 if p.css == N.CSS_GRAY else 3
         h = C.c_void_p()
         rc = self._L.b2j_create(C.byref(p), C.byref(h))
         if rc:
@@ -49,7 +55,13 @@ class Engine:
     # ---------------------------------------------------------------- host API
     def encode(self, img, out=None):
         img = np.asarray(img)
-        assert img.dtype == np.uint8 and img.ndim == 3 and img.shape[2] == 3 and img.strides[2] == 1 and img.strides[1] == 3
+        if self.channels == 1:
+            if img.ndim == 3 and img.shape[2] == 1:
+                img = img[:, :, 0]
+            assert img.dtype == np.uint8 and img.ndim == 2 and (img.strides[1] == 1 or img.shape[1] == 1), \
+                "a gray context encodes (H, W) uint8 rows"
+        else:
+            assert img.dtype == np.uint8 and img.ndim == 3 and img.shape[2] == 3 and img.strides[2] == 1 and img.strides[1] == 3
         H, W = img.shape[:2]
         if out is None:
             out = np.empty(min(self._L.b2j_encode_bound(self._h), W * H * 3 * 2 + 65536), np.uint8)
@@ -66,8 +78,9 @@ class Engine:
         jpg = np.ascontiguousarray(jpg, np.uint8)
         W, H = C.c_int(0), C.c_int(0)
         self._ck(self._L.b2j_decode(self._h, _ptr(jpg), jpg.size, None, 0, C.byref(W), C.byref(H)))
-        out = np.empty((H.value, W.value, 3), np.uint8)
-        self._ck(self._L.b2j_decode(self._h, _ptr(jpg), jpg.size, _ptr(out), W.value * 3, C.byref(W), C.byref(H)))
+        shape = (H.value, W.value) if self.channels == 1 else (H.value, W.value, 3)
+        out = np.empty(shape, np.uint8)
+        self._ck(self._L.b2j_decode(self._h, _ptr(jpg), jpg.size, _ptr(out), W.value * self.channels, C.byref(W), C.byref(H)))
         return out
 
     def decode_ptr(self, jpg, out_ptr, step):
@@ -260,6 +273,9 @@ class MultiEngine:
 
     def __init__(self, width, height, quality=95, optimize=True, css="422", devices=(0,)):
         self._L = N.lib()
+        self._h = None
+        if css_id(css) == N.CSS_GRAY:
+            raise B2JError(-1, "MultiEngine: gray images are encoded on one GPU (Engine); the strips assume three components")
         p = N.Params()
         self._L.b2j_default_params(C.byref(p))
         p.width, p.height, p.quality, p.optimize = int(width), int(height), int(quality), int(bool(optimize))

@@ -29,6 +29,7 @@ import torch
 import torch.distributed as dist
 
 from . import _native as N
+from .engine import B2JError
 
 _HS = {0: 1, 1: 2, 2: 1, 3: 2, 4: 4}
 _VS = {0: 1, 1: 1, 2: 2, 3: 2, 4: 1}
@@ -121,6 +122,8 @@ class StripEncoder:
                  group=None, peer=None):
         self.W, self.H = W, H
         self.css = N.CSS[css] if isinstance(css, str) else int(css)
+        if self.css == N.CSS_GRAY:
+            raise B2JError(-1, "StripEncoder: gray images are not supported (the strips' records and seams assume three components)")
         self.optimize = bool(optimize)
         self.group = group
         self.rank = dist.get_rank(group) if rank is None else rank
@@ -252,6 +255,8 @@ class StripSecondary:
         from .engine import Engine
         self.W, self.H, self.mode, self.group = W, H, int(diff_mode), group
         css_id = N.CSS[css] if isinstance(css, str) else int(css)
+        if css_id == N.CSS_GRAY:
+            raise B2JError(-1, "StripSecondary: gray images are not supported")
         self.enc1 = StripEncoder(W, H, quality, optimize, css_id, rank, world, None, device, group)
         self.enc2 = StripEncoder(W, H, quality, optimize, css_id, rank, world, None, device, group)
         self.rank, self.world = self.enc1.rank, self.enc1.world
