@@ -14,6 +14,7 @@ public:
     b2j_params p;
     b2j_ctx *enc = nullptr, *dec = nullptr;
     int ngpus = 1, restart_rows = 0;
+    int decode_scale = 1;         // setDecodeScale: decode() returns the image at 1 / decode_scale
     b2j_multi *multi = nullptr;   // compress() over several GPUs (ngpus > 1)
     static bool quiet() { return getenv("B2J_QUIET") != nullptr; }
     int ensure(b2j_ctx **c) {
@@ -117,20 +118,35 @@ std::vector<unsigned char> NvjpegCompressRunner::compress(cv::Mat image, int *ru
     return obuffer;
 }
 
-cv::Mat NvjpegCompressRunner::reconstruct(const std::vector<unsigned char> &jpg, int *run_state) {
+// JPEG bytes -> pixels at 1 / scale. The scale is set on the (possibly shared) context for this call only: compress()
+// and reconstruct() keep seeing full-size decodes.
+static cv::Mat decode_at(NvjpegCompressRunnerImpl *m, const std::vector<unsigned char> &jpg, int scale) {
     cv::Mat result;
-    b2j_ctx *c = compressor->dec ? compressor->dec : compressor->enc;
+    b2j_ctx *c = m->dec ? m->dec : m->enc;
+    if (!c || jpg.empty()) return result;
+    if (b2j_set_decode_scale(c, scale) != B2J_OK) {
+        std::cerr << "[ERROR] decode: invalid decode scale " << scale << " (1, 2, 4 or 8)" << std::endl;
+        return result;
+    }
     int w = 0, h = 0;
-    if (c && !jpg.empty() && b2j_decode(c, jpg.data(), jpg.size(), nullptr, 0, &w, &h) == B2J_OK) {
-        result.create(h, w, compressor->mat_type());
+    if (b2j_decode(c, jpg.data(), jpg.size(), nullptr, 0, &w, &h) == B2J_OK) {
+        result.create(h, w, m->mat_type());
         if (b2j_decode(c, jpg.data(), jpg.size(), result.data, result.step, &w, &h) != B2J_OK) {
             std::cerr << "[ERROR] decode: " << b2j_last_error(c) << std::endl;
             result = cv::Mat();
         }
     }
+    b2j_set_decode_scale(c, 1);
+    return result;
+}
+
+cv::Mat NvjpegCompressRunner::reconstruct(const std::vector<unsigned char> &jpg, int *run_state) {
+    cv::Mat result = decode_at(compressor, jpg, 1);   // full size: differenceMap / psnr compare it with the original
     if (run_state) *run_state = result.empty() ? 0 : 1;
     return result;
 }
+
+void NvjpegCompressRunner::setDecodeScale(int denom) { compressor->decode_scale = denom; }
 
 cv::Mat NvjpegCompressRunner::decode(std::string image_path, int *run_state) {
     FILE *f = fopen(image_path.c_str(), "rb");
@@ -147,7 +163,7 @@ cv::Mat NvjpegCompressRunner::decode(std::string image_path, int *run_state) {
     const size_t rd = jpg.empty() ? 0 : fread(jpg.data(), 1, jpg.size(), f);
     fclose(f);
     cv::Mat result;
-    if (rd == jpg.size() && !jpg.empty()) result = reconstruct(jpg, nullptr);
+    if (rd == jpg.size() && !jpg.empty()) result = decode_at(compressor, jpg, compressor->decode_scale);
     else std::cerr << "[INFO] Failed to read the entire JPEG data." << std::endl;
     if (run_state) *run_state = result.empty() ? 0 : 1;
     auto ms = std::chrono::duration_cast<std::chrono::milliseconds>(std::chrono::steady_clock::now() - t0).count();

@@ -8,7 +8,8 @@
 //     (README default 4:2:2) and the stream is baseline sequential, not progressive (ImageCompressorImpl.cu:28)
 //   * CUDA failures never exit(1) (ImageCompressorImpl.cuh:16-34); they produce the documented failure signal
 //   * reconstruct / differenceMap / psnr / secondaryCompress implement the README's feature bullet (README.md:8)
-//   * a defaulted 6th constructor argument spreads compress() over several GPUs; setRestartRows() turns DRI/RSTn on
+//   * a defaulted 6th constructor argument spreads compress() over several GPUs; setRestartRows() turns DRI/RSTn on;
+//     setDecodeScale() makes decode() return a reduced image (cv::IMREAD_REDUCED_*)
 #ifndef IMAGECOMPRESSOR_H_
 #define IMAGECOMPRESSOR_H_
 
@@ -75,6 +76,11 @@ public:
     // nvjpegEncoderParamsSetRestartInterval / cv2 IMWRITE_JPEG_RST_INTERVAL at the reference's parameter site
     // (ImageCompressorImpl.cu:28-31). decode() / reconstruct() accept any restart interval and progressive files.
     void setRestartRows(int mcu_rows);
+    // decode() returns the image at 1 / denom (denom 1, 2, 4 or 8; 1 = full size, the default), as
+    // cv::imread(path, IMREAD_REDUCED_COLOR_denom) does (IMREAD_REDUCED_GRAYSCALE_denom with sampling 400): libjpeg's DCT
+    // scaling, ceil(W / denom) x ceil(H / denom) pixels. Any other value makes decode() give the failure signal.
+    // reconstruct() stays full size (differenceMap / psnr compare it with the original).
+    void setDecodeScale(int denom);
 
     // README.md:8 -- reconstruction, difference map, secondary compression, PSNR
     cv::Mat reconstruct(const std::vector<unsigned char> &obuffer, int *run_state);

@@ -136,6 +136,15 @@ B2J_API int b2j_decode_device(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint
  * allocation, which every CUDA allocation granule (>= 256 bytes) contains. */
 B2J_API int b2j_decode_scan_device(b2j_ctx *ctx, const uint8_t *hdr, size_t hdr_len, const uint8_t *d_scan, size_t scan_len,
                                    int height_override, uint8_t *d_bgr, size_t step, int *width, int *height);
+/* Reduced-size decode: libjpeg's scale_num = 1, scale_denom = denom (cv2 IMREAD_REDUCED_COLOR_denom /
+ * IMREAD_REDUCED_GRAYSCALE_denom), denom in {1, 2, 4, 8}; 1 (full size) is the default. Any other value returns
+ * B2J_EINVAL and leaves the setting unchanged. It applies to b2j_decode, b2j_decode_device / b2j_decode_finish and
+ * b2j_decode_scan_device, for baseline, restart-marker and progressive files, on colour and gray contexts: their
+ * width / height report the output size ceil(W / denom) x ceil(H / denom) (also with a NULL image, to size buffers),
+ * and `step` is checked against that width. The samples equal libjpeg-turbo's DCT-scaled decode (jidctred.c, jdsample.c).
+ * A context sized W x H decodes files up to that size at every scale. b2j_peek still reports the file's size; the
+ * encoders, the strips, b2j_reconstruct_* and b2j_secondary* are not affected. */
+B2J_API int b2j_set_decode_scale(b2j_ctx *ctx, int denom);
 /* Completes the last b2j_decode_device: waits for it and validates it. The decode runs a fixed schedule of Huffman
  * synchronisation launches without asking the host; in the rare case that was too short the image is decoded again
  * here with the checked schedule. `jpg` of the b2j_decode_device call must stay valid until this returns. */

@@ -53,6 +53,7 @@ SYMBOLS = ["b2j_default_params", "b2j_create", "b2j_destroy", "b2j_last_error", 
            "b2j_multi_create", "b2j_multi_destroy", "b2j_multi_encode", "b2j_multi_encode_begin", "b2j_multi_encode_fetch",
            "b2j_multi_last_error",
            "b2j_strip_state_get", "b2j_strip_phase1", "b2j_strip_phase1b", "b2j_strip_phase2", "b2j_strip_phase3", "b2j_strip_phase3_dev", "b2j_strip_phase1x", "b2j_strip_phase2x", "b2j_peer_export", "b2j_peer_open", "b2j_peer_connect", "b2j_set_restart_rows",
+           "b2j_set_decode_scale",
            "b2j_debug_read", "b2j_set_debug", "b2j_last_timings", "b2j_enable_timing", "b2j_launch_count", "b2j_host_alloc",
            "b2j_host_free"]
 
@@ -128,6 +129,7 @@ def lib():
     L.b2j_peer_open.argtypes = [vp, vp, C.POINTER(vp)]
     L.b2j_peer_connect.argtypes = [vp, i, i, C.POINTER(vp)]
     L.b2j_set_restart_rows.argtypes = [vp, i]
+    L.b2j_set_decode_scale.argtypes = [vp, i]
     L.b2j_debug_read.argtypes = [vp, i, vp, sz, C.POINTER(sz)]
     L.b2j_set_debug.argtypes = [vp, i]
     L.b2j_last_timings.argtypes = [vp, C.POINTER(Timings)]

@@ -94,6 +94,8 @@ struct b2j_ctx {
     const uint8_t *last_jpg;
     size_t last_len, last_step;
     uint8_t *last_bgr;
+    int last_scale;                // ... and the scale it was issued with (its checked retry keeps it)
+    int dec_scale;                 // decode output at 1 / dec_scale (1, 2, 4, 8); b2j_set_decode_scale
     b2j_ctx *second;  // encoder for the difference image (secondary compression)
     uint8_t *d_rplanes; size_t rplanes_bytes;   // reconstruction from the encoder's coefficients: sample planes
     void *d_rtb;                                // ... and de-quantisation tables (a DecTables with q filled)
@@ -260,6 +262,7 @@ int b2j_create(const b2j_params *p, b2j_ctx **out) {
     int rc = make_geom(p->width, p->height, p->css, &ctx->cap_g);
     if (rc) { delete ctx; return rc; }
     ctx->g = ctx->cap_g;
+    ctx->dec_scale = 1;
     make_quant(p->quality, &ctx->hq);
     cudaError_t e;
     if (p->device >= 0) {
@@ -316,6 +319,13 @@ size_t b2j_encode_bound(const b2j_ctx *ctx) { return ctx ? (size_t)ctx->cap_g.nb
 int b2j_set_restart_rows(b2j_ctx *ctx, int rows) {
     if (!ctx || rows < 0 || (long long)rows * ctx->cap_g.mcux > 65535) return B2J_EINVAL;
     ctx->rst_rows = rows;
+    return B2J_OK;
+}
+// Reduced-size decode: libjpeg's scale_num = 1, scale_denom = denom (cv2 IMREAD_REDUCED_*_denom). The entropy stages are
+// unchanged; the back end runs jidctred.c's smaller inverse DCTs (dec_scaled.cu).
+int b2j_set_decode_scale(b2j_ctx *ctx, int denom) {
+    if (!ctx || (denom != 1 && denom != 2 && denom != 4 && denom != 8)) return B2J_EINVAL;
+    ctx->dec_scale = denom;
     return B2J_OK;
 }
 uint64_t b2j_launch_count(const b2j_ctx *ctx) { return ctx ? ctx->launches : 0; }
@@ -1003,6 +1013,7 @@ static int check_components(b2j_ctx *ctx, int file_css) {
 }
 
 // progressive (SOF2) files: parsed and decoded scan by scan (dec_prog.cu); returns B2J_EFORMAT if it is not one
+// width / height: the output size (the file's at the context's decode scale)
 static int decode_progressive_to(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *d_bgr, size_t step, bool alloc_recon,
                                  int *width, int *height) {
     ProgInfo pi;
@@ -1010,46 +1021,47 @@ static int decode_progressive_to(b2j_ctx *ctx, const uint8_t *jpg, size_t len, u
     if (rc) return rc;
     rc = check_components(ctx, pi.css);
     if (rc) { prog_free(&pi); return rc; }
-    const int ch = chans(ctx);
-    if (width) *width = pi.W;
-    if (height) *height = pi.H;
+    const int ch = chans(ctx), scale = ctx->dec_scale;
+    const int ow = dec_scaled_size(pi.W, scale), oh = dec_scaled_size(pi.H, scale);
+    if (width) *width = ow;
+    if (height) *height = oh;
     Geom g;
     rc = make_geom(pi.W, pi.H, pi.css, &g);
     if (!rc && (d_bgr || alloc_recon)) {
         size_t dstep = step;
         if (alloc_recon) {
-            dstep = ((size_t)pi.W * ch + 15) & ~(size_t)15;
-            if (ctx->d_recon_bytes < dstep * pi.H) {
+            dstep = ((size_t)ow * ch + 15) & ~(size_t)15;
+            if (ctx->d_recon_bytes < dstep * oh) {
                 cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0;
-                if (cudaMalloc(&ctx->d_recon, dstep * pi.H) != cudaSuccess) { prog_free(&pi); return B2J_ECUDA; }
-                ctx->d_recon_bytes = dstep * pi.H;
+                if (cudaMalloc(&ctx->d_recon, dstep * oh) != cudaSuccess) { prog_free(&pi); return B2J_ECUDA; }
+                ctx->d_recon_bytes = dstep * oh;
             }
             d_bgr = ctx->d_recon;
         }
-        if (dstep < (size_t)pi.W * ch) rc = B2J_EINVAL;
+        if (dstep < (size_t)ow * ch) rc = B2J_EINVAL;
         if (!rc) rc = dec_ensure(ctx);
-        if (!rc) rc = dec_run_progressive(ctx->dec, jpg, len, pi, g, d_bgr, dstep, ch == 1, ctx->stream, &ctx->launches);
+        if (!rc) rc = dec_run_progressive(ctx->dec, jpg, len, pi, g, d_bgr, dstep, ch == 1, ctx->stream, &ctx->launches, scale);
     }
     prog_free(&pi);
     return rc;
 }
 
 static int decode_parsed(b2j_ctx *ctx, const uint8_t *jpg, size_t len, const JpegInfo &info, uint8_t *d_bgr, size_t step, bool careful,
-                         const uint8_t *d_scan_src = nullptr) {
-    if (step < (size_t)info.W * chans(ctx)) return B2J_EINVAL;
+                         int scale, const uint8_t *d_scan_src = nullptr) {
+    if (step < (size_t)dec_scaled_size(info.W, scale) * chans(ctx)) return B2J_EINVAL;
     int rc = dec_ensure(ctx); if (rc) return rc;
     Geom g; rc = make_geom(info.W, info.H, info.css, &g); if (rc) return rc;
     dec_set_spec_launches(ctx->dec, (ctx->debug & 4) ? 1 : 3);
     return dec_run(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, ctx->timing ? &ctx->tm : nullptr,
-                   &ctx->launches, careful, d_scan_src);
+                   &ctx->launches, careful, d_scan_src, scale);
 }
 
 static int parse_for(b2j_ctx *ctx, const uint8_t *jpg, size_t len, JpegInfo *info, int *width, int *height) {
     int rc = parse_jpeg(jpg, len, info);
     if (rc) { snprintf(ctx->err, sizeof(ctx->err), "unsupported or corrupt JPEG (parse rc=%d)", rc); return B2J_EFORMAT; }
     rc = check_components(ctx, info->css); if (rc) return rc;
-    if (width) *width = info->W;
-    if (height) *height = info->H;
+    if (width) *width = dec_scaled_size(info->W, ctx->dec_scale);
+    if (height) *height = dec_scaled_size(info->H, ctx->dec_scale);
     return B2J_OK;
 }
 
@@ -1068,8 +1080,8 @@ int b2j_decode_device(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *d_b
     // one decode in flight per context: an unfinished predecessor is finished (validated, retried if needed) first
     if (ctx->last_jpg) { rc = b2j_decode_finish(ctx); if (rc) return rc; }
     // remembered for b2j_decode_finish: the caller keeps `jpg` alive until then
-    ctx->last_jpg = jpg; ctx->last_len = len; ctx->last_bgr = d_bgr; ctx->last_step = step;
-    return decode_parsed(ctx, jpg, len, info, d_bgr, step, false);
+    ctx->last_jpg = jpg; ctx->last_len = len; ctx->last_bgr = d_bgr; ctx->last_step = step; ctx->last_scale = ctx->dec_scale;
+    return decode_parsed(ctx, jpg, len, info, d_bgr, step, false, ctx->last_scale);
 }
 
 // A baseline JPEG whose entropy-coded segment is already in DEVICE memory (the output of b2j_encode_device, a slice
@@ -1088,10 +1100,11 @@ int b2j_decode_scan_device(b2j_ctx *ctx, const uint8_t *hdr, size_t hdr_len, con
     if (info.scan_offset != hdr_len) { snprintf(ctx->err, sizeof(ctx->err), "hdr must end with the SOS header"); return B2J_EINVAL; }
     if (height_override > 0) info.H = height_override;
     info.scan_offset = 0; info.scan_len = scan_len;
-    if (width) *width = info.W;
-    if (height) *height = info.H;
+    const int scale = ctx->dec_scale;
+    if (width) *width = dec_scaled_size(info.W, scale);
+    if (height) *height = dec_scaled_size(info.H, scale);
     for (int attempt = 0; attempt < 2; attempt++) {
-        rc = decode_parsed(ctx, hdr, hdr_len, info, d_bgr, step, attempt == 1, d_scan); if (rc) return rc;
+        rc = decode_parsed(ctx, hdr, hdr_len, info, d_bgr, step, attempt == 1, scale, d_scan); if (rc) return rc;
         rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
         if (rc != DEC_RETRY) break;
     }
@@ -1106,7 +1119,7 @@ int b2j_decode_finish(b2j_ctx *ctx) {
     if (rc == DEC_RETRY) {   // the speculative synchronisation schedule was too short for this stream: decode again, checked
         JpegInfo info;
         rc = parse_for(ctx, ctx->last_jpg, ctx->last_len, &info, nullptr, nullptr); if (rc) return rc;
-        rc = decode_parsed(ctx, ctx->last_jpg, ctx->last_len, info, ctx->last_bgr, ctx->last_step, true); if (rc) return rc;
+        rc = decode_parsed(ctx, ctx->last_jpg, ctx->last_len, info, ctx->last_bgr, ctx->last_step, true, ctx->last_scale); if (rc) return rc;
         rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
     }
     ctx->last_jpg = nullptr;
@@ -1133,17 +1146,18 @@ int b2j_decode(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *bgr, size_
     }
     if (rc) return rc;
     if (!bgr) return B2J_OK;
-    if (step < (size_t)info.W * ch) return B2J_EINVAL;
-    const size_t dstep = ((size_t)info.W * ch + 15) & ~(size_t)15;
-    if (ctx->d_recon_bytes < dstep * info.H) {
+    const int scale = ctx->dec_scale, ow = dec_scaled_size(info.W, scale), oh = dec_scaled_size(info.H, scale);
+    if (step < (size_t)ow * ch) return B2J_EINVAL;
+    const size_t dstep = ((size_t)ow * ch + 15) & ~(size_t)15;
+    if (ctx->d_recon_bytes < dstep * oh) {
         cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0;
-        CK(cudaMalloc(&ctx->d_recon, dstep * info.H));
-        ctx->d_recon_bytes = dstep * info.H;
+        CK(cudaMalloc(&ctx->d_recon, dstep * oh));
+        ctx->d_recon_bytes = dstep * oh;
     }
     for (int attempt = 0; attempt < 2; attempt++) {
-        rc = decode_parsed(ctx, jpg, len, info, ctx->d_recon, dstep, attempt == 1);
+        rc = decode_parsed(ctx, jpg, len, info, ctx->d_recon, dstep, attempt == 1, scale);
         if (rc) return rc;
-        rc = download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)info.W * ch, info.H, ctx->stream); if (rc) return rc;
+        rc = download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)ow * ch, oh, ctx->stream); if (rc) return rc;
         rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
         if (rc != DEC_RETRY) break;   // else: the speculative synchronisation schedule was too short: once more, checked
     }

@@ -156,7 +156,8 @@ static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interv
 }
 
 int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr, size_t step,
-            bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src) {
+            bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src,
+            int scale) {
     const int rst = info.restart_interval;   // MCUs per restart interval (0: none)
     if (rst && info.scan_len >= 0xFFFFFFF0ull) { snprintf(d->err, d->errlen, "restart-marker scans of 4 GB and more are not supported"); return B2J_EFORMAT; }
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
@@ -269,7 +270,17 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
     DCK(launch_dc_scan(d->d_dc, g, gray_out ? 1 : g.nc, d->d_desc + 2 * d->desc_cap, &d->d_ctrl->ticket[2], d->desc_cap,
                        &d->d_ctrl->err, s));
     if (tm) cudaEventRecord(d->ev[3], s);
-    if (gray_out) {   // Y straight from the IDCT into the caller's image: no planes, no colour pass (dec_color stays 0)
+    if (scale > 1) {   // reduced size: the scaled IDCT (gray: straight into the caller's image), colour on the scaled view
+        uint8_t *py = d->d_planes;
+        uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
+        uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
+        const DecScale sc = dec_scale_setup(g, scale);
+        DCK(launch_idct_scaled(d->d_coef, d->d_dc, g, sc, d->d_tb, gray_out ? d_bgr : py, pcb, pcr, gray_out, step, rst, s));
+        if (tm) cudaEventRecord(d->ev[4], s);
+        if (!gray_out) DCK(launch_upcolor(py, pcb, pcr, sc.view, d_bgr, step, s));
+        if (tm) cudaEventRecord(d->ev[5], s);
+        if (launches) (*launches) += gray_out ? 4 : 5;
+    } else if (gray_out) {   // Y straight from the IDCT into the caller's image: no planes, no colour pass (dec_color stays 0)
         DCK(launch_idct_gray(d->d_coef, d->d_dc, g, d->d_tb, d_bgr, step, rst, s));
         if (tm) { cudaEventRecord(d->ev[4], s); cudaEventRecord(d->ev[5], s); }
         if (launches) (*launches) += 4;
@@ -296,7 +307,7 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
 }
 
 int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, uint8_t *d_bgr,
-                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches) {
+                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches, int scale) {
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
     int rc = ensure(d, 4096, g, 0);
     if (rc) return rc;
@@ -304,7 +315,8 @@ int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const ProgIn
     d->speculated = false;
     d->last_stream = s;
     DCK(cudaMemsetAsync(&d->d_ctrl->err, 0, 4, s));
-    return dec_progressive(jpg, len, info, g, d->d_coef, d->d_tb, d->d_planes, d_bgr, step, gray_out, s, launches, d->err, d->errlen);
+    return dec_progressive(jpg, len, info, g, d->d_coef, d->d_tb, d->d_planes, d_bgr, step, gray_out, s, launches, d->err, d->errlen,
+                           scale);
 }
 
 int dec_check(Decoder *d, char *err, size_t errlen) {

@@ -27,8 +27,10 @@ void dec_destroy(Decoder *d);
 // careful = false: no host synchronisation inside (dec_check may then answer DEC_RETRY: run again with careful = true)
 // d_scan_src != NULL: the scan's stuffed bytes are already in device memory (info.scan_len of them): nothing is uploaded
 // gray_out: d_bgr receives one byte per pixel, the Y samples (JCS_GRAYSCALE; chroma blocks are decoded, not transformed)
+// scale 2 / 4 / 8: d_bgr receives the image at 1 / scale (dec_kernels.h dec_scale_setup), 1: full size
 int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr, size_t step,
-            bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src = nullptr);
+            bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src = nullptr,
+            int scale = 1);
 constexpr int DEC_RETRY = 1;
 int dec_check(Decoder *d, char *err, size_t errlen);   // synchronises the decode's stream
 // optional: how host bytes reach the device (the API layer stages pageable memory through pinned buffers); the
@@ -62,6 +64,6 @@ int parse_progressive(const uint8_t *jpg, size_t len, ProgInfo *info);
 void prog_free(ProgInfo *info);
 // every scan is absorbed into the coefficient array in file order, then the baseline back end runs
 int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, uint8_t *d_bgr,
-                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches);
+                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches, int scale = 1);
 
 }  // namespace b2j

@@ -58,10 +58,50 @@ cudaError_t launch_idct_gray(const int16_t *coef, const int16_t *dcarr, const Ge
 cudaError_t launch_upcolor(const uint8_t *py, const uint8_t *pcb, const uint8_t *pcr, const Geom &g, uint8_t *bgr, size_t step,
                            cudaStream_t s, int halo_top = 0, int halo_bottom = 0);
 
+// ---- reduced-size decode (dec_scaled.cu): libjpeg's DCT scaling with scale_num = 1, scale_denom = 2 / 4 / 8 (jdmaster.c)
+// Output W' x H' = ceil(W / denom) x ceil(H / denom). A luma block gives S x S samples (S = 8 / denom); a chroma block
+// Sc x Sc, where Sc starts at S and doubles while it is below 8 and both (hs S) % (2 Sc) and (vs S) % (2 Sc) are 0
+// (4:2:0: Sc = 2 S). The true chroma size is ceil(W Sc / (hs 8)) x ceil(H Sc / (vs 8)). Chroma reaches the output size
+// through k_upcolor unchanged, on `view`: a Geom whose W / H are the output size, dw[1] / dh[1] the true chroma size, hs /
+// vs the k_upcolor instantiation (hs S / Sc x vs S / Sc) and mcux the file's (the planes' pitches mcux 8 hs and mcux 8
+// hold the scaled rows). jdsample.c turns its fancy filters off when Sc = 1: 4:2:2 and 4:4:0 at 1/8 replicate, which
+// the IDCT does itself (rep) so that the view is 1 x 1.
+inline int dec_scaled_size(int n, int denom) { return (n + denom - 1) / denom; }
+struct DecScale {
+    int S, Sc;      // output size of a luma / chroma block
+    int rep;        // 0, or every chroma sample stored twice: 1 side by side (4:2:2 at 1/8), 2 one above the other (4:4:0)
+    Geom view;
+};
+inline DecScale dec_scale_setup(const Geom &g, int denom) {
+    DecScale d;
+    d.S = 8 / denom;
+    d.Sc = d.S;
+    while (d.Sc < 8 && (g.hs * d.S) % (2 * d.Sc) == 0 && (g.vs * d.S) % (2 * d.Sc) == 0) d.Sc *= 2;
+    int hx = g.hs * d.S / d.Sc, vx = g.vs * d.S / d.Sc;
+    d.rep = 0;
+    if (d.Sc == 1 && hx == 2 && vx == 1) { d.rep = 1; hx = 1; }
+    if (d.Sc == 1 && hx == 1 && vx == 2) { d.rep = 2; vx = 1; }
+    d.view = g;
+    d.view.W = dec_scaled_size(g.W, denom);
+    d.view.H = dec_scaled_size(g.H, denom);
+    d.view.hs = hx; d.view.vs = vx;
+    d.view.dw[0] = d.view.W; d.view.dh[0] = d.view.H;
+    for (int c = 1; c < g.nc; c++) {
+        d.view.dw[c] = (g.W * d.Sc + g.hs * 8 - 1) / (g.hs * 8);
+        d.view.dh[c] = (g.H * d.Sc + g.vs * 8 - 1) / (g.vs * 8);
+    }
+    return d;
+}
+// gray: the luma blocks only, clipped into the caller's 8-bit image (py, pitch out_step); else Y into py (pitch
+// mcux 8 view.hs) and Cb / Cr into pcb / pcr (pitch mcux 8), for launch_upcolor(py, pcb, pcr, sc.view, ...)
+cudaError_t launch_idct_scaled(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecScale &sc, const void *tb,
+                               uint8_t *py, uint8_t *pcb, uint8_t *pcr, bool gray, size_t out_step, int rst_mcus, cudaStream_t s);
+
 // progressive files (dec_prog.cu): all scans into d_coef, then IDCT + upsampling; synchronises the stream before returning
 // gray_out: 8-bit Y samples into d_bgr (launch_idct_gray) instead of IDCT + upsampling + colour conversion
+// scale: 1, or the reduced-size back end (launch_idct_scaled) at 1 / scale
 int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
                     uint8_t *d_planes, uint8_t *d_bgr, size_t step, bool gray_out, cudaStream_t s, uint64_t *launches,
-                    char *err, size_t errlen);
+                    char *err, size_t errlen, int scale = 1);
 
 }  // namespace b2j

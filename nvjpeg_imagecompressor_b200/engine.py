@@ -127,6 +127,12 @@ class Engine:
         """Restart markers every `rows` MCU rows (0 = none); the stream equals cv2's with RST_INTERVAL = rows * mcux."""
         self._ck(self._L.b2j_set_restart_rows(self._h, int(rows)))
 
+    def set_decode_scale(self, denom):
+        """Decode at 1/denom (1, 2, 4 or 8; 1 = full size, the default): libjpeg's DCT scaling, the pixels of
+        cv2.imdecode(IMREAD_REDUCED_COLOR_denom) / IMREAD_REDUCED_GRAYSCALE_denom on a gray context. decode returns and
+        decode_device / decode_scan_device write and report the reduced size ceil(W / denom) x ceil(H / denom)."""
+        self._ck(self._L.b2j_set_decode_scale(self._h, int(denom)))
+
     # ---------------------------------------------------------------- device API (pointers from torch tensors)
     def decode_scan_device(self, hdr, d_scan_ptr, scan_len, d_bgr_ptr, step, height_override=0):
         """Baseline JPEG with its scan bytes already in device memory (hdr: host bytes SOI .. SOS header) -> (W, H)."""
