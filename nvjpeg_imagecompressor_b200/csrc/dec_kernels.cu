@@ -31,6 +31,8 @@ namespace b2j {
 // RST (streams with restart markers, jdmarker.c read_restart_marker): the two bytes of every FF Dn are dropped as well
 // and the output offset where the next interval begins goes to bnd[j], j = ordinal of the marker (the look-back
 // carries the marker count in the upper bits of its sums); bnd[number of markers] = 0xFFFFFFFF closes the list.
+// So is every 0xFF followed by 0xFF: the fill bytes a marker may have in front of it (T.81 B.1.1.2; an 0xFF of
+// entropy data is always followed by a stuffed zero). Fill before the terminating marker is cut off by the parser.
 constexpr int DS_MK_SHIFT = 38;   // look-back value: kept bytes | markers << 38
 constexpr int DS_THREADS = 256, DS_NP = 4;
 static_assert(DS_THREADS * 16 * DS_NP == DS_CHUNK, "chunk = four 16-byte pieces per thread");
@@ -107,7 +109,7 @@ k_destuff(const uint8_t *__restrict__ in, size_t n, uint8_t *__restrict__ out, u
                 if (RST) d0[q] = lanes_zero((x[p][q] & 0xF8F8F8F8u) ^ 0xD0D0D0D0u);   // bytes D0 .. D7
             }
             const uint32_t ffprev = prevb == 0xFFu ? 0x80000000u : 0u;
-            const uint32_t d0next = (nextb & 0xF8u) == 0xD0u ? 0x80u : 0u;
+            const uint32_t d0next = (nextb & 0xF8u) == 0xD0u ? 0x80u : 0u, ffnext = nextb == 0xFFu ? 0x80u : 0u;
             uint32_t k16 = 0, m16 = 0;
 #pragma unroll
             for (int q = 0; q < 4; q++) {
@@ -116,7 +118,8 @@ k_destuff(const uint8_t *__restrict__ in, size_t n, uint8_t *__restrict__ out, u
                 if (RST) {
                     sec[q] = pf & d0[q];                                                        // second byte of FF Dn
                     const uint32_t nd = __funnelshift_r(d0[q], q < 3 ? d0[q + 1] : d0next, 8);  // the byte after is Dn
-                    drop[q] |= sec[q] | (ff[q] & nd);                                           // ... and its first byte
+                    const uint32_t nf = __funnelshift_r(ff[q], q < 3 ? ff[q + 1] : ffnext, 8);  // the byte after is 0xFF
+                    drop[q] |= sec[q] | (ff[q] & (nd | nf));                                    // ... and its first byte
                     m16 |= lanes_to_bits(sec[q]) << (4 * q);
                 }
                 k16 |= lanes_to_bits(drop[q] ^ 0x80808080u) << (4 * q);

@@ -10,6 +10,44 @@ namespace b2j {
 
 static inline int be16(const uint8_t *p) { return (p[0] << 8) | p[1]; }
 
+// The colour-space markers, as jdmarker.c get_interesting_appn reads them: a JFIF APP0 ("JFIF\0", at least 14 bytes)
+// and an Adobe APP14 ("Adobe", at least 12 bytes, the transform in byte 11; the last one seen counts).
+struct ColourMarkers {
+    bool jfif = false;
+    int adobe = -1;   // the Adobe transform, -1: no Adobe marker
+    void note(int m, const uint8_t *s, int n) {
+        if (m == 0xE0 && n >= 14 && !memcmp(s, "JFIF", 5)) jfif = true;
+        if (m == 0xEE && n >= 12 && !memcmp(s, "Adobe", 5)) adobe = s[11];
+    }
+    // jdapimin.c default_decompress_parms for three components: JFIF means YCbCr; else an Adobe marker decides
+    // (transform 0: RGB); else the component ids 'R', 'G', 'B' mean RGB; anything else is YCbCr. RGB-coded files
+    // have no colour transform, which the back end always applies, so they are refused.
+    bool rgb(const int cid[3]) const {
+        if (jfif) return false;
+        if (adobe >= 0) return adobe == 0;
+        return cid[0] == 'R' && cid[1] == 'G' && cid[2] == 'B';
+    }
+};
+
+// The end of an entropy-coded segment: the first marker that is neither a stuffed zero nor RSTn, less the fill bytes
+// (0xFF, T.81 B.1.1.2) in front of it. An 0xFF of entropy data is always followed by a stuffed zero, so an 0xFF right
+// before a marker is fill.
+static size_t segment_end(const uint8_t *jpg, size_t len, size_t e) {
+    const size_t e0 = e;
+    const uint8_t *f = nullptr;
+    while (e < len && (f = (const uint8_t *)memchr(jpg + e, 0xFF, len - e)) != nullptr) {
+        e = (size_t)(f - jpg);
+        if (e + 1 >= len) { e = len; break; }
+        const uint8_t nx = jpg[e + 1];
+        if (nx == 0x00 || (nx >= 0xD0 && nx <= 0xD7)) { e += 2; continue; }
+        if (nx == 0xFF) { e += 1; continue; }
+        break;
+    }
+    if (e > len || f == nullptr) e = len;
+    while (e > e0 && jpg[e - 1] == 0xFF) e--;
+    return e;
+}
+
 int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
     static const uint8_t ZZ[64] = {0,  1,  8,  16, 9,  2,  3,  10, 17, 24, 32, 25, 18, 11, 4,  5,  12, 19, 26, 33, 40, 48,
                                    41, 34, 27, 20, 13, 6,  7,  14, 21, 28, 35, 42, 49, 56, 57, 50, 43, 36, 29, 22, 15, 23,
@@ -23,6 +61,7 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
     memset(hb, 0, sizeof(hb));
     memset(hv, 0, sizeof(hv));
     int cid[3] = {0, 0, 0}, chv[3] = {0, 0, 0}, ctq[3] = {0, 0, 0}, ncomp = 0;
+    ColourMarkers cm;
     size_t p = 2;
     while (p + 4 <= len) {
         if (jpg[p] != 0xFF) return B2J_EFORMAT;
@@ -49,7 +88,10 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
         case 0xC0: case 0xC1:
             if (n < 9 || s[0] != 8 || (s[5] != 3 && s[5] != 1) || n < 6 + 3 * s[5]) return B2J_EFORMAT;
             info->H = be16(s + 1); info->W = be16(s + 3); ncomp = s[5];
-            for (int c = 0; c < ncomp; c++) { cid[c] = s[6 + 3 * c]; chv[c] = s[7 + 3 * c]; ctq[c] = s[8 + 3 * c] & 3; }
+            for (int c = 0; c < ncomp; c++) {
+                cid[c] = s[6 + 3 * c]; chv[c] = s[7 + 3 * c]; ctq[c] = s[8 + 3 * c];
+                if (ctq[c] > 3) return B2J_EFORMAT;   // jdinput.c latch_quant_tables: JERR_NO_QUANT_TABLE
+            }
             break;
         case 0xC2: case 0xC3: case 0xC5: case 0xC6: case 0xC7: case 0xC9: case 0xCA: case 0xCB: case 0xCD: case 0xCE: case 0xCF:
             return B2J_EFORMAT;  // progressive / lossless / arithmetic (SURVEY.md 8f N4)
@@ -99,6 +141,7 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
                 if (td[c] > 3 || ta[c] > 3 || !have_h[0][td[c]] || !have_h[1][ta[c]]) return B2J_EFORMAT;
             }
             if (ncomp == 3) {
+                if (cm.rgb(cid)) return B2J_EFORMAT;
                 if (chv[1] != 0x11 || chv[2] != 0x11 || td[1] != td[2] || ta[1] != ta[2] || ctq[1] != ctq[2]) return B2J_EFORMAT;
                 if (!have_q[ctq[0]] || !have_q[ctq[1]]) return B2J_EFORMAT;
                 info->hs = chv[0] >> 4; info->vs = chv[0] & 15;
@@ -113,27 +156,19 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
                 memcpy(info->bits[3], hb[1][ta[1]], 17); memcpy(info->vals[3], hv[1][ta[1]], 256);
             }
             info->scan_offset = p + L;
-            // the entropy-coded segment ends at the first marker that is neither a stuffed zero nor RSTn. Fast path for
-            // the files this engine and libjpeg write (one scan, EOI as the last two bytes): no 0xFF search at all.
+            // the entropy-coded segment (segment_end). Fast path for the files this engine and libjpeg write (one scan,
+            // EOI as the last two bytes): no 0xFF search at all.
             size_t e = info->scan_offset;
             if (len >= e + 2 && jpg[len - 2] == 0xFF && jpg[len - 1] == 0xD9) {
                 e = len - 2;
+                while (e > info->scan_offset && jpg[e - 1] == 0xFF) e--;   // fill bytes before EOI
             } else {
-                const uint8_t *f = nullptr;
-                while (e < len && (f = (const uint8_t *)memchr(jpg + e, 0xFF, len - e)) != nullptr) {
-                    e = (size_t)(f - jpg);
-                    if (e + 1 >= len) { e = len; break; }
-                    const uint8_t nx = jpg[e + 1];
-                    if (nx == 0x00 || (nx >= 0xD0 && nx <= 0xD7)) { e += 2; continue; }
-                    if (nx == 0xFF) { e += 1; continue; }
-                    break;
-                }
-                if (e > len || f == nullptr) e = len;
+                e = segment_end(jpg, len, e);
             }
             info->scan_len = e - info->scan_offset;
             return B2J_OK;
         }
-        default: break;  // APPn, COM, ...
+        default: cm.note(m, s, n); break;  // APPn, COM, ...
         }
         p += L;
     }
@@ -159,6 +194,7 @@ int parse_progressive(const uint8_t *jpg, size_t len, ProgInfo *info) {
     int cid[3] = {0, 0, 0}, chv[3] = {0, 0, 0}, ctq[3] = {0, 0, 0};
     int ri = 0, cap = 0;
     bool have_sof = false;
+    ColourMarkers cm;
     size_t p = 2;
     int rc = B2J_EFORMAT;
     while (p + 2 <= len) {
@@ -187,15 +223,15 @@ int parse_progressive(const uint8_t *jpg, size_t len, ProgInfo *info) {
             if (have_sof || n < 9 || s[0] != 8 || (s[5] != 3 && s[5] != 1) || n < 6 + 3 * s[5]) { bad = true; }
             else if (s[5] == 1) {   // one component (gray): any sampling factor, laid out 1x1
                 info->H = be16(s + 1); info->W = be16(s + 3);
-                cid[0] = s[6]; ctq[0] = ctq[1] = ctq[2] = s[8] & 3;
+                cid[0] = s[6]; ctq[0] = ctq[1] = ctq[2] = s[8];
                 cid[1] = cid[2] = -1;   // no scan can name them
                 info->hs = info->vs = 1; info->css = B2J_CSS_GRAY;
-                if (info->W <= 0 || info->H <= 0) bad = true;
+                if (info->W <= 0 || info->H <= 0 || ctq[0] > 3) bad = true;
                 have_sof = !bad;
             } else {
                 info->H = be16(s + 1); info->W = be16(s + 3);
-                for (int c = 0; c < 3; c++) { cid[c] = s[6 + 3 * c]; chv[c] = s[7 + 3 * c]; ctq[c] = s[8 + 3 * c] & 3; }
-                if (chv[1] != 0x11 || chv[2] != 0x11 || ctq[1] != ctq[2]) bad = true;
+                for (int c = 0; c < 3; c++) { cid[c] = s[6 + 3 * c]; chv[c] = s[7 + 3 * c]; ctq[c] = s[8 + 3 * c]; }
+                if (chv[1] != 0x11 || chv[2] != 0x11 || ctq[1] != ctq[2] || ctq[0] > 3 || ctq[1] > 3) bad = true;
                 info->hs = chv[0] >> 4; info->vs = chv[0] & 15;
                 static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
                 info->css = -1;
@@ -225,7 +261,8 @@ int parse_progressive(const uint8_t *jpg, size_t len, ProgInfo *info) {
         } else if (m == 0xDD) {
             if (n < 2) bad = true; else ri = be16(s);
         } else if (m == 0xDA) {
-            if (!have_sof || n < 6) { bad = true; }
+            // the colour space is settled by the markers before the first scan (jpeg_read_header)
+            if (!have_sof || n < 6 || (info->nscans == 0 && info->css != B2J_CSS_GRAY && cm.rgb(cid))) { bad = true; }
             else {
                 ProgScan sc;
                 memset(&sc, 0, sizeof(sc));
@@ -256,17 +293,7 @@ int parse_progressive(const uint8_t *jpg, size_t len, ProgInfo *info) {
                 if (!bad) {
                     sc.restart_interval = ri;
                     sc.seg_off = p + L;
-                    size_t e = sc.seg_off;   // the segment ends at the first marker that is neither a stuffed zero nor RSTn
-                    const uint8_t *f = nullptr;
-                    while (e < len && (f = (const uint8_t *)memchr(jpg + e, 0xFF, len - e)) != nullptr) {
-                        e = (size_t)(f - jpg);
-                        if (e + 1 >= len) { e = len; break; }
-                        const uint8_t nx = jpg[e + 1];
-                        if (nx == 0x00 || (nx >= 0xD0 && nx <= 0xD7)) { e += 2; continue; }
-                        if (nx == 0xFF) { e += 1; continue; }
-                        break;
-                    }
-                    if (e > len || f == nullptr) e = len;
+                    const size_t e = segment_end(jpg, len, sc.seg_off);
                     sc.seg_len = e - sc.seg_off;
                     if (info->nscans == cap) {
                         cap = cap ? cap * 2 : 16;
@@ -285,6 +312,8 @@ int parse_progressive(const uint8_t *jpg, size_t len, ProgInfo *info) {
                     }
                 }
             }
+        } else {
+            cm.note(m, s, n);   // APPn, COM, ...
         }
         if (bad) break;
         p += L;

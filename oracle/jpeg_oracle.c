@@ -747,12 +747,25 @@ int orc_encode_progressive(const uint8_t *bgr, size_t step, int W, int H, int cs
 
 static int rd16(const uint8_t *p) { return (p[0] << 8) | p[1]; }
 
+/* jdmarker.c get_interesting_appn: JFIF APP0 ("JFIF\0", 14+ bytes) and Adobe APP14 ("Adobe", 12+ bytes, transform in
+ * byte 11); jdapimin.c default_decompress_parms then takes three components as RGB (no colour transform, which this
+ * checker does not restate: such files are refused) for Adobe transform 0, or without either marker for ids R, G, B. */
+static void note_appn(int m, const uint8_t *s, int n, int *jfif, int *adobe) {
+    if (m == 0xE0 && n >= 14 && !memcmp(s, "JFIF", 5)) *jfif = 1;
+    if (m == 0xEE && n >= 12 && !memcmp(s, "Adobe", 5)) *adobe = s[11];
+}
+static int rgb_coded(int jfif, int adobe, const int id[3]) {
+    if (jfif) return 0;
+    if (adobe >= 0) return adobe == 0;
+    return id[0] == 'R' && id[1] == 'G' && id[2] == 'B';
+}
+
 int orc_parse(const uint8_t *jpg, size_t len, orc_info *info) {
     memset(info, 0, sizeof(*info));
     if (len < 4 || jpg[0] != 0xFF || jpg[1] != 0xD8) return -1;
     uint16_t qtabs[4][64]; int have_q[4] = {0, 0, 0, 0};
     uint8_t hb[2][4][17], hv[2][4][256]; memset(hb, 0, sizeof(hb)); memset(hv, 0, sizeof(hv));
-    int comp_id[3], comp_hv[3], comp_tq[3], ncomp = 0;
+    int comp_id[3], comp_hv[3], comp_tq[3], ncomp = 0, jfif = 0, adobe = -1;
     size_t p = 2;
     while (p + 4 <= len) {
         if (jpg[p] != 0xFF) return -2;
@@ -779,6 +792,7 @@ int orc_parse(const uint8_t *jpg, size_t len, orc_info *info) {
             info->H = rd16(s + 1); info->W = rd16(s + 3); ncomp = s[5];
             if (ncomp != 3) return -7;
             for (int c = 0; c < 3; c++) { comp_id[c] = s[6 + 3 * c]; comp_hv[c] = s[7 + 3 * c]; comp_tq[c] = s[8 + 3 * c]; }
+            if (comp_tq[0] > 3 || comp_tq[1] > 3 || comp_tq[2] > 3) return -14;
         } else if (m == 0xC2 || (m >= 0xC5 && m <= 0xCF && m != 0xC4 && m != 0xC8 && m != 0xCC)) {
             return -8; /* progressive / lossless / arithmetic: not baseline */
         } else if (m == 0xC4) {
@@ -795,6 +809,7 @@ int orc_parse(const uint8_t *jpg, size_t len, orc_info *info) {
             info->restart_interval = rd16(s);
         } else if (m == 0xDA) {
             if (ncomp != 3 || s[0] != 3) return -10;
+            if (rgb_coded(jfif, adobe, comp_id)) return -17;
             int td[3], ta[3];
             for (int c = 0; c < 3; c++) {
                 if (s[1 + 2 * c] != comp_id[c]) return -10;
@@ -817,12 +832,15 @@ int orc_parse(const uint8_t *jpg, size_t len, orc_info *info) {
             /* find end of entropy data: first marker that is not RSTn / stuffed zero */
             size_t e = info->scan_offset;
             while (e + 1 < len) {
-                if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
+                if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && jpg[e + 1] != 0xFF && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
                 e++;
             }
             if (e + 1 >= len) e = len;
+            while (e > info->scan_offset && jpg[e - 1] == 0xFF) e--;   /* fill bytes before the marker */
             info->scan_len = e - info->scan_offset;
             return 0;
+        } else {
+            note_appn(m, s, n, &jfif, &adobe);
         }
         p += L;
     }
@@ -848,9 +866,11 @@ static int get_bit(bitr *r) {
         uint8_t b = 0;
         if (r->pos < r->n && !r->marker) {
             b = r->d[r->pos];
-            if (b == 0xFF) {
-                uint8_t b2 = r->pos + 1 < r->n ? r->d[r->pos + 1] : 0xD9;
-                if (b2 == 0) r->pos += 2; else { r->marker = b2; b = 0; }
+            if (b == 0xFF) {   /* jdhuff.c fill_bit_buffer: any number of 0xFF, then 00 (data) or a marker */
+                size_t q = r->pos + 1;
+                while (q < r->n && r->d[q] == 0xFF) q++;
+                uint8_t b2 = q < r->n ? r->d[q] : 0xD9;
+                if (b2 == 0) r->pos = q + 1; else { r->marker = b2; r->pos = q - 1; b = 0; }
             } else r->pos++;
         }
         r->acc = b; r->cnt = 8;
@@ -882,6 +902,7 @@ int orc_decode_coefs(const uint8_t *jpg, size_t len, const orc_info *info, int16
     for (long long m = 0; m < nmcu; m++) {
         if (ri && togo == 0) { /* process restart marker */
             r.cnt = 0;
+            while (!r.marker && r.pos + 1 < r.n && r.d[r.pos] == 0xFF && r.d[r.pos + 1] == 0xFF) r.pos++;   /* fill */
             if (r.marker) { r.pos += 2; r.marker = 0; }
             else if (r.pos + 1 < r.n && r.d[r.pos] == 0xFF && r.d[r.pos + 1] >= 0xD0 && r.d[r.pos + 1] <= 0xD7) r.pos += 2;
             pred[0] = pred[1] = pred[2] = 0; togo = ri;
@@ -1033,6 +1054,7 @@ int orc_inverse(const int16_t *coef, const orc_info *info, uint8_t *bgr, size_t 
  * back end (IDCT, upsampling, colour) runs: block smoothing never triggers on a complete file. */
 static void prog_restart(bitr *r, int pred[3], int *eobrun) {
     r->cnt = 0;
+    while (!r->marker && r->pos + 1 < r->n && r->d[r->pos] == 0xFF && r->d[r->pos + 1] == 0xFF) r->pos++;   /* fill */
     if (r->marker) { r->pos += 2; r->marker = 0; }
     else if (r->pos + 1 < r->n && r->d[r->pos] == 0xFF && r->d[r->pos + 1] >= 0xD0 && r->d[r->pos + 1] <= 0xD7) r->pos += 2;
     pred[0] = pred[1] = pred[2] = 0; *eobrun = 0;
@@ -1102,6 +1124,7 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
     static uint8_t hb[2][4][17], hv[2][4][256];
     memset(hb, 0, sizeof(hb)); memset(hv, 0, sizeof(hv));
     int comp_id[3] = {0, 0, 0}, comp_hv[3] = {0, 0, 0}, comp_tq[3] = {0, 0, 0}, ncomp = 0, ri = 0, have_sof = 0;
+    int jfif = 0, adobe = -1, nscans = 0;
     orc_geom g; memset(&g, 0, sizeof(g));
     int16_t *coef = NULL;
     size_t p = 2;
@@ -1130,6 +1153,7 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
             if (ncomp != 3) { rc = -7; break; }
             for (int c = 0; c < 3; c++) { comp_id[c] = s[6 + 3 * c]; comp_hv[c] = s[7 + 3 * c]; comp_tq[c] = s[8 + 3 * c]; }
             if (comp_hv[1] != 0x11 || comp_hv[2] != 0x11 || comp_tq[1] != comp_tq[2]) { rc = -11; break; }
+            if (comp_tq[0] > 3 || comp_tq[1] > 3) { rc = -14; break; }
             info.hs = comp_hv[0] >> 4; info.vs = comp_hv[0] & 15;
             static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
             info.css = -1;
@@ -1155,8 +1179,11 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
             }
         } else if (m == 0xDD) {
             ri = rd16(s);
-        } else if (m == 0xDA) {
+        } else if (m != 0xDA) {
+            note_appn(m, s, n, &jfif, &adobe);
+        } else {
             if (!have_sof) { rc = -10; break; }
+            if (nscans++ == 0 && rgb_coded(jfif, adobe, comp_id)) { rc = -17; break; }
             pscan sc; sc.ncomp = s[0];
             if (sc.ncomp < 1 || sc.ncomp > 3) { rc = -10; break; }
             for (int i = 0; i < sc.ncomp; i++) {
@@ -1173,10 +1200,11 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
             /* entropy-coded segment of this scan */
             size_t e0 = p + L, e = e0;
             while (e + 1 < len) {
-                if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
+                if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && jpg[e + 1] != 0xFF && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
                 e++;
             }
             if (e + 1 >= len) e = len;
+            while (e > e0 && jpg[e - 1] == 0xFF) e--;   /* fill bytes before the marker */
             bitr r = {jpg + e0, e - e0, 0, 0, 0, 0};
             dtbl dct[3], act[3];
             for (int i = 0; i < sc.ncomp; i++) {
