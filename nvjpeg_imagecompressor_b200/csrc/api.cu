@@ -988,16 +988,8 @@ static int dec_ensure(b2j_ctx *ctx) {
 
 int b2j_peek(const uint8_t *jpg, size_t len, int *width, int *height, int *css) {
     JpegInfo info;
-    int rc = parse_jpeg(jpg, len, &info);
-    if (rc) {   // progressive (SOF2) files are decoded too
-        ProgInfo pi;
-        if (parse_progressive(jpg, len, &pi) != B2J_OK) return rc;
-        if (width) *width = pi.W;
-        if (height) *height = pi.H;
-        if (css) *css = pi.css;
-        prog_free(&pi);
-        return B2J_OK;
-    }
+    const int rc = parse_jpeg(jpg, len, &info);
+    if (rc) return rc;
     if (width) *width = info.W;
     if (height) *height = info.H;
     if (css) *css = info.css;
@@ -1012,45 +1004,14 @@ static int check_components(b2j_ctx *ctx, int file_css) {
     return B2J_EFORMAT;
 }
 
-// progressive (SOF2) files: parsed and decoded scan by scan (dec_prog.cu); returns B2J_EFORMAT if it is not one
-// width / height: the output size (the file's at the context's decode scale)
-static int decode_progressive_to(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *d_bgr, size_t step, bool alloc_recon,
-                                 int *width, int *height) {
-    ProgInfo pi;
-    int rc = parse_progressive(jpg, len, &pi);
-    if (rc) return rc;
-    rc = check_components(ctx, pi.css);
-    if (rc) { prog_free(&pi); return rc; }
-    const int ch = chans(ctx), scale = ctx->dec_scale;
-    const int ow = dec_scaled_size(pi.W, scale), oh = dec_scaled_size(pi.H, scale);
-    if (width) *width = ow;
-    if (height) *height = oh;
-    Geom g;
-    rc = make_geom(pi.W, pi.H, pi.css, &g);
-    if (!rc && (d_bgr || alloc_recon)) {
-        size_t dstep = step;
-        if (alloc_recon) {
-            dstep = ((size_t)ow * ch + 15) & ~(size_t)15;
-            if (ctx->d_recon_bytes < dstep * oh) {
-                cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0;
-                if (cudaMalloc(&ctx->d_recon, dstep * oh) != cudaSuccess) { prog_free(&pi); return B2J_ECUDA; }
-                ctx->d_recon_bytes = dstep * oh;
-            }
-            d_bgr = ctx->d_recon;
-        }
-        if (dstep < (size_t)ow * ch) rc = B2J_EINVAL;
-        if (!rc) rc = dec_ensure(ctx);
-        if (!rc) rc = dec_run_progressive(ctx->dec, jpg, len, pi, g, d_bgr, dstep, ch == 1, ctx->stream, &ctx->launches, scale);
-    }
-    prog_free(&pi);
-    return rc;
-}
-
+// sequential files: asynchronous (careful = false: dec_check may ask for a checked retry); progressive files: scan by
+// scan (dec_prog.cu), synchronous
 static int decode_parsed(b2j_ctx *ctx, const uint8_t *jpg, size_t len, const JpegInfo &info, uint8_t *d_bgr, size_t step, bool careful,
                          int scale, const uint8_t *d_scan_src = nullptr) {
     if (step < (size_t)dec_scaled_size(info.W, scale) * chans(ctx)) return B2J_EINVAL;
     int rc = dec_ensure(ctx); if (rc) return rc;
     Geom g; rc = make_geom(info.W, info.H, info.css, &g); if (rc) return rc;
+    if (info.progressive) return dec_run_progressive(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, &ctx->launches, scale);
     dec_set_spec_launches(ctx->dec, (ctx->debug & 4) ? 1 : 3);
     return dec_run(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, ctx->timing ? &ctx->tm : nullptr,
                    &ctx->launches, careful, d_scan_src, scale);
@@ -1065,20 +1026,25 @@ static int parse_for(b2j_ctx *ctx, const uint8_t *jpg, size_t len, JpegInfo *inf
     return B2J_OK;
 }
 
+// ctx->d_recon of at least `bytes`: b2j_decode's image before it is downloaded, the secondary compression's reconstruction
+static int ensure_recon(b2j_ctx *ctx, size_t bytes) {
+    if (ctx->d_recon_bytes >= bytes) return B2J_OK;
+    cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0;
+    CK(cudaMalloc(&ctx->d_recon, bytes));
+    ctx->d_recon_bytes = bytes;
+    return B2J_OK;
+}
+
 int b2j_decode_device(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *d_bgr, size_t step, int *width, int *height) {
     if (!ctx || !jpg) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     JpegInfo info;
     int rc = parse_for(ctx, jpg, len, &info, width, height);
-    if (rc == B2J_EFORMAT && info.css != B2J_CSS_GRAY) {   // not a baseline file: progressive? (decoded synchronously, nothing left for b2j_decode_finish)
-        if (ctx->last_jpg) { const int rf = b2j_decode_finish(ctx); if (rf) return rf; }
-        const int rp = decode_progressive_to(ctx, jpg, len, d_bgr, step, false, width, height);
-        if (rp != B2J_EFORMAT) return rp;
-    }
-    if (rc) return rc;
-    if (!d_bgr) return B2J_OK;
+    if (rc || !d_bgr) return rc;
     // one decode in flight per context: an unfinished predecessor is finished (validated, retried if needed) first
     if (ctx->last_jpg) { rc = b2j_decode_finish(ctx); if (rc) return rc; }
+    // progressive files decode synchronously: nothing is left for b2j_decode_finish
+    if (info.progressive) return decode_parsed(ctx, jpg, len, info, d_bgr, step, false, ctx->dec_scale);
     // remembered for b2j_decode_finish: the caller keeps `jpg` alive until then
     ctx->last_jpg = jpg; ctx->last_len = len; ctx->last_bgr = d_bgr; ctx->last_step = step; ctx->last_scale = ctx->dec_scale;
     return decode_parsed(ctx, jpg, len, info, d_bgr, step, false, ctx->last_scale);
@@ -1097,9 +1063,11 @@ int b2j_decode_scan_device(b2j_ctx *ctx, const uint8_t *hdr, size_t hdr_len, con
     if (ctx->last_jpg) { int rf = b2j_decode_finish(ctx); if (rf) return rf; }
     JpegInfo info;
     int rc = parse_for(ctx, hdr, hdr_len, &info, nullptr, nullptr); if (rc) return rc;
-    if (info.scan_offset != hdr_len) { snprintf(ctx->err, sizeof(ctx->err), "hdr must end with the SOS header"); return B2J_EINVAL; }
+    if (info.progressive) { snprintf(ctx->err, sizeof(ctx->err), "progressive JPEG: one scan in device memory cannot be decoded"); return B2J_EFORMAT; }
+    JpegScan &sc = info.scans[0];
+    if (sc.seg_off != hdr_len) { snprintf(ctx->err, sizeof(ctx->err), "hdr must end with the SOS header"); return B2J_EINVAL; }
     if (height_override > 0) info.H = height_override;
-    info.scan_offset = 0; info.scan_len = scan_len;
+    sc.seg_off = 0; sc.seg_len = scan_len;
     const int scale = ctx->dec_scale;
     if (width) *width = dec_scaled_size(info.W, scale);
     if (height) *height = dec_scaled_size(info.H, scale);
@@ -1131,29 +1099,11 @@ int b2j_decode(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *bgr, size_
     CK(cudaSetDevice(ctx->device));
     JpegInfo info;
     int rc = parse_for(ctx, jpg, len, &info, width, height);
-    const int ch = chans(ctx);
-    if (rc == B2J_EFORMAT && info.css != B2J_CSS_GRAY) {   // not a baseline file: progressive?
-        int pw = 0, ph = 0;
-        const int rp = decode_progressive_to(ctx, jpg, len, nullptr, 0, bgr != nullptr, &pw, &ph);
-        if (rp != B2J_EFORMAT) {
-            if (width) *width = pw;
-            if (height) *height = ph;
-            if (rp || !bgr) return rp;
-            if (step < (size_t)pw * ch) return B2J_EINVAL;
-            const size_t dstep = ((size_t)pw * ch + 15) & ~(size_t)15;
-            return download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)pw * ch, ph, ctx->stream);
-        }
-    }
-    if (rc) return rc;
-    if (!bgr) return B2J_OK;
-    const int scale = ctx->dec_scale, ow = dec_scaled_size(info.W, scale), oh = dec_scaled_size(info.H, scale);
+    if (rc || !bgr) return rc;
+    const int ch = chans(ctx), scale = ctx->dec_scale, ow = dec_scaled_size(info.W, scale), oh = dec_scaled_size(info.H, scale);
     if (step < (size_t)ow * ch) return B2J_EINVAL;
     const size_t dstep = ((size_t)ow * ch + 15) & ~(size_t)15;
-    if (ctx->d_recon_bytes < dstep * oh) {
-        cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0;
-        CK(cudaMalloc(&ctx->d_recon, dstep * oh));
-        ctx->d_recon_bytes = dstep * oh;
-    }
+    rc = ensure_recon(ctx, dstep * oh); if (rc) return rc;
     for (int attempt = 0; attempt < 2; attempt++) {
         rc = decode_parsed(ctx, jpg, len, info, ctx->d_recon, dstep, attempt == 1, scale);
         if (rc) return rc;
@@ -1294,7 +1244,7 @@ int b2j_secondary_device(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int wi
     if (!d_bgr || step != (size_t)width * 3 || (diff_mode != 0 && diff_mode != 1)) return B2J_EINVAL;   // contiguous rows
     CK(cudaSetDevice(ctx->device));
     const size_t bytes = (size_t)width * 3 * height;
-    if (ctx->d_recon_bytes < bytes) { cudaFree(ctx->d_recon); ctx->d_recon = nullptr; ctx->d_recon_bytes = 0; CK(cudaMalloc(&ctx->d_recon, bytes)); ctx->d_recon_bytes = bytes; }
+    int rc = ensure_recon(ctx, bytes); if (rc) return rc;
     if (ctx->d_diff_bytes < bytes) { cudaFree(ctx->d_diff); ctx->d_diff = nullptr; ctx->d_diff_bytes = 0; CK(cudaMalloc(&ctx->d_diff, bytes)); ctx->d_diff_bytes = bytes; }
     if (!ctx->second) {
         b2j_params p2 = ctx->p; p2.flags = 0; p2.device = ctx->device;
@@ -1303,7 +1253,7 @@ int b2j_secondary_device(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int wi
     b2j_set_stream(ctx->second, ctx->stream);
     const int dbg = ctx->debug;
     ctx->debug |= 1;
-    int rc = ensure_debug(ctx);
+    rc = ensure_debug(ctx);
     const uint8_t *o1 = nullptr, *o2 = nullptr; const uint64_t *l1, *l2;
     if (!rc) rc = b2j_encode_device(ctx, d_bgr, step, width, height, &o1, &l1);
     if (!rc) rc = b2j_reconstruct_device(ctx, ctx->d_recon, (size_t)width * 3);

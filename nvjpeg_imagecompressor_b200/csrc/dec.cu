@@ -111,6 +111,20 @@ void dec_set_spec_launches(Decoder *d, int n) { d->spec_launches = n < 1 ? 1 : n
 
 const void *dec_coef_ptr(Decoder *d, size_t *bytes) { *bytes = (size_t)d->nblocks_cap * 128; return d->d_coef; }
 
+// the back end's sample planes in one buffer: Y (mcux 8 hs x mcuy 8 vs), then Cb and Cr (mcux 8 x mcuy 8 each), every
+// plane at a multiple of 64 bytes
+struct PlaneLayout {
+    size_t cb, cr, bytes;   // offsets of Cb and Cr; the buffer size
+};
+static PlaneLayout plane_layout(const Geom &g) {
+    const size_t y = (size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs, c = (size_t)g.mcux * 8 * g.mcuy * 8;
+    PlaneLayout l;
+    l.cb = (y + 63) & ~(size_t)63;
+    l.cr = l.cb + ((c + 63) & ~(size_t)63);
+    l.bytes = y + 2 * c + 256;
+    return l;
+}
+
 static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interval) {
     if (restart_interval > 0) {
         const size_t need = ((size_t)g.mcux * g.mcuy + restart_interval - 1) / restart_interval + 2;
@@ -146,7 +160,7 @@ static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interv
         DCK(cudaMalloc(&d->d_desc, nd * 5 * 8));
         d->desc_cap = nd;
     }
-    const size_t pl = (size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 2 * (size_t)g.mcux * 8 * g.mcuy * 8 + 256;
+    const size_t pl = plane_layout(g).bytes;
     if (pl > d->planes_cap) {
         cudaFree(d->d_planes); d->d_planes = nullptr; d->planes_cap = 0;
         DCK(cudaMalloc(&d->d_planes, pl));
@@ -155,16 +169,41 @@ static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interv
     return B2J_OK;
 }
 
+cudaError_t dec_back_end(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *planes, uint8_t *d_bgr,
+                         size_t step, bool gray_out, int scale, int rst_mcus, cudaStream_t s, cudaEvent_t ev_idct,
+                         cudaEvent_t ev_color, uint64_t *launches) {
+    const PlaneLayout pl = plane_layout(g);
+    uint8_t *py = planes, *pcb = planes + pl.cb, *pcr = planes + pl.cr;
+    cudaError_t e;
+    Geom view = g;   // the geometry of the colour pass
+    if (scale > 1) {   // reduced size: the scaled IDCT (gray: straight into the caller's image), colour on the scaled view
+        const DecScale sc = dec_scale_setup(g, scale);
+        e = launch_idct_scaled(coef, dcarr, g, sc, tb, gray_out ? d_bgr : py, pcb, pcr, gray_out, step, rst_mcus, s);
+        view = sc.view;
+    } else if (gray_out) {   // Y straight from the IDCT into the caller's image: no planes
+        e = launch_idct_gray(coef, dcarr, g, tb, d_bgr, step, rst_mcus, s);
+    } else {
+        e = launch_idct(coef, dcarr, g, tb, py, pcb, pcr, rst_mcus, s);
+    }
+    if (e != cudaSuccess) return e;
+    if (ev_idct) cudaEventRecord(ev_idct, s);
+    if (!gray_out && (e = launch_upcolor(py, pcb, pcr, view, d_bgr, step, s)) != cudaSuccess) return e;
+    if (ev_color) cudaEventRecord(ev_color, s);   // gray: no colour pass (dec_color stays 0)
+    if (launches) (*launches) += gray_out ? 1 : 2;
+    return cudaSuccess;
+}
+
 int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr, size_t step,
             bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src,
             int scale) {
-    const int rst = info.restart_interval;   // MCUs per restart interval (0: none)
-    if (rst && info.scan_len >= 0xFFFFFFF0ull) { snprintf(d->err, d->errlen, "restart-marker scans of 4 GB and more are not supported"); return B2J_EFORMAT; }
+    const JpegScan &sc = info.scans[0];
+    const int rst = sc.restart_interval;   // MCUs per restart interval (0: none)
+    if (rst && sc.seg_len >= 0xFFFFFFF0ull) { snprintf(d->err, d->errlen, "restart-marker scans of 4 GB and more are not supported"); return B2J_EFORMAT; }
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
-    if ((!d_scan_src && info.scan_offset + info.scan_len > len) || info.scan_len == 0) return B2J_EFORMAT;
-    int rc = ensure(d, info.scan_len, g, rst);
+    if ((!d_scan_src && sc.seg_off + sc.seg_len > len) || sc.seg_len == 0) return B2J_EFORMAT;
+    int rc = ensure(d, sc.seg_len, g, rst);
     if (rc) return rc;
-    const size_t n = info.scan_len;
+    const size_t n = sc.seg_len;
     const size_t nsub_max = (n * 8 + DEC_SUB_BITS - 1) / DEC_SUB_BITS;
     const int hv = g.hs * g.vs;   // luma blocks per MCU (gray: 1 of 1)
     if (tm) cudaEventRecord(d->ev[0], s);
@@ -205,10 +244,10 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
         const size_t b0 = std::min(n, (size_t)j * piece), b1 = std::min(n, b0 + piece);
         if (b1 > b0 && !d_scan_src) {
             if (d->upload) {
-                const int urc = d->upload(d->upload_user, d->d_scan + b0, jpg + info.scan_offset + b0, b1 - b0, d->up_stream);
+                const int urc = d->upload(d->upload_user, d->d_scan + b0, jpg + sc.seg_off + b0, b1 - b0, d->up_stream);
                 if (urc) return urc;
             } else {
-                DCK(cudaMemcpyAsync(d->d_scan + b0, jpg + info.scan_offset + b0, b1 - b0, cudaMemcpyHostToDevice, d->up_stream));
+                DCK(cudaMemcpyAsync(d->d_scan + b0, jpg + sc.seg_off + b0, b1 - b0, cudaMemcpyHostToDevice, d->up_stream));
             }
         }
         DCK(cudaEventRecord(d->ev_up[j], d->up_stream));
@@ -270,30 +309,9 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
     DCK(launch_dc_scan(d->d_dc, g, gray_out ? 1 : g.nc, d->d_desc + 2 * d->desc_cap, &d->d_ctrl->ticket[2], d->desc_cap,
                        &d->d_ctrl->err, s));
     if (tm) cudaEventRecord(d->ev[3], s);
-    if (scale > 1) {   // reduced size: the scaled IDCT (gray: straight into the caller's image), colour on the scaled view
-        uint8_t *py = d->d_planes;
-        uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
-        uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
-        const DecScale sc = dec_scale_setup(g, scale);
-        DCK(launch_idct_scaled(d->d_coef, d->d_dc, g, sc, d->d_tb, gray_out ? d_bgr : py, pcb, pcr, gray_out, step, rst, s));
-        if (tm) cudaEventRecord(d->ev[4], s);
-        if (!gray_out) DCK(launch_upcolor(py, pcb, pcr, sc.view, d_bgr, step, s));
-        if (tm) cudaEventRecord(d->ev[5], s);
-        if (launches) (*launches) += gray_out ? 4 : 5;
-    } else if (gray_out) {   // Y straight from the IDCT into the caller's image: no planes, no colour pass (dec_color stays 0)
-        DCK(launch_idct_gray(d->d_coef, d->d_dc, g, d->d_tb, d_bgr, step, rst, s));
-        if (tm) { cudaEventRecord(d->ev[4], s); cudaEventRecord(d->ev[5], s); }
-        if (launches) (*launches) += 4;
-    } else {
-        uint8_t *py = d->d_planes;
-        uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
-        uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
-        DCK(launch_idct(d->d_coef, d->d_dc, g, d->d_tb, py, pcb, pcr, rst, s));
-        if (tm) cudaEventRecord(d->ev[4], s);
-        DCK(launch_upcolor(py, pcb, pcr, g, d_bgr, step, s));
-        if (tm) cudaEventRecord(d->ev[5], s);
-        if (launches) (*launches) += 5;
-    }
+    DCK(dec_back_end(d->d_coef, d->d_dc, g, d->d_tb, d->d_planes, d_bgr, step, gray_out, scale, rst, s, tm ? d->ev[4] : nullptr,
+                     tm ? d->ev[5] : nullptr, launches));
+    if (launches) (*launches) += 3;
     if (tm) {
         DCK(cudaStreamSynchronize(s));
         cudaEventElapsedTime(&tm->dec_parse, d->ev[0], d->ev[1]);
@@ -306,7 +324,7 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
     return B2J_OK;
 }
 
-int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, uint8_t *d_bgr,
+int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr,
                         size_t step, bool gray_out, cudaStream_t s, uint64_t *launches, int scale) {
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
     int rc = ensure(d, 4096, g, 0);

@@ -5,7 +5,8 @@
 
 namespace b2j {
 
-constexpr int DEC_LUT_BITS = 10;
+constexpr int DEC_LUT_BITS = 10;    // sequential decode tables (DecTables)
+constexpr int PROG_LUT_BITS = 9;    // progressive decode tables (dec_prog.cu ProgTable)
 constexpr int DEC_SUB_BITS = 1024;
 
 struct DecTables {                 // device copy, one per decode
@@ -18,6 +19,10 @@ struct DecTables {                 // device copy, one per decode
 size_t dec_tables_size();
 // host side (dec_parse.cpp); B2J_EFORMAT for a table with more codes than its lengths allow
 int dec_build_tables(const JpegInfo &info, void *dst_host);
+// one Huffman table at a LUT of lut_bits: lut[1 << lut_bits] = (len << 8) | symbol for codes of length <= lut_bits, else
+// 0; maxcode[18]: largest code of length l, -1 if none, [17] a sentinel; valoff[17]: valptr[l] - mincode[l]; vals_out[256]
+int huff_derive(const uint8_t bits[17], const uint8_t vals[256], int lut_bits, uint16_t *lut, int32_t *maxcode, int32_t *valoff,
+                uint8_t *vals_out);
 
 // Chunks [c0, c1) of the n-byte scan (DS_CHUNK bytes of the 16-byte aligned stream that contains `in`: destuff_chunks()
 // of them in all); `ticket`: a zeroed counter per launch; *avail = bytes produced so far
@@ -97,10 +102,17 @@ inline DecScale dec_scale_setup(const Geom &g, int denom) {
 cudaError_t launch_idct_scaled(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecScale &sc, const void *tb,
                                uint8_t *py, uint8_t *pcb, uint8_t *pcr, bool gray, size_t out_step, int rst_mcus, cudaStream_t s);
 
-// progressive files (dec_prog.cu): all scans into d_coef, then IDCT + upsampling; synchronises the stream before returning
-// gray_out: 8-bit Y samples into d_bgr (launch_idct_gray) instead of IDCT + upsampling + colour conversion
-// scale: 1, or the reduced-size back end (launch_idct_scaled) at 1 / scale
-int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
+// The back end (dec.cu): de-quantisation, IDCT and colour conversion of the coefficient array into d_bgr (pitch step).
+// dcarr: the DC array of k_dc_scan, NULL if the blocks hold their own DCs (progressive); rst_mcus: the restart interval
+// (0: none); planes: the decoder's buffer of Y / Cb / Cr sample planes; gray_out: 8-bit Y samples only
+// (launch_idct_gray), no colour pass; scale: 1, or the reduced-size back end (launch_idct_scaled) at 1 / scale.
+// ev_idct / ev_color (optional) are recorded after the IDCT and after the colour pass; *launches counts the kernels.
+cudaError_t dec_back_end(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *planes, uint8_t *d_bgr,
+                         size_t step, bool gray_out, int scale, int rst_mcus, cudaStream_t s, cudaEvent_t ev_idct,
+                         cudaEvent_t ev_color, uint64_t *launches);
+
+// progressive files (dec_prog.cu): all scans into d_coef, then dec_back_end; synchronises the stream before returning
+int dec_progressive(const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
                     uint8_t *d_planes, uint8_t *d_bgr, size_t step, bool gray_out, cudaStream_t s, uint64_t *launches,
                     char *err, size_t errlen, int scale = 1);
 

@@ -28,8 +28,7 @@
 
 namespace b2j {
 
-constexpr int PROG_LUT_BITS = 9;
-struct ProgTable {                       // one Huffman table (jdhuff.c jpeg_make_d_derived_tbl)
+struct ProgTable {                       // one Huffman table (dec_parse.cpp huff_derive)
     uint16_t lut[1 << PROG_LUT_BITS];    // (len << 8) | symbol for codes of length <= PROG_LUT_BITS, else 0
     int32_t maxcode[18];
     int32_t valoff[17];
@@ -45,26 +44,6 @@ struct ProgCtl {                         // device words of one scan's front end
     uint64_t u_len, avail;
     uint32_t ticket, nmark, err, pad;
 };
-
-static int build_table(const uint8_t bits[17], const uint8_t vals[256], ProgTable *t) {
-    memset(t, 0, sizeof(*t));
-    int code = 0, p = 0;
-    for (int l = 1; l <= 16; l++) {
-        const int n = bits[l];
-        if (code + n > (1 << l) || p + n > 256) return B2J_EFORMAT;
-        t->valoff[l] = p - code;
-        for (int i = 0; i < n; i++, p++, code++)
-            if (l <= PROG_LUT_BITS) {
-                const int lo = code << (PROG_LUT_BITS - l), cnt = 1 << (PROG_LUT_BITS - l);
-                for (int j = 0; j < cnt; j++) t->lut[lo + j] = (uint16_t)((l << 8) | vals[p]);
-            }
-        t->maxcode[l] = n ? code - 1 : -1;
-        code <<= 1;
-    }
-    t->maxcode[17] = 0x7fffffff;
-    memcpy(t->vals, vals, 256);
-    return B2J_OK;
-}
 
 // streaming bit reader over UNSTUFFED bytes: the next `nav` bits left-aligned in acc; words come from a four-word
 // register queue refilled with 16-byte loads issued one vector ahead (the load latency stays off the symbol chain)
@@ -327,7 +306,7 @@ k_prog_apply(const uint64_t *__restrict__ cm, const uint64_t *__restrict__ corr,
         }                                                                                                          \
     } while (0)
 
-int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
+int dec_progressive(const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
                     uint8_t *d_planes, uint8_t *d_bgr, size_t step, bool gray_out, cudaStream_t s, uint64_t *launches,
                     char *err, size_t errlen, int scale) {
     int rc = B2J_OK;
@@ -336,18 +315,20 @@ int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const 
     ProgCtl *d_ctl = nullptr;
     uint64_t *d_desc = nullptr, *d_mask = nullptr, *d_tmp = nullptr;
     uint32_t *d_bnd = nullptr;
-    std::vector<ProgScanDev> hsc(info.nscans);
+    const int nscans = (int)info.scans.size();
+    std::vector<ProgScanDev> hsc(nscans);
     DecTables *htb = nullptr;
     size_t max_seg = 0, max_units = 0, max_int = 1;
-    for (int i = 0; i < info.nscans; i++) {
-        const ProgScan &ps = info.scans[i];
+    for (int i = 0; i < nscans; i++) {
+        const JpegScan &ps = info.scans[i];
         ProgScanDev &sd = hsc[i];
         memset(&sd, 0, sizeof(sd));
         sd.ncomp = ps.ncomp; sd.Ss = ps.Ss; sd.Se = ps.Se; sd.Ah = ps.Ah; sd.Al = ps.Al; sd.ri = ps.restart_interval;
         for (int c = 0; c < ps.ncomp; c++) {
             sd.comp[c] = ps.comp[c];
-            if ((ps.Ss == 0 && ps.Ah == 0 && build_table(ps.bits[0][c], ps.vals[0][c], &sd.tb[0][c])) ||
-                (ps.Ss > 0 && build_table(ps.bits[1][c], ps.vals[1][c], &sd.tb[1][c]))) {
+            const int k = ps.Ss > 0;   // the table the scan decodes with: DC (first DC scans, Ah = 0) or AC
+            ProgTable &t = sd.tb[k][c];
+            if ((k || ps.Ah == 0) && huff_derive(ps.bits[k][c], ps.vals[k][c], PROG_LUT_BITS, t.lut, t.maxcode, t.valoff, t.vals)) {
                 snprintf(err, errlen, "invalid Huffman table in scan %d", i);
                 return B2J_EFORMAT;
             }
@@ -364,7 +345,7 @@ int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const 
     {   // one allocation for everything the scans need (allocations and frees synchronise: a handful of them per decode
         // would cost more than a small file's kernels)
         auto up = [](size_t x) { return (x + 255) & ~(size_t)255; };
-        const size_t o_file = 0, o_u = o_file + up(len + 64), o_sc = o_u + up(max_seg + 4096), o_ctl = o_sc + up(sizeof(ProgScanDev) * info.nscans),
+        const size_t o_file = 0, o_u = o_file + up(len + 64), o_sc = o_u + up(max_seg + 4096), o_ctl = o_sc + up(sizeof(ProgScanDev) * nscans),
                      o_desc = o_ctl + up(sizeof(ProgCtl)), o_bnd = o_desc + up(ndesc * 8), o_mask = o_bnd + up((max_int + 2) * 4),
                      o_tmp = o_mask + up((size_t)g.nblocks * 8), total = o_tmp + up(max_units * 8 * 4);
         PCK(cudaMalloc(&d_all, total));
@@ -374,11 +355,11 @@ int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const 
         d_tmp = reinterpret_cast<uint64_t *>(d_all + o_tmp);
     }
     PCK(cudaMemcpyAsync(d_file, jpg, len, cudaMemcpyDefault, s));
-    PCK(cudaMemcpyAsync(d_sc, hsc.data(), sizeof(ProgScanDev) * info.nscans, cudaMemcpyHostToDevice, s));
+    PCK(cudaMemcpyAsync(d_sc, hsc.data(), sizeof(ProgScanDev) * nscans, cudaMemcpyHostToDevice, s));
     PCK(cudaMemsetAsync(d_coef, 0, (size_t)g.nblocks * 128, s));
     PCK(cudaMemsetAsync(d_mask, 0, (size_t)g.nblocks * 8, s));
-    for (int i = 0; i < info.nscans; i++) {
-        const ProgScan &ps = info.scans[i];
+    for (int i = 0; i < nscans; i++) {
+        const JpegScan &ps = info.scans[i];
         const ProgScanDev &sd = hsc[i];
         if (ps.seg_len == 0) continue;
         // front end: stuffing and RSTn markers out, interval starts recorded (the baseline decoder's kernel)
@@ -406,22 +387,8 @@ int dec_progressive(const uint8_t *jpg, size_t len, const ProgInfo &info, const 
         if (!htb) { rc = B2J_ENOMEM; goto done; }
         memcpy(htb->q, info.qt, sizeof(htb->q));
         PCK(cudaMemcpyAsync(d_tb, htb, dec_tables_size(), cudaMemcpyHostToDevice, s));
-        uint8_t *py = d_planes;
-        uint8_t *pcb = py + (((size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs + 63) & ~(size_t)63);
-        uint8_t *pcr = pcb + (((size_t)g.mcux * 8 * g.mcuy * 8 + 63) & ~(size_t)63);
-        if (scale > 1) {   // reduced size: the blocks hold their own DCs (dcarr NULL), as for the full-size back end
-            const DecScale sc = dec_scale_setup(g, scale);
-            PCK(launch_idct_scaled(d_coef, nullptr, g, sc, d_tb, gray_out ? d_bgr : py, pcb, pcr, gray_out, step, 0, s));
-            if (!gray_out) PCK(launch_upcolor(py, pcb, pcr, sc.view, d_bgr, step, s));
-            if (launches) (*launches) += gray_out ? 1 : 2;
-        } else if (gray_out) {
-            PCK(launch_idct_gray(d_coef, nullptr, g, d_tb, d_bgr, step, 0, s));
-            if (launches) (*launches) += 1;
-        } else {
-            PCK(launch_idct(d_coef, nullptr, g, d_tb, py, pcb, pcr, 0, s));
-            PCK(launch_upcolor(py, pcb, pcr, g, d_bgr, step, s));
-            if (launches) (*launches) += 2;
-        }
+        // the blocks hold their own DCs (dcarr NULL)
+        PCK(dec_back_end(d_coef, nullptr, g, d_tb, d_planes, d_bgr, step, gray_out, scale, 0, s, nullptr, nullptr, launches));
     }
     PCK(cudaStreamSynchronize(s));   // the host vectors and the temporary buffers go away below
 done:

@@ -1,5 +1,5 @@
-// ASAN fuzz harness for the product's JPEG header parser (csrc/dec_parse.cpp: parse_jpeg + dec_build_tables): every mutated input is copied into an
-// exact-size heap block so that any read past the end is reported.
+// ASAN fuzz harness for the product's JPEG header parser (csrc/dec_parse.cpp: parse_jpeg, dec_build_tables, huff_derive):
+// every mutated input is copied into an exact-size heap block so that any read past the end is reported.
 #include <cstdio>
 #include <cstdlib>
 #include <cstring>
@@ -35,20 +35,24 @@ int main(int argc, char **argv) {
         int rc = b2j::parse_jpeg(heap, s.size(), &info);
         if (rc == 0) {
             ok++;
-            if (info.scan_offset + info.scan_len > s.size()) { printf("BAD RANGE it=%d\n", it); return 2; }
-            // the table builder writes a fixed-size block: exact-size heap copy so ASAN sees any overflow
-            void *tb = malloc(b2j::dec_tables_size());
-            b2j::dec_build_tables(info, tb);
-            free(tb);
-            if (info.W <= 0 || info.H <= 0 || info.css < 0 || info.css > 4) { printf("BAD INFO it=%d\n", it); return 2; }
-        }
-        {   // the progressive parser on the same bytes
-            b2j::ProgInfo pi;
-            if (b2j::parse_progressive(heap, s.size(), &pi) == 0) {
-                ok++;
-                for (int i = 0; i < pi.nscans; i++)
-                    if (pi.scans[i].seg_off + pi.scans[i].seg_len > s.size() || pi.scans[i].ncomp < 1 || pi.scans[i].ncomp > 3) { printf("BAD SCAN it=%d\n", it); return 2; }
-                b2j::prog_free(&pi);
+            if (info.W <= 0 || info.H <= 0 || info.css < 0 || info.css > 4 || info.scans.empty()) { printf("BAD INFO it=%d\n", it); return 2; }
+            for (const b2j::JpegScan &sc : info.scans)
+                if (sc.seg_off + sc.seg_len > s.size() || sc.ncomp < 1 || sc.ncomp > 3) { printf("BAD SCAN it=%d\n", it); return 2; }
+            // the table builders write fixed-size blocks: exact-size heap copies so ASAN sees any overflow
+            if (!info.progressive) {
+                void *tb = malloc(b2j::dec_tables_size());
+                b2j::dec_build_tables(info, tb);
+                free(tb);
+            } else {   // dec_prog.cu: one table per component and class of every scan
+                for (const b2j::JpegScan &sc : info.scans)
+                    for (int k = 0; k < 2; k++)
+                        for (int c = 0; c < sc.ncomp; c++) {
+                            uint16_t *lut = (uint16_t *)malloc(sizeof(uint16_t) << b2j::PROG_LUT_BITS);
+                            int32_t *maxcode = (int32_t *)malloc(18 * 4), *valoff = (int32_t *)malloc(17 * 4);
+                            uint8_t *vals = (uint8_t *)malloc(256);
+                            b2j::huff_derive(sc.bits[k][c], sc.vals[k][c], b2j::PROG_LUT_BITS, lut, maxcode, valoff, vals);
+                            free(lut); free(maxcode); free(valoff); free(vals);
+                        }
             }
         }
         total++;

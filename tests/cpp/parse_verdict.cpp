@@ -1,5 +1,5 @@
 // The product's JPEG header parser (csrc/dec_parse.cpp) on files named on the command line: one line per file,
-// "<parse_jpeg rc> <parse_progressive rc> <css>" (css of the parser that accepted the file, -1 if none did).
+// "<parse_jpeg rc> <progressive> <css>" (progressive and css as parsed, 0 and -1 for a refused file).
 #include <cstdio>
 #include <vector>
 #include <cuda_runtime.h>
@@ -13,11 +13,8 @@ int main(int argc, char **argv) {
         size_t got = fread(b.data(), 1, n, f);
         fclose(f);
         b2j::JpegInfo info;
-        b2j::ProgInfo pi;
-        const int rb = b2j::parse_jpeg(b.data(), got, &info);
-        const int rp = b2j::parse_progressive(b.data(), got, &pi);
-        printf("%d %d %d\n", rb, rp, rb == 0 ? info.css : rp == 0 ? pi.css : -1);
-        if (rp == 0) b2j::prog_free(&pi);
+        const int rc = b2j::parse_jpeg(b.data(), got, &info);
+        printf("%d %d %d\n", rc, rc == 0 && info.progressive ? 1 : 0, rc == 0 ? info.css : -1);
     }
     return 0;
 }

@@ -116,8 +116,8 @@ def test_parser_verdicts(corpus, parse_verdict, tmp_path):
     assert r.returncode == 0, r.stderr
     lines = r.stdout.split("\n")
     for e, line in zip(corpus, lines):
-        rb, rp, css = (int(x) for x in line.split())
+        rc, progressive, css = (int(x) for x in line.split())
         if e["accept"]:
-            assert (rp if e["progressive"] else rb) == 0 and 0 <= css <= 4, (e["name"], line)
+            assert rc == 0 and progressive == int(e["progressive"]) and 0 <= css <= 4, (e["name"], line)
         else:
-            assert rb == -5 and rp == -5, (e["name"], line)
+            assert rc == -5, (e["name"], line)
