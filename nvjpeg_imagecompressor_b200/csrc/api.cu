@@ -1021,6 +1021,11 @@ static int parse_for(b2j_ctx *ctx, const uint8_t *jpg, size_t len, JpegInfo *inf
     int rc = parse_jpeg(jpg, len, info);
     if (rc) { snprintf(ctx->err, sizeof(ctx->err), "unsupported or corrupt JPEG (parse rc=%d)", rc); return B2J_EFORMAT; }
     rc = check_components(ctx, info->css); if (rc) return rc;
+    if (info->progressive && info->smoothed[chans(ctx) == 1]) {
+        snprintf(ctx->err, sizeof(ctx->err), "incomplete progressive JPEG (low-frequency coefficients unfinished): "
+                 "libjpeg would block-smooth it, which this decoder does not do");
+        return B2J_EFORMAT;
+    }
     if (width) *width = dec_scaled_size(info->W, ctx->dec_scale);
     if (height) *height = dec_scaled_size(info->H, ctx->dec_scale);
     return B2J_OK;

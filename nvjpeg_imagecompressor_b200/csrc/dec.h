@@ -24,6 +24,10 @@ struct JpegInfo {
     bool progressive;              // SOF2: scans up to EOI; else SOF0 / SOF1: the first scan only
     uint16_t qt[2][64];            // natural order: luma, chroma (gray: both the component's table), as at the last SOS
     std::vector<JpegScan> scans;
+    // a progressive file that leaves low-frequency coefficients unfinished: libjpeg-turbo block-smooths such output
+    // (jdcoefct.c smoothing_ok), which this decoder does not restate, so the decode entry points refuse it.
+    // [0]: BGR output (any component unfinished), [1]: gray output (the Y plane: Y unfinished)
+    bool smoothed[2];
 };
 
 // jdmarker.c subset: SOF0 / SOF1 / SOF2, 3 components, chroma 1x1, luma in {1x1,2x1,1x2,2x2,4x1}; or one component (any

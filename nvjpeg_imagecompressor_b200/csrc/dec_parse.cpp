@@ -63,6 +63,8 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
     memset(hb, 0, sizeof(hb));
     memset(hv, 0, sizeof(hv));
     int cid[3] = {0, 0, 0}, chv[3] = {0, 0, 0}, ctq[3] = {0, 0, 0}, ncomp = 0, ri = 0;
+    int coef_bits[3][10];   // jdphuff.c coef_bits for zig-zag 0..9: the Al of the last scan that sent it, -1: none yet
+    memset(coef_bits, 0xFF, sizeof(coef_bits));
     ColourMarkers cm;
     size_t p = 2;
     while (p + 2 <= len) {
@@ -162,8 +164,12 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
             if (info->progressive) {
                 sc.Ss = s[1 + 2 * sc.ncomp]; sc.Se = s[2 + 2 * sc.ncomp];
                 sc.Ah = s[3 + 2 * sc.ncomp] >> 4; sc.Al = s[3 + 2 * sc.ncomp] & 15;
-                if (sc.Ss > sc.Se || sc.Se > 63 || (sc.Ss == 0 && sc.Se != 0) || (sc.Ss > 0 && sc.ncomp != 1) || sc.Al > 13 || sc.Ah > 13)
+                // jdphuff.c start_pass_phuff_decoder: a refinement scan refines by exactly one bit
+                if (sc.Ss > sc.Se || sc.Se > 63 || (sc.Ss == 0 && sc.Se != 0) || (sc.Ss > 0 && sc.ncomp != 1) || sc.Al > 13 ||
+                    (sc.Ah != 0 && sc.Al != sc.Ah - 1))
                     return B2J_EFORMAT;
+                for (int i = 0; i < sc.ncomp; i++)
+                    for (int k = sc.Ss; k <= sc.Se && k < 10; k++) coef_bits[sc.comp[i]][k] = sc.Al;
             } else {
                 sc.Se = 63;
                 if (sc.ncomp == 3 && (td[1] != td[2] || ta[1] != ta[2])) return B2J_EFORMAT;   // one table pair for Cb and Cr
@@ -199,7 +205,19 @@ int parse_jpeg(const uint8_t *jpg, size_t len, JpegInfo *info) {
         p += L;
     }
     // EOI, or the end of the bytes: a progressive file may end right after its last scan (a sequential one has returned)
-    return info->scans.empty() ? B2J_EFORMAT : B2J_OK;
+    if (info->scans.empty()) return B2J_EFORMAT;
+    // jdcoefct.c smoothing_ok (libjpeg-turbo 2.1 and later): every component's DC has been sent, the quantisers of
+    // zig-zag 0..9 are non-zero, and some coefficient among zig-zag 1..9 is unfinished (never sent, or sent with Al > 0).
+    // Smoothing then changes a component only where that component is unfinished: on gray output, only Y counts.
+    bool ok = true, unfinished[3] = {false, false, false};
+    for (int c = 0; c < ncomp; c++) {
+        ok = ok && coef_bits[c][0] >= 0;
+        for (int k = 0; k < 10; k++) ok = ok && info->qt[c > 0][ZZ[k]] != 0;
+        for (int k = 1; k < 10; k++) unfinished[c] = unfinished[c] || coef_bits[c][k] != 0;
+    }
+    info->smoothed[0] = ok && (unfinished[0] || unfinished[1] || unfinished[2]);
+    info->smoothed[1] = ok && unfinished[0];
+    return B2J_OK;
 }
 
 size_t dec_tables_size() { return sizeof(DecTables); }

@@ -46,7 +46,9 @@ struct ProgCtl {                         // device words of one scan's front end
 };
 
 // streaming bit reader over UNSTUFFED bytes: the next `nav` bits left-aligned in acc; words come from a four-word
-// register queue refilled with 16-byte loads issued one vector ahead (the load latency stays off the symbol chain)
+// register queue refilled with 16-byte loads issued one vector ahead (the load latency stays off the symbol chain).
+// Bytes at and after `end` (the end of the interval's data) read as zeros, as jdhuff.c jpeg_fill_bit_buffer feeds
+// zero bits at a marker; over() tells that a bit past the end has been consumed (libjpeg's insufficient_data).
 struct WordReader {
     const uint4 *u4;
     uint64_t acc;
@@ -54,6 +56,7 @@ struct WordReader {
     uint32_t w0, w1, w2, w3;
     uint4 ahead;
     size_t vidx;
+    int64_t wpos, end;   // byte offset of the next word into acc; end of the data (-1: an interval the file lacks)
     __device__ __forceinline__ uint32_t next_word() {
         if (qn == 0) {
             w0 = ahead.x; w1 = ahead.y; w2 = ahead.z; w3 = ahead.w;
@@ -61,12 +64,18 @@ struct WordReader {
             vidx++;
             ahead = u4[vidx];
         }
-        const uint32_t w = w0;
+        const uint32_t w = __byte_perm(w0, 0, 0x0123);
         w0 = w1; w1 = w2; w2 = w3;
         qn--;
-        return __byte_perm(w, 0, 0x0123);
+        const int64_t rem = end - wpos;
+        wpos += 4;
+        if (rem >= 4) return w;
+        return rem <= 0 ? 0u : w & ~(0xFFFFFFFFu >> (8 * (int)rem));
     }
-    __device__ __forceinline__ void seek(const uint8_t *u, uint64_t byte_pos) {   // interval starts are byte aligned
+    __device__ __forceinline__ bool over() const { return wpos * 8 - nav > end * 8; }
+    __device__ __forceinline__ void seek(const uint8_t *u, uint64_t byte_pos, int64_t end_pos) {   // interval starts are byte aligned
+        end = end_pos;
+        wpos = (int64_t)(byte_pos & ~(uint64_t)3);
         u4 = reinterpret_cast<const uint4 *>(u);
         const size_t widx = (size_t)(byte_pos >> 2);
         vidx = widx >> 2;
@@ -178,89 +187,109 @@ k_prog_scan(const uint8_t *__restrict__ u, const ProgCtl *__restrict__ ctl, cons
     __syncwarp();
     const uint32_t j = blockIdx.x * 32 + threadIdx.x;
     const uint32_t nint = sc.ri ? ctl->nmark + 1u : 1u;
-    if (j >= nint || j >= sc.nint_max) return;   // intervals a truncated file does not have keep their zeros
+    // Interval j ends where the next begins, the last one where the data ends. A cut file lacks the intervals from
+    // nint on: they read as out of data from their start, so they leave their blocks alone (jdphuff.c insufficient_data)
+    // and a refinement scan writes zero words for them. Interval nint is the previous thread's: when the data ends
+    // exactly at its start, libjpeg still decodes one MCU of zero bits there.
+    if (j >= sc.nint_max || j == nint) return;
     WordReader r;
-    r.seek(u, j == 0 ? 0 : (uint64_t)bnd[j - 1]);
-    int pred[3] = {0, 0, 0}, eobrun = 0;
-    const uint64_t u0 = sc.ri ? (uint64_t)j * sc.ri : 0, u1 = sc.ri ? min(sc.units, u0 + sc.ri) : sc.units;
+    if (j < nint) r.seek(u, j == 0 ? 0 : (uint64_t)bnd[j - 1], j < ctl->nmark ? (int64_t)bnd[j] : (int64_t)ctl->u_len);
+    else r.seek(u, 0, -1);
+    int pred[3], eobrun;
     const int Al = sc.Al;
     const uint32_t p1 = 1u << Al;
-    if (sc.Ss == 0) {
-        // ---- DC scans (interleaved: MCU order, every block of the MCU, padding blocks too; or one component)
-        UnitWalk wk;
-        wk.init(g, sc.comp[0], u0);
-        for (uint64_t un = u0; un < u1; un++, wk.next()) {
-            for (int i = 0; i < sc.ncomp; i++) {
-                const int c = sc.comp[i];
-                const int nb = sc.ncomp > 1 ? (c ? 1 : g.hs * g.vs) : 1;
-                for (int b = 0; b < nb; b++) {
-                    const size_t blk = sc.ncomp > 1 ? (size_t)un * g.bpm + (c ? g.bpm - 3 + c : b) : wk.block(g);
-                    if (sc.Ah == 0) {          // decode_mcu_DC_first
-                        const int s = r.sym(sc.tb[0][i]);
-                        const int diff = s ? prog_extend((int)r.get(s), s) : 0;
-                        pred[i] += diff;
-                        coef[blk * 64] = (int16_t)(pred[i] * (1 << Al));
-                    } else if (r.get(1)) {     // decode_mcu_DC_refine: a posted OR on the word that holds coefficient 0
-                        atomicOr(reinterpret_cast<unsigned int *>(coef + blk * 64), p1);
+    const int c = sc.comp[0], Ss = sc.Ss, Se = sc.Se;
+    const ProgTable &ac = sc.tb[1][0];
+    const uint64_t band = bits_range(Ss, Se);
+    // the chain over units [u0, u1) of one interval; an MCU that starts after the data ran out is left alone, and so is
+    // every later one of the interval
+    auto chain = [&](uint64_t u0, uint64_t u1) {
+        pred[0] = pred[1] = pred[2] = 0;
+        eobrun = 0;
+        if (sc.Ss == 0) {
+            // ---- DC scans (interleaved: MCU order, every block of the MCU, padding blocks too; or one component)
+            UnitWalk wk;
+            wk.init(g, sc.comp[0], u0);
+            for (uint64_t un = u0; un < u1 && !r.over(); un++, wk.next()) {
+                for (int i = 0; i < sc.ncomp; i++) {
+                    const int ci = sc.comp[i];
+                    const int nb = sc.ncomp > 1 ? (ci ? 1 : g.hs * g.vs) : 1;
+                    for (int b = 0; b < nb; b++) {
+                        const size_t blk = sc.ncomp > 1 ? (size_t)un * g.bpm + (ci ? g.bpm - 3 + ci : b) : wk.block(g);
+                        if (sc.Ah == 0) {          // decode_mcu_DC_first
+                            const int s = r.sym(sc.tb[0][i]);
+                            const int diff = s ? prog_extend((int)r.get(s), s) : 0;
+                            pred[i] += diff;
+                            coef[blk * 64] = (int16_t)(pred[i] * (1 << Al));
+                        } else if (r.get(1)) {     // decode_mcu_DC_refine: a posted OR on the word that holds coefficient 0
+                            atomicOr(reinterpret_cast<unsigned int *>(coef + blk * 64), p1);
+                        }
                     }
                 }
             }
+            return;
         }
-        return;
-    }
-    const int c = sc.comp[0], Ss = sc.Ss, Se = sc.Se;
-    const ProgTable &ac = sc.tb[1][0];
-    if (sc.Ah == 0) {
-        // ---- decode_mcu_AC_first: coefficients by posted stores, new positions OR-ed into the block's mask
-        UnitWalk wk;
-        wk.init(g, c, u0);
-        for (uint64_t un = u0; un < u1; un++, wk.next()) {
-            if (eobrun > 0) { eobrun--; continue; }
-            const size_t blk = wk.block(g);
-            uint64_t bits = 0;
-            for (int k = Ss; k <= Se; k++) {
-                const int rs = r.sym(ac), rr = rs >> 4, ss = rs & 15;
-                if (ss) {
-                    k += rr;
-                    const int v = prog_extend((int)r.get(ss), ss);
-                    if (k <= 63) { coef[blk * 64 + k] = (int16_t)(v * (1 << Al)); bits |= 1ull << k; }
-                } else {
-                    if (rr == 15) k += 15;
-                    else { eobrun = 1 << rr; if (rr) eobrun += (int)r.get(rr); eobrun--; break; }
+        if (sc.Ah == 0) {
+            // ---- decode_mcu_AC_first: coefficients by posted stores, new positions OR-ed into the block's mask
+            UnitWalk wk;
+            wk.init(g, c, u0);
+            for (uint64_t un = u0; un < u1 && !r.over(); un++, wk.next()) {
+                if (eobrun > 0) { eobrun--; continue; }
+                const size_t blk = wk.block(g);
+                uint64_t bits = 0;
+                for (int k = Ss; k <= Se; k++) {
+                    const int rs = r.sym(ac), rr = rs >> 4, ss = rs & 15;
+                    if (ss) {
+                        k += rr;
+                        const int v = prog_extend((int)r.get(ss), ss);
+                        if (k <= 63) { coef[blk * 64 + k] = (int16_t)(v * (1 << Al)); bits |= 1ull << k; }
+                    } else {
+                        if (rr == 15) k += 15;
+                        else { eobrun = 1 << rr; if (rr) eobrun += (int)r.get(rr); eobrun--; break; }
+                    }
+                }
+                if (bits) atomicOr(reinterpret_cast<unsigned long long *>(mask + blk), (unsigned long long)bits);
+            }
+            return;
+        }
+        // ---- decode_mcu_AC_refine, parsing only: correction bits, new positions and their signs per block
+        for (uint64_t un = u0; un < u1; un++) {
+            const uint64_t m = cm[un] & band;     // coefficients of the band that are already non-zero
+            uint64_t cbits = 0, nm = 0, ns = 0;
+            int k = Ss;
+            if (r.over()) { corr[un] = 0; newm[un] = 0; news[un] = 0; continue; }
+            if (eobrun == 0) {
+                while (k <= Se) {
+                    const int rs = r.sym(ac), rr = rs >> 4, ss = rs & 15;
+                    uint32_t positive = 0;
+                    if (ss) positive = r.get(1);                       // the size of a new coefficient is always 1
+                    else if (rr != 15) { eobrun = 1 << rr; if (rr) eobrun += (int)r.get(rr); break; }
+                    // pass over rr still-zero coefficients, stop at the next one; the non-zero ones on the way take a bit each
+                    const uint64_t z = ~m & bits_range(k, Se);
+                    const int p = min(select_bit(z, rr), Se + 1);
+                    const uint64_t nzs = m & bits_range(k, p - 1);
+                    const int n = __popcll(nzs);
+                    cbits = (cbits << n) | r.get64(n);
+                    if (ss && p <= Se) { nm |= 1ull << p; if (positive) ns |= 1ull << p; }
+                    k = p + 1;
                 }
             }
-            if (bits) atomicOr(reinterpret_cast<unsigned long long *>(mask + blk), (unsigned long long)bits);
-        }
-        return;
-    }
-    // ---- decode_mcu_AC_refine, parsing only: correction bits, new positions and their signs per block
-    const uint64_t band = bits_range(Ss, Se);
-    for (uint64_t un = u0; un < u1; un++) {
-        const uint64_t m = cm[un] & band;     // coefficients of the band that are already non-zero
-        uint64_t cbits = 0, nm = 0, ns = 0;
-        int k = Ss;
-        if (eobrun == 0) {
-            while (k <= Se) {
-                const int rs = r.sym(ac), rr = rs >> 4, ss = rs & 15;
-                uint32_t positive = 0;
-                if (ss) positive = r.get(1);                       // the size of a new coefficient is always 1
-                else if (rr != 15) { eobrun = 1 << rr; if (rr) eobrun += (int)r.get(rr); break; }
-                // pass over rr still-zero coefficients, stop at the next one; the non-zero ones on the way take a bit each
-                const uint64_t z = ~m & bits_range(k, Se);
-                const int p = min(select_bit(z, rr), Se + 1);
-                const uint64_t nzs = m & bits_range(k, p - 1);
-                const int n = __popcll(nzs);
+            if (eobrun > 0) {
+                const int n = __popcll(m & bits_range(k, Se));
                 cbits = (cbits << n) | r.get64(n);
-                if (ss && p <= Se) { nm |= 1ull << p; if (positive) ns |= 1ull << p; }
-                k = p + 1;
+                eobrun--;
             }
+            corr[un] = cbits; newm[un] = nm; news[un] = ns;
         }
-        if (eobrun > 0) {
-            const int n = __popcll(m & bits_range(k, Se));
-            cbits = (cbits << n) | r.get64(n);
-            eobrun--;
-        }
-        corr[un] = cbits; newm[un] = nm; news[un] = ns;
+    };
+    uint64_t u0 = sc.ri ? (uint64_t)j * sc.ri : 0, u1 = sc.ri ? min(sc.units, u0 + sc.ri) : sc.units;
+    for (uint32_t jj = j;; jj++) {
+        chain(u0, u1);
+        if (jj + 1 != nint || nint >= sc.nint_max) break;
+        // interval nint: one MCU of zero bits if this interval ended without running out of data, nothing otherwise
+        r.seek(u, ctl->u_len, r.over() ? -1 : (int64_t)ctl->u_len);
+        u0 = u1;
+        u1 = min(sc.units, u0 + sc.ri);
     }
 }
 

@@ -860,7 +860,9 @@ static void make_dtbl(const uint8_t bits[17], const uint8_t *vals, dtbl *t) {
     }
     t->maxcode[17] = 0x7fffffff; t->vals = vals;
 }
-typedef struct { const uint8_t *d; size_t n, pos; uint32_t acc; int cnt; int marker; } bitr;
+/* insufficient: a bit past the data (a marker or the end of the segment) was read; jdhuff.c jpeg_fill_bit_buffer then
+ * feeds zero bits and sets the entropy decoder's insufficient_data */
+typedef struct { const uint8_t *d; size_t n, pos; uint32_t acc; int cnt; int marker; int insufficient; } bitr;
 static int get_bit(bitr *r) {
     if (r->cnt == 0) {
         uint8_t b = 0;
@@ -870,9 +872,9 @@ static int get_bit(bitr *r) {
                 size_t q = r->pos + 1;
                 while (q < r->n && r->d[q] == 0xFF) q++;
                 uint8_t b2 = q < r->n ? r->d[q] : 0xD9;
-                if (b2 == 0) r->pos = q + 1; else { r->marker = b2; r->pos = q - 1; b = 0; }
+                if (b2 == 0) r->pos = q + 1; else { r->marker = b2; r->pos = q - 1; b = 0; r->insufficient = 1; }
             } else r->pos++;
-        }
+        } else r->insufficient = 1;
         r->acc = b; r->cnt = 8;
     }
     r->cnt--;
@@ -894,7 +896,7 @@ int orc_decode_coefs(const uint8_t *jpg, size_t len, const orc_info *info, int16
     dtbl t[4];
     for (int i = 0; i < 4; i++) make_dtbl(info->bits[i], info->vals[i], &t[i]);
     if (info->scan_offset + info->scan_len > len) return -2;
-    bitr r = {jpg + info->scan_offset, info->scan_len, 0, 0, 0, 0};
+    bitr r = {jpg + info->scan_offset, info->scan_len, 0, 0, 0, 0, 0};
     memset(coef, 0, (size_t)g.nblocks * 128);
     int pred[3] = {0, 0, 0};
     long long nmcu = (long long)g.mcux * g.mcuy;
@@ -1052,12 +1054,40 @@ int orc_inverse(const int16_t *coef, const orc_info *info, uint8_t *bgr, size_t 
  * What the reference as shipped writes (NVJPEG_ENCODING_PROGRESSIVE_DCT_HUFFMAN, ImageCompressorImpl.cu:28; SURVEY.md
  * 8f N4). All scans are absorbed into the coefficient array (jdapimin.c without buffered-image mode), then the baseline
  * back end (IDCT, upsampling, colour) runs: block smoothing never triggers on a complete file. */
+/* jdphuff.c process_restart. Where the data ends instead of an RSTn (a cut file), insufficient_data stays as it is: the
+ * rest of the scan is left alone, except that an interval that ended cleanly lets the next one decode one MCU of zero
+ * bits before it runs out */
 static void prog_restart(bitr *r, int pred[3], int *eobrun) {
     r->cnt = 0;
     while (!r->marker && r->pos + 1 < r->n && r->d[r->pos] == 0xFF && r->d[r->pos + 1] == 0xFF) r->pos++;   /* fill */
-    if (r->marker) { r->pos += 2; r->marker = 0; }
-    else if (r->pos + 1 < r->n && r->d[r->pos] == 0xFF && r->d[r->pos + 1] >= 0xD0 && r->d[r->pos + 1] <= 0xD7) r->pos += 2;
+    if (r->marker) { r->pos += 2; r->marker = 0; r->insufficient = 0; }
+    else if (r->pos + 1 < r->n && r->d[r->pos] == 0xFF && r->d[r->pos + 1] >= 0xD0 && r->d[r->pos + 1] <= 0xD7) {
+        r->pos += 2; r->insufficient = 0;
+    }
     pred[0] = pred[1] = pred[2] = 0; *eobrun = 0;
+}
+
+/* jdphuff.c start_pass_phuff_decoder: scan parameters libjpeg accepts (a refinement refines by one bit), and coef_bits
+ * (the Al of the last scan that sent each of zig-zag 0..9, -1: none yet) */
+static int prog_scan_ok(const pscan *sc) {
+    return !(sc->Ss > sc->Se || sc->Se > 63 || (sc->Ss == 0 && sc->Se != 0) || (sc->Ss > 0 && sc->ncomp != 1) ||
+             sc->Al > 13 || (sc->Ah != 0 && sc->Al != sc->Ah - 1));
+}
+static void note_coef_bits(int cb[3][10], const pscan *sc) {
+    for (int i = 0; i < sc->ncomp; i++)
+        for (int k = sc->Ss; k <= sc->Se && k < 10; k++) cb[sc->comp[i]][k] = sc->Al;
+}
+/* jdcoefct.c smoothing_ok (libjpeg-turbo 2.1 and later): every component's DC sent, the quantisers of zig-zag 0..9
+ * non-zero, and some coefficient among zig-zag 1..9 of an output component (0..nout-1) unfinished. libjpeg would then
+ * block-smooth the output, which this checker does not restate: -18. */
+static int prog_smoothed(const int cb[3][10], int ncomp, int nout, const uint16_t *qt[3]) {
+    int unfinished = 0;
+    for (int c = 0; c < ncomp; c++) {
+        if (cb[c][0] < 0) return 0;
+        for (int k = 0; k < 10; k++) if (qt[c][ZIGZAG[k]] == 0) return 0;
+        for (int k = 1; k < 10; k++) if (c < nout && cb[c][k] != 0) unfinished = 1;
+    }
+    return unfinished ? -18 : 0;
 }
 
 static void prog_block(bitr *r, const pscan *sc, int ci, const dtbl *dc, const dtbl *ac, int16_t *blk, int *pred, int *eobrun) {
@@ -1124,7 +1154,8 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
     static uint8_t hb[2][4][17], hv[2][4][256];
     memset(hb, 0, sizeof(hb)); memset(hv, 0, sizeof(hv));
     int comp_id[3] = {0, 0, 0}, comp_hv[3] = {0, 0, 0}, comp_tq[3] = {0, 0, 0}, ncomp = 0, ri = 0, have_sof = 0;
-    int jfif = 0, adobe = -1, nscans = 0;
+    int jfif = 0, adobe = -1, nscans = 0, coef_bits[3][10];
+    memset(coef_bits, 0xFF, sizeof(coef_bits));
     orc_geom g; memset(&g, 0, sizeof(g));
     int16_t *coef = NULL;
     size_t p = 2;
@@ -1194,7 +1225,8 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
             }
             sc.Ss = s[1 + 2 * sc.ncomp]; sc.Se = s[2 + 2 * sc.ncomp];
             sc.Ah = s[3 + 2 * sc.ncomp] >> 4; sc.Al = s[3 + 2 * sc.ncomp] & 15;
-            if (sc.Ss > sc.Se || sc.Se > 63 || (sc.Ss == 0 && sc.Se != 0) || (sc.Ss > 0 && sc.ncomp != 1)) { rc = -16; break; }
+            if (!prog_scan_ok(&sc)) { rc = -16; break; }
+            note_coef_bits(coef_bits, &sc);
             for (int c = 0; c < 3; c++) if (!have_q[comp_tq[c]]) { rc = -14; goto done; }
             memcpy(info.qt[0], qtabs[comp_tq[0]], 128); memcpy(info.qt[1], qtabs[comp_tq[1]], 128);
             /* entropy-coded segment of this scan */
@@ -1205,17 +1237,18 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
             }
             if (e + 1 >= len) e = len;
             while (e > e0 && jpg[e - 1] == 0xFF) e--;   /* fill bytes before the marker */
-            bitr r = {jpg + e0, e - e0, 0, 0, 0, 0};
+            bitr r = {jpg + e0, e - e0, 0, 0, 0, 0, 0};
             dtbl dct[3], act[3];
             for (int i = 0; i < sc.ncomp; i++) {
                 make_dtbl(hb[0][sc.td[i]], hv[0][sc.td[i]], &dct[i]);
                 make_dtbl(hb[1][sc.ta[i]], hv[1][sc.ta[i]], &act[i]);
             }
             int pred[3] = {0, 0, 0}, eobrun = 0, togo = ri;
+            /* an MCU that starts after the data ran out (insufficient_data) is left alone */
             if (sc.ncomp > 1) {            /* interleaved: MCU order, every block of the MCU (padding blocks too) */
                 for (long long mi = 0; mi < (long long)g.mcux * g.mcuy; mi++) {
                     if (ri && togo == 0) { prog_restart(&r, pred, &eobrun); togo = ri; }
-                    for (int i = 0; i < sc.ncomp; i++) {
+                    for (int i = 0; i < sc.ncomp && !r.insufficient; i++) {
                         int c = sc.comp[i], nb = c ? 1 : g.hs * g.vs, b0 = c ? g.bpm - 3 + c : 0;
                         for (int b = 0; b < nb; b++)
                             prog_block(&r, &sc, i, &dct[i], &act[i], coef + ((size_t)mi * g.bpm + b0 + b) * 64, pred, &eobrun);
@@ -1227,7 +1260,8 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
                 for (int by = 0; by < g.hib[c]; by++)
                     for (int bx = 0; bx < g.wib[c]; bx++) {
                         if (ri && togo == 0) { prog_restart(&r, pred, &eobrun); togo = ri; }
-                        prog_block(&r, &sc, 0, &dct[0], &act[0], coef + block_index(&g, c, bx, by) * 64, pred, &eobrun);
+                        if (!r.insufficient)
+                            prog_block(&r, &sc, 0, &dct[0], &act[0], coef + block_index(&g, c, bx, by) * 64, pred, &eobrun);
                         if (ri) togo--;
                     }
             }
@@ -1236,7 +1270,12 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
         }
         p += L;
     }
+    if (rc == -15 && nscans > 0 && coef) rc = 0;   /* the data ended after a scan without EOI: jdatasrc.c inserts one */
 done:
+    if (rc == 0) {
+        const uint16_t *qt[3] = {qtabs[comp_tq[0]], qtabs[comp_tq[1]], qtabs[comp_tq[2]]};
+        rc = prog_smoothed((const int(*)[10])coef_bits, 3, 3, qt);
+    }
     if (rc == 0) rc = orc_inverse(coef, &info, bgr, step);
     free(coef);
     return rc;

@@ -112,12 +112,16 @@ int orc_encode_gray(const uint8_t *gray, size_t step, int W, int H, int quality,
     return 0;
 }
 
-static size_t scan_end(const uint8_t *jpg, size_t len, size_t e) {   /* first marker that is not RSTn / stuffed zero */
+/* the first marker that is not RSTn / stuffed zero, less the fill bytes (0xFF) in front of it */
+static size_t scan_end(const uint8_t *jpg, size_t len, size_t e0) {
+    size_t e = e0;
     while (e + 1 < len) {
-        if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
+        if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && jpg[e + 1] != 0xFF && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
         e++;
     }
-    return e + 1 >= len ? len : e;
+    if (e + 1 >= len) e = len;
+    while (e > e0 && jpg[e - 1] == 0xFF) e--;
+    return e;
 }
 
 /* Coefficients of the files orc_parse / orc_decode_progressive reject for having one component, and of progressive
@@ -129,7 +133,8 @@ static int other_coefs(const uint8_t *jpg, size_t len, int want, orc_geom *g, ui
     uint16_t qtabs[4][64]; int have_q[4] = {0, 0, 0, 0};
     static uint8_t hb[2][4][17], hv[2][4][256];
     memset(hb, 0, sizeof(hb)); memset(hv, 0, sizeof(hv));
-    int comp_id[3] = {-1, -1, -1}, comp_hv[3] = {0, 0, 0}, comp_tq[3] = {0, 0, 0}, ncomp = 0, ri = 0, sof = 0;
+    int comp_id[3] = {-1, -1, -1}, comp_hv[3] = {0, 0, 0}, comp_tq[3] = {0, 0, 0}, ncomp = 0, ri = 0, sof = 0, coef_bits[3][10];
+    memset(coef_bits, 0xFF, sizeof(coef_bits));
     int16_t *coef = NULL;
     size_t p = 2;
     int rc = -15;
@@ -201,7 +206,7 @@ static int other_coefs(const uint8_t *jpg, size_t len, int want, orc_geom *g, ui
             if (!have_q[comp_tq[0]]) { rc = -14; break; }
             memcpy(qt_out, qtabs[comp_tq[0]], 128);
             const size_t e0 = p + L, e = scan_end(jpg, len, e0);
-            bitr r = {jpg + e0, e - e0, 0, 0, 0, 0};
+            bitr r = {jpg + e0, e - e0, 0, 0, 0, 0, 0};
             dtbl dct[3], act[3];
             for (int i = 0; i < sc.ncomp; i++) {
                 make_dtbl(hb[0][sc.td[i]], hv[0][sc.td[i]], &dct[i]);
@@ -223,11 +228,13 @@ static int other_coefs(const uint8_t *jpg, size_t len, int want, orc_geom *g, ui
                     if (ri) togo--;
                 }
             } else {
-                if (sc.Ss > sc.Se || sc.Se > 63 || (sc.Ss == 0 && sc.Se != 0) || (sc.Ss > 0 && sc.ncomp != 1)) { rc = -16; break; }
+                if (!prog_scan_ok(&sc)) { rc = -16; break; }
+                note_coef_bits(coef_bits, &sc);
+                /* an MCU that starts after the data ran out (insufficient_data) is left alone */
                 if (sc.ncomp > 1) {        /* interleaved (three components): MCU order, every block of the MCU */
                     for (long long mi = 0; mi < (long long)g->mcux * g->mcuy; mi++) {
                         if (ri && togo == 0) { prog_restart(&r, pred, &eobrun); togo = ri; }
-                        for (int i = 0; i < sc.ncomp; i++) {
+                        for (int i = 0; i < sc.ncomp && !r.insufficient; i++) {
                             const int c = sc.comp[i], nb = c ? 1 : g->hs * g->vs, b0 = c ? g->bpm - 3 + c : 0;
                             for (int b = 0; b < nb; b++)
                                 prog_block(&r, &sc, i, &dct[i], &act[i], coef + ((size_t)mi * g->bpm + b0 + b) * 64, pred, &eobrun);
@@ -239,7 +246,8 @@ static int other_coefs(const uint8_t *jpg, size_t len, int want, orc_geom *g, ui
                     for (int by = 0; by < g->hib[c]; by++)
                         for (int bx = 0; bx < g->wib[c]; bx++) {
                             if (ri && togo == 0) { prog_restart(&r, pred, &eobrun); togo = ri; }
-                            prog_block(&r, &sc, 0, &dct[0], &act[0], coef + block_index(g, c, bx, by) * 64, pred, &eobrun);
+                            if (!r.insufficient)
+                                prog_block(&r, &sc, 0, &dct[0], &act[0], coef + block_index(g, c, bx, by) * 64, pred, &eobrun);
                             if (ri) togo--;
                         }
                 }
@@ -248,6 +256,11 @@ static int other_coefs(const uint8_t *jpg, size_t len, int want, orc_geom *g, ui
             continue;
         }
         p += L;
+    }
+    if (rc == -15 && sof == 0xC2 && coef) rc = 0;   /* a progressive file may end after a scan without EOI */
+    if (rc == 0 && sof == 0xC2 && want) {             /* on gray output only Y's history counts (jdcoefct.c) */
+        const uint16_t *qt[3] = {qtabs[comp_tq[0]], qtabs[comp_tq[1]], qtabs[comp_tq[2]]};
+        rc = prog_smoothed((const int(*)[10])coef_bits, ncomp, 1, qt);
     }
 done:
     if (rc == 0) *coef_out = coef;
