@@ -14,11 +14,13 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB = os.path.join(_HERE, "liborc.so")
 
 CSS = {"444": 0, "422": 1, "440": 2, "420": 3, "411": 4}
+CSS_GRAY = 6      # B2J_CSS_GRAY: one component
+SCALES = (2, 4, 8)
 
 
 def build(force=False):
-    src = os.path.join(_HERE, "jpeg_oracle.c")
-    if force or not os.path.exists(_LIB) or os.path.getmtime(_LIB) < os.path.getmtime(src):
+    newest = max(os.path.getmtime(os.path.join(_HERE, f)) for f in ("jpeg_oracle.c", "jpeg_oracle.h"))
+    if force or not os.path.exists(_LIB) or os.path.getmtime(_LIB) < newest:
         subprocess.check_call(["make", "-C", _HERE, "-s"] + (["-B"] if force else []))
     return _LIB
 
@@ -166,6 +168,25 @@ def encode(img, css, quality, optimize, restart_interval=0):
     return out[: n.value].copy()
 
 
+def encode_gray(img, quality, optimize, restart_interval=0):
+    """cv2.imencode(".jpg", gray, [QUALITY, OPTIMIZE(, RST_INTERVAL)]) of an (H, W) or (H, W, 1) uint8 image restated;
+    restart_interval in blocks (MCUs of the one-component scan)."""
+    img = np.asarray(img)
+    if img.ndim == 3 and img.shape[2] == 1:
+        img = img[:, :, 0]
+    if img.ndim != 2 or img.dtype != np.uint8 or img.strides[1] != 1:
+        img = np.ascontiguousarray(img, np.uint8)
+    H, W = img.shape
+    cap = W * H * 4 + 4096 + (2 * W * H // 64 if restart_interval else 0)
+    out = np.empty(cap, np.uint8)
+    n = C.c_size_t(0)
+    rc = lib().orc_encode_rst(_p(img), C.c_size_t(img.strides[0]), W, H, CSS_GRAY, int(quality), int(bool(optimize)),
+                              int(restart_interval), _p(out), C.c_size_t(cap), C.byref(n))
+    if rc:
+        raise RuntimeError(f"orc_encode_rst rc={rc}")
+    return out[: n.value].copy()
+
+
 def encode_progressive(img, css, quality):
     """cv2.imencode(..., IMWRITE_JPEG_PROGRESSIVE=1) restated (progressive mode always optimises its tables)."""
     img = np.ascontiguousarray(img)
@@ -200,17 +221,40 @@ def decode_coefs(jpg):
     return coef, info
 
 
-def decode(jpg):
+def reduced_size(W, H, denom):
+    """(W', H') of a decode at 1/denom: libjpeg's jdiv_round_up(W, denom)."""
+    return (W + denom - 1) // denom, (H + denom - 1) // denom
+
+
+def _decode(name, jpg, gray, *args):
+    """name(jpg, len, *args, out, step, &W, &H): first the output size, then the pixels"""
+    fn = getattr(lib(), name)
     jpg = np.ascontiguousarray(jpg, np.uint8)
     W, H = C.c_int(0), C.c_int(0)
-    rc = lib().orc_decode(_p(jpg), C.c_size_t(jpg.size), None, C.c_size_t(0), C.byref(W), C.byref(H))
+    rc = fn(_p(jpg), C.c_size_t(jpg.size), *args, None, C.c_size_t(0), C.byref(W), C.byref(H))
+    if not rc:
+        out = np.empty((H.value, W.value) + (() if gray else (3,)), np.uint8)
+        rc = fn(_p(jpg), C.c_size_t(jpg.size), *args, _p(out), C.c_size_t(out.strides[0]), C.byref(W), C.byref(H))
     if rc:
-        raise RuntimeError(f"orc_decode rc={rc}")
-    out = np.empty((H.value, W.value, 3), np.uint8)
-    rc = lib().orc_decode(_p(jpg), C.c_size_t(jpg.size), _p(out), C.c_size_t(W.value * 3), C.byref(W), C.byref(H))
-    if rc:
-        raise RuntimeError(f"orc_decode rc={rc}")
+        raise RuntimeError(f"{name} rc={rc}")
     return out
+
+
+def decode(jpg):
+    """cv2.imdecode(jpg, IMREAD_COLOR) as (H, W, 3) BGR"""
+    return _decode("orc_decode", jpg, False)
+
+
+def decode_gray(jpg):
+    """(H, W) uint8: cv2.imdecode(IMREAD_UNCHANGED) of a one-component file, IMREAD_GRAYSCALE (the Y plane) of a
+    three-component one."""
+    return _decode("orc_decode_output", jpg, True, 1, 1)
+
+
+def decode_scaled(jpg, denom, gray=False):
+    """cv2.imdecode(jpg, IMREAD_REDUCED_COLOR_denom) as (H', W', 3) BGR, or IMREAD_REDUCED_GRAYSCALE_denom as (H', W')
+    with gray=True (denom 1: IMREAD_COLOR / IMREAD_GRAYSCALE)."""
+    return _decode("orc_decode_output", jpg, gray, int(denom), int(bool(gray)))
 
 
 def diff(a, b, mode=0):

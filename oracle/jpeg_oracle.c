@@ -2,8 +2,8 @@
  * jpeg_oracle.c -- TEST INFRASTRUCTURE, NOT PRODUCT CODE (see jpeg_oracle.h).
  *
  * Plain-C restatement of libjpeg-turbo 3.1.2 baseline JPEG (DCT_ISLOW, fancy upsampling; restart intervals
- * in orc_encode_rst / the decoder; progressive mode in orc_encode_progressive / orc_decode_progressive) following
- * SURVEY.md Appendix A section by section. The reference repository contains no
+ * in orc_encode_rst / the decoder; progressive mode in orc_encode_progressive / the decoder; one-component files;
+ * gray and reduced-size output) following SURVEY.md Appendix A section by section. The reference repository contains no
  * JPEG arithmetic of its own (it calls nvjpegEncodeImage at ImageCompressorImpl.cu:280 and the
  * nvjpegDecodeJpeg* trio at :364-366); the north-star pins results to libjpeg-turbo instead.
  * Pinned by tests/test_oracle_golden.py (live cv2 = libjpeg-turbo 3.1.2) and tests/golden/.
@@ -64,16 +64,24 @@ static int clampi(int v, int lo, int hi) { return v < lo ? lo : (v > hi ? hi : v
 
 /* ------------------------------------------------------------------ geometry (jcmaster.c initial_setup / per_scan_setup) */
 
-int orc_geometry(int W, int H, int css, orc_geom *g) {
-    static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
-    if (W <= 0 || H <= 0 || css < 0 || css > 4) return -1;
+static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
+
+static int css_of(int hs, int vs) {
+    for (int i = 0; i < 5; i++) if (HS[i] == hs && VS[i] == vs) return i;
+    return -1;
+}
+
+/* css 0..4: three components, chroma 1x1; ORC_CSS_GRAY: one component, one block per MCU (a one-component scan is
+ * non-interleaved, so its sampling factors do not matter) */
+static void layout(int W, int H, int css, orc_geom *g) {
+    const int nc = css == ORC_CSS_GRAY ? 1 : 3;
     memset(g, 0, sizeof(*g));
     g->W = W; g->H = H; g->css = css;
-    g->hs = HS[css]; g->vs = VS[css];
+    g->hs = nc == 1 ? 1 : HS[css]; g->vs = nc == 1 ? 1 : VS[css];
     g->mcux = ceil_div(W, 8 * g->hs);
     g->mcuy = ceil_div(H, 8 * g->vs);
-    g->bpm = g->hs * g->vs + 2;
-    for (int c = 0; c < 3; c++) {
+    g->bpm = nc == 1 ? 1 : g->hs * g->vs + 2;
+    for (int c = 0; c < nc; c++) {
         int h = c ? 1 : g->hs, v = c ? 1 : g->vs;
         g->dw[c] = ceil_div(W * h, g->hs);
         g->dh[c] = ceil_div(H * v, g->vs);
@@ -81,6 +89,11 @@ int orc_geometry(int W, int H, int css, orc_geom *g) {
         g->hib[c] = ceil_div(g->dh[c], 8);
     }
     g->nblocks = (long long)g->mcux * g->mcuy * g->bpm;
+}
+
+int orc_geometry(int W, int H, int css, orc_geom *g) {
+    if (W <= 0 || H <= 0 || css < 0 || css > 4) return -1;
+    layout(W, H, css, g);
     return 0;
 }
 
@@ -270,6 +283,7 @@ int orc_forward(const uint8_t *bgr, size_t step, int W, int H, int css, int qual
 
 /* ------------------------------------------------------------------ scan-order helpers */
 
+/* bpm 1 (one component): every block is the last component's, so its tables are slots 2 / 3 (DC1 / AC1) */
 static int comp_of_block(int blkn, int bpm) { return blkn < bpm - 2 ? 0 : (blkn == bpm - 2 ? 1 : 2); }
 static int nbits_of(int v) { int a = v < 0 ? -v : v, n = 0; while (a) { n++; a >>= 1; } return n; }
 
@@ -410,128 +424,138 @@ size_t orc_stuff(const uint8_t *in, uint64_t nbits, uint8_t *out, size_t cap) {
 
 /* ------------------------------------------------------------------ A.8 markers (jcmarker.c) */
 
-static size_t headers_ri(int W, int H, int css, const uint16_t qt[2][64], const uint8_t bits[4][17],
-                         const uint8_t vals[4][256], int restart_interval, uint8_t *out, size_t cap) {
-    orc_geom g; if (orc_geometry(W, H, css, &g)) return 0;
-    uint8_t buf[2048]; size_t n = 0;
-#define PUT(b) buf[n++] = (uint8_t)(b)
-    PUT(0xFF); PUT(0xD8);
-    PUT(0xFF); PUT(0xE0); PUT(0); PUT(16); PUT('J'); PUT('F'); PUT('I'); PUT('F'); PUT(0); PUT(1); PUT(1); PUT(0);
-    PUT(0); PUT(1); PUT(0); PUT(1); PUT(0); PUT(0);
-    for (int t = 0; t < 2; t++) {
-        PUT(0xFF); PUT(0xDB); PUT(0); PUT(67); PUT(t);
-        for (int k = 0; k < 64; k++) PUT(qt[t][ZIGZAG[k]]);
+typedef struct { uint8_t *out; size_t n, cap; } bytew;   /* counts past cap without writing */
+static void put(bytew *w, int b) { if (w->n < w->cap) w->out[w->n] = (uint8_t)b; w->n++; }
+static void put16(bytew *w, int v) { put(w, v >> 8); put(w, v & 255); }
+
+/* SOI, JFIF APP0, one DQT per table in use, SOF (marker byte `sof`) with component ids 1, 2, 3 */
+static void put_frame(bytew *w, int sof, const orc_geom *g, const uint16_t qt[2][64]) {
+    static const uint8_t app0[18] = {0xFF, 0xE0, 0, 16, 'J', 'F', 'I', 'F', 0, 1, 1, 0, 0, 1, 0, 1, 0, 0};
+    const int nc = g->css == ORC_CSS_GRAY ? 1 : 3;
+    put16(w, 0xFFD8);
+    for (int i = 0; i < 18; i++) put(w, app0[i]);
+    for (int t = 0; t < (nc == 1 ? 1 : 2); t++) {
+        put16(w, 0xFFDB); put16(w, 67); put(w, t);
+        for (int k = 0; k < 64; k++) put(w, qt[t][ZIGZAG[k]]);
     }
-    PUT(0xFF); PUT(0xC0); PUT(0); PUT(17); PUT(8); PUT(H >> 8); PUT(H & 255); PUT(W >> 8); PUT(W & 255); PUT(3);
-    PUT(1); PUT((g.hs << 4) | g.vs); PUT(0);
-    PUT(2); PUT(0x11); PUT(1);
-    PUT(3); PUT(0x11); PUT(1);
-    static const uint8_t tc_th[4] = {0x00, 0x10, 0x01, 0x11};
-    for (int t = 0; t < 4; t++) {
-        int ns = 0; for (int l = 1; l <= 16; l++) ns += bits[t][l];
-        PUT(0xFF); PUT(0xC4); PUT((19 + ns) >> 8); PUT((19 + ns) & 255); PUT(tc_th[t]);
-        for (int l = 1; l <= 16; l++) PUT(bits[t][l]);
-        for (int i = 0; i < ns; i++) PUT(vals[t][i]);
-    }
-    if (restart_interval) { /* jcmarker.c write_scan_header: emit_dri after the scan's DHTs, before SOS */
-        PUT(0xFF); PUT(0xDD); PUT(0); PUT(4); PUT(restart_interval >> 8); PUT(restart_interval & 255);
-    }
-    PUT(0xFF); PUT(0xDA); PUT(0); PUT(12); PUT(3); PUT(1); PUT(0x00); PUT(2); PUT(0x11); PUT(3); PUT(0x11);
-    PUT(0); PUT(63); PUT(0);
-#undef PUT
-    if (n > cap) return 0;
-    memcpy(out, buf, n);
-    return n;
+    put16(w, 0xFF00 | sof); put16(w, 8 + 3 * nc); put(w, 8); put16(w, g->H); put16(w, g->W); put(w, nc);
+    for (int c = 0; c < nc; c++) { put(w, c + 1); put(w, c ? 0x11 : (g->hs << 4) | g->vs); put(w, c ? 1 : 0); }
+}
+static void put_dht(bytew *w, int tc_th, const uint8_t bits[17], const uint8_t *vals) {
+    int ns = 0; for (int l = 1; l <= 16; l++) ns += bits[l];
+    put16(w, 0xFFC4); put16(w, 19 + ns); put(w, tc_th);
+    for (int l = 1; l <= 16; l++) put(w, bits[l]);
+    for (int i = 0; i < ns; i++) put(w, vals[i]);
+}
+/* SOS of components comp[0..n-1] (ids comp + 1), table selector bytes sel[] */
+static void put_sos(bytew *w, int n, const int comp[], const int sel[], int Ss, int Se, int Ah_Al) {
+    put16(w, 0xFFDA); put16(w, 6 + 2 * n); put(w, n);
+    for (int i = 0; i < n; i++) { put(w, comp[i] + 1); put(w, sel[i]); }
+    put(w, Ss); put(w, Se); put(w, Ah_Al);
+}
+/* a one-scan baseline file: the frame, DHT DC0 AC0 (DC1 AC1) from bits / vals [0..3] ([0..1] for one component), DRI
+ * when there are restart intervals (write_scan_header: after the scan's DHTs, before SOS), SOS */
+static void put_baseline_headers(bytew *w, const orc_geom *g, const uint16_t qt[2][64], const uint8_t bits[][17],
+                                 const uint8_t vals[][256], int ri) {
+    static const int comp[3] = {0, 1, 2}, sel[3] = {0x00, 0x11, 0x11};
+    const int nc = g->css == ORC_CSS_GRAY ? 1 : 3;
+    put_frame(w, 0xC0, g, qt);
+    for (int t = 0; t < 2 * (nc == 1 ? 1 : 2); t++) put_dht(w, (t & 1) << 4 | t >> 1, bits[t], vals[t]);
+    if (ri) { put16(w, 0xFFDD); put16(w, 4); put16(w, ri); }
+    put_sos(w, nc, comp, sel, 0, 63, 0);
 }
 
 size_t orc_headers(int W, int H, int css, const uint16_t qt[2][64], const uint8_t bits[4][17],
                    const uint8_t vals[4][256], uint8_t *out, size_t cap) {
-    return headers_ri(W, H, css, qt, bits, vals, 0, out, cap);
+    orc_geom g; if (orc_geometry(W, H, css, &g)) return 0;
+    bytew w = {out, 0, cap};
+    put_baseline_headers(&w, &g, qt, bits, vals, 0);
+    return w.n > cap ? 0 : w.n;
+}
+
+/* one component (jccolor.c grayscale_convert): the samples as they stand, edges replicated to whole blocks
+ * (jcsample.c expand_right_edge, jcprepct.c), quantised with the luma table */
+static void forward_gray(const uint8_t *gray, size_t step, const orc_geom *g, const uint16_t qt[64], int16_t *coef) {
+    int nat[64]; uint8_t blk8[64];
+    for (int by = 0; by < g->mcuy; by++)
+        for (int bx = 0; bx < g->mcux; bx++) {
+            for (int r = 0; r < 8; r++)
+                for (int c = 0; c < 8; c++) {
+                    int y = by * 8 + r, x = bx * 8 + c;
+                    blk8[r * 8 + c] = gray[(size_t)(y < g->H ? y : g->H - 1) * step + (x < g->W ? x : g->W - 1)];
+                }
+            fdct_block(blk8, 8, nat);
+            int16_t *blk = coef + ((size_t)by * g->mcux + bx) * 64;
+            for (int k = 0; k < 64; k++) blk[k] = quantise(nat[ZIGZAG[k]], qt[ZIGZAG[k]]);
+        }
+}
+
+/* The baseline encoder, three components (BGR pixels) or one (gray samples, g->css == ORC_CSS_GRAY: the stream's DC0 /
+ * AC0 tables are slots 2 / 3 of orc_histogram and orc_entropy_bits). Restart intervals (jchuff.c
+ * emit_restart, jcmarker.c emit_dri): every `ri` MCUs (0 = none; a one-component MCU is one block) the bit buffer is
+ * flushed (1-padding to a byte boundary, stuffing applies to the padded byte), RSTn (n = 0..7 cycling) is written
+ * unstuffed and the DC predictors return to 0; no marker follows the last interval. Symbol statistics use the same
+ * predictor resets. */
+static int encode_baseline(const uint8_t *px, size_t step, const orc_geom *g, int quality, int optimize, int ri,
+                           uint8_t *out, size_t cap, size_t *len) {
+    if (g->W > 65535 || g->H > 65535 || ri < 0 || ri > 65535) return -1;
+    const int t0 = g->bpm == 1 ? 2 : 0;   /* the slots of the stream's tables: t0 .. 3 */
+    const long long nmcu = (long long)g->mcux * g->mcuy, iv = ri ? ri : nmcu;
+    int16_t *coef = (int16_t *)malloc((size_t)g->nblocks * 128);
+    uint8_t *raw = (uint8_t *)malloc((size_t)iv * g->bpm * 208 + 16);   /* worst case 64 coefs * 26 bits */
+    uint16_t qt[2][64]; orc_quant_tables(quality, qt);
+    uint8_t bits[4][17], vals[4][256];
+    memset(bits, 0, sizeof(bits)); memset(vals, 0, sizeof(vals));
+    int rc = coef && raw ? 0 : -2;
+    if (!rc) {
+        if (g->bpm == 1) forward_gray(px, step, g, qt[0], coef);
+        else rc = orc_forward(px, step, g->W, g->H, g->css, quality, coef);
+    }
+    if (!rc && optimize) {
+        uint32_t hist[4][257], h1[4][257];
+        memset(hist, 0, sizeof(hist));
+        for (long long m0 = 0; m0 < nmcu; m0 += iv) {
+            orc_histogram(coef + m0 * g->bpm * 64, (nmcu - m0 < iv ? nmcu - m0 : iv) * g->bpm, g->bpm, NULL, h1);
+            for (int t = 0; t < 4; t++) for (int i = 0; i < 257; i++) hist[t][i] += h1[t][i];
+        }
+        for (int t = t0; t < 4; t++) if (orc_gen_optimal_table(hist[t], bits[t], vals[t]) < 0) rc = -3;
+    } else if (!rc) {
+        for (int t = t0; t < 4; t++) orc_std_table(t - t0, bits[t], vals[t]);
+    }
+    bytew w = {out, 0, cap};
+    if (!rc) {
+        put_baseline_headers(&w, g, qt, (const uint8_t(*)[17])bits + t0, (const uint8_t(*)[256])vals + t0, ri);
+        if (w.n > cap) rc = -4;
+    }
+    size_t o = w.n;
+    int rstn = 0;
+    for (long long m0 = 0; !rc && m0 < nmcu; m0 += iv) {
+        uint64_t nbits = 0;
+        if (orc_entropy_bits(coef + m0 * g->bpm * 64, (nmcu - m0 < iv ? nmcu - m0 : iv) * g->bpm, g->bpm, NULL,
+                             (const uint8_t(*)[17])bits, (const uint8_t(*)[256])vals, raw, (size_t)iv * g->bpm * 208 + 16,
+                             &nbits)) { rc = -5; break; }
+        o += orc_stuff(raw, nbits, out + o, cap > o ? cap - o : 0);
+        if (o + 2 > cap) { rc = -6; break; }
+        if (m0 + iv < nmcu) { out[o++] = 0xFF; out[o++] = (uint8_t)(0xD0 + rstn); rstn = (rstn + 1) & 7; }
+    }
+    free(coef); free(raw);
+    if (rc) return rc;
+    out[o++] = 0xFF; out[o++] = 0xD9;
+    *len = o;
+    return 0;
 }
 
 int orc_encode(const uint8_t *bgr, size_t step, int W, int H, int css, int quality, int optimize, uint8_t *out,
                size_t cap, size_t *len) {
-    orc_geom g; if (orc_geometry(W, H, css, &g)) return -1;
-    if (W > 65535 || H > 65535) return -1;
-    int16_t *coef = (int16_t *)malloc((size_t)g.nblocks * 128);
-    if (!coef) return -2;
-    int rc = orc_forward(bgr, step, W, H, css, quality, coef);
-    if (rc) { free(coef); return rc; }
-    uint16_t qt[2][64]; orc_quant_tables(quality, qt);
-    uint8_t bits[4][17], vals[4][256];
-    if (optimize) {
-        uint32_t hist[4][257];
-        orc_histogram(coef, g.nblocks, g.bpm, NULL, hist);
-        for (int t = 0; t < 4; t++) if (orc_gen_optimal_table(hist[t], bits[t], vals[t]) < 0) { free(coef); return -3; }
-    } else {
-        for (int t = 0; t < 4; t++) orc_std_table(t, bits[t], vals[t]);
-    }
-    size_t hl = orc_headers(W, H, css, qt, bits, vals, out, cap);
-    if (!hl) { free(coef); return -4; }
-    size_t raw_cap = (size_t)g.nblocks * 208 + 16; /* worst case 64 coefs * 26 bits */
-    uint8_t *raw = (uint8_t *)malloc(raw_cap);
-    if (!raw) { free(coef); return -2; }
-    uint64_t nbits = 0;
-    rc = orc_entropy_bits(coef, g.nblocks, g.bpm, NULL, bits, vals, raw, raw_cap, &nbits);
-    free(coef);
-    if (rc) { free(raw); return -5; }
-    size_t sl = orc_stuff(raw, nbits, out + hl, cap - hl > 2 ? cap - hl - 2 : 0);
-    free(raw);
-    if (hl + sl + 2 > cap) return -6;
-    out[hl + sl] = 0xFF; out[hl + sl + 1] = 0xD9;
-    *len = hl + sl + 2;
-    return 0;
+    return orc_encode_rst(bgr, step, W, H, css, quality, optimize, 0, out, cap, len);
 }
 
-/* Restart intervals (jchuff.c emit_restart, jcmarker.c emit_dri): every `ri` MCUs the bit buffer is flushed (1-padding
- * to a byte boundary, stuffing applies to the padded byte), RSTn (n = 0..7 cycling) is written unstuffed and the DC
- * predictors return to 0; no marker follows the last interval. Symbol statistics use the same predictor resets. */
-int orc_encode_rst(const uint8_t *bgr, size_t step, int W, int H, int css, int quality, int optimize, int ri,
+int orc_encode_rst(const uint8_t *px, size_t step, int W, int H, int css, int quality, int optimize, int ri,
                    uint8_t *out, size_t cap, size_t *len) {
-    if (ri <= 0) return orc_encode(bgr, step, W, H, css, quality, optimize, out, cap, len);
-    if (ri > 65535) return -1;
-    orc_geom g; if (orc_geometry(W, H, css, &g)) return -1;
-    if (W > 65535 || H > 65535) return -1;
-    int16_t *coef = (int16_t *)malloc((size_t)g.nblocks * 128);
-    if (!coef) return -2;
-    int rc = orc_forward(bgr, step, W, H, css, quality, coef);
-    if (rc) { free(coef); return rc; }
-    uint16_t qt[2][64]; orc_quant_tables(quality, qt);
-    uint8_t bits[4][17], vals[4][256];
-    const long long nmcu = (long long)g.mcux * g.mcuy;
-    if (optimize) {
-        uint32_t hist[4][257], h1[4][257];
-        memset(hist, 0, sizeof(hist));
-        for (long long m0 = 0; m0 < nmcu; m0 += ri) {
-            long long nm = nmcu - m0 < ri ? nmcu - m0 : ri;
-            orc_histogram(coef + m0 * g.bpm * 64, nm * g.bpm, g.bpm, NULL, h1);
-            for (int t = 0; t < 4; t++) for (int i = 0; i < 257; i++) hist[t][i] += h1[t][i];
-        }
-        for (int t = 0; t < 4; t++) if (orc_gen_optimal_table(hist[t], bits[t], vals[t]) < 0) { free(coef); return -3; }
-    } else {
-        for (int t = 0; t < 4; t++) orc_std_table(t, bits[t], vals[t]);
-    }
-    size_t o = headers_ri(W, H, css, qt, bits, vals, ri, out, cap);
-    if (!o) { free(coef); return -4; }
-    size_t raw_cap = (size_t)ri * g.bpm * 208 + 16;
-    uint8_t *raw = (uint8_t *)malloc(raw_cap);
-    if (!raw) { free(coef); return -2; }
-    int rstn = 0;
-    for (long long m0 = 0; m0 < nmcu; m0 += ri) {
-        long long nm = nmcu - m0 < ri ? nmcu - m0 : ri;
-        uint64_t nbits = 0;
-        rc = orc_entropy_bits(coef + m0 * g.bpm * 64, nm * g.bpm, g.bpm, NULL, bits, vals, raw, raw_cap, &nbits);
-        if (rc) { free(coef); free(raw); return -5; }
-        size_t sl = orc_stuff(raw, nbits, out + o, cap > o ? cap - o : 0);
-        o += sl;
-        if (o + 2 > cap) { free(coef); free(raw); return -6; }
-        if (m0 + ri < nmcu) { out[o++] = 0xFF; out[o++] = (uint8_t)(0xD0 + rstn); rstn = (rstn + 1) & 7; }
-    }
-    free(coef); free(raw);
-    if (o + 2 > cap) return -6;
-    out[o++] = 0xFF; out[o++] = 0xD9;
-    *len = o;
-    return 0;
+    orc_geom g;
+    if (css == ORC_CSS_GRAY && W > 0 && H > 0) layout(W, H, css, &g);
+    else if (orc_geometry(W, H, css, &g)) return -1;
+    return encode_baseline(px, step, &g, quality, optimize, ri < 0 ? 0 : ri, out, cap, len);
 }
 
 /* scan parameters and the scan-order index of block (bx, by) of component c (shared by both progressive halves) */
@@ -677,19 +701,8 @@ int orc_encode_progressive(const uint8_t *bgr, size_t step, int W, int H, int cs
     int rc = orc_forward(bgr, step, W, H, css, quality, coef);
     if (rc) { free(coef); return rc; }
     uint16_t qt[2][64]; orc_quant_tables(quality, qt);
-    size_t n = 0;
-#define PUT(b) do { if (n < cap) out[n] = (uint8_t)(b); n++; } while (0)
-    PUT(0xFF); PUT(0xD8);
-    PUT(0xFF); PUT(0xE0); PUT(0); PUT(16); PUT('J'); PUT('F'); PUT('I'); PUT('F'); PUT(0); PUT(1); PUT(1); PUT(0);
-    PUT(0); PUT(1); PUT(0); PUT(1); PUT(0); PUT(0);
-    for (int t = 0; t < 2; t++) {
-        PUT(0xFF); PUT(0xDB); PUT(0); PUT(67); PUT(t);
-        for (int k = 0; k < 64; k++) PUT(qt[t][ZIGZAG[k]]);
-    }
-    PUT(0xFF); PUT(0xC2); PUT(0); PUT(17); PUT(8); PUT(H >> 8); PUT(H & 255); PUT(W >> 8); PUT(W & 255); PUT(3);
-    PUT(1); PUT((g.hs << 4) | g.vs); PUT(0);
-    PUT(2); PUT(0x11); PUT(1);
-    PUT(3); PUT(0x11); PUT(1);
+    bytew w = {out, 0, cap};
+    put_frame(&w, 0xC2, &g, qt);
     /* jcparam.c jpeg_simple_progression, YCbCr: {comps, Ss, Se, Ah, Al} */
     static const int script[10][5] = {{-1, 0, 0, 0, 1}, {0, 1, 5, 0, 2}, {2, 1, 63, 0, 1}, {1, 1, 63, 0, 1}, {0, 6, 63, 0, 2},
                                       {0, 1, 63, 2, 1}, {-1, 0, 0, 1, 0}, {2, 1, 63, 1, 0}, {1, 1, 63, 1, 0}, {0, 1, 63, 1, 0}};
@@ -714,140 +727,29 @@ int orc_encode_progressive(const uint8_t *bgr, size_t step, int W, int H, int cs
                 if (!used) continue;
                 if (orc_gen_optimal_table(cnt, bits[t], vals[t]) < 0) { free(coef); free(raw); free(e); return -3; }
                 orc_derive_codes(bits[t], vals[t], e->code[t], e->size[t]);
-                int ns = 0; for (int l = 1; l <= 16; l++) ns += bits[t][l];
-                PUT(0xFF); PUT(0xC4); PUT((19 + ns) >> 8); PUT((19 + ns) & 255); PUT((is_dc ? 0x00 : 0x10) | t);
-                for (int l = 1; l <= 16; l++) PUT(bits[t][l]);
-                for (int i = 0; i < ns; i++) PUT(vals[t][i]);
+                put_dht(&w, (is_dc ? 0x00 : 0x10) | t, bits[t], vals[t]);
             }
         }
-        PUT(0xFF); PUT(0xDA); PUT(0); PUT(6 + 2 * sc.ncomp); PUT(sc.ncomp);
-        for (int i = 0; i < sc.ncomp; i++) {
-            int c = sc.comp[i], t = c ? 1 : 0;
-            PUT(c + 1);
-            PUT(is_dc ? (sc.Ah == 0 ? (t << 4) : 0) : t);
-        }
-        PUT(sc.Ss); PUT(sc.Se); PUT((sc.Ah << 4) | sc.Al);
+        int sel[3];
+        for (int i = 0; i < sc.ncomp; i++) { int t = sc.comp[i] ? 1 : 0; sel[i] = is_dc ? (sc.Ah == 0 ? t << 4 : 0) : t; }
+        put_sos(&w, sc.ncomp, sc.comp, sel, sc.Ss, sc.Se, (sc.Ah << 4) | sc.Al);
         e->gather = 0;
         memset(raw, 0, raw_cap);
         e->w.out = raw; e->w.cap = raw_cap; e->w.nbits = 0; e->w.overflow = 0;
         p_scan(e, &g, coef, &sc, 0);
         if (e->w.overflow) { free(coef); free(raw); free(e); return -5; }
-        size_t sl = orc_stuff(raw, e->w.nbits, n < cap ? out + n : out, n < cap ? cap - n : 0);
-        n += sl;
+        w.n += orc_stuff(raw, e->w.nbits, w.n < cap ? out + w.n : out, w.n < cap ? cap - w.n : 0);
     }
-    PUT(0xFF); PUT(0xD9);
-#undef PUT
+    put16(&w, 0xFFD9);
     free(coef); free(raw); free(e);
-    if (n > cap) return -6;
-    *len = n;
+    if (w.n > cap) return -6;
+    *len = w.n;
     return 0;
 }
 
-/* ------------------------------------------------------------------ decoder: markers (jdmarker.c) */
+/* ------------------------------------------------------------------ decoder: Huffman (jdhuff.c) */
 
 static int rd16(const uint8_t *p) { return (p[0] << 8) | p[1]; }
-
-/* jdmarker.c get_interesting_appn: JFIF APP0 ("JFIF\0", 14+ bytes) and Adobe APP14 ("Adobe", 12+ bytes, transform in
- * byte 11); jdapimin.c default_decompress_parms then takes three components as RGB (no colour transform, which this
- * checker does not restate: such files are refused) for Adobe transform 0, or without either marker for ids R, G, B. */
-static void note_appn(int m, const uint8_t *s, int n, int *jfif, int *adobe) {
-    if (m == 0xE0 && n >= 14 && !memcmp(s, "JFIF", 5)) *jfif = 1;
-    if (m == 0xEE && n >= 12 && !memcmp(s, "Adobe", 5)) *adobe = s[11];
-}
-static int rgb_coded(int jfif, int adobe, const int id[3]) {
-    if (jfif) return 0;
-    if (adobe >= 0) return adobe == 0;
-    return id[0] == 'R' && id[1] == 'G' && id[2] == 'B';
-}
-
-int orc_parse(const uint8_t *jpg, size_t len, orc_info *info) {
-    memset(info, 0, sizeof(*info));
-    if (len < 4 || jpg[0] != 0xFF || jpg[1] != 0xD8) return -1;
-    uint16_t qtabs[4][64]; int have_q[4] = {0, 0, 0, 0};
-    uint8_t hb[2][4][17], hv[2][4][256]; memset(hb, 0, sizeof(hb)); memset(hv, 0, sizeof(hv));
-    int comp_id[3], comp_hv[3], comp_tq[3], ncomp = 0, jfif = 0, adobe = -1;
-    size_t p = 2;
-    while (p + 4 <= len) {
-        if (jpg[p] != 0xFF) return -2;
-        int m = jpg[p + 1];
-        if (m == 0xFF) { p++; continue; }
-        p += 2;
-        if (m == 0xD8 || (m >= 0xD0 && m <= 0xD7) || m == 0x01) continue;
-        if (m == 0xD9) return -3;
-        int L = rd16(jpg + p);
-        if (p + L > len) return -4;
-        const uint8_t *s = jpg + p + 2; int n = L - 2;
-        if (m == 0xDB) {
-            while (n > 0) {
-                int pq = s[0] >> 4, tq = s[0] & 15; s++; n--;
-                if (tq > 3) return -5;
-                for (int k = 0; k < 64; k++) {
-                    int v = pq ? rd16(s + 2 * k) : s[k];
-                    qtabs[tq][ZIGZAG[k]] = (uint16_t)v;
-                }
-                s += pq ? 128 : 64; n -= pq ? 128 : 64; have_q[tq] = 1;
-            }
-        } else if (m == 0xC0 || m == 0xC1) {
-            if (s[0] != 8) return -6;
-            info->H = rd16(s + 1); info->W = rd16(s + 3); ncomp = s[5];
-            if (ncomp != 3) return -7;
-            for (int c = 0; c < 3; c++) { comp_id[c] = s[6 + 3 * c]; comp_hv[c] = s[7 + 3 * c]; comp_tq[c] = s[8 + 3 * c]; }
-            if (comp_tq[0] > 3 || comp_tq[1] > 3 || comp_tq[2] > 3) return -14;
-        } else if (m == 0xC2 || (m >= 0xC5 && m <= 0xCF && m != 0xC4 && m != 0xC8 && m != 0xCC)) {
-            return -8; /* progressive / lossless / arithmetic: not baseline */
-        } else if (m == 0xC4) {
-            while (n > 0) {
-                int tc = s[0] >> 4, th = s[0] & 15; s++; n--;
-                if (tc > 1 || th > 3) return -9;
-                int ns = 0; hb[tc][th][0] = 0;
-                for (int l = 1; l <= 16; l++) { hb[tc][th][l] = s[l - 1]; ns += s[l - 1]; }
-                s += 16; n -= 16;
-                if (ns > 256) return -9;
-                memset(hv[tc][th], 0, 256); memcpy(hv[tc][th], s, ns); s += ns; n -= ns;
-            }
-        } else if (m == 0xDD) {
-            info->restart_interval = rd16(s);
-        } else if (m == 0xDA) {
-            if (ncomp != 3 || s[0] != 3) return -10;
-            if (rgb_coded(jfif, adobe, comp_id)) return -17;
-            int td[3], ta[3];
-            for (int c = 0; c < 3; c++) {
-                if (s[1 + 2 * c] != comp_id[c]) return -10;
-                td[c] = s[2 + 2 * c] >> 4; ta[c] = s[2 + 2 * c] & 15;
-            }
-            if (comp_hv[1] != 0x11 || comp_hv[2] != 0x11) return -11;
-            if (td[1] != td[2] || ta[1] != ta[2] || comp_tq[1] != comp_tq[2]) return -12;
-            info->hs = comp_hv[0] >> 4; info->vs = comp_hv[0] & 15;
-            static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
-            info->css = -1;
-            for (int i = 0; i < 5; i++) if (HS[i] == info->hs && VS[i] == info->vs) info->css = i;
-            if (info->css < 0) return -13;
-            if (!have_q[comp_tq[0]] || !have_q[comp_tq[1]]) return -14;
-            memcpy(info->qt[0], qtabs[comp_tq[0]], 128); memcpy(info->qt[1], qtabs[comp_tq[1]], 128);
-            memcpy(info->bits[0], hb[0][td[0]], 17); memcpy(info->vals[0], hv[0][td[0]], 256);
-            memcpy(info->bits[1], hb[1][ta[0]], 17); memcpy(info->vals[1], hv[1][ta[0]], 256);
-            memcpy(info->bits[2], hb[0][td[1]], 17); memcpy(info->vals[2], hv[0][td[1]], 256);
-            memcpy(info->bits[3], hb[1][ta[1]], 17); memcpy(info->vals[3], hv[1][ta[1]], 256);
-            info->scan_offset = p + L;
-            /* find end of entropy data: first marker that is not RSTn / stuffed zero */
-            size_t e = info->scan_offset;
-            while (e + 1 < len) {
-                if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && jpg[e + 1] != 0xFF && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
-                e++;
-            }
-            if (e + 1 >= len) e = len;
-            while (e > info->scan_offset && jpg[e - 1] == 0xFF) e--;   /* fill bytes before the marker */
-            info->scan_len = e - info->scan_offset;
-            return 0;
-        } else {
-            note_appn(m, s, n, &jfif, &adobe);
-        }
-        p += L;
-    }
-    return -15;
-}
-
-/* ------------------------------------------------------------------ decoder: Huffman (jdhuff.c) */
 
 typedef struct { int mincode[17], maxcode[18], valptr[17]; const uint8_t *vals; } dtbl;
 static void make_dtbl(const uint8_t bits[17], const uint8_t *vals, dtbl *t) {
@@ -891,172 +793,22 @@ static int decode_sym(bitr *r, const dtbl *t) {
 }
 static int extend(int v, int n) { return n == 0 ? 0 : (v < (1 << (n - 1)) ? v - (1 << n) + 1 : v); }
 
-int orc_decode_coefs(const uint8_t *jpg, size_t len, const orc_info *info, int16_t *coef) {
-    orc_geom g; if (orc_geometry(info->W, info->H, info->css, &g)) return -1;
-    dtbl t[4];
-    for (int i = 0; i < 4; i++) make_dtbl(info->bits[i], info->vals[i], &t[i]);
-    if (info->scan_offset + info->scan_len > len) return -2;
-    bitr r = {jpg + info->scan_offset, info->scan_len, 0, 0, 0, 0, 0};
-    memset(coef, 0, (size_t)g.nblocks * 128);
-    int pred[3] = {0, 0, 0};
-    long long nmcu = (long long)g.mcux * g.mcuy;
-    int ri = info->restart_interval, togo = ri;
-    for (long long m = 0; m < nmcu; m++) {
-        if (ri && togo == 0) { /* process restart marker */
-            r.cnt = 0;
-            while (!r.marker && r.pos + 1 < r.n && r.d[r.pos] == 0xFF && r.d[r.pos + 1] == 0xFF) r.pos++;   /* fill */
-            if (r.marker) { r.pos += 2; r.marker = 0; }
-            else if (r.pos + 1 < r.n && r.d[r.pos] == 0xFF && r.d[r.pos + 1] >= 0xD0 && r.d[r.pos + 1] <= 0xD7) r.pos += 2;
-            pred[0] = pred[1] = pred[2] = 0; togo = ri;
-        }
-        for (int blkn = 0; blkn < g.bpm; blkn++) {
-            int c = comp_of_block(blkn, g.bpm);
-            int16_t *blk = coef + (m * g.bpm + blkn) * 64;
-            int s = decode_sym(&r, &t[c ? 2 : 0]);
-            int diff = s ? extend(get_bits(&r, s), s) : 0;
-            pred[c] += diff; blk[0] = (int16_t)pred[c];
-            for (int k = 1; k < 64; k++) {
-                int rs = decode_sym(&r, &t[c ? 3 : 1]);
-                int rr = rs >> 4, ss = rs & 15;
-                if (ss) { k += rr; if (k > 63) break; blk[k] = (int16_t)extend(get_bits(&r, ss), ss); }
-                else { if (rr != 15) break; k += 15; }
-            }
-        }
-        if (ri) togo--;
+/* the end of a scan's entropy-coded data: the first marker that is not RSTn / stuffed zero, less the fill bytes (0xFF)
+ * in front of it */
+static size_t entropy_end(const uint8_t *jpg, size_t len, size_t e0) {
+    size_t e = e0;
+    while (e + 1 < len) {
+        if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && jpg[e + 1] != 0xFF && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
+        e++;
     }
-    return 0;
+    if (e + 1 >= len) e = len;
+    while (e > e0 && jpg[e - 1] == 0xFF) e--;
+    return e;
 }
 
-/* ------------------------------------------------------------------ A.9 IDCT (jidctint.c jpeg_idct_islow) */
-
-static void idct_1d(const int *in, int stride, int *out, int sh) {
-    int i0 = in[0], i1 = in[stride], i2 = in[2 * stride], i3 = in[3 * stride], i4 = in[4 * stride],
-        i5 = in[5 * stride], i6 = in[6 * stride], i7 = in[7 * stride];
-    int z1 = (i2 + i6) * F_0_541;
-    int t2 = z1 - i6 * F_1_847, t3 = z1 + i2 * F_0_765;
-    int t0 = (i0 + i4) << 13, t1 = (i0 - i4) << 13;
-    int t10 = t0 + t3, t13 = t0 - t3, t11 = t1 + t2, t12 = t1 - t2;
-    int a0 = i7, a1 = i5, a2 = i3, a3 = i1;
-    z1 = a0 + a3; int z2 = a1 + a2, z3 = a0 + a2, z4 = a1 + a3;
-    int z5 = (z3 + z4) * F_1_175;
-    a0 *= F_0_298; a1 *= F_2_053; a2 *= F_3_072; a3 *= F_1_501;
-    z1 *= -F_0_899; z2 *= -F_2_562; z3 = z3 * (-F_1_961) + z5; z4 = z4 * (-F_0_390) + z5;
-    a0 += z1 + z3; a1 += z2 + z4; a2 += z2 + z3; a3 += z1 + z4;
-    out[0] = DESCALE(t10 + a3, sh); out[7 * stride] = DESCALE(t10 - a3, sh);
-    out[stride] = DESCALE(t11 + a2, sh); out[6 * stride] = DESCALE(t11 - a2, sh);
-    out[2 * stride] = DESCALE(t12 + a1, sh); out[5 * stride] = DESCALE(t12 - a1, sh);
-    out[3 * stride] = DESCALE(t13 + a0, sh); out[4 * stride] = DESCALE(t13 - a0, sh);
-}
-
-static void idct_block(const int16_t *zz, const uint16_t *q, uint8_t *dst, int stride) {
-    int w[64];
-    for (int k = 0; k < 64; k++) w[ZIGZAG[k]] = (int)zz[k] * (int)q[ZIGZAG[k]];
-    for (int c = 0; c < 8; c++) idct_1d(w + c, 8, w + c, 11);
-    for (int r = 0; r < 8; r++) {
-        idct_1d(w + r * 8, 1, w + r * 8, 18);
-        for (int c = 0; c < 8; c++) dst[r * stride + c] = (uint8_t)clampi(w[r * 8 + c] + 128, 0, 255);
-    }
-}
-
-int orc_inverse(const int16_t *coef, const orc_info *info, uint8_t *bgr, size_t step) {
-    orc_geom g; if (orc_geometry(info->W, info->H, info->css, &g)) return -1;
-    int W = g.W, H = g.H;
-    /* per-component sample planes covering the whole MCU grid */
-    uint8_t *pl[3]; int pw[3], ph[3];
-    for (int c = 0; c < 3; c++) {
-        int h = c ? 1 : g.hs, v = c ? 1 : g.vs;
-        pw[c] = g.mcux * h * 8; ph[c] = g.mcuy * v * 8;
-        pl[c] = (uint8_t *)malloc((size_t)pw[c] * ph[c]); if (!pl[c]) return -2;
-    }
-    for (int my = 0; my < g.mcuy; my++)
-        for (int mx = 0; mx < g.mcux; mx++) {
-            const int16_t *mcu = coef + ((size_t)my * g.mcux + mx) * g.bpm * 64;
-            int blkn = 0;
-            for (int c = 0; c < 3; c++) {
-                int h = c ? 1 : g.hs, v = c ? 1 : g.vs;
-                for (int by = 0; by < v; by++)
-                    for (int bx = 0; bx < h; bx++, blkn++)
-                        idct_block(mcu + blkn * 64, info->qt[c ? 1 : 0],
-                                   pl[c] + (size_t)(my * v + by) * 8 * pw[c] + (size_t)(mx * h + bx) * 8, pw[c]);
-            }
-        }
-    /* upsample chroma to full resolution (jdsample.c), using the TRUE downsampled size */
-    uint8_t *up[3]; up[0] = NULL;
-    int hx = g.hs, vx = g.vs;
-    for (int c = 1; c < 3; c++) {
-        int dw = g.dw[c], dh = g.dh[c];
-        const uint8_t *in = pl[c]; int is = pw[c];
-        int ow = dw * hx, oh = dh * vx;
-        uint8_t *o = (uint8_t *)malloc((size_t)ow * oh); if (!o) return -2;
-        up[c] = o;
-#define IN(r, i) ((int)in[(size_t)(r) * is + (i)])
-        if (hx == 1 && vx == 1) {
-            for (int r = 0; r < dh; r++) memcpy(o + (size_t)r * ow, in + (size_t)r * is, dw);
-        } else if (hx == 2 && vx == 1) {
-            for (int r = 0; r < dh; r++) {
-                uint8_t *d = o + (size_t)r * ow;
-                if (dw > 2) { /* h2v1_fancy_upsample */
-                    for (int i = 0; i < dw; i++) {
-                        d[2 * i] = (uint8_t)(i == 0 ? IN(r, 0) : (3 * IN(r, i) + IN(r, i - 1) + 1) >> 2);
-                        d[2 * i + 1] = (uint8_t)(i == dw - 1 ? IN(r, dw - 1) : (3 * IN(r, i) + IN(r, i + 1) + 2) >> 2);
-                    }
-                } else for (int i = 0; i < dw; i++) d[2 * i] = d[2 * i + 1] = (uint8_t)IN(r, i);
-            }
-        } else if (hx == 1 && vx == 2) { /* h1v2_fancy_upsample */
-            for (int r = 0; r < dh; r++) {
-                int ra = r > 0 ? r - 1 : 0, rb = r < dh - 1 ? r + 1 : dh - 1;
-                for (int i = 0; i < dw; i++) {
-                    o[(size_t)(2 * r) * ow + i] = (uint8_t)((3 * IN(r, i) + IN(ra, i) + 1) >> 2);
-                    o[(size_t)(2 * r + 1) * ow + i] = (uint8_t)((3 * IN(r, i) + IN(rb, i) + 2) >> 2);
-                }
-            }
-        } else if (hx == 2 && vx == 2) {
-            if (dw > 2) { /* h2v2_fancy_upsample */
-                for (int r = 0; r < dh; r++)
-                    for (int half = 0; half < 2; half++) {
-                        int rn = half == 0 ? (r > 0 ? r - 1 : 0) : (r < dh - 1 ? r + 1 : dh - 1);
-                        uint8_t *d = o + (size_t)(2 * r + half) * ow;
-                        for (int i = 0; i < dw; i++) {
-                            int s = 3 * IN(r, i) + IN(rn, i);
-                            int sl = i > 0 ? 3 * IN(r, i - 1) + IN(rn, i - 1) : 0;
-                            int sr = i < dw - 1 ? 3 * IN(r, i + 1) + IN(rn, i + 1) : 0;
-                            d[2 * i] = (uint8_t)(i == 0 ? (4 * s + 8) >> 4 : (3 * s + sl + 8) >> 4);
-                            d[2 * i + 1] = (uint8_t)(i == dw - 1 ? (4 * s + 7) >> 4 : (3 * s + sr + 7) >> 4);
-                        }
-                    }
-            } else {
-                for (int r = 0; r < oh; r++)
-                    for (int i = 0; i < ow; i++) o[(size_t)r * ow + i] = (uint8_t)IN(r / 2, i / 2);
-            }
-        } else { /* int_upsample: replication */
-            for (int r = 0; r < oh; r++)
-                for (int i = 0; i < ow; i++) o[(size_t)r * ow + i] = (uint8_t)IN(r / vx, i / hx);
-        }
-#undef IN
-    }
-    /* colour (jdcolor.c ycc_rgb_convert) */
-    for (int y = 0; y < H; y++)
-        for (int x = 0; x < W; x++) {
-            int Y = pl[0][(size_t)y * pw[0] + x];
-            int cb = up[1][(size_t)y * (g.dw[1] * hx) + x] - 128, cr = up[2][(size_t)y * (g.dw[2] * hx) + x] - 128;
-            int r = Y + ((91881 * cr + 32768) >> 16);
-            int b = Y + ((116130 * cb + 32768) >> 16);
-            int gg = Y + ((-22554 * cb - 46802 * cr + 32768) >> 16);
-            uint8_t *p = bgr + (size_t)y * step + (size_t)x * 3;
-            p[0] = (uint8_t)clampi(b, 0, 255); p[1] = (uint8_t)clampi(gg, 0, 255); p[2] = (uint8_t)clampi(r, 0, 255);
-        }
-    for (int c = 0; c < 3; c++) free(pl[c]);
-    free(up[1]); free(up[2]);
-    return 0;
-}
-
-/* ------------------------------------------------------------------ progressive (SOF2) decode: jdphuff.c
- * What the reference as shipped writes (NVJPEG_ENCODING_PROGRESSIVE_DCT_HUFFMAN, ImageCompressorImpl.cu:28; SURVEY.md
- * 8f N4). All scans are absorbed into the coefficient array (jdapimin.c without buffered-image mode), then the baseline
- * back end (IDCT, upsampling, colour) runs: block smoothing never triggers on a complete file. */
-/* jdphuff.c process_restart. Where the data ends instead of an RSTn (a cut file), insufficient_data stays as it is: the
- * rest of the scan is left alone, except that an interval that ended cleanly lets the next one decode one MCU of zero
- * bits before it runs out */
+/* jdhuff.c / jdphuff.c process_restart. Where the data ends instead of an RSTn (a cut file), insufficient_data stays as
+ * it is: the rest of a progressive scan is left alone, except that an interval that ended cleanly lets the next one
+ * decode one MCU of zero bits before it runs out */
 static void prog_restart(bitr *r, int pred[3], int *eobrun) {
     r->cnt = 0;
     while (!r->marker && r->pos + 1 < r->n && r->d[r->pos] == 0xFF && r->d[r->pos + 1] == 0xFF) r->pos++;   /* fill */
@@ -1066,6 +818,23 @@ static void prog_restart(bitr *r, int pred[3], int *eobrun) {
     }
     pred[0] = pred[1] = pred[2] = 0; *eobrun = 0;
 }
+
+/* jdhuff.c decode_mcu, one block of a sequential scan */
+static void seq_block(bitr *r, const dtbl *dc, const dtbl *ac, int16_t *blk, int *pred) {
+    int s = decode_sym(r, dc);
+    *pred += s ? extend(get_bits(r, s), s) : 0;
+    blk[0] = (int16_t)*pred;
+    for (int k = 1; k < 64; k++) {
+        int rs = decode_sym(r, ac), rr = rs >> 4, ss = rs & 15;
+        if (ss) { k += rr; if (k > 63) break; blk[k] = (int16_t)extend(get_bits(r, ss), ss); }
+        else { if (rr != 15) break; k += 15; }
+    }
+}
+
+/* ------------------------------------------------------------------ progressive (SOF2) decode: jdphuff.c
+ * What the reference as shipped writes (NVJPEG_ENCODING_PROGRESSIVE_DCT_HUFFMAN, ImageCompressorImpl.cu:28; SURVEY.md
+ * 8f N4). All scans are absorbed into the coefficient array (jdapimin.c without buffered-image mode), then the common
+ * back end runs: block smoothing never triggers on a complete file. */
 
 /* jdphuff.c start_pass_phuff_decoder: scan parameters libjpeg accepts (a refinement refines by one bit), and coef_bits
  * (the Al of the last scan that sent each of zig-zag 0..9, -1: none yet) */
@@ -1147,17 +916,74 @@ static void prog_block(bitr *r, const pscan *sc, int ci, const dtbl *dc, const d
     }
 }
 
-int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t step, int *W, int *H) {
+/* One scan into the scan-order coefficient array. A sequential scan and an interleaved progressive one run in MCU
+ * order over every block of the MCU (padding blocks too), a one-component progressive scan in raster order over the
+ * component's own blocks (real data only). In a progressive scan an MCU that starts after the data ran out
+ * (insufficient_data) is left alone. dc[i] / ac[i]: the tables of the scan's i-th component. */
+static void decode_scan(bitr *r, const orc_geom *g, const pscan *sc, int prog, int ri, const dtbl *dc, const dtbl *ac,
+                        int16_t *coef) {
+    int pred[3] = {0, 0, 0}, eobrun = 0, togo = ri;
+    if (!prog || sc->ncomp > 1) {
+        for (long long mi = 0; mi < (long long)g->mcux * g->mcuy; mi++) {
+            if (ri && togo == 0) { prog_restart(r, pred, &eobrun); togo = ri; }
+            for (int i = 0; i < sc->ncomp && !(prog && r->insufficient); i++) {
+                int c = sc->comp[i], nb = c ? 1 : g->hs * g->vs, b0 = c ? g->bpm - 3 + c : 0;
+                for (int b = 0; b < nb; b++) {
+                    int16_t *blk = coef + ((size_t)mi * g->bpm + b0 + b) * 64;
+                    if (prog) prog_block(r, sc, i, &dc[i], &ac[i], blk, pred, &eobrun);
+                    else seq_block(r, &dc[i], &ac[i], blk, &pred[i]);
+                }
+            }
+            if (ri) togo--;
+        }
+    } else {
+        int c = sc->comp[0];
+        for (int by = 0; by < g->hib[c]; by++)
+            for (int bx = 0; bx < g->wib[c]; bx++) {
+                if (ri && togo == 0) { prog_restart(r, pred, &eobrun); togo = ri; }
+                if (!r->insufficient) prog_block(r, sc, 0, &dc[0], &ac[0], coef + block_index(g, c, bx, by) * 64, pred, &eobrun);
+                if (ri) togo--;
+            }
+    }
+}
+
+/* ------------------------------------------------------------------ decoder: the file reader (jdmarker.c) */
+
+/* jdmarker.c get_interesting_appn: JFIF APP0 ("JFIF\0", 14+ bytes) and Adobe APP14 ("Adobe", 12+ bytes, transform in
+ * byte 11); jdapimin.c default_decompress_parms then takes three components as RGB (no colour transform, which this
+ * checker does not restate: such files are refused) for Adobe transform 0, or without either marker for ids R, G, B. */
+static void note_appn(int m, const uint8_t *s, int n, int *jfif, int *adobe) {
+    if (m == 0xE0 && n >= 14 && !memcmp(s, "JFIF", 5)) *jfif = 1;
+    if (m == 0xEE && n >= 12 && !memcmp(s, "Adobe", 5)) *adobe = s[11];
+}
+static int rgb_coded(int jfif, int adobe, const int id[3]) {
+    if (jfif) return 0;
+    if (adobe >= 0) return adobe == 0;
+    return id[0] == 'R' && id[1] == 'G' && id[2] == 'B';
+}
+
+typedef struct {
+    orc_geom g;           /* three components: css 0..4; one: ORC_CSS_GRAY, laid out 1x1 whatever its SOF says */
+    int ncomp, sof;       /* 1 or 3; 0xC0 / 0xC1 (sequential) or 0xC2 (progressive) */
+    uint16_t qt[3][64];   /* natural order, per component, as the last scan found them */
+    int16_t *coef;        /* scan-order blocks of g, zig-zag order (malloc'ed) */
+} jfile;
+
+enum { READ_FRAME, READ_HEADERS, READ_ALL };
+
+/* The one marker walker: SOF0/1/2 with one or three components, DQT (8 and 16 bit), DHT, DRI, APP0/APP14 and every SOS.
+ * READ_FRAME stops after the SOF (a size query); READ_HEADERS stops at the first SOS of a three-component sequential
+ * file and describes it in *info (orc_parse); READ_ALL decodes every scan into f->coef and applies the smoothing rule to
+ * output components 0..nout-1. A three-component sequential file is what the product decodes: one interleaved scan,
+ * components in SOF order, chroma sharing their tables; nothing after that scan is read. */
+static int read_file(const uint8_t *jpg, size_t len, int upto, int nout, jfile *f, orc_info *info) {
+    memset(f, 0, sizeof(*f));
     if (len < 4 || jpg[0] != 0xFF || jpg[1] != 0xD8) return -1;
-    orc_info info; memset(&info, 0, sizeof(info));
     uint16_t qtabs[4][64]; int have_q[4] = {0, 0, 0, 0};
-    static uint8_t hb[2][4][17], hv[2][4][256];
+    uint8_t hb[2][4][17], hv[2][4][256];
     memset(hb, 0, sizeof(hb)); memset(hv, 0, sizeof(hv));
-    int comp_id[3] = {0, 0, 0}, comp_hv[3] = {0, 0, 0}, comp_tq[3] = {0, 0, 0}, ncomp = 0, ri = 0, have_sof = 0;
-    int jfif = 0, adobe = -1, nscans = 0, coef_bits[3][10];
-    memset(coef_bits, 0xFF, sizeof(coef_bits));
-    orc_geom g; memset(&g, 0, sizeof(g));
-    int16_t *coef = NULL;
+    int id[3] = {-1, -1, -1}, tq[3] = {0, 0, 0}, seq3 = 0, ri = 0, jfif = 0, adobe = -1, nscans = 0, cb[3][10];
+    memset(cb, 0xFF, sizeof(cb));
     size_t p = 2;
     int rc = -15;
     while (p + 2 <= len) {
@@ -1166,38 +992,40 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
         if (m == 0xFF) { p++; continue; }
         p += 2;
         if (m == 0xD8 || (m >= 0xD0 && m <= 0xD7) || m == 0x01) continue;
-        if (m == 0xD9) { rc = have_sof && coef ? 0 : -3; break; }
+        if (m == 0xD9) { rc = f->coef && !seq3 ? 0 : -3; break; }
         if (p + 2 > len) { rc = -4; break; }
         int L = rd16(jpg + p);
-        if (p + L > len) { rc = -4; break; }
+        if (L < 2 || p + L > len) { rc = -4; break; }
         const uint8_t *s = jpg + p + 2; int n = L - 2;
         if (m == 0xDB) {
             while (n > 0) {
-                int pq = s[0] >> 4, tq = s[0] & 15; s++; n--;
-                if (tq > 3) { rc = -5; goto done; }
-                for (int k = 0; k < 64; k++) qtabs[tq][ZIGZAG[k]] = (uint16_t)(pq ? rd16(s + 2 * k) : s[k]);
-                s += pq ? 128 : 64; n -= pq ? 128 : 64; have_q[tq] = 1;
+                int pq = s[0] >> 4, t = s[0] & 15; s++; n--;
+                if (t > 3) { rc = -5; goto done; }
+                for (int k = 0; k < 64; k++) qtabs[t][ZIGZAG[k]] = (uint16_t)(pq ? rd16(s + 2 * k) : s[k]);
+                s += pq ? 128 : 64; n -= pq ? 128 : 64; have_q[t] = 1;
             }
-        } else if (m == 0xC2) {
-            if (s[0] != 8) { rc = -6; break; }
-            info.H = rd16(s + 1); info.W = rd16(s + 3); ncomp = s[5];
-            if (ncomp != 3) { rc = -7; break; }
-            for (int c = 0; c < 3; c++) { comp_id[c] = s[6 + 3 * c]; comp_hv[c] = s[7 + 3 * c]; comp_tq[c] = s[8 + 3 * c]; }
-            if (comp_hv[1] != 0x11 || comp_hv[2] != 0x11 || comp_tq[1] != comp_tq[2]) { rc = -11; break; }
-            if (comp_tq[0] > 3 || comp_tq[1] > 3) { rc = -14; break; }
-            info.hs = comp_hv[0] >> 4; info.vs = comp_hv[0] & 15;
-            static const int HS[5] = {1, 2, 1, 2, 4}, VS[5] = {1, 1, 2, 2, 1};
-            info.css = -1;
-            for (int i = 0; i < 5; i++) if (HS[i] == info.hs && VS[i] == info.vs) info.css = i;
-            if (info.css < 0 || orc_geometry(info.W, info.H, info.css, &g)) { rc = -13; break; }
-            if (W) *W = info.W;
-            if (H) *H = info.H;
-            if (!bgr) return 0;
-            coef = (int16_t *)calloc((size_t)g.nblocks * 64, 2);
-            if (!coef) return -2;
-            have_sof = 1;
-        } else if (m == 0xC0 || m == 0xC1) {
-            rc = -8; break;   /* not progressive: orc_decode handles it */
+        } else if (m == 0xC0 || m == 0xC1 || m == 0xC2) {
+            if (f->sof || s[0] != 8) { rc = -6; break; }
+            int nc = s[5], H = rd16(s + 1), W = rd16(s + 3), samp[3] = {0, 0, 0}, css = ORC_CSS_GRAY;
+            if (nc != 1 && nc != 3) { rc = -7; break; }
+            for (int c = 0; c < nc; c++) {
+                id[c] = s[6 + 3 * c]; samp[c] = s[7 + 3 * c]; tq[c] = s[8 + 3 * c];
+                if (tq[c] > 3) { rc = -14; goto done; }
+            }
+            if (W <= 0 || H <= 0) { rc = -13; break; }
+            if (nc == 3) {
+                if (samp[1] != 0x11 || samp[2] != 0x11 || tq[1] != tq[2]) { rc = -11; break; }
+                css = css_of(samp[0] >> 4, samp[0] & 15);
+                if (css < 0) { rc = -13; break; }
+            }
+            seq3 = m != 0xC2 && nc == 3;
+            if (upto == READ_HEADERS && !seq3) { rc = m == 0xC2 ? -8 : -7; break; }
+            f->ncomp = nc; f->sof = m;
+            layout(W, H, css, &f->g);
+            if (upto == READ_FRAME) return 0;
+            if (upto == READ_ALL && !(f->coef = (int16_t *)calloc((size_t)f->g.nblocks * 64, 2))) { rc = -2; break; }
+        } else if (m >= 0xC3 && m <= 0xCF && m != 0xC4 && m != 0xC8 && m != 0xCC) {
+            rc = -8; break;   /* lossless / arithmetic */
         } else if (m == 0xC4) {
             while (n > 0) {
                 int tc = s[0] >> 4, th = s[0] & 15; s++; n--;
@@ -1210,92 +1038,298 @@ int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t 
             }
         } else if (m == 0xDD) {
             ri = rd16(s);
-        } else if (m != 0xDA) {
-            note_appn(m, s, n, &jfif, &adobe);
-        } else {
-            if (!have_sof) { rc = -10; break; }
-            if (nscans++ == 0 && rgb_coded(jfif, adobe, comp_id)) { rc = -17; break; }
-            pscan sc; sc.ncomp = s[0];
-            if (sc.ncomp < 1 || sc.ncomp > 3) { rc = -10; break; }
+        } else if (m == 0xDA) {
+            if (!f->sof) { rc = -10; break; }
+            if (nscans++ == 0 && f->ncomp == 3 && rgb_coded(jfif, adobe, id)) { rc = -17; break; }
+            pscan sc; memset(&sc, 0, sizeof(sc));
+            sc.ncomp = s[0];
+            if (sc.ncomp < 1 || sc.ncomp > f->ncomp) { rc = -10; break; }
             for (int i = 0; i < sc.ncomp; i++) {
-                int id = s[1 + 2 * i]; sc.comp[i] = -1;
-                for (int c = 0; c < 3; c++) if (comp_id[c] == id) sc.comp[i] = c;
-                if (sc.comp[i] < 0) { rc = -10; goto done; }
+                sc.comp[i] = -1;
+                for (int c = 0; c < f->ncomp; c++) if (id[c] == s[1 + 2 * i]) sc.comp[i] = c;
                 sc.td[i] = s[2 + 2 * i] >> 4; sc.ta[i] = s[2 + 2 * i] & 15;
+                if (sc.comp[i] < 0 || sc.td[i] > 3 || sc.ta[i] > 3) { rc = -10; goto done; }
             }
             sc.Ss = s[1 + 2 * sc.ncomp]; sc.Se = s[2 + 2 * sc.ncomp];
             sc.Ah = s[3 + 2 * sc.ncomp] >> 4; sc.Al = s[3 + 2 * sc.ncomp] & 15;
-            if (!prog_scan_ok(&sc)) { rc = -16; break; }
-            note_coef_bits(coef_bits, &sc);
-            for (int c = 0; c < 3; c++) if (!have_q[comp_tq[c]]) { rc = -14; goto done; }
-            memcpy(info.qt[0], qtabs[comp_tq[0]], 128); memcpy(info.qt[1], qtabs[comp_tq[1]], 128);
-            /* entropy-coded segment of this scan */
-            size_t e0 = p + L, e = e0;
-            while (e + 1 < len) {
-                if (jpg[e] == 0xFF && jpg[e + 1] != 0x00 && jpg[e + 1] != 0xFF && !(jpg[e + 1] >= 0xD0 && jpg[e + 1] <= 0xD7)) break;
-                e++;
+            if (seq3) {
+                if (sc.ncomp != 3 || sc.comp[0] != 0 || sc.comp[1] != 1 || sc.comp[2] != 2) { rc = -10; break; }
+                if (sc.td[1] != sc.td[2] || sc.ta[1] != sc.ta[2]) { rc = -12; break; }
             }
-            if (e + 1 >= len) e = len;
-            while (e > e0 && jpg[e - 1] == 0xFF) e--;   /* fill bytes before the marker */
+            if (f->sof == 0xC2) {
+                if (!prog_scan_ok(&sc)) { rc = -16; break; }
+                note_coef_bits(cb, &sc);
+            }
+            for (int c = 0; c < f->ncomp; c++) {
+                if (!have_q[tq[c]]) { rc = -14; goto done; }
+                memcpy(f->qt[c], qtabs[tq[c]], 128);
+            }
+            size_t e0 = p + L, e = entropy_end(jpg, len, e0);
+            if (upto == READ_HEADERS) {
+                info->W = f->g.W; info->H = f->g.H; info->css = f->g.css; info->hs = f->g.hs; info->vs = f->g.vs;
+                info->restart_interval = ri; info->scan_offset = e0; info->scan_len = e - e0;
+                memcpy(info->qt, f->qt, sizeof(info->qt));
+                for (int t = 0; t < 4; t++) {   /* DC0, AC0, DC1, AC1 */
+                    int sel = t & 1 ? sc.ta[t >> 1] : sc.td[t >> 1];
+                    memcpy(info->bits[t], hb[t & 1][sel], 17); memcpy(info->vals[t], hv[t & 1][sel], 256);
+                }
+                return 0;
+            }
             bitr r = {jpg + e0, e - e0, 0, 0, 0, 0, 0};
             dtbl dct[3], act[3];
             for (int i = 0; i < sc.ncomp; i++) {
                 make_dtbl(hb[0][sc.td[i]], hv[0][sc.td[i]], &dct[i]);
                 make_dtbl(hb[1][sc.ta[i]], hv[1][sc.ta[i]], &act[i]);
             }
-            int pred[3] = {0, 0, 0}, eobrun = 0, togo = ri;
-            /* an MCU that starts after the data ran out (insufficient_data) is left alone */
-            if (sc.ncomp > 1) {            /* interleaved: MCU order, every block of the MCU (padding blocks too) */
-                for (long long mi = 0; mi < (long long)g.mcux * g.mcuy; mi++) {
-                    if (ri && togo == 0) { prog_restart(&r, pred, &eobrun); togo = ri; }
-                    for (int i = 0; i < sc.ncomp && !r.insufficient; i++) {
-                        int c = sc.comp[i], nb = c ? 1 : g.hs * g.vs, b0 = c ? g.bpm - 3 + c : 0;
-                        for (int b = 0; b < nb; b++)
-                            prog_block(&r, &sc, i, &dct[i], &act[i], coef + ((size_t)mi * g.bpm + b0 + b) * 64, pred, &eobrun);
-                    }
-                    if (ri) togo--;
-                }
-            } else {                       /* one component: raster order over its own blocks (real data only) */
-                int c = sc.comp[0];
-                for (int by = 0; by < g.hib[c]; by++)
-                    for (int bx = 0; bx < g.wib[c]; bx++) {
-                        if (ri && togo == 0) { prog_restart(&r, pred, &eobrun); togo = ri; }
-                        if (!r.insufficient)
-                            prog_block(&r, &sc, 0, &dct[0], &act[0], coef + block_index(&g, c, bx, by) * 64, pred, &eobrun);
-                        if (ri) togo--;
-                    }
-            }
+            decode_scan(&r, &f->g, &sc, f->sof == 0xC2, ri, dct, act, f->coef);
+            if (seq3) { rc = 0; break; }
             p = e;
             continue;
+        } else {
+            note_appn(m, s, n, &jfif, &adobe);
         }
         p += L;
     }
-    if (rc == -15 && nscans > 0 && coef) rc = 0;   /* the data ended after a scan without EOI: jdatasrc.c inserts one */
-done:
-    if (rc == 0) {
-        const uint16_t *qt[3] = {qtabs[comp_tq[0]], qtabs[comp_tq[1]], qtabs[comp_tq[2]]};
-        rc = prog_smoothed((const int(*)[10])coef_bits, 3, 3, qt);
+    /* the data ended after a scan without EOI: jdatasrc.c inserts one */
+    if (rc == -15 && f->sof == 0xC2 && f->coef && nscans > 0) rc = 0;
+    if (rc == 0 && f->sof == 0xC2) {
+        const uint16_t *q[3] = {qtabs[tq[0]], qtabs[tq[1]], qtabs[tq[2]]};
+        rc = prog_smoothed((const int(*)[10])cb, f->ncomp, nout, q);
     }
-    if (rc == 0) rc = orc_inverse(coef, &info, bgr, step);
-    free(coef);
+done:
+    if (rc) { free(f->coef); f->coef = NULL; }
+    return rc;
+}
+
+int orc_parse(const uint8_t *jpg, size_t len, orc_info *info) {
+    jfile f;
+    memset(info, 0, sizeof(*info));
+    return read_file(jpg, len, READ_HEADERS, 3, &f, info);
+}
+
+int orc_decode_coefs(const uint8_t *jpg, size_t len, const orc_info *info, int16_t *coef) {
+    orc_geom g; if (orc_geometry(info->W, info->H, info->css, &g)) return -1;
+    if (info->scan_offset + info->scan_len > len) return -2;
+    dtbl dc[3], ac[3];
+    for (int c = 0; c < 3; c++) {
+        make_dtbl(info->bits[c ? 2 : 0], info->vals[c ? 2 : 0], &dc[c]);
+        make_dtbl(info->bits[c ? 3 : 1], info->vals[c ? 3 : 1], &ac[c]);
+    }
+    pscan sc = {3, {0, 1, 2}, {0, 0, 0}, {0, 0, 0}, 0, 63, 0, 0};
+    bitr r = {jpg + info->scan_offset, info->scan_len, 0, 0, 0, 0, 0};
+    memset(coef, 0, (size_t)g.nblocks * 128);
+    decode_scan(&r, &g, &sc, 0, info->restart_interval, dc, ac, coef);
+    return 0;
+}
+
+/* ------------------------------------------------------------------ A.9 back end: IDCT (jidctint.c jpeg_idct_islow,
+ * jidctred.c), upsampling (jdsample.c), colour (jdcolor.c) */
+
+static void idct_1d(const int *in, int stride, int *out, int sh) {
+    int i0 = in[0], i1 = in[stride], i2 = in[2 * stride], i3 = in[3 * stride], i4 = in[4 * stride],
+        i5 = in[5 * stride], i6 = in[6 * stride], i7 = in[7 * stride];
+    int z1 = (i2 + i6) * F_0_541;
+    int t2 = z1 - i6 * F_1_847, t3 = z1 + i2 * F_0_765;
+    int t0 = (i0 + i4) << 13, t1 = (i0 - i4) << 13;
+    int t10 = t0 + t3, t13 = t0 - t3, t11 = t1 + t2, t12 = t1 - t2;
+    int a0 = i7, a1 = i5, a2 = i3, a3 = i1;
+    z1 = a0 + a3; int z2 = a1 + a2, z3 = a0 + a2, z4 = a1 + a3;
+    int z5 = (z3 + z4) * F_1_175;
+    a0 *= F_0_298; a1 *= F_2_053; a2 *= F_3_072; a3 *= F_1_501;
+    z1 *= -F_0_899; z2 *= -F_2_562; z3 = z3 * (-F_1_961) + z5; z4 = z4 * (-F_0_390) + z5;
+    a0 += z1 + z3; a1 += z2 + z4; a2 += z2 + z3; a3 += z1 + z4;
+    out[0] = DESCALE(t10 + a3, sh); out[7 * stride] = DESCALE(t10 - a3, sh);
+    out[stride] = DESCALE(t11 + a2, sh); out[6 * stride] = DESCALE(t11 - a2, sh);
+    out[2 * stride] = DESCALE(t12 + a1, sh); out[5 * stride] = DESCALE(t12 - a1, sh);
+    out[3 * stride] = DESCALE(t13 + a0, sh); out[4 * stride] = DESCALE(t13 - a0, sh);
+}
+
+static void idct_block(const int16_t *zz, const uint16_t *q, uint8_t *dst, int stride) {
+    int w[64];
+    for (int k = 0; k < 64; k++) w[ZIGZAG[k]] = (int)zz[k] * (int)q[ZIGZAG[k]];
+    for (int c = 0; c < 8; c++) idct_1d(w + c, 8, w + c, 11);
+    for (int r = 0; r < 8; r++) {
+        idct_1d(w + r * 8, 1, w + r * 8, 18);
+        for (int c = 0; c < 8; c++) dst[r * stride + c] = (uint8_t)clampi(w[r * 8 + c] + 128, 0, 255);
+    }
+}
+
+/* k x k samples of one block: jidctint.c's 8 x 8, jidctred.c jpeg_idct_4x4 / 2x2 / 1x1 */
+static void idct_scaled(const int16_t *zz, const uint16_t *q, int k, uint8_t *dst, int stride) {
+    if (k == 8) { idct_block(zz, q, dst, stride); return; }
+    int x[64], ws[64];
+    for (int i = 0; i < 64; i++) x[ZIGZAG[i]] = (int)zz[i] * (int)q[ZIGZAG[i]];
+    if (k == 1) { dst[0] = (uint8_t)clampi(DESCALE(x[0], 3) + 128, 0, 255); return; }
+    if (k == 2) {
+        for (int c = 0; c < 8; c++) {   /* columns 2, 4, 6 are never read */
+            const int *in = x + c;
+            const int t10 = in[0] << 15;
+            const int t0 = -5906 * in[56] + 6967 * in[40] - 10426 * in[24] + 29692 * in[8];
+            ws[c] = DESCALE(t10 + t0, 13);
+            ws[8 + c] = DESCALE(t10 - t0, 13);
+        }
+        for (int r = 0; r < 2; r++) {
+            const int *w = ws + 8 * r;
+            const int t10 = w[0] << 15;
+            const int t0 = -5906 * w[7] + 6967 * w[5] - 10426 * w[3] + 29692 * w[1];
+            dst[r * stride] = (uint8_t)clampi(DESCALE(t10 + t0, 20) + 128, 0, 255);
+            dst[r * stride + 1] = (uint8_t)clampi(DESCALE(t10 - t0, 20) + 128, 0, 255);
+        }
+        return;
+    }
+    /* k == 4: row / column 4 is never read */
+    for (int pass = 0; pass < 2; pass++) {
+        const int n = pass ? 4 : 8, sh = pass ? 19 : 12;
+        for (int i = 0; i < n; i++) {
+            int v[8];
+            for (int j = 0; j < 8; j++) v[j] = pass ? ws[i * 8 + j] : x[j * 8 + i];
+            const int t0e = v[0] << 14, t2e = 15137 * v[2] - 6270 * v[6];
+            const int t10 = t0e + t2e, t12 = t0e - t2e;
+            const int z1 = v[7], z2 = v[5], z3 = v[3], z4 = v[1];
+            const int t0 = -1730 * z1 + 11893 * z2 - 17799 * z3 + 8697 * z4;
+            const int t2 = -4176 * z1 - 4926 * z2 + 7373 * z3 + 20995 * z4;
+            const int o[4] = {DESCALE(t10 + t2, sh), DESCALE(t12 + t0, sh), DESCALE(t12 - t0, sh), DESCALE(t10 - t2, sh)};
+            for (int j = 0; j < 4; j++) {
+                if (pass) dst[i * stride + j] = (uint8_t)clampi(o[j] + 128, 0, 255);
+                else ws[j * 8 + i] = o[j];
+            }
+        }
+    }
+}
+
+/* jdmaster.c: chroma DCT output size for luma size S */
+static int chroma_size(int hs, int vs, int S) {
+    int sc = S;
+    while (sc < 8 && (hs * S) % (2 * sc) == 0 && (vs * S) % (2 * sc) == 0) sc *= 2;
+    return sc;
+}
+
+/* jdsample.c: a plane of true size dw x dh (row pitch is) expanded hx x vx into o (row pitch dw * hx). The fancy
+ * (triangle) filters run only when the chroma output size is above 1 (do_fancy), h2v1 / h2v2 only on planes wider than
+ * 2 samples; everything else is replication (fullsize, int_upsample). */
+static void upsample(const uint8_t *in, int is, int dw, int dh, int hx, int vx, int fancy, uint8_t *o) {
+    const int ow = dw * hx, oh = dh * vx;
+#define IN(r, i) ((int)in[(size_t)(r) * is + (i)])
+    if (hx == 2 && vx == 1 && fancy && dw > 2) {          /* h2v1_fancy_upsample */
+        for (int r = 0; r < dh; r++) {
+            uint8_t *d = o + (size_t)r * ow;
+            for (int i = 0; i < dw; i++) {
+                d[2 * i] = (uint8_t)(i == 0 ? IN(r, 0) : (3 * IN(r, i) + IN(r, i - 1) + 1) >> 2);
+                d[2 * i + 1] = (uint8_t)(i == dw - 1 ? IN(r, dw - 1) : (3 * IN(r, i) + IN(r, i + 1) + 2) >> 2);
+            }
+        }
+    } else if (hx == 1 && vx == 2 && fancy) {             /* h1v2_fancy_upsample */
+        for (int r = 0; r < dh; r++) {
+            int ra = r > 0 ? r - 1 : 0, rb = r < dh - 1 ? r + 1 : dh - 1;
+            for (int i = 0; i < dw; i++) {
+                o[(size_t)(2 * r) * ow + i] = (uint8_t)((3 * IN(r, i) + IN(ra, i) + 1) >> 2);
+                o[(size_t)(2 * r + 1) * ow + i] = (uint8_t)((3 * IN(r, i) + IN(rb, i) + 2) >> 2);
+            }
+        }
+    } else if (hx == 2 && vx == 2 && fancy && dw > 2) {   /* h2v2_fancy_upsample */
+        for (int r = 0; r < dh; r++)
+            for (int half = 0; half < 2; half++) {
+                int rn = half == 0 ? (r > 0 ? r - 1 : 0) : (r < dh - 1 ? r + 1 : dh - 1);
+                uint8_t *d = o + (size_t)(2 * r + half) * ow;
+                for (int i = 0; i < dw; i++) {
+                    int s = 3 * IN(r, i) + IN(rn, i);
+                    int sl = i > 0 ? 3 * IN(r, i - 1) + IN(rn, i - 1) : 0;
+                    int sr = i < dw - 1 ? 3 * IN(r, i + 1) + IN(rn, i + 1) : 0;
+                    d[2 * i] = (uint8_t)(i == 0 ? (4 * s + 8) >> 4 : (3 * s + sl + 8) >> 4);
+                    d[2 * i + 1] = (uint8_t)(i == dw - 1 ? (4 * s + 7) >> 4 : (3 * s + sr + 7) >> 4);
+                }
+            }
+    } else {
+        for (int r = 0; r < oh; r++)
+            for (int i = 0; i < ow; i++) o[(size_t)r * ow + i] = (uint8_t)IN(r / vx, i / hx);
+    }
+#undef IN
+}
+
+/* Coefficients -> what libjpeg returns with scale_denom 8 / S (jdmaster.c): ceil(W S / 8) x ceil(H S / 8) gray samples
+ * (luma only: no chroma IDCT, no upsampling, no colour conversion) or BGR. Luma blocks come out S x S, chroma blocks at
+ * chroma_size's size, the chroma planes at their true size ceil(W Sc / (hs 8)) x ceil(H Sc / (vs 8)). */
+static int render(const orc_geom *g, const uint16_t qt[3][64], const int16_t *coef, int S, int gray, uint8_t *out,
+                  size_t step) {
+    const int nc = gray ? 1 : 3, Sc = chroma_size(g->hs, g->vs, S);
+    const int Wo = ceil_div(g->W * S, 8), Ho = ceil_div(g->H * S, 8);
+    const int hx = g->hs * S / Sc, vx = g->vs * S / Sc;
+    const int dw = ceil_div(g->W * Sc, g->hs * 8), dh = ceil_div(g->H * Sc, g->vs * 8), ow = dw * hx;
+    uint8_t *pl[3] = {NULL, NULL, NULL}, *up[3] = {NULL, NULL, NULL};
+    int pw[3], k[3], rc = 0;
+    for (int c = 0; c < nc; c++) {
+        int h = c ? 1 : g->hs, v = c ? 1 : g->vs;
+        k[c] = c ? Sc : S;
+        pw[c] = g->mcux * h * k[c];
+        pl[c] = (uint8_t *)malloc((size_t)pw[c] * g->mcuy * v * k[c]);
+        if (c) up[c] = (uint8_t *)malloc((size_t)ow * dh * vx);
+        if (!pl[c] || (c && !up[c])) { rc = -2; goto done; }
+    }
+    for (int my = 0; my < g->mcuy; my++)
+        for (int mx = 0; mx < g->mcux; mx++) {
+            const int16_t *mcu = coef + ((size_t)my * g->mcux + mx) * g->bpm * 64;
+            int blkn = 0;
+            for (int c = 0; c < nc; c++) {
+                int h = c ? 1 : g->hs, v = c ? 1 : g->vs;
+                for (int by = 0; by < v; by++)
+                    for (int bx = 0; bx < h; bx++, blkn++)
+                        idct_scaled(mcu + blkn * 64, qt[c], k[c],
+                                   pl[c] + (size_t)(my * v + by) * k[c] * pw[c] + (size_t)(mx * h + bx) * k[c], pw[c]);
+            }
+        }
+    if (gray) {
+        for (int y = 0; y < Ho; y++) memcpy(out + (size_t)y * step, pl[0] + (size_t)y * pw[0], (size_t)Wo);
+        goto done;
+    }
+    for (int c = 1; c < 3; c++) upsample(pl[c], pw[c], dw, dh, hx, vx, Sc > 1, up[c]);
+    for (int y = 0; y < Ho; y++)   /* jdcolor.c ycc_rgb_convert */
+        for (int x = 0; x < Wo; x++) {
+            int Y = pl[0][(size_t)y * pw[0] + x];
+            int cb = up[1][(size_t)y * ow + x] - 128, cr = up[2][(size_t)y * ow + x] - 128;
+            int r = Y + ((91881 * cr + 32768) >> 16);
+            int b = Y + ((116130 * cb + 32768) >> 16);
+            int gg = Y + ((-22554 * cb - 46802 * cr + 32768) >> 16);
+            uint8_t *p = out + (size_t)y * step + (size_t)x * 3;
+            p[0] = (uint8_t)clampi(b, 0, 255); p[1] = (uint8_t)clampi(gg, 0, 255); p[2] = (uint8_t)clampi(r, 0, 255);
+        }
+done:
+    for (int c = 0; c < 3; c++) { free(pl[c]); free(up[c]); }
+    return rc;
+}
+
+int orc_inverse(const int16_t *coef, const orc_info *info, uint8_t *bgr, size_t step) {
+    orc_geom g; if (orc_geometry(info->W, info->H, info->css, &g)) return -1;
+    uint16_t qt[3][64];
+    memcpy(qt[0], info->qt[0], 128); memcpy(qt[1], info->qt[1], 128); memcpy(qt[2], info->qt[1], 128);
+    return render(&g, (const uint16_t(*)[64])qt, coef, 8, 0, bgr, step);
+}
+
+/* ------------------------------------------------------------------ decoder: entry points */
+
+int orc_decode_output(const uint8_t *jpg, size_t len, int denom, int gray_out, uint8_t *out, size_t step, int *W, int *H) {
+    if (denom != 1 && denom != 2 && denom != 4 && denom != 8) return -20;
+    jfile f;
+    int rc = read_file(jpg, len, out ? READ_ALL : READ_FRAME, gray_out ? 1 : 3, &f, NULL);
+    if (rc) return rc;
+    if (!gray_out && f.ncomp == 1) rc = -21;
+    else {
+        if (W) *W = ceil_div(f.g.W, denom);
+        if (H) *H = ceil_div(f.g.H, denom);
+        if (out) rc = render(&f.g, (const uint16_t(*)[64])f.qt, f.coef, 8 / denom, gray_out, out, step);
+    }
+    free(f.coef);
     return rc;
 }
 
 int orc_decode(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t step, int *W, int *H) {
-    orc_info info;
-    int rc = orc_parse(jpg, len, &info);
-    if (rc == -8) return orc_decode_progressive(jpg, len, bgr, step, W, H);
-    if (rc) return rc;
-    if (W) *W = info.W;
-    if (H) *H = info.H;
-    if (!bgr) return 0;
-    orc_geom g; orc_geometry(info.W, info.H, info.css, &g);
-    int16_t *coef = (int16_t *)malloc((size_t)g.nblocks * 128);
-    if (!coef) return -2;
-    rc = orc_decode_coefs(jpg, len, &info, coef);
-    if (!rc) rc = orc_inverse(coef, &info, bgr, step);
-    free(coef);
-    return rc;
+    return orc_decode_output(jpg, len, 1, 0, bgr, step, W, H);
+}
+
+int orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t step, int *W, int *H) {
+    jfile f;
+    int rc = read_file(jpg, len, READ_FRAME, 3, &f, NULL);
+    if (!rc && f.sof != 0xC2) rc = -8;
+    return rc ? rc : orc_decode(jpg, len, bgr, step, W, H);
 }
 
 /* ------------------------------------------------------------------ a-12: difference map + PSNR */

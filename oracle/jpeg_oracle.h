@@ -8,9 +8,9 @@
  * (jccolor.c, jcsample.c, jcprepct.c, jfdctint.c, jcdctmgr.c, jccoefct.c, jchuff.c, jcparam.c,
  * jcmarker.c / jdhuff.c, jidctint.c, jdsample.c, jdcolor.c) as written down in SURVEY.md Appendix A.
  *
- * Parity pin: tests/test_oracle_vs_cv2.py compares every function here byte-for-byte with
- * cv2.imencode / cv2.imdecode (OpenCV 4.13.0 wheel = libjpeg-turbo 3.1.2) and tests/golden/ holds
- * committed digests produced by that library (tests/golden/make_golden.py).
+ * Parity pin: tests/test_oracle_golden.py, test_oracle_gray.py, test_oracle_scaled.py and test_prog_streams.py compare
+ * the functions here byte-for-byte with cv2.imencode / cv2.imdecode (OpenCV 4.13.0 wheel = libjpeg-turbo 3.1.2), and
+ * tests/golden/ holds committed digests produced by that library (tests/golden/make_golden*.py).
  *
  * Only tests/, __graft_entry__.smoke() and bench.py's cpu_baseline / reference leg may link or call this.
  */
@@ -24,14 +24,14 @@
 extern "C" {
 #endif
 
-/* chroma subsampling codes shared with include/b2jpeg.h */
-enum { ORC_CSS_444 = 0, ORC_CSS_422 = 1, ORC_CSS_440 = 2, ORC_CSS_420 = 3, ORC_CSS_411 = 4 };
+/* chroma subsampling codes shared with include/b2jpeg.h; GRAY: one component (orc_geometry refuses it) */
+enum { ORC_CSS_444 = 0, ORC_CSS_422 = 1, ORC_CSS_440 = 2, ORC_CSS_420 = 3, ORC_CSS_411 = 4, ORC_CSS_GRAY = 6 };
 
 typedef struct {
     int W, H, css;
     int hs, vs;          /* luma sampling factors (chroma is 1x1) */
     int mcux, mcuy;      /* MCU grid */
-    int bpm;             /* blocks per MCU = hs*vs + 2 */
+    int bpm;             /* blocks per MCU = hs*vs + 2 (gray: 1) */
     int wib[3], hib[3];  /* per-component width/height in blocks (real data) */
     int dw[3], dh[3];    /* per-component true downsampled size in samples */
     long long nblocks;   /* mcux*mcuy*bpm (scan order) */
@@ -51,7 +51,8 @@ void orc_synth_rows(int W, int H, int y0, int rows, uint32_t seed, int amp, uint
  * 64 int16 per block in ZIG-ZAG order. coef must hold g.nblocks*64 int16. */
 int  orc_forward(const uint8_t *bgr, size_t step, int W, int H, int css, int quality, int16_t *coef);
 
-/* Stage 3: symbol histograms. hist[4][257]: DC0, AC0, DC1, AC1 (index 256 unused, left 0).
+/* Stage 3: symbol histograms. hist[4][257]: DC0, AC0, DC1, AC1 (index 256 unused, left 0). bpm 1: one component,
+ * counted as the last component (DC1, AC1); orc_entropy_bits codes it with tables 2 / 3 likewise.
  * pred_in/pred_out: optional DC predictors per component at strip start/end (NULL = 0 / ignored). */
 void orc_histogram(const int16_t *coef, long long nblocks, int bpm, const int16_t *pred_in,
                    uint32_t hist[4][257]);
@@ -83,8 +84,10 @@ size_t orc_headers(int W, int H, int css, const uint16_t qt[2][64], const uint8_
 int  orc_encode(const uint8_t *bgr, size_t step, int W, int H, int css, int quality, int optimize,
                 uint8_t *out, size_t cap, size_t *len);
 /* Same with restart markers every `restart_interval` MCUs (0 = none): DRI before SOS, RSTn between the intervals,
- * DC predictors and the bit buffer restart (jchuff.c emit_restart). Pinned against cv2 IMWRITE_JPEG_RST_INTERVAL. */
-int  orc_encode_rst(const uint8_t *bgr, size_t step, int W, int H, int css, int quality, int optimize,
+ * DC predictors and the bit buffer restart (jchuff.c emit_restart). Pinned against cv2 IMWRITE_JPEG_RST_INTERVAL.
+ * css ORC_CSS_GRAY: one component (JCS_GRAYSCALE) from 8-bit samples with row pitch `step`; DQT 0, SOF0 and SOS with
+ * one component, DHT DC0 and AC0; the restart interval counts blocks (one block per MCU). */
+int  orc_encode_rst(const uint8_t *px, size_t step, int W, int H, int css, int quality, int optimize,
                     int restart_interval, uint8_t *out, size_t cap, size_t *len);
 
 /* Parsed header info */
@@ -99,12 +102,14 @@ typedef struct {
     uint8_t vals[4][256];
 } orc_info;
 
+/* Headers of a three-component sequential file up to its (only) scan; -8 for a progressive file, -7 for one with one
+ * component. */
 int  orc_parse(const uint8_t *jpg, size_t len, orc_info *info);
 
 /* Decode entropy data to scan-order quantised coefficients (zig-zag order), DC already un-differenced. */
 int  orc_decode_coefs(const uint8_t *jpg, size_t len, const orc_info *info, int16_t *coef);
 
-/* Stage 5: coefficients -> BGR (islow IDCT, fancy upsampling, jdcolor) */
+/* Stage 5: coefficients of orc_decode_coefs -> BGR (islow IDCT, fancy upsampling, jdcolor) */
 int  orc_inverse(const int16_t *coef, const orc_info *info, uint8_t *bgr, size_t step);
 
 /* Progressive (SOF2) encode: jpeg_simple_progression's 10 scans, optimal tables per scan (jcphuff.c); what
@@ -112,11 +117,19 @@ int  orc_inverse(const int16_t *coef, const orc_info *info, uint8_t *bgr, size_t
 int  orc_encode_progressive(const uint8_t *bgr, size_t step, int W, int H, int css, int quality, uint8_t *out,
                             size_t cap, size_t *len);
 
-/* Progressive (SOF2) streams: all scans absorbed, then the baseline back end (jdphuff.c). orc_decode dispatches here. */
-int  orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t step, int *W, int *H);
+/* The decoders read sequential (SOF0/1) and progressive (SOF2) files with one or three components; a progressive
+ * file's scans are all absorbed (jdphuff.c) before the one back end runs. *W, *H: the output size; the output may be
+ * NULL to query it. 0 on success; -18 for a progressive file libjpeg would block-smooth (an output component's
+ * low-frequency coefficients unfinished); other negative values: a file the product refuses. */
 
-/* Whole decoder; *W,*H returned; bgr may be NULL to query size */
+/* what libjpeg returns with scale_num = 1, scale_denom = d (1, 2, 4, 8; else -20; cv2 IMREAD_REDUCED_*_d): BGR
+ * (H', W', 3) or, with gray_out, the luma plane (H', W') (JCS_GRAYSCALE: no chroma IDCT, upsampling or colour
+ * conversion), row pitch `step`. Colour output of a one-component file: -21. */
+int  orc_decode_output(const uint8_t *jpg, size_t len, int denom, int gray_out, uint8_t *out, size_t step, int *W, int *H);
+/* full-size BGR (IMREAD_COLOR): orc_decode_output(jpg, len, 1, 0, ...) */
 int  orc_decode(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t step, int *W, int *H);
+/* orc_decode of progressive files only (-8 otherwise) */
+int  orc_decode_progressive(const uint8_t *jpg, size_t len, uint8_t *bgr, size_t step, int *W, int *H);
 
 /* a-12 definitions (SURVEY.md 8a-12): mode 0 = absdiff, 1 = clamp(a-b+128) */
 void   orc_diff(const uint8_t *a, const uint8_t *b, size_t n, int mode, uint8_t *out);

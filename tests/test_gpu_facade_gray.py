@@ -6,7 +6,7 @@ import subprocess
 import numpy as np
 import pytest
 
-import gray_oracle as G
+import oracle as O
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,7 +41,7 @@ def test_cpp_gray_demo_sequence(tmp_path, oracle):
     assert r.stdout.count("[INFO] Successful.") == 4
     for name, img in (("1", a), ("2", b)):
         jpg = np.fromfile(tmp_path / f"{name}.jpeg", np.uint8)
-        want = G.encode_gray(img, 95, 1)
+        want = O.encode_gray(img, 95, 1)
         assert np.array_equal(jpg, want)
         dec = np.fromfile(tmp_path / f"{name}.dec.gray", np.uint8).reshape(H, W)
-        assert np.array_equal(dec, G.decode_gray(want))
+        assert np.array_equal(dec, O.decode_gray(want))

@@ -7,7 +7,7 @@ import subprocess
 import numpy as np
 import pytest
 
-import scaled_oracle as SO
+import oracle as O
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -41,7 +41,7 @@ def test_cpp_scaled_decode(tmp_path, oracle):
     assert r.returncode == 0, r.stdout + r.stderr
     for name in ("bgr", "gray"):
         jpg = np.fromfile(tmp_path / f"{name}.jpeg", np.uint8)
-        for d in SO.SCALES:
-            want = SO.decode_scaled(jpg, d, gray=name == "gray")
+        for d in O.SCALES:
+            want = O.decode_scaled(jpg, d, gray=name == "gray")
             got = np.fromfile(tmp_path / f"{name}.d{d}.raw", np.uint8).reshape(want.shape)
             assert np.array_equal(got, want), (name, d)

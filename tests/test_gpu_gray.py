@@ -1,4 +1,4 @@
-"""GPU: gray (B2J_CSS_GRAY, one byte per pixel) contexts against the grayscale CPU checker (tests/gray_oracle.py,
+"""GPU: gray (B2J_CSS_GRAY, one byte per pixel) contexts against the grayscale CPU checker (oracle/,
 pinned to libjpeg-turbo by tests/test_oracle_gray.py) and the committed digests of tests/golden/golden_gray.json."""
 import ctypes as C
 import hashlib
@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-import gray_oracle as G
+import oracle as O
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -62,7 +62,7 @@ def test_encode_matrix_vs_checker_and_golden(P, oracle, golden_gray):
         img = gray_img(oracle, W, H, c["seed"])
         jpg = eng.encode(img)
         assert jpg.size == c["jpeg_len"] and sha(jpg)[:32] == c["jpeg_sha256_128"], c
-        assert np.array_equal(jpg, G.encode_gray(img, c["quality"], c["optimize"], c["restart_interval"])), c
+        assert np.array_equal(jpg, O.encode_gray(img, c["quality"], c["optimize"], c["restart_interval"])), c
 
 
 @pytest.mark.parametrize("W,H", SIZES)
@@ -72,7 +72,7 @@ def test_encode_pinned_pitch_and_shapes(P, oracle, W, H):
     for q, opt, rows in ((95, 1, 0), (75, 0, 1), (100, 1, 2)):
         eng = P.Engine(W, H, q, bool(opt), "400", device=0)
         eng.set_restart_rows(rows)
-        want = G.encode_gray(img, q, opt, rows * ((W + 7) // 8))
+        want = O.encode_gray(img, q, opt, rows * ((W + 7) // 8))
         assert np.array_equal(eng.encode(img), want), (W, H, q, opt, rows, "pageable, pitch")
         assert np.array_equal(eng.encode(np.ascontiguousarray(img)[:, :, None]), want), (W, H, q, opt, rows, "(H, W, 1)")
         buf, p = pinned_copy(P, np.ascontiguousarray(img))
@@ -91,7 +91,7 @@ def test_special_images(P, oracle):
     for q, opt in ((100, 1), (95, 0), (40, 1)):
         eng = P.Engine(W, H, q, bool(opt), "gray", device=0)
         for img in imgs:
-            assert np.array_equal(eng.encode(img), G.encode_gray(img, q, opt)), (q, opt)
+            assert np.array_equal(eng.encode(img), O.encode_gray(img, q, opt)), (q, opt)
 
 
 def test_device_entry_points(P, oracle):
@@ -105,7 +105,7 @@ def test_device_entry_points(P, oracle):
                 eng = P.Engine(W, H, 90, bool(opt), "gray", device=0)
                 eng.set_restart_rows(rows)
                 eng.set_debug(dbg)
-                want = G.encode_gray(img, 90, opt, rows * mcux)
+                want = O.encode_gray(img, 90, opt, rows * mcux)
                 d = torch.from_numpy(img).cuda()
                 o, _ = eng.encode_device(d.data_ptr(), W, W, H)
                 n = eng.encode_finish()
@@ -137,15 +137,15 @@ def test_decode_gray_files_and_matrix(P, oracle, golden_gray):
     for f in golden_gray["files"]:
         jpg = np.fromfile(os.path.join(HERE, "golden", f["file"]), np.uint8)
         eng = P.Engine(f["W"], f["H"], 95, True, "gray", device=0)
-        want = G.decode_gray(jpg)
+        want = O.decode_gray(jpg)
         assert sha(want) == f["decoded_sha256"]
         _decode_all_ways(P, eng, jpg, want, f["file"])
     for (W, H) in SIZES:
         img = gray_img(oracle, W, H, W + 3 * H)
         eng = P.Engine(W, H, 95, True, "gray", device=0)
         for q, opt, ri in ((95, 1, 0), (75, 0, 1), (90, 1, (W + 7) // 8)):
-            jpg = G.encode_gray(img, q, opt, ri)
-            _decode_all_ways(P, eng, jpg, G.decode_gray(jpg), (W, H, q, opt, ri))
+            jpg = O.encode_gray(img, q, opt, ri)
+            _decode_all_ways(P, eng, jpg, O.decode_gray(jpg), (W, H, q, opt, ri))
 
 
 def test_decode_y_plane_of_colour_files(P, oracle, golden_gray):
@@ -159,7 +159,7 @@ def test_decode_y_plane_of_colour_files(P, oracle, golden_gray):
         key = (c["W"], c["H"])
         if key not in engines:
             engines[key] = P.Engine(c["W"], c["H"], 95, True, "gray", device=0)
-        want = G.decode_gray(jpg)
+        want = O.decode_gray(jpg)
         assert sha(want)[:32] == c["gray_sha256_128"], c
         _decode_all_ways(P, engines[key], jpg, want, c)
 
@@ -169,7 +169,7 @@ def test_decode_scan_device_restart_file(P, oracle):
     W, H = 257, 63
     img = gray_img(oracle, W, H, 17)
     mcux = (W + 7) // 8
-    jpg = G.encode_gray(img, 90, 1, 2 * mcux)
+    jpg = O.encode_gray(img, 90, 1, 2 * mcux)
     b = jpg.tobytes()
     p = 2
     while b[p + 1] != 0xDA:
@@ -179,15 +179,15 @@ def test_decode_scan_device_restart_file(P, oracle):
     out = torch.zeros((H, W), dtype=torch.uint8, device="cuda")
     eng = P.Engine(W, H, 90, True, "gray", device=0)
     assert eng.decode_scan_device(jpg[:hdr_len], scan.data_ptr(), scan.numel(), out.data_ptr(), W) == (W, H)
-    assert np.array_equal(out.cpu().numpy(), G.decode_gray(jpg))
+    assert np.array_equal(out.cpu().numpy(), O.decode_gray(jpg))
 
 
 def test_colour_gray_cross(P, oracle):
     W, H = 135, 121
-    gray_file = G.encode_gray(gray_img(oracle, W, H, 1), 90, 1)
+    gray_file = O.encode_gray(gray_img(oracle, W, H, 1), 90, 1)
     colour_file = oracle.encode(oracle.synth(W, H, 1, 8), 1, 90, 1)
     g = P.Engine(W, H, 90, True, "gray", device=0)
-    assert np.array_equal(g.decode(colour_file), G.decode_gray(colour_file))
+    assert np.array_equal(g.decode(colour_file), O.decode_gray(colour_file))
     c = P.Engine(W, H, 90, True, "422", device=0)
     for f in (gray_file, cv2_progressive_gray(gray_img(oracle, W, H, 1))):
         if f is None:

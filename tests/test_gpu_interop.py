@@ -7,7 +7,7 @@ import cv2
 import numpy as np
 import pytest
 
-import gray_oracle as GO
+import oracle as O
 import jpeg_streams as J
 
 pytestmark = pytest.mark.gpu
@@ -127,7 +127,7 @@ def test_size_limit_frames(P, oracle, W, H):
                 try:
                     if css == "gray":
                         jpg = eng.encode(g)
-                        want = GO.encode_gray(g, q, opt)
+                        want = O.encode_gray(g, q, opt)
                         cv = cv2.imencode(".jpg", g, [cv2.IMWRITE_JPEG_QUALITY, q, cv2.IMWRITE_JPEG_OPTIMIZE, opt])[1].ravel()
                         flags = (cv2.IMREAD_GRAYSCALE, cv2.IMREAD_REDUCED_GRAYSCALE_8)
                     else:
@@ -163,8 +163,8 @@ def test_width_65535(P, oracle, H):
         try:
             if css == "gray":
                 jpg = eng.encode(g)
-                assert np.array_equal(jpg, GO.encode_gray(g, 90, 1)), css
-                assert np.array_equal(eng.decode(jpg), GO.decode_gray(jpg)), css
+                assert np.array_equal(jpg, O.encode_gray(g, 90, 1)), css
+                assert np.array_equal(eng.decode(jpg), O.decode_gray(jpg)), css
             else:
                 jpg = eng.encode(img)
                 assert np.array_equal(jpg, oracle.encode(img, css, 90, 1)), css
@@ -191,8 +191,8 @@ def test_restart_rows_at_the_dri_limit(P, oracle, W):
             eng.set_restart_rows(rows)
             if css == "gray":
                 jpg = eng.encode(g)
-                assert np.array_equal(jpg, GO.encode_gray(g, 90, 1, rows * mcux)), css
-                assert np.array_equal(eng.decode(jpg), GO.decode_gray(jpg)), css
+                assert np.array_equal(jpg, O.encode_gray(g, 90, 1, rows * mcux)), css
+                assert np.array_equal(eng.decode(jpg), O.decode_gray(jpg)), css
             else:
                 jpg = eng.encode(img)
                 assert np.array_equal(jpg, oracle.encode(img, css, 90, 1, rows * mcux)), css

@@ -1,5 +1,5 @@
 """GPU: reduced-size decode (b2j_set_decode_scale, libjpeg's DCT scaling at 1/2, 1/4, 1/8) against the CPU checker
-(tests/scaled_oracle.py, pinned to libjpeg-turbo by tests/test_oracle_scaled.py) and the committed digests of
+(oracle/, pinned to libjpeg-turbo by tests/test_oracle_scaled.py) and the committed digests of
 tests/golden/golden_scaled.json."""
 import ctypes as C
 import hashlib
@@ -9,7 +9,7 @@ import os
 import numpy as np
 import pytest
 
-import scaled_oracle as SO
+import oracle as O
 
 pytestmark = pytest.mark.gpu
 HERE = os.path.dirname(os.path.abspath(__file__))
@@ -92,12 +92,12 @@ def test_matrix_every_entry_point(P, oracle, css):
         gray = P.Engine(W + 32, H + 32, 95, True, "gray", device=0)
         for q, rst in ((90, 0), (100, 0), (75, mcux)):
             jpg = oracle.encode(img, css, q, 1, rst)
-            for d in SO.SCALES:
+            for d in O.SCALES:
                 col.set_decode_scale(d)
                 gray.set_decode_scale(d)
                 tag = (W, H, css, q, rst, d)
-                decode_every_way(P, col, jpg, SO.decode_scaled(jpg, d), tag + ("colour",))
-                decode_every_way(P, gray, jpg, SO.decode_scaled(jpg, d, gray=True), tag + ("gray",))
+                decode_every_way(P, col, jpg, O.decode_scaled(jpg, d), tag + ("colour",))
+                decode_every_way(P, gray, jpg, O.decode_scaled(jpg, d, gray=True), tag + ("gray",))
         col.close()
         gray.close()
 
@@ -109,9 +109,9 @@ def test_one_component_files(P, golden_scaled):
             continue
         jpg = np.fromfile(os.path.join(HERE, "golden", f["file"]), np.uint8)
         eng = P.Engine(f["W"], f["H"], 95, True, "gray", device=0)
-        for d in SO.SCALES:
+        for d in O.SCALES:
             eng.set_decode_scale(d)
-            want = SO.decode_scaled(jpg, d, gray=True)
+            want = O.decode_scaled(jpg, d, gray=True)
             assert sha(want)[:32] == f["g%d" % d], (f["file"], d)
             decode_every_way(P, eng, jpg, want, (f["file"], d), scan_device="prog" not in f["file"])
         eng.close()
@@ -126,10 +126,10 @@ def test_progressive_and_nvjpeg_files(P, golden_scaled):
         css = P.Engine.peek(jpg)[2]
         col = P.Engine(f["W"], f["H"], 95, True, CSS_NAMES[css], device=0)
         gray = P.Engine(f["W"], f["H"], 95, True, "gray", device=0)
-        for d in SO.SCALES:
+        for d in O.SCALES:
             col.set_decode_scale(d)
             gray.set_decode_scale(d)
-            W, H = SO.reduced_size(f["W"], f["H"], d)
+            W, H = O.reduced_size(f["W"], f["H"], d)
             out = col.decode(jpg)
             assert out.shape == (H, W, 3) and sha(out)[:32] == f["c%d" % d], (f["file"], d, "colour")
             assert sha(gray.decode(jpg))[:32] == f["g%d" % d], (f["file"], d, "gray")
@@ -168,7 +168,7 @@ def test_invalid_scales_leave_setting(P, oracle):
             eng.set_decode_scale(bad)
     assert L.b2j_set_decode_scale(None, 2) == -1
     out = eng.decode(jpg)
-    assert out.shape == (12, 16, 3) and np.array_equal(out, SO.decode_scaled(jpg, 4))
+    assert out.shape == (12, 16, 3) and np.array_equal(out, O.decode_scaled(jpg, 4))
     assert P.Engine.peek(jpg) == (W, H, 1)   # peek reports the file's size
     # a step that fits the reduced width but not the full one is accepted; one below the reduced width is not
     dst = np.empty((12, 16 * 3), np.uint8)
@@ -182,9 +182,9 @@ def test_timings_filled(P, oracle):
     jpg = oracle.encode(oracle.synth(W, H, 4, 8), 1, 90, 1)
     eng = P.Engine(W, H, 95, True, "422", device=0)
     eng.enable_timing(True)
-    for d in SO.SCALES:
+    for d in O.SCALES:
         eng.set_decode_scale(d)
-        assert np.array_equal(eng.decode(jpg), SO.decode_scaled(jpg, d))
+        assert np.array_equal(eng.decode(jpg), O.decode_scaled(jpg, d))
         t = eng.timings()
         assert t["dec_idct"] > 0 and t["dec_color"] > 0, d
 
@@ -209,8 +209,8 @@ def test_headline_reduced_digests(P, oracle, golden_scaled):
     jpg = buf.numpy()
     assert sha(jpg) == h["jpeg_sha256"]
     gray = P.Engine(W, H, h["quality"], True, "gray", device=0)
-    for dn in SO.SCALES:
-        ow, oh = SO.reduced_size(W, H, dn)
+    for dn in O.SCALES:
+        ow, oh = O.reduced_size(W, H, dn)
         eng.set_decode_scale(dn)
         gray.set_decode_scale(dn)
         out = torch.empty((oh, ow * 3), dtype=torch.uint8, device="cuda")

@@ -91,6 +91,26 @@ def test_pillow_corpus_present(corpus):
     assert b"\xff\xc1" in big   # SOF1: extended sequential, 16-bit tables
 
 
+def test_checker_refuses_what_the_product_refuses(corpus, oracle):
+    """every output of the checker -- colour, gray, reduced size -- refuses the streams the product refuses"""
+    calls = [("colour", oracle.decode), ("gray", oracle.decode_gray)]
+    calls += [(f"1/{d} {'gray' if g else 'colour'}", lambda j, d=d, g=g: oracle.decode_scaled(j, d, g))
+              for d in oracle.SCALES for g in (False, True)]
+
+    def refused(call, jpg):
+        try:
+            call(jpg)
+        except RuntimeError:
+            return True
+        return False
+
+    refusals = [e for e in corpus if not e["accept"]]
+    for e in refusals:
+        for name, call in calls:
+            assert refused(call, e["jpg"]), (e["name"], name)
+    assert len(refusals) >= 30
+
+
 @pytest.fixture(scope="module")
 def parse_verdict(tmp_path_factory):
     nvcc = shutil.which("nvcc") or "/usr/local/cuda/bin/nvcc"

@@ -1,4 +1,4 @@
-"""The grayscale CPU checker (tests/gray_oracle.py: encode_gray / decode_gray) against libjpeg-turbo: live cv2 where it is
+"""The grayscale CPU checker (oracle/: encode_gray / decode_gray) against libjpeg-turbo: live cv2 where it is
 importable, and the committed digests of tests/golden/golden_gray.json (tests/golden/make_golden_gray.py) always.
 Also b2j_peek on one-component files, which needs no GPU."""
 import hashlib
@@ -8,7 +8,7 @@ import os
 import numpy as np
 import pytest
 
-import gray_oracle as G
+import oracle as O
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 SIZES = ((1, 1), (2, 2), (8, 8), (17, 33), (33, 17), (135, 121), (257, 63), (640, 360))
@@ -38,14 +38,14 @@ def colour_stream(oracle, c):
 def test_encode_gray_matches_golden(oracle, golden_gray):
     for c in golden_gray["encode"]:
         img = gray_img(oracle, c["W"], c["H"], c["seed"])
-        jpg = G.encode_gray(img, c["quality"], c["optimize"], c["restart_interval"])
+        jpg = O.encode_gray(img, c["quality"], c["optimize"], c["restart_interval"])
         assert jpg.size == c["jpeg_len"] and sha(jpg)[:32] == c["jpeg_sha256_128"], c
-        assert sha(G.decode_gray(jpg))[:32] == c["decoded_sha256_128"], c
+        assert sha(O.decode_gray(jpg))[:32] == c["decoded_sha256_128"], c
 
 
 def test_gray_stream_layout(oracle):
     img = gray_img(oracle, 40, 24, 3)
-    jpg = G.encode_gray(img, 90, 1, 5).tobytes()
+    jpg = O.encode_gray(img, 90, 1, 5).tobytes()
     markers = []
     p = 2
     while jpg[p + 1] != 0xDA:
@@ -61,14 +61,14 @@ def test_decode_gray_of_colour_matches_golden(oracle, golden_gray):
     for c in golden_gray["ydecode"]:
         jpg = colour_stream(oracle, c)
         assert sha(jpg)[:32] == c["jpeg_sha256_128"], c
-        assert sha(G.decode_gray(jpg))[:32] == c["gray_sha256_128"], c
+        assert sha(O.decode_gray(jpg))[:32] == c["gray_sha256_128"], c
 
 
 def test_decode_gray_files(oracle, golden_gray):
     for f in golden_gray["files"]:
         jpg = np.fromfile(os.path.join(HERE, "golden", f["file"]), np.uint8)
         assert sha(jpg) == f["jpeg_sha256"]
-        dec = G.decode_gray(jpg)
+        dec = O.decode_gray(jpg)
         assert dec.shape == (f["H"], f["W"])
         assert sha(dec) == f["decoded_sha256"], f["file"]
 
@@ -78,7 +78,7 @@ def test_colour_functions_still_reject_gray(oracle, golden_gray):
     with pytest.raises(RuntimeError):
         oracle.decode(jpg)
     with pytest.raises(ValueError):
-        oracle.geometry(8, 8, G.CSS_GRAY)
+        oracle.geometry(8, 8, O.CSS_GRAY)
 
 
 def test_peek_gray_files(golden_gray):
@@ -111,9 +111,9 @@ def test_encode_gray_vs_cv2(oracle, W, H):
         for opt in (0, 1):
             for rst in sorted({0, 1, 5, mcux, 2 * mcux}):
                 ref = cv_gray(img, q, opt, rst)
-                jpg = G.encode_gray(img, q, opt, rst)
+                jpg = O.encode_gray(img, q, opt, rst)
                 assert np.array_equal(jpg, ref), (W, H, q, opt, rst)
-                assert np.array_equal(G.decode_gray(jpg), cv2.imdecode(ref, cv2.IMREAD_UNCHANGED)), (W, H, q, opt, rst)
+                assert np.array_equal(O.decode_gray(jpg), cv2.imdecode(ref, cv2.IMREAD_UNCHANGED)), (W, H, q, opt, rst)
 
 
 @pytest.mark.parametrize("kind", ["flat", "saturated", "checker"])
@@ -127,13 +127,13 @@ def test_encode_gray_special_images_vs_cv2(oracle, kind):
     else:
         img = ((np.indices((H, W)).sum(0) & 1) * 255).astype(np.uint8)
     for q, opt in ((100, 1), (95, 0), (40, 1)):
-        assert np.array_equal(G.encode_gray(img, q, opt), cv_gray(img, q, opt)), (kind, q, opt)
+        assert np.array_equal(O.encode_gray(img, q, opt), cv_gray(img, q, opt)), (kind, q, opt)
 
 
 def test_encode_gray_pitch(oracle):
     big = gray_img(oracle, 160, 50, 11)
     img = big[:, 3:140]   # pitch 160 != width 137
-    assert np.array_equal(G.encode_gray(img, 90, 1, 3), cv_gray(np.ascontiguousarray(img), 90, 1, 3))
+    assert np.array_equal(O.encode_gray(img, 90, 1, 3), cv_gray(np.ascontiguousarray(img), 90, 1, 3))
 
 
 @pytest.mark.parametrize("css", range(5))
@@ -142,14 +142,14 @@ def test_decode_gray_of_colour_vs_cv2(oracle, css):
     mcux = oracle.geometry(135, 121, css).mcux
     for jpg in (oracle.encode(img, css, 90, 1), oracle.encode(img, css, 75, 0, mcux), oracle.encode(img, css, 95, 1, 7),
                 oracle.encode_progressive(img, css, 85)):
-        assert np.array_equal(G.decode_gray(jpg), cv2.imdecode(jpg, cv2.IMREAD_GRAYSCALE))
+        assert np.array_equal(O.decode_gray(jpg), cv2.imdecode(jpg, cv2.IMREAD_GRAYSCALE))
 
 
 def test_decode_gray_progressive_and_patched_vs_cv2(oracle):
     img = gray_img(oracle, 135, 121, 4)
     for rst in (0, 4):
         jpg = cv_gray(img, 85, 1, rst, prog=1)
-        assert np.array_equal(G.decode_gray(jpg), cv2.imdecode(jpg, cv2.IMREAD_UNCHANGED))
+        assert np.array_equal(O.decode_gray(jpg), cv2.imdecode(jpg, cv2.IMREAD_UNCHANGED))
     for f in ("gray/gray_135x121_q90_sof22.jpg", "gray/gray_135x121_q90_prog.jpg", "gray/gray_135x121_q90_rst5.jpg"):
         jpg = np.fromfile(os.path.join(HERE, "golden", f), np.uint8)
-        assert np.array_equal(G.decode_gray(jpg), cv2.imdecode(jpg, cv2.IMREAD_UNCHANGED)), f
+        assert np.array_equal(O.decode_gray(jpg), cv2.imdecode(jpg, cv2.IMREAD_UNCHANGED)), f

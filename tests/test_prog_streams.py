@@ -7,7 +7,7 @@ import cv2
 import numpy as np
 import pytest
 
-import gray_oracle as GO
+import oracle as O
 import jpeg_streams as J
 import prog_streams as PS
 
@@ -62,7 +62,7 @@ def test_checkers_match_cv2_on_the_catalogue(oracle):
     for tag, jpg, ncomp in PS.catalogue(oracle, big=False):
         if ncomp == 3:
             assert np.array_equal(oracle.decode(jpg), dec(jpg)), tag
-        assert np.array_equal(GO.decode_gray(jpg), dec(jpg, cv2.IMREAD_GRAYSCALE)), tag
+        assert np.array_equal(O.decode_gray(jpg), dec(jpg, cv2.IMREAD_GRAYSCALE)), tag
 
 
 def test_incomplete_files_checkers(oracle):
@@ -73,10 +73,10 @@ def test_incomplete_files_checkers(oracle):
         for gray in ((False, True) if ncomp == 3 else (True,)):
             if PS.smoothed(received, ncomp, gray):
                 with pytest.raises(RuntimeError, match="rc=-18"):
-                    GO.decode_gray(jpg) if gray else oracle.decode(jpg)
+                    O.decode_gray(jpg) if gray else oracle.decode(jpg)
                 n_refused += 1
             else:
-                got = GO.decode_gray(jpg) if gray else oracle.decode(jpg)
+                got = O.decode_gray(jpg) if gray else oracle.decode(jpg)
                 assert np.array_equal(got, dec(ref, cv2.IMREAD_GRAYSCALE if gray else cv2.IMREAD_COLOR)), (tag, gray)
                 n_equal += 1
     assert n_refused >= 100 and n_equal >= 60
