@@ -38,6 +38,7 @@ struct Ctrl {  // zeroed before every encode with one memset
     uint32_t huff_err;   // k_tables
     // ----
     int seam[2];         // [0] skip bits, [1] ext byte XOR 0xFF (so that all-zero means "whole image": skip 0, pad with ones)
+    uint32_t fdct_ticket[32];   // k_fdct's tile tickets, one per launch (MCU-row group) of an encode
 };
 
 struct HostRet {  // pinned
@@ -142,14 +143,12 @@ static int make_geom(int W, int H, int css, Geom *g) {
     const long long nb = (long long)g->mcux * g->mcuy * g->bpm;
     if (nb > 0x7fffffffLL / 64) return B2J_EINVAL;
     g->nblocks = (int)nb;
-    // fdct tiles: as even as possible, an even MCU count per tile (16-byte alignment of the bulk copies)
-    const int tmax = fdct_tm_max(g->hs, g->vs, g->nc);
-    g->tiles_x = (g->mcux + tmax - 1) / tmax;
-    int tm = (g->mcux + g->tiles_x - 1) / g->tiles_x;
-    tm = (tm + 1) & ~1;
-    if (tm > tmax) tm = tmax;
-    g->tm = tm;
-    g->tiles_x = (g->mcux + tm - 1) / tm;
+    // fdct tiles: TM_MAX MCUs each (even, so every tile's rows start 16-byte aligned for the bulk copies), the last
+    // tile of a row takes the remainder. k_fdct's CTAs are persistent, so a short tile costs only its own blocks, and
+    // every other tile fills whole warps of stage B. The remainder has the parity of mcux, as it had with any even
+    // tile width, so the bulk-copy alignment rule for the last tile decides as before.
+    g->tm = fdct_tm_max(g->hs, g->vs, g->nc);
+    g->tiles_x = (g->mcux + g->tm - 1) / g->tm;
     g->ntiles = g->tiles_x * g->mcuy;
     return B2J_OK;
 }
@@ -367,7 +366,7 @@ int b2j_strip_phase1(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width,
     rc = set_strip_geom(ctx, width, rows); if (rc) return rc;
     rc = enc_reset(ctx); if (rc) return rc;
     tick(ctx, 1);
-    CK(launch_fdct(d_bgr, step, ctx->g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, ctx->d_recs, ctx->d_ctrl->hist, ctx->p.optimize, 0, ctx->g.mcuy, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
+    CK(launch_fdct(d_bgr, step, ctx->g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, &ctx->d_ctrl->fdct_ticket[0], ctx->d_recs, ctx->d_ctrl->hist, ctx->p.optimize, 0, ctx->g.mcuy, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
     CK(launch_dc_edge_hist(ctx->d_recs, ctx->g, ctx->d_pred_in, ctx->d_ctrl->hist, ctx->d_ctrl->rec.last_dc, 0, ctx->d_pool, 0, nullptr, 0, ctx->stream));
     ctx->launches += 2;
     tick(ctx, 2);
@@ -463,7 +462,7 @@ int b2j_strip_phase1x(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width
     rc = enc_reset(ctx); if (rc) return rc;
     tick(ctx, 1);
     // symbol counts are always taken: they also give every strip's bit count once the tables are known
-    CK(launch_fdct(d_bgr, step, ctx->g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, ctx->d_recs, ctx->d_ctrl->hist, 1, 0, ctx->g.mcuy, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
+    CK(launch_fdct(d_bgr, step, ctx->g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, &ctx->d_ctrl->fdct_ticket[0], ctx->d_recs, ctx->d_ctrl->hist, 1, 0, ctx->g.mcuy, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
     tick(ctx, 2);
     CK(launch_dc_edge_hist(ctx->d_recs, ctx->g, ctx->d_pred_in, ctx->d_ctrl->hist, ctx->d_ctrl->rec.last_dc, 1, ctx->d_pool, 1, &ctx->d_ctrl->rec, 0, ctx->stream));
     ctx->launches += 2;
@@ -575,7 +574,7 @@ int b2j_encode_device(b2j_ctx *ctx, const uint8_t *d_bgr, size_t step, int width
     tick(ctx, 0);
     rc = enc_reset(ctx); if (rc) return rc;
     tick(ctx, 1);
-    CK(launch_fdct(d_bgr, step, ctx->g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, ctx->d_recs, ctx->d_ctrl->hist, ctx->p.optimize, 0, ctx->g.mcuy, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
+    CK(launch_fdct(d_bgr, step, ctx->g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, &ctx->d_ctrl->fdct_ticket[0], ctx->d_recs, ctx->d_ctrl->hist, ctx->p.optimize, 0, ctx->g.mcuy, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
     ctx->launches += 1;
     tick(ctx, 2);
     rc = enc_tail(ctx, width, height); if (rc) return rc;
@@ -717,6 +716,7 @@ static int upload_fdct_group(b2j_ctx *ctx, const uint8_t *bgr, size_t step, size
     const int rows_per = (g.mcuy + ngroups - 1) / ngroups;
     const int my0 = gi * rows_per;
     if (my0 >= g.mcuy) return B2J_OK;
+    if (gi >= 32) return B2J_EINVAL;   // one k_fdct ticket per group (Ctrl::fdct_ticket)
     const int mcu_h = 8 * g.vs, width = g.W, height = g.H;
     const size_t row_bytes = (size_t)width * chans(ctx);
     const int nr = std::min(rows_per, g.mcuy - my0);
@@ -740,7 +740,7 @@ static int upload_fdct_group(b2j_ctx *ctx, const uint8_t *bgr, size_t step, size
     }
     CK(cudaEventRecord(ctx->ev_copy[gi], ctx->copy_stream));
     CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_copy[gi], 0));
-    CK(launch_fdct(ctx->d_img, dstep, g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, ctx->d_recs, ctx->d_ctrl->hist, do_hist, my0, nr, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
+    CK(launch_fdct(ctx->d_img, dstep, g, ctx->d_quant, ctx->d_pool, &ctx->d_ctrl->pool_count, &ctx->d_ctrl->fdct_ticket[gi], ctx->d_recs, ctx->d_ctrl->hist, do_hist, my0, nr, (ctx->debug & 1) ? ctx->d_coef : nullptr, ctx->stream));
     ctx->launches += 1;
     return B2J_OK;
 }

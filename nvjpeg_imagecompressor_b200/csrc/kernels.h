@@ -8,8 +8,8 @@ namespace b2j {
 int fdct_tm_max(int hs, int vs, int nc);   // MCUs per fdct tile (even); nc = components per image
 // MCU rows [my0, my0+nrows) of the image `img` (img points at pixel row 0); coef_dump != NULL also writes coefficients
 cudaError_t launch_fdct(const uint8_t *img, size_t step, const Geom &g, const QuantDev *qd, uint32_t *pool,
-                        uint32_t *pool_count, TileRec *recs, uint32_t *hist, int do_hist, int my0, int nrows,
-                        int16_t *coef_dump, cudaStream_t s);
+                        uint32_t *pool_count, uint32_t *ticket, TileRec *recs, uint32_t *hist, int do_hist, int my0, int nrows,
+                        int16_t *coef_dump, cudaStream_t s);   // ticket: zeroed, one per launch
 // xr != NULL: one-collective strip exchange (first MCU left to k_strip_merge, record fields filled)
 // resolve != 0: also rewrite each tile's three raw-DC tokens in `pool` as final DC-difference tokens
 cudaError_t launch_dc_edge_hist(const TileRec *recs, const Geom &g, const int16_t *pred_in, uint32_t *hist,
