@@ -15,6 +15,7 @@ public:
     b2j_ctx *enc = nullptr, *dec = nullptr;
     int ngpus = 1, restart_rows = 0;
     int decode_scale = 1;         // setDecodeScale: decode() returns the image at 1 / decode_scale
+    int decode_region[4] = {0, 0, 0, 0};   // setDecodeRegion: ... and of that, the rectangle x, y, w, h (w = 0: all of it)
     b2j_multi *multi = nullptr;   // compress() over several GPUs (ngpus > 1)
     static bool quiet() { return getenv("B2J_QUIET") != nullptr; }
     int ensure(b2j_ctx **c) {
@@ -118,14 +119,20 @@ std::vector<unsigned char> NvjpegCompressRunner::compress(cv::Mat image, int *ru
     return obuffer;
 }
 
-// JPEG bytes -> pixels at 1 / scale. The scale is set on the (possibly shared) context for this call only: compress()
-// and reconstruct() keep seeing full-size decodes.
-static cv::Mat decode_at(NvjpegCompressRunnerImpl *m, const std::vector<unsigned char> &jpg, int scale) {
+// JPEG bytes -> pixels at 1 / scale, the rectangle `region` of them (NULL: all). Scale and region are set on the
+// (possibly shared) context for this call only: compress() and reconstruct() keep seeing full-size decodes.
+static cv::Mat decode_at(NvjpegCompressRunnerImpl *m, const std::vector<unsigned char> &jpg, int scale, const int *region) {
     cv::Mat result;
     b2j_ctx *c = m->dec ? m->dec : m->enc;
     if (!c || jpg.empty()) return result;
     if (b2j_set_decode_scale(c, scale) != B2J_OK) {
         std::cerr << "[ERROR] decode: invalid decode scale " << scale << " (1, 2, 4 or 8)" << std::endl;
+        return result;
+    }
+    if (region && b2j_set_decode_region(c, region[0], region[1], region[2], region[3]) != B2J_OK) {
+        std::cerr << "[ERROR] decode: invalid decode region " << region[2] << "x" << region[3] << " at (" << region[0] << ", "
+                  << region[1] << ")" << std::endl;
+        b2j_set_decode_scale(c, 1);
         return result;
     }
     int w = 0, h = 0;
@@ -137,16 +144,20 @@ static cv::Mat decode_at(NvjpegCompressRunnerImpl *m, const std::vector<unsigned
         }
     }
     b2j_set_decode_scale(c, 1);
+    b2j_set_decode_region(c, 0, 0, 0, 0);
     return result;
 }
 
 cv::Mat NvjpegCompressRunner::reconstruct(const std::vector<unsigned char> &jpg, int *run_state) {
-    cv::Mat result = decode_at(compressor, jpg, 1);   // full size: differenceMap / psnr compare it with the original
+    cv::Mat result = decode_at(compressor, jpg, 1, nullptr);   // full size: differenceMap / psnr compare it with the original
     if (run_state) *run_state = result.empty() ? 0 : 1;
     return result;
 }
 
 void NvjpegCompressRunner::setDecodeScale(int denom) { compressor->decode_scale = denom; }
+void NvjpegCompressRunner::setDecodeRegion(int x, int y, int w, int h) {
+    compressor->decode_region[0] = x; compressor->decode_region[1] = y; compressor->decode_region[2] = w; compressor->decode_region[3] = h;
+}
 
 cv::Mat NvjpegCompressRunner::decode(std::string image_path, int *run_state) {
     FILE *f = fopen(image_path.c_str(), "rb");
@@ -163,7 +174,7 @@ cv::Mat NvjpegCompressRunner::decode(std::string image_path, int *run_state) {
     const size_t rd = jpg.empty() ? 0 : fread(jpg.data(), 1, jpg.size(), f);
     fclose(f);
     cv::Mat result;
-    if (rd == jpg.size() && !jpg.empty()) result = decode_at(compressor, jpg, compressor->decode_scale);
+    if (rd == jpg.size() && !jpg.empty()) result = decode_at(compressor, jpg, compressor->decode_scale, compressor->decode_region);
     else std::cerr << "[INFO] Failed to read the entire JPEG data." << std::endl;
     if (run_state) *run_state = result.empty() ? 0 : 1;
     auto ms = std::chrono::duration_cast<std::chrono::milliseconds>(std::chrono::steady_clock::now() - t0).count();

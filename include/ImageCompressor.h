@@ -9,7 +9,7 @@
 //   * CUDA failures never exit(1) (ImageCompressorImpl.cuh:16-34); they produce the documented failure signal
 //   * reconstruct / differenceMap / psnr / secondaryCompress implement the README's feature bullet (README.md:8)
 //   * a defaulted 6th constructor argument spreads compress() over several GPUs; setRestartRows() turns DRI/RSTn on;
-//     setDecodeScale() makes decode() return a reduced image (cv::IMREAD_REDUCED_*)
+//     setDecodeScale() makes decode() return a reduced image (cv::IMREAD_REDUCED_*), setDecodeRegion() one rectangle of it
 #ifndef IMAGECOMPRESSOR_H_
 #define IMAGECOMPRESSOR_H_
 
@@ -81,6 +81,10 @@ public:
     // scaling, ceil(W / denom) x ceil(H / denom) pixels. Any other value makes decode() give the failure signal.
     // reconstruct() stays full size (differenceMap / psnr compare it with the original).
     void setDecodeScale(int denom);
+    // decode() returns only columns x .. x + w - 1 and rows y .. y + h - 1 of what it would return without it (after the
+    // decode scale); (0, 0, 0, 0), the default, is the whole image. A region that is invalid or does not lie inside the
+    // file's output size makes decode() give the failure signal. reconstruct() stays full size.
+    void setDecodeRegion(int x, int y, int w, int h);
 
     // README.md:8 -- reconstruction, difference map, secondary compression, PSNR
     cv::Mat reconstruct(const std::vector<unsigned char> &obuffer, int *run_state);

@@ -145,6 +145,17 @@ B2J_API int b2j_decode_scan_device(b2j_ctx *ctx, const uint8_t *hdr, size_t hdr_
  * A context sized W x H decodes files up to that size at every scale. b2j_peek still reports the file's size; the
  * encoders, the strips, b2j_reconstruct_* and b2j_secondary* are not affected. */
 B2J_API int b2j_set_decode_scale(b2j_ctx *ctx, int denom);
+/* Region decode: the decodes return only columns x .. x + w - 1 and rows y .. y + h - 1 of what they would return
+ * without it, in output coordinates (after the decode scale; with height_override, of the overridden image).
+ * (0, 0, 0, 0), the default, is the whole image. A negative value, only one of w and h zero, or w = h = 0 with x or y
+ * non-zero return B2J_EINVAL and leave the setting unchanged. It applies to b2j_decode, b2j_decode_device /
+ * b2j_decode_finish and b2j_decode_scan_device: their width / height report w x h (also with a NULL image), `step` is
+ * checked against w, and not one byte of the caller's image outside the w x h rectangle (pitch padding included) is
+ * written. A rectangle that does not lie inside the file's output size returns B2J_EINVAL before anything runs. Only
+ * the MCUs around the rectangle are transformed; in a file with restart markers only the intervals that hold them are
+ * entropy-decoded. A b2j_decode_device keeps the region it was issued with until b2j_decode_finish. b2j_peek, the
+ * encoders, the strips, b2j_reconstruct_* and b2j_secondary* are not affected. */
+B2J_API int b2j_set_decode_region(b2j_ctx *ctx, int x, int y, int w, int h);
 /* Completes the last b2j_decode_device: waits for it and validates it. The decode runs a fixed schedule of Huffman
  * synchronisation launches without asking the host; in the rare case that was too short the image is decoded again
  * here with the checked schedule. `jpg` of the b2j_decode_device call must stay valid until this returns. */

@@ -96,7 +96,9 @@ struct b2j_ctx {
     size_t last_len, last_step;
     uint8_t *last_bgr;
     int last_scale;                // ... and the scale it was issued with (its checked retry keeps it)
+    int last_region[4];            // ... and the region
     int dec_scale;                 // decode output at 1 / dec_scale (1, 2, 4, 8); b2j_set_decode_scale
+    int dec_region[4];             // x, y, w, h of the decode output (w = 0: all of it); b2j_set_decode_region
     b2j_ctx *second;  // encoder for the difference image (secondary compression)
     uint8_t *d_rplanes; size_t rplanes_bytes;   // reconstruction from the encoder's coefficients: sample planes
     void *d_rtb;                                // ... and de-quantisation tables (a DecTables with q filled)
@@ -325,6 +327,13 @@ int b2j_set_restart_rows(b2j_ctx *ctx, int rows) {
 int b2j_set_decode_scale(b2j_ctx *ctx, int denom) {
     if (!ctx || (denom != 1 && denom != 2 && denom != 4 && denom != 8)) return B2J_EINVAL;
     ctx->dec_scale = denom;
+    return B2J_OK;
+}
+// Region decode: one rectangle of the output (after the scale). The back end transforms only the MCUs around it; with
+// restart markers the entropy stages decode only the intervals that hold them (dec.cu dec_run).
+int b2j_set_decode_region(b2j_ctx *ctx, int x, int y, int w, int h) {
+    if (!ctx || x < 0 || y < 0 || w < 0 || h < 0 || (w == 0) != (h == 0) || (w == 0 && (x || y))) return B2J_EINVAL;
+    ctx->dec_region[0] = x; ctx->dec_region[1] = y; ctx->dec_region[2] = w; ctx->dec_region[3] = h;
     return B2J_OK;
 }
 uint64_t b2j_launch_count(const b2j_ctx *ctx) { return ctx ? ctx->launches : 0; }
@@ -1004,20 +1013,37 @@ static int check_components(b2j_ctx *ctx, int file_css) {
     return B2J_EFORMAT;
 }
 
-// sequential files: asynchronous (careful = false: dec_check may ask for a checked retry); progressive files: scan by
-// scan (dec_prog.cu), synchronous
-static int decode_parsed(b2j_ctx *ctx, const uint8_t *jpg, size_t len, const JpegInfo &info, uint8_t *d_bgr, size_t step, bool careful,
-                         int scale, const uint8_t *d_scan_src = nullptr) {
-    if (step < (size_t)dec_scaled_size(info.W, scale) * chans(ctx)) return B2J_EINVAL;
-    int rc = dec_ensure(ctx); if (rc) return rc;
-    Geom g; rc = make_geom(info.W, info.H, info.css, &g); if (rc) return rc;
-    if (info.progressive) return dec_run_progressive(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, &ctx->launches, scale);
-    dec_set_spec_launches(ctx->dec, (ctx->debug & 4) ? 1 : 3);
-    return dec_run(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, ctx->timing ? &ctx->tm : nullptr,
-                   &ctx->launches, careful, d_scan_src, scale);
+// The output size of a decode of `info` at `scale` with `region` (w = 0: the whole image); B2J_EINVAL with an error
+// text if the region does not lie inside the image
+static int out_size(b2j_ctx *ctx, const JpegInfo &info, int scale, const int region[4], int *ow, int *oh) {
+    const int W = dec_scaled_size(info.W, scale), H = dec_scaled_size(info.H, scale);
+    if (region[2] == 0) { *ow = W; *oh = H; return B2J_OK; }
+    if ((long long)region[0] + region[2] > W || (long long)region[1] + region[3] > H) {
+        snprintf(ctx->err, sizeof(ctx->err), "decode region %dx%d at (%d, %d) does not lie inside the %dx%d output", region[2], region[3],
+                 region[0], region[1], W, H);
+        return B2J_EINVAL;
+    }
+    *ow = region[2]; *oh = region[3];
+    return B2J_OK;
 }
 
-static int parse_for(b2j_ctx *ctx, const uint8_t *jpg, size_t len, JpegInfo *info, int *width, int *height) {
+// sequential files: asynchronous (careful = false: dec_check may ask for a checked retry); progressive files: scan by
+// scan (dec_prog.cu), synchronous. d_bgr receives the region (the whole output if region[2] = 0).
+static int decode_parsed(b2j_ctx *ctx, const uint8_t *jpg, size_t len, const JpegInfo &info, uint8_t *d_bgr, size_t step, bool careful,
+                         int scale, const int region[4], const uint8_t *d_scan_src = nullptr) {
+    int ow, oh;
+    int rc = out_size(ctx, info, scale, region, &ow, &oh); if (rc) return rc;
+    if (step < (size_t)ow * chans(ctx)) return B2J_EINVAL;
+    rc = dec_ensure(ctx); if (rc) return rc;
+    Geom g; rc = make_geom(info.W, info.H, info.css, &g); if (rc) return rc;
+    if (info.progressive) return dec_run_progressive(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, &ctx->launches, scale, region);
+    dec_set_spec_launches(ctx->dec, (ctx->debug & 4) ? 1 : 3);
+    return dec_run(ctx->dec, jpg, len, info, g, d_bgr, step, chans(ctx) == 1, ctx->stream, ctx->timing ? &ctx->tm : nullptr,
+                   &ctx->launches, careful, d_scan_src, scale, region);
+}
+
+// region != NULL: the output size with that region (checked against the file) goes to *width / *height
+static int parse_for(b2j_ctx *ctx, const uint8_t *jpg, size_t len, JpegInfo *info, int *width, int *height, const int *region) {
     int rc = parse_jpeg(jpg, len, info);
     if (rc) { snprintf(ctx->err, sizeof(ctx->err), "unsupported or corrupt JPEG (parse rc=%d)", rc); return B2J_EFORMAT; }
     rc = check_components(ctx, info->css); if (rc) return rc;
@@ -1026,8 +1052,11 @@ static int parse_for(b2j_ctx *ctx, const uint8_t *jpg, size_t len, JpegInfo *inf
                  "libjpeg would block-smooth it, which this decoder does not do");
         return B2J_EFORMAT;
     }
-    if (width) *width = dec_scaled_size(info->W, ctx->dec_scale);
-    if (height) *height = dec_scaled_size(info->H, ctx->dec_scale);
+    if (!region) return B2J_OK;
+    int ow, oh;
+    rc = out_size(ctx, *info, ctx->dec_scale, region, &ow, &oh); if (rc) return rc;
+    if (width) *width = ow;
+    if (height) *height = oh;
     return B2J_OK;
 }
 
@@ -1044,15 +1073,16 @@ int b2j_decode_device(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *d_b
     if (!ctx || !jpg) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     JpegInfo info;
-    int rc = parse_for(ctx, jpg, len, &info, width, height);
+    int rc = parse_for(ctx, jpg, len, &info, width, height, ctx->dec_region);
     if (rc || !d_bgr) return rc;
     // one decode in flight per context: an unfinished predecessor is finished (validated, retried if needed) first
     if (ctx->last_jpg) { rc = b2j_decode_finish(ctx); if (rc) return rc; }
     // progressive files decode synchronously: nothing is left for b2j_decode_finish
-    if (info.progressive) return decode_parsed(ctx, jpg, len, info, d_bgr, step, false, ctx->dec_scale);
+    if (info.progressive) return decode_parsed(ctx, jpg, len, info, d_bgr, step, false, ctx->dec_scale, ctx->dec_region);
     // remembered for b2j_decode_finish: the caller keeps `jpg` alive until then
     ctx->last_jpg = jpg; ctx->last_len = len; ctx->last_bgr = d_bgr; ctx->last_step = step; ctx->last_scale = ctx->dec_scale;
-    return decode_parsed(ctx, jpg, len, info, d_bgr, step, false, ctx->last_scale);
+    memcpy(ctx->last_region, ctx->dec_region, sizeof(ctx->last_region));
+    return decode_parsed(ctx, jpg, len, info, d_bgr, step, false, ctx->last_scale, ctx->last_region);
 }
 
 // A baseline JPEG whose entropy-coded segment is already in DEVICE memory (the output of b2j_encode_device, a slice
@@ -1067,17 +1097,19 @@ int b2j_decode_scan_device(b2j_ctx *ctx, const uint8_t *hdr, size_t hdr_len, con
     CK(cudaSetDevice(ctx->device));
     if (ctx->last_jpg) { int rf = b2j_decode_finish(ctx); if (rf) return rf; }
     JpegInfo info;
-    int rc = parse_for(ctx, hdr, hdr_len, &info, nullptr, nullptr); if (rc) return rc;
+    int rc = parse_for(ctx, hdr, hdr_len, &info, nullptr, nullptr, nullptr); if (rc) return rc;
     if (info.progressive) { snprintf(ctx->err, sizeof(ctx->err), "progressive JPEG: one scan in device memory cannot be decoded"); return B2J_EFORMAT; }
     JpegScan &sc = info.scans[0];
     if (sc.seg_off != hdr_len) { snprintf(ctx->err, sizeof(ctx->err), "hdr must end with the SOS header"); return B2J_EINVAL; }
     if (height_override > 0) info.H = height_override;
     sc.seg_off = 0; sc.seg_len = scan_len;
     const int scale = ctx->dec_scale;
-    if (width) *width = dec_scaled_size(info.W, scale);
-    if (height) *height = dec_scaled_size(info.H, scale);
+    int ow, oh;
+    rc = out_size(ctx, info, scale, ctx->dec_region, &ow, &oh); if (rc) return rc;
+    if (width) *width = ow;
+    if (height) *height = oh;
     for (int attempt = 0; attempt < 2; attempt++) {
-        rc = decode_parsed(ctx, hdr, hdr_len, info, d_bgr, step, attempt == 1, scale, d_scan); if (rc) return rc;
+        rc = decode_parsed(ctx, hdr, hdr_len, info, d_bgr, step, attempt == 1, scale, ctx->dec_region, d_scan); if (rc) return rc;
         rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
         if (rc != DEC_RETRY) break;
     }
@@ -1091,8 +1123,9 @@ int b2j_decode_finish(b2j_ctx *ctx) {
     int rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
     if (rc == DEC_RETRY) {   // the speculative synchronisation schedule was too short for this stream: decode again, checked
         JpegInfo info;
-        rc = parse_for(ctx, ctx->last_jpg, ctx->last_len, &info, nullptr, nullptr); if (rc) return rc;
-        rc = decode_parsed(ctx, ctx->last_jpg, ctx->last_len, info, ctx->last_bgr, ctx->last_step, true, ctx->last_scale); if (rc) return rc;
+        rc = parse_for(ctx, ctx->last_jpg, ctx->last_len, &info, nullptr, nullptr, nullptr); if (rc) return rc;
+        rc = decode_parsed(ctx, ctx->last_jpg, ctx->last_len, info, ctx->last_bgr, ctx->last_step, true, ctx->last_scale, ctx->last_region);
+        if (rc) return rc;
         rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
     }
     ctx->last_jpg = nullptr;
@@ -1103,14 +1136,16 @@ int b2j_decode(b2j_ctx *ctx, const uint8_t *jpg, size_t len, uint8_t *bgr, size_
     if (!ctx || !jpg) return B2J_EINVAL;
     CK(cudaSetDevice(ctx->device));
     JpegInfo info;
-    int rc = parse_for(ctx, jpg, len, &info, width, height);
+    int rc = parse_for(ctx, jpg, len, &info, width, height, ctx->dec_region);
     if (rc || !bgr) return rc;
-    const int ch = chans(ctx), scale = ctx->dec_scale, ow = dec_scaled_size(info.W, scale), oh = dec_scaled_size(info.H, scale);
+    const int ch = chans(ctx), scale = ctx->dec_scale;
+    int ow, oh;
+    rc = out_size(ctx, info, scale, ctx->dec_region, &ow, &oh); if (rc) return rc;
     if (step < (size_t)ow * ch) return B2J_EINVAL;
     const size_t dstep = ((size_t)ow * ch + 15) & ~(size_t)15;
     rc = ensure_recon(ctx, dstep * oh); if (rc) return rc;
     for (int attempt = 0; attempt < 2; attempt++) {
-        rc = decode_parsed(ctx, jpg, len, info, ctx->d_recon, dstep, attempt == 1, scale);
+        rc = decode_parsed(ctx, jpg, len, info, ctx->d_recon, dstep, attempt == 1, scale, ctx->dec_region);
         if (rc) return rc;
         rc = download_2d(ctx, bgr, step, ctx->d_recon, dstep, (size_t)ow * ch, oh, ctx->stream); if (rc) return rc;
         rc = dec_check(ctx->dec, ctx->err, sizeof(ctx->err));
@@ -1203,7 +1238,7 @@ int b2j_reconstruct_planes(b2j_ctx *ctx, b2j_recon_planes *out) {
         CK(cudaMalloc(&ctx->d_rtb, dec_tables_size()));
         CK(cudaMemcpy(ctx->d_rtb, h.data(), h.size(), cudaMemcpyHostToDevice));
     }
-    CK(launch_idct(ctx->d_coef, nullptr, g, ctx->d_rtb, py, pcb, pcr, 0, ctx->stream));
+    CK(launch_idct(ctx->d_coef, nullptr, g, nullptr, ctx->d_rtb, py, pcb, pcr, 0, ctx->stream));
     ctx->launches += 1;
     if (out) {
         const size_t cs = (size_t)g.mcux * 8;
@@ -1227,7 +1262,7 @@ int b2j_reconstruct_color(b2j_ctx *ctx, uint8_t *d_bgr, size_t step, int halo_to
     CK(cudaSetDevice(ctx->device));
     uint8_t *py, *pcb, *pcr;
     int rc = recon_layout(ctx, &py, &pcb, &pcr); if (rc) return rc;
-    CK(launch_upcolor(py, pcb, pcr, g, d_bgr, step, ctx->stream, halo_top, halo_bottom));
+    CK(launch_upcolor(py, pcb, pcr, g, nullptr, d_bgr, step, ctx->stream, halo_top, halo_bottom));
     ctx->launches += 1;
     return B2J_OK;
 }

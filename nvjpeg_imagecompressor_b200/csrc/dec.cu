@@ -22,6 +22,8 @@ struct DecCtrl {
     uint32_t changed;
     uint32_t changed_alt;   // the launches of the fixed schedule alternate between the two flags
     uint32_t nmark;      // restart markers found by k_destuff
+    uint64_t r_len;      // decode region: bytes of the restart intervals it needs (k_dec_range) ...
+    uint32_t r_nmark;    // ... and the markers between them
 };
 
 struct Decoder {
@@ -34,8 +36,8 @@ struct Decoder {
     uint64_t *d_st_in = nullptr, *d_st_out = nullptr;
     uint32_t *d_nblk = nullptr, *d_blk_start = nullptr;
     uint8_t *d_done = nullptr;   // per decoder chunk (256 subsequences): first synchronisation pass has run
-    uint32_t *d_bnd = nullptr;   // restart intervals: start offsets in the unstuffed stream (k_destuff<true>)
-    size_t bnd_cap = 0;
+    uint32_t *d_bnd = nullptr;   // restart intervals: start offsets in the unstuffed stream (k_destuff<true>); a second
+    size_t bnd_cap = 0;          // array of bnd_cap entries behind it: those of a decode region's intervals (k_dec_range)
     size_t nsub_cap = 0;
     cudaStream_t up_stream = nullptr;   // uploads of the scan pieces
     cudaEvent_t ev_up[33] = {};
@@ -111,26 +113,27 @@ void dec_set_spec_launches(Decoder *d, int n) { d->spec_launches = n < 1 ? 1 : n
 
 const void *dec_coef_ptr(Decoder *d, size_t *bytes) { *bytes = (size_t)d->nblocks_cap * 128; return d->d_coef; }
 
-// the back end's sample planes in one buffer: Y (mcux 8 hs x mcuy 8 vs), then Cb and Cr (mcux 8 x mcuy 8 each), every
-// plane at a multiple of 64 bytes
+// the back end's sample planes in one buffer: Y (pitch ys, yrows rows), then Cb and Cr (pitch cs, crows rows each),
+// every plane at a multiple of 64 bytes; the window (dec_window) says what they hold
 struct PlaneLayout {
     size_t cb, cr, bytes;   // offsets of Cb and Cr; the buffer size
 };
-static PlaneLayout plane_layout(const Geom &g) {
-    const size_t y = (size_t)g.mcux * 8 * g.hs * g.mcuy * 8 * g.vs, c = (size_t)g.mcux * 8 * g.mcuy * 8;
+static PlaneLayout plane_layout(const DecWin &w) {
+    const size_t y = (size_t)w.ys * w.yrows, c = (size_t)w.cs * w.crows;
     PlaneLayout l;
     l.cb = (y + 63) & ~(size_t)63;
     l.cr = l.cb + ((c + 63) & ~(size_t)63);
     l.bytes = y + 2 * c + 256;
     return l;
 }
+size_t dec_planes_bytes(const DecWin &w) { return plane_layout(w).bytes; }
 
-static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interval) {
+static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interval, size_t planes_bytes) {
     if (restart_interval > 0) {
         const size_t need = ((size_t)g.mcux * g.mcuy + restart_interval - 1) / restart_interval + 2;
         if (need > d->bnd_cap) {
             cudaFree(d->d_bnd); d->d_bnd = nullptr; d->bnd_cap = 0;
-            DCK(cudaMalloc(&d->d_bnd, (need + need / 4) * 4));
+            DCK(cudaMalloc(&d->d_bnd, (need + need / 4) * 4 * 2));
             d->bnd_cap = need + need / 4;
         }
     }
@@ -160,7 +163,7 @@ static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interv
         DCK(cudaMalloc(&d->d_desc, nd * 5 * 8));
         d->desc_cap = nd;
     }
-    const size_t pl = plane_layout(g).bytes;
+    const size_t pl = planes_bytes;
     if (pl > d->planes_cap) {
         cudaFree(d->d_planes); d->d_planes = nullptr; d->planes_cap = 0;
         DCK(cudaMalloc(&d->d_planes, pl));
@@ -169,25 +172,25 @@ static int ensure(Decoder *d, size_t scan_len, const Geom &g, int restart_interv
     return B2J_OK;
 }
 
-cudaError_t dec_back_end(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *planes, uint8_t *d_bgr,
-                         size_t step, bool gray_out, int scale, int rst_mcus, cudaStream_t s, cudaEvent_t ev_idct,
+cudaError_t dec_back_end(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecWin &w, const void *tb, uint8_t *planes,
+                         uint8_t *d_bgr, size_t step, bool gray_out, int scale, int rst_mcus, cudaStream_t s, cudaEvent_t ev_idct,
                          cudaEvent_t ev_color, uint64_t *launches) {
-    const PlaneLayout pl = plane_layout(g);
+    const PlaneLayout pl = plane_layout(w);
     uint8_t *py = planes, *pcb = planes + pl.cb, *pcr = planes + pl.cr;
     cudaError_t e;
     Geom view = g;   // the geometry of the colour pass
     if (scale > 1) {   // reduced size: the scaled IDCT (gray: straight into the caller's image), colour on the scaled view
         const DecScale sc = dec_scale_setup(g, scale);
-        e = launch_idct_scaled(coef, dcarr, g, sc, tb, gray_out ? d_bgr : py, pcb, pcr, gray_out, step, rst_mcus, s);
+        e = launch_idct_scaled(coef, dcarr, g, sc, w, tb, gray_out ? d_bgr : py, pcb, pcr, gray_out, step, rst_mcus, s);
         view = sc.view;
     } else if (gray_out) {   // Y straight from the IDCT into the caller's image: no planes
-        e = launch_idct_gray(coef, dcarr, g, tb, d_bgr, step, rst_mcus, s);
+        e = launch_idct_gray(coef, dcarr, g, w, tb, d_bgr, step, rst_mcus, s);
     } else {
-        e = launch_idct(coef, dcarr, g, tb, py, pcb, pcr, rst_mcus, s);
+        e = launch_idct(coef, dcarr, g, &w, tb, py, pcb, pcr, rst_mcus, s);
     }
     if (e != cudaSuccess) return e;
     if (ev_idct) cudaEventRecord(ev_idct, s);
-    if (!gray_out && (e = launch_upcolor(py, pcb, pcr, view, d_bgr, step, s)) != cudaSuccess) return e;
+    if (!gray_out && (e = launch_upcolor(py, pcb, pcr, view, &w, d_bgr, step, s)) != cudaSuccess) return e;
     if (ev_color) cudaEventRecord(ev_color, s);   // gray: no colour pass (dec_color stays 0)
     if (launches) (*launches) += gray_out ? 1 : 2;
     return cudaSuccess;
@@ -195,13 +198,23 @@ cudaError_t dec_back_end(const int16_t *coef, const int16_t *dcarr, const Geom &
 
 int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr, size_t step,
             bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src,
-            int scale) {
+            int scale, const int *region) {
     const JpegScan &sc = info.scans[0];
     const int rst = sc.restart_interval;   // MCUs per restart interval (0: none)
     if (rst && sc.seg_len >= 0xFFFFFFF0ull) { snprintf(d->err, d->errlen, "restart-marker scans of 4 GB and more are not supported"); return B2J_EFORMAT; }
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
     if ((!d_scan_src && sc.seg_off + sc.seg_len > len) || sc.seg_len == 0) return B2J_EFORMAT;
-    int rc = ensure(d, sc.seg_len, g, rst);
+    const int whole[4] = {0, 0, 0, 0};
+    DecWin win = dec_window(g, scale, region ? region : whole);
+    // A region that does not need every MCU: the entropy stages decode up to its last needed block and store whole
+    // blocks for its needed MCUs only; with restart markers they decode only the intervals j0 .. j1 that hold needed
+    // MCUs (k_dec_range), and block 0 is then the first block of interval j0.
+    const bool part = !dec_window_full(win, g);
+    const int fm = win.my0 * g.mcux + win.mx0, lm = (win.my1 - 1) * g.mcux + win.mx1 - 1;   // first / last needed MCU
+    const uint32_t j0 = rst ? (uint32_t)(fm / rst) : 0, j1 = rst ? (uint32_t)(lm / rst) : 0;
+    if (part && rst) win.m0 = (int)j0 * rst;
+    const uint32_t nblk_dec = part ? (uint32_t)((lm + 1 - win.m0) * g.bpm) : (uint32_t)g.nblocks;   // blocks the write stage stores
+    int rc = ensure(d, sc.seg_len, g, rst, dec_planes_bytes(win));
     if (rc) return rc;
     const size_t n = sc.seg_len;
     const size_t nsub_max = (n * 8 + DEC_SUB_BITS - 1) / DEC_SUB_BITS;
@@ -236,7 +249,7 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
     // restart markers: one piece (a marker's two bytes may straddle pieces: k_destuff looks one byte ahead)
     const int npieces = (spec && n >= (16u << 20) && !rst && !d_scan_src) ? 8 : 1;   // fewer, larger pieces: a piece should fill the GPU
     uint32_t *bnd = rst ? d->d_bnd : nullptr;
-    const uint32_t *nmark = rst ? &d->d_ctrl->nmark : nullptr;
+    const uint32_t *nmark = rst ? &d->d_ctrl->nmark : nullptr;   // (the stages after the front end: a region's intervals)
     const size_t piece = ((n + npieces - 1) / npieces + DS_CHUNK - 1) & ~(size_t)(DS_CHUNK - 1);
     DCK(cudaEventRecord(d->ev_up[32], s));                       // the scan buffer is free once earlier work on s is done
     DCK(cudaStreamWaitEvent(d->up_stream, d->ev_up[32], 0));
@@ -264,6 +277,15 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
             if (launches) (*launches)++;
         }
     }
+    // the entropy stages' stream: the whole scan, or a region's restart intervals
+    const uint8_t *u = d->d_u;
+    const uint64_t *u_len = &d->d_ctrl->u_len;
+    if (part && rst) {   // (the scan buffer is free: k_destuff has read it)
+        DCK(launch_dec_range(d->d_u, &d->d_ctrl->u_len, d->d_bnd, &d->d_ctrl->nmark, j0, j1, d->d_scan, &d->d_ctrl->r_len,
+                             d->d_bnd + d->bnd_cap, &d->d_ctrl->r_nmark, s));
+        if (launches) (*launches)++;
+        u = d->d_scan; u_len = &d->d_ctrl->r_len; bnd = d->d_bnd + d->bnd_cap; nmark = &d->d_ctrl->r_nmark;
+    }
     if (tm) cudaEventRecord(d->ev[1], s);
     int rounds = 0;
     if (spec) {
@@ -273,7 +295,7 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
             // a launch whose predecessor in this loop moved nothing returns at once (its own flag stays 0)
             flag = (rounds & 1) ? &d->d_ctrl->changed_alt : &d->d_ctrl->changed;
             DCK(cudaMemsetAsync(flag, 0, 4, s));
-            DCK(launch_dec_sync(d->d_u, &d->d_ctrl->u_len, d->d_tb, d->d_st_in, d->d_st_out, d->d_nblk, g.bpm, hv, 8, 0, d->d_done,
+            DCK(launch_dec_sync(u, u_len, d->d_tb, d->d_st_in, d->d_st_out, d->d_nblk, g.bpm, hv, 8, 0, d->d_done,
                                 flag, nsub_max, bnd, nmark, prev, s));
             prev = flag;
             if (launches) (*launches)++;
@@ -291,7 +313,7 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
         for (;; rounds++) {
             if (rounds >= 65536) { snprintf(d->err, d->errlen, "Huffman synchronisation did not converge"); return B2J_EINTERNAL; }
             DCK(cudaMemsetAsync(&d->d_ctrl->changed, 0, 4, s));
-            DCK(launch_dec_sync_long(d->d_u, &d->d_ctrl->u_len, d->d_tb, d->d_st_in, d->d_st_out, d->d_nblk, g.bpm, hv, rounds == 0, group,
+            DCK(launch_dec_sync_long(u, u_len, d->d_tb, d->d_st_in, d->d_st_out, d->d_nblk, g.bpm, hv, rounds == 0, group,
                                      &d->d_ctrl->changed, nsub_max, bnd, nmark, s));
             if (launches) (*launches)++;
             if (rounds == 0) continue;  // the first launch always moves states
@@ -304,12 +326,12 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
     if (getenv("B2J_DEC_VERBOSE")) fprintf(stderr, "[b2j decode] %s synchronisation: %d launches, scan %zu bytes, %.1f bits/block\n", spec ? "scheduled" : "checked", d->last_rounds, n, (double)n * 8.0 / (double)g.nblocks);
     if (tm) cudaEventRecord(d->ev[2], s);
     DCK(launch_scan_u32(d->d_nblk, d->d_blk_start, nsub_max, d->d_desc + d->desc_cap, &d->d_ctrl->ticket[1], &d->d_ctrl->err, s));
-    DCK(launch_dec_write(d->d_u, &d->d_ctrl->u_len, d->d_tb, d->d_st_out, d->d_blk_start, g.bpm, hv, d->d_coef, d->d_dc, (uint32_t)g.nblocks,
-                         &d->d_ctrl->err, nsub_max, bnd, nmark, s));
-    DCK(launch_dc_scan(d->d_dc, g, gray_out ? 1 : g.nc, d->d_desc + 2 * d->desc_cap, &d->d_ctrl->ticket[2], d->desc_cap,
+    DCK(launch_dec_write(u, u_len, d->d_tb, d->d_st_out, d->d_blk_start, g.bpm, hv, d->d_coef, d->d_dc, nblk_dec,
+                         &d->d_ctrl->err, nsub_max, bnd, nmark, g, part ? &win : nullptr, s));
+    DCK(launch_dc_scan(d->d_dc, g, nblk_dec / g.bpm, gray_out ? 1 : g.nc, d->d_desc + 2 * d->desc_cap, &d->d_ctrl->ticket[2], d->desc_cap,
                        &d->d_ctrl->err, s));
     if (tm) cudaEventRecord(d->ev[3], s);
-    DCK(dec_back_end(d->d_coef, d->d_dc, g, d->d_tb, d->d_planes, d_bgr, step, gray_out, scale, rst, s, tm ? d->ev[4] : nullptr,
+    DCK(dec_back_end(d->d_coef, d->d_dc, g, win, d->d_tb, d->d_planes, d_bgr, step, gray_out, scale, rst, s, tm ? d->ev[4] : nullptr,
                      tm ? d->ev[5] : nullptr, launches));
     if (launches) (*launches) += 3;
     if (tm) {
@@ -325,16 +347,18 @@ int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, co
 }
 
 int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr,
-                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches, int scale) {
+                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches, int scale, const int *region) {
     if (g.nblocks > d->nblocks_cap) { snprintf(d->err, d->errlen, "image exceeds the context's size"); return B2J_ESIZE; }
-    int rc = ensure(d, 4096, g, 0);
+    const int whole[4] = {0, 0, 0, 0};
+    const DecWin win = dec_window(g, scale, region ? region : whole);   // every scan decodes whole: only the back end is windowed
+    int rc = ensure(d, 4096, g, 0, dec_planes_bytes(win));
     if (rc) return rc;
     if (d->in_flight) { DCK(cudaStreamSynchronize(d->last_stream)); d->in_flight = false; }
     d->speculated = false;
     d->last_stream = s;
     DCK(cudaMemsetAsync(&d->d_ctrl->err, 0, 4, s));
     return dec_progressive(jpg, len, info, g, d->d_coef, d->d_tb, d->d_planes, d_bgr, step, gray_out, s, launches, d->err, d->errlen,
-                           scale);
+                           scale, win);
 }
 
 int dec_check(Decoder *d, char *err, size_t errlen) {

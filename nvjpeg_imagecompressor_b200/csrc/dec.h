@@ -43,9 +43,11 @@ void dec_destroy(Decoder *d);
 // d_scan_src != NULL: the scan's stuffed bytes are already in device memory (seg_len of them): nothing is uploaded
 // gray_out: d_bgr receives one byte per pixel, the Y samples (JCS_GRAYSCALE; chroma blocks are decoded, not transformed)
 // scale 2 / 4 / 8: d_bgr receives the image at 1 / scale (dec_kernels.h dec_scale_setup), 1: full size
+// region != NULL: {x, y, w, h} of the output (w = 0: all of it), inside the output size; d_bgr receives that rectangle
+// (its pixel (x, y) at d_bgr) and nothing else (dec_kernels.h DecWin)
 int dec_run(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr, size_t step,
             bool gray_out, cudaStream_t s, b2j_timings *tm, uint64_t *launches, bool careful, const uint8_t *d_scan_src = nullptr,
-            int scale = 1);
+            int scale = 1, const int *region = nullptr);
 constexpr int DEC_RETRY = 1;
 int dec_check(Decoder *d, char *err, size_t errlen);   // synchronises the decode's stream
 // optional: how host bytes reach the device (the API layer stages pageable memory through pinned buffers); the
@@ -58,6 +60,6 @@ const void *dec_coef_ptr(Decoder *d, size_t *bytes);
 // progressive files (SOF2, what the reference as shipped writes, ImageCompressorImpl.cu:28): every scan is absorbed into
 // the coefficient array in file order, then the back end of dec_run runs
 int dec_run_progressive(Decoder *d, const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, uint8_t *d_bgr,
-                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches, int scale = 1);
+                        size_t step, bool gray_out, cudaStream_t s, uint64_t *launches, int scale = 1, const int *region = nullptr);
 
 }  // namespace b2j

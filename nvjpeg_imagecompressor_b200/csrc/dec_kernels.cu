@@ -663,12 +663,15 @@ struct DecWriteShared {
     uint32_t blk[DEC_THREADS][32];                   // word w of thread t's block at [t][w ^ (t & 31)]
 };
 
-template <bool RST>
+// WIN (a decode region): block b belongs to MCU m0 + b / bpm; the blocks of the needed MCUs (columns [mx0, mx1), rows
+// from my0 on; nblocks ends with the last needed block) are stored whole, the others only as DC differences (k_dc_scan
+// sums them), and the subsequences that begin at or after block nblocks have nothing to store.
+template <bool RST, bool WIN>
 __global__ void __launch_bounds__(DEC_THREADS)
 k_dec_write(const uint8_t *__restrict__ u, const uint64_t *__restrict__ u_len, const DecTables *__restrict__ tb,
             const uint64_t *__restrict__ st_out, const uint32_t *__restrict__ blk_start, int bpm, int hv,
             int16_t *__restrict__ coef, int16_t *__restrict__ dcarr, uint32_t nblocks, uint32_t *__restrict__ err,
-            const uint32_t *__restrict__ bnd, const uint32_t *__restrict__ nmark_p) {
+            const uint32_t *__restrict__ bnd, const uint32_t *__restrict__ nmark_p, int mcux, int m0, int mx0, int mx1, int my0) {
     extern __shared__ __align__(16) uint8_t smem_raw[];
     DecWriteShared &sh = *reinterpret_cast<DecWriteShared *>(smem_raw);
     const int tid = threadIdx.x, lane = tid & 31;
@@ -677,6 +680,7 @@ k_dec_write(const uint8_t *__restrict__ u, const uint64_t *__restrict__ u_len, c
     const size_t cta = blockIdx.x;
     const uint64_t chunk_bit0 = (uint64_t)cta * SUB_BITS * DEC_THREADS;
     if (chunk_bit0 >= total_bits) return;
+    if (WIN && blk_start[cta * DEC_THREADS] >= nblocks) return;
     {   // the chunk's words + two subsequences of lookahead, tables, empty block cells
         const uint32_t *uw = reinterpret_cast<const uint32_t *>(u);
         const size_t w0 = cta * (size_t)(SUB_WORDS * DEC_THREADS);
@@ -696,7 +700,7 @@ k_dec_write(const uint8_t *__restrict__ u, const uint64_t *__restrict__ u_len, c
     __syncthreads();
     const size_t i = cta * DEC_THREADS + tid;
     const uint64_t my_bit0 = chunk_bit0 + (uint64_t)tid * SUB_BITS;
-    const bool live = my_bit0 < total_bits;
+    const bool live = my_bit0 < total_bits && (!WIN || blk_start[i] < nblocks);
     const uint64_t in = (!live || i == 0) ? pack_state(live ? 0 : my_bit0, 0, 0) : st_out[i - 1];
     uint32_t q = (uint32_t)((in >> 16) - chunk_bit0);
     int c = (int)((in >> 8) & 0xFF), k = (int)(in & 0xFF);
@@ -770,7 +774,12 @@ k_dec_write(const uint8_t *__restrict__ u, const uint64_t *__restrict__ u_len, c
             const uint32_t w = src[lane ^ L];
             src[lane ^ L] = 0;
             if (b < nblocks) {
-                reinterpret_cast<uint32_t *>(coef)[(size_t)b * 32 + lane] = w;
+                bool store = true;
+                if (WIN) {
+                    const int m = m0 + (int)(b / (uint32_t)bpm), my = m / mcux, mx = m - my * mcux;
+                    store = mx >= mx0 && mx < mx1 && my >= my0;
+                }
+                if (store) reinterpret_cast<uint32_t *>(coef)[(size_t)b * 32 + lane] = w;
                 if (lane == 0) dcarr[b] = (int16_t)(w & 0xFFFFu);   // the DC differences also go to a compact array (k_dc_scan)
             }
         }
@@ -778,6 +787,40 @@ k_dec_write(const uint8_t *__restrict__ u, const uint64_t *__restrict__ u_len, c
         __syncwarp();
     }
     if (live && (!crossed || end_state != st_out[i])) atomicOr(err, 4u);  // the states were not a fixed point
+}
+
+// ------------------------------------------------------------------------------------------------------
+// k_dec_range: restart intervals j0 .. j1 of the de-stuffed stream as a stream of their own (a decode region needs
+// them only). Interval j spans [j ? bnd[j - 1] : 0, j < nmark ? bnd[j] : u_len). Every thread reads the two ends;
+// 4-byte words of the copy are funnel-shifted from two aligned source words (the source has k_destuff's 64 bytes of
+// padding behind its end); the copy is followed by 0xFF padding like k_destuff's output. CTA 0 writes the length and
+// the intervals' starts relative to the copy.
+__global__ void __launch_bounds__(256)
+k_dec_range(const uint8_t *__restrict__ u, const uint64_t *__restrict__ u_len, const uint32_t *__restrict__ bnd,
+            const uint32_t *__restrict__ nmark_p, uint32_t j0, uint32_t j1, uint32_t *__restrict__ dst, uint64_t *__restrict__ dst_len,
+            uint32_t *__restrict__ dst_bnd, uint32_t *__restrict__ dst_nmark) {
+    const uint64_t ul = *u_len;
+    const uint32_t nmark = *nmark_p;
+    const uint64_t off = j0 == 0 ? 0 : (j0 <= nmark ? bnd[j0 - 1] : ul);
+    const uint64_t end = j1 < nmark ? bnd[j1] : ul;
+    const uint64_t len = end > off ? end - off : 0;
+    const uint32_t nm = (uint32_t)max(0, (int)min(j1, nmark) - (int)j0);   // markers inside the range
+    const uint32_t *src = reinterpret_cast<const uint32_t *>(u) + (off >> 2);
+    const uint32_t sh = (uint32_t)(off & 3) * 8;
+    const size_t nw = (size_t)((len + 64 + 3) >> 2);
+    for (size_t k = (size_t)blockIdx.x * blockDim.x + threadIdx.x; k < nw; k += (size_t)gridDim.x * blockDim.x) {
+        uint32_t v = 0xFFFFFFFFu;
+        if (4 * k < len) {
+            v = __funnelshift_r(src[k], src[k + 1], sh);
+            const uint64_t left = len - 4 * k;
+            if (left < 4) v |= 0xFFFFFFFFu << (8 * left);
+        }
+        dst[k] = v;
+    }
+    if (blockIdx.x == 0) {
+        for (uint32_t j = threadIdx.x; j < nm; j += blockDim.x) dst_bnd[j] = (uint32_t)(bnd[j0 + j] - off);
+        if (threadIdx.x == 0) { dst_bnd[nm] = 0xFFFFFFFFu; *dst_nmark = nm; *dst_len = len; }
+    }
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -904,23 +947,35 @@ template <int N>
 __device__ __forceinline__ void cp_async_wait() { asm volatile("cp.async.wait_group %0;" ::"n"(N) : "memory"); }
 
 // GRAY: only the luma blocks are transformed and their samples go straight to the caller's 8-bit image (py, pitch
-// out_step), cut at the image's right and bottom edges: no Y plane in between (it would cost two more passes over W * H
-// bytes) and no colour kernel behind it.
-template <bool GRAY>
+// out_step), cut at the region's edges: no Y plane in between (it would cost two more passes over W * H bytes) and no
+// colour kernel behind it.
+// WIN (a decode region): the blocks walked are those of the window's MCUs (w.mx0 .. w.mx1 of each of the rows w.my0 ..
+// w.my1, in scan order): window block wb is coefficient block cbase + row * (mcux bpm) + (wb - row * wbpr). Without
+// WIN the whole image is walked with its own addressing (w is not read): the full-size decode pays nothing for regions.
+template <bool GRAY, bool WIN>
 __global__ void __launch_bounds__(256, 2)
-k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom g, const DecTables *__restrict__ tb,
+k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom g, DecWin w, const DecTables *__restrict__ tb,
        uint8_t *__restrict__ py, uint8_t *__restrict__ pcb, uint8_t *__restrict__ pcr, int rst_mcus, size_t out_step) {
     extern __shared__ __align__(16) uint4 s_c[];   // [2][IDCT_TILE * 8], chunk c of block b at b * 8 + (c ^ (b & 7))
     __shared__ __align__(16) int s_q[2][64];       // zig-zag order
     const int tid = threadIdx.x;
-    const int ntile = (g.nblocks + IDCT_TILE - 1) / IDCT_TILE;
+    const int rowb = g.mcux * g.bpm;                                              // blocks per image row
+    const int wbpr = WIN ? (w.mx1 - w.mx0) * g.bpm : rowb;                        // ... per window row
+    const int nwb = WIN ? (w.my1 - w.my0) * wbpr : g.nblocks;
+    const int cbase = WIN ? (w.my0 * g.mcux + w.mx0 - w.m0) * g.bpm : 0;
+    const int ntile = (nwb + IDCT_TILE - 1) / IDCT_TILE;
     const uint4 *coef4 = reinterpret_cast<const uint4 *>(coef);
     auto issue = [&](int tile, int buf) {
-        const int b0 = tile * IDCT_TILE, nb = min(IDCT_TILE, g.nblocks - b0);
+        const int b0 = tile * IDCT_TILE, nb = min(IDCT_TILE, nwb - b0);
         uint4 *dstb = s_c + buf * (IDCT_TILE * 8);
         for (int i = tid; i < nb * 8; i += 256) {
             const int b = i >> 3, c = i & 7;
-            cp_async16(dstb + b * 8 + (c ^ (b & 7)), coef4 + (size_t)b0 * 8 + i);
+            if (WIN) {
+                const int wb = b0 + b, r = wb / wbpr;
+                cp_async16(dstb + b * 8 + (c ^ (b & 7)), coef4 + (size_t)(cbase + r * rowb + (wb - r * wbpr)) * 8 + c);
+            } else {
+                cp_async16(dstb + b * 8 + (c ^ (b & 7)), coef4 + (size_t)b0 * 8 + i);
+            }
         }
         cp_async_commit();
     };
@@ -933,12 +988,20 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
         if (tn < ntile) { issue(tn, (k + 1) & 1); cp_async_wait<1>(); }
         else cp_async_wait<0>();
         __syncthreads();   // tile t has landed (every thread waited for its own requests)
-        const int b0 = t * IDCT_TILE, nb = min(IDCT_TILE, g.nblocks - b0);
-        if (tid < nb && (!GRAY || (b0 + tid) % g.bpm < hv)) {
+        const int b0 = t * IDCT_TILE, nb = min(IDCT_TILE, nwb - b0);
+        int b, m, bn, my, mx;   // coefficient block, its MCU, its index in the MCU, MCU row and column
+        if (WIN) {
+            const int wb = b0 + tid, r = wb / wbpr, o = wb - r * wbpr, mm = o / g.bpm;
+            bn = o - mm * g.bpm;
+            b = cbase + r * rowb + o;
+            my = w.my0 + r; mx = w.mx0 + mm; m = my * g.mcux + mx;
+        } else {
+            b = b0 + tid;
+            m = b / g.bpm; bn = b - m * g.bpm;
+            my = m / g.mcux; mx = m - my * g.mcux;
+        }
+        if (tid < nb && (!GRAY || bn < hv)) {
             const uint4 *sc = s_c + (k & 1) * (IDCT_TILE * 8);
-            const int b = b0 + tid;
-            const int m = b / g.bpm, bn = b - m * g.bpm;
-            const int my = m / g.mcux, mx = m - my * g.mcux;
             const bool isY = bn < hv;
             const int4 *q4 = reinterpret_cast<const int4 *>(s_q[isY ? 0 : 1]);
             int v[64];
@@ -960,9 +1023,11 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
             // the un-differenced DC (the coefficient array holds the difference): k_dc_scan's running sum, taken from the
             // start of the block's restart interval (predictors return to 0 there; 16-bit modular differences are exact)
             // (dcarr == NULL: the blocks come from the encoder and hold the quantised DC itself -- b2j_reconstruct_*)
+            // (the sum starts at block 0, the first block of MCU m0: an interval start)
+            const int m0 = WIN ? w.m0 : 0;
             int dcv = dcarr ? (int)dcarr[b] : c0raw;
-            if (dcarr && rst_mcus > 0 && m >= rst_mcus) {
-                const int pm = (m / rst_mcus) * rst_mcus - 1;   // last MCU of the previous interval
+            if (dcarr && rst_mcus > 0 && (WIN ? (m / rst_mcus) * rst_mcus > m0 : m >= rst_mcus)) {
+                const int pm = (m / rst_mcus) * rst_mcus - 1 - m0;   // last MCU of the previous interval
                 dcv = (int16_t)(dcv - (int)dcarr[pm * g.bpm + (isY ? hv - 1 : bn)]);
             }
             v[0] = dcv * s_q[isY ? 0 : 1][0];
@@ -970,21 +1035,25 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
             for (int c = 0; c < 8; c++) idct8<11>(v[c], v[8 + c], v[16 + c], v[24 + c], v[32 + c], v[40 + c], v[48 + c], v[56 + c]);
             uint8_t *dst;
             size_t stride;
-            int gx0 = 0, nrow = 8;   // GRAY: the block's first column and its rows inside the image
+            // GRAY: the block's columns [c0, c1) and rows [r0, r1) inside the region (without WIN: the image)
+            // (WIN: the block's first row and column relative to the region, gy0 / gx0, may be negative: dst is the region's
+            // first row, and row r of the block is region row gy0 + r, its column c at gx0 + c)
+            int c0 = 0, c1 = 8, r0 = 0, r1 = 8, gy0 = 0, gx0 = 0;
             if (GRAY) {
                 const int by = bn / g.hs, bx = bn - by * g.hs;
-                const int gy0 = (my * g.vs + by) * 8;
-                gx0 = (mx * g.hs + bx) * 8;
-                nrow = min(8, g.H - gy0);
+                gy0 = (my * g.vs + by) * 8 - (WIN ? w.oy : 0); gx0 = (mx * g.hs + bx) * 8 - (WIN ? w.ox : 0);
+                if (WIN) { c0 = max(0, -gx0); r0 = max(0, -gy0); }
+                c1 = min(8, (WIN ? w.ow : g.W) - gx0);
+                r1 = min(8, (WIN ? w.oh : g.H) - gy0);
                 stride = out_step;
-                dst = py + (size_t)gy0 * stride + (size_t)gx0;
+                dst = WIN ? py : py + (size_t)gy0 * stride + (size_t)gx0;
             } else if (isY) {
                 const int by = bn / g.hs, bx = bn - by * g.hs;
-                stride = (size_t)g.mcux * 8 * g.hs;
-                dst = py + ((size_t)(my * g.vs + by) * 8) * stride + (size_t)(mx * g.hs + bx) * 8;
+                stride = WIN ? (size_t)w.ys : (size_t)g.mcux * 8 * g.hs;
+                dst = py + ((size_t)((my - (WIN ? w.my0 : 0)) * g.vs + by) * 8) * stride + (size_t)((mx * g.hs + bx) * 8 - (WIN ? w.px : 0));
             } else {
-                stride = (size_t)g.mcux * 8;
-                dst = (bn == hv ? pcb : pcr) + ((size_t)my * 8) * stride + (size_t)mx * 8;
+                stride = WIN ? (size_t)w.cs : (size_t)g.mcux * 8;
+                dst = (bn == hv ? pcb : pcr) + ((size_t)(my - (WIN ? w.my0 : 0)) * 8) * stride + (size_t)(mx * 8 - (WIN ? w.cx : 0));
             }
 #pragma unroll
             for (int r = 0; r < 8; r++) {
@@ -996,10 +1065,18 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
                 const uint32_t hi = __byte_perm(__byte_perm(x[4], x[5], 0x0040), __byte_perm(x[6], x[7], 0x0040), 0x5410);
                 if (!GRAY) {
                     *reinterpret_cast<uint2 *>(dst + r * stride) = make_uint2(lo, hi);
-                } else if (r < nrow) {
-                    uint8_t *d = dst + r * stride;
-                    if (gx0 + 8 <= g.W && ((reinterpret_cast<uintptr_t>(d) & 7) == 0)) *reinterpret_cast<uint2 *>(d) = make_uint2(lo, hi);
-                    else for (int c = 0; c < min(8, g.W - gx0); c++) d[c] = (uint8_t)x[c];
+                } else if (r >= r0 && r < r1) {
+                    uint8_t *d = WIN ? dst + (size_t)(gy0 + r) * stride : dst + r * stride;
+                    const int cb = WIN ? gx0 : 0;
+                    if (c0 == 0 && c1 == 8 && ((reinterpret_cast<uintptr_t>(d + cb) & 7) == 0)) {
+                        *reinterpret_cast<uint2 *>(d + cb) = make_uint2(lo, hi);
+                    } else if (!WIN) {
+                        for (int c = 0; c < c1; c++) d[c] = (uint8_t)x[c];
+                    } else {   // unrolled with a predicate: x stays in registers
+#pragma unroll
+                        for (int c = 0; c < 8; c++)
+                            if (c >= c0 && c < c1) d[cb + c] = (uint8_t)x[c];
+                    }
                 }
             }
         }
@@ -1010,35 +1087,41 @@ k_idct(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom
 // ------------------------------------------------------------------------------------------------------
 // k_upcolor: jdsample.c fancy upsampling (h2v1 / h2v2 / h1v2 triangle filters, h4v1 replication) on the TRUE
 // downsampled size + jdcolor.c YCbCr->RGB, 8 pixels per thread, stored interleaved B,G,R (cv::Mat CV_8UC3).
+// Coordinates x, y and the edge rules (dw, rlo, rhi) are the true image's; the plane holds chroma rows from cy and
+// columns from cx on (a decode region's window; 0, 0 for the whole image): chroma sample (i, r) at p[(r - cy) stride + i - cx].
 template <int HS, int VS>
-__device__ __forceinline__ int chroma_at(const uint8_t *__restrict__ p, size_t stride, int dw, int rlo, int rhi, int x, int y) {
-    if (HS == 1 && VS == 1) return p[(size_t)y * stride + x];
-    if (HS == 4) return p[(size_t)y * stride + (x >> 2)];
+__device__ __forceinline__ int chroma_at(const uint8_t *__restrict__ p, size_t stride, int cx, int cy, int dw, int rlo, int rhi, int x, int y) {
+    auto row = [&](int r) { return p + (size_t)(r - cy) * stride; };
+    if (HS == 1 && VS == 1) return row(y)[x - cx];
+    if (HS == 4) return row(y)[(x >> 2) - cx];
     if (HS == 2 && VS == 1) {
-        const uint8_t *row = p + (size_t)y * stride;
+        const uint8_t *rw = row(y);
         const int i = x >> 1;
-        if (dw <= 2) return row[i];
-        if (x & 1) return i < dw - 1 ? (3 * row[i] + row[i + 1] + 2) >> 2 : row[dw - 1];
-        return i > 0 ? (3 * row[i] + row[i - 1] + 1) >> 2 : row[0];
+        if (dw <= 2) return rw[i - cx];
+        if (x & 1) return i < dw - 1 ? (3 * rw[i - cx] + rw[i + 1 - cx] + 2) >> 2 : rw[dw - 1 - cx];
+        return i > 0 ? (3 * rw[i - cx] + rw[i - 1 - cx] + 1) >> 2 : rw[-cx];
     }
     if (HS == 1 && VS == 2) {
         const int r = y >> 1;
         const int rn = (y & 1) ? min(r + 1, rhi) : max(r - 1, rlo);
-        return (3 * p[(size_t)r * stride + x] + p[(size_t)rn * stride + x] + ((y & 1) ? 2 : 1)) >> 2;
+        return (3 * row(r)[x - cx] + row(rn)[x - cx] + ((y & 1) ? 2 : 1)) >> 2;
     }
     // h2v2
-    const int r = y >> 1, i = x >> 1;
-    if (dw <= 2) return p[(size_t)r * stride + i];
+    const int r = y >> 1, i = x >> 1, ir = i - cx;   // ir: the column in the plane
+    if (dw <= 2) return row(r)[ir];
     const int rn = (y & 1) ? min(r + 1, rhi) : max(r - 1, rlo);
-    const uint8_t *r0 = p + (size_t)r * stride, *r1 = p + (size_t)rn * stride;
-    const int s = 3 * r0[i] + r1[i];
-    if (x & 1) return i < dw - 1 ? (3 * s + 3 * r0[i + 1] + r1[i + 1] + 7) >> 4 : (4 * s + 7) >> 4;
-    return i > 0 ? (3 * s + 3 * r0[i - 1] + r1[i - 1] + 8) >> 4 : (4 * s + 8) >> 4;
+    const uint8_t *r0 = row(r), *r1 = row(rn);
+    const int s = 3 * r0[ir] + r1[ir];
+    if (x & 1) return i < dw - 1 ? (3 * s + 3 * r0[ir + 1] + r1[ir + 1] + 7) >> 4 : (4 * s + 7) >> 4;
+    return i > 0 ? (3 * s + 3 * r0[ir - 1] + r1[ir - 1] + 8) >> 4 : (4 * s + 8) >> 4;
 }
 
-// the same eight upsampled chroma samples for an INTERIOR group (every neighbour exists): word loads, no edge tests
+// the same eight upsampled chroma samples for an INTERIOR group (every neighbour exists): word loads, no edge tests.
+// The plane as in chroma_at; cx is a multiple of 8, so the word loads stay aligned
 template <int HS, int VS>
-__device__ __forceinline__ void chroma8_interior(const uint8_t *__restrict__ p, size_t stride, int rlo, int rhi, int x0, int y, int (&c)[8]) {
+__device__ __forceinline__ void chroma8_interior(const uint8_t *__restrict__ p, size_t stride, int cx, int cy, int rlo, int rhi, int x0, int y, int (&c)[8]) {
+    auto prow = [&](int r) { return p + (size_t)(r - cy) * stride; };
+    const int xr = x0 - cx * HS;   // the group's first column relative to the plane, in luma samples
     auto six = [](const uint8_t *row, int i0, int (&s)[6]) {   // samples i0 - 1 .. i0 + 4 (i0 % 4 == 0)
         const uint32_t w = *reinterpret_cast<const uint32_t *>(row + i0);
         s[0] = row[i0 - 1];
@@ -1046,17 +1129,17 @@ __device__ __forceinline__ void chroma8_interior(const uint8_t *__restrict__ p, 
         s[5] = row[i0 + 4];
     };
     if (HS == 1 && VS == 1) {
-        const uint2 w = *reinterpret_cast<const uint2 *>(p + (size_t)y * stride + x0);
+        const uint2 w = *reinterpret_cast<const uint2 *>(prow(y) + xr);
 #pragma unroll
         for (int i = 0; i < 4; i++) { c[i] = (w.x >> (8 * i)) & 0xFF; c[4 + i] = (w.y >> (8 * i)) & 0xFF; }
     } else if (HS == 4) {
-        const uint8_t *row = p + (size_t)y * stride + (x0 >> 2);
+        const uint8_t *row = prow(y) + (xr >> 2);
         const int s0 = row[0], s1 = row[1];
 #pragma unroll
         for (int i = 0; i < 4; i++) { c[i] = s0; c[4 + i] = s1; }
     } else if (HS == 2 && VS == 1) {
         int s[6];
-        six(p + (size_t)y * stride, x0 >> 1, s);
+        six(prow(y), xr >> 1, s);
 #pragma unroll
         for (int j = 0; j < 4; j++) {
             c[2 * j] = (3 * s[j + 1] + s[j] + 1) >> 2;
@@ -1065,8 +1148,8 @@ __device__ __forceinline__ void chroma8_interior(const uint8_t *__restrict__ p, 
     } else if (HS == 1 && VS == 2) {
         const int r = y >> 1;
         const int rn = (y & 1) ? min(r + 1, rhi) : max(r - 1, rlo);
-        const uint2 a = *reinterpret_cast<const uint2 *>(p + (size_t)r * stride + x0);
-        const uint2 bq = *reinterpret_cast<const uint2 *>(p + (size_t)rn * stride + x0);
+        const uint2 a = *reinterpret_cast<const uint2 *>(prow(r) + xr);
+        const uint2 bq = *reinterpret_cast<const uint2 *>(prow(rn) + xr);
         const int bias = (y & 1) ? 2 : 1;
 #pragma unroll
         for (int i = 0; i < 4; i++) {
@@ -1077,8 +1160,8 @@ __device__ __forceinline__ void chroma8_interior(const uint8_t *__restrict__ p, 
         const int r = y >> 1;
         const int rn = (y & 1) ? min(r + 1, rhi) : max(r - 1, rlo);
         int s0[6], s1[6], t[6];
-        six(p + (size_t)r * stride, x0 >> 1, s0);
-        six(p + (size_t)rn * stride, x0 >> 1, s1);
+        six(prow(r), xr >> 1, s0);
+        six(prow(rn), xr >> 1, s1);
 #pragma unroll
         for (int j = 0; j < 6; j++) t[j] = 3 * s0[j] + s1[j];
 #pragma unroll
@@ -1089,25 +1172,32 @@ __device__ __forceinline__ void chroma8_interior(const uint8_t *__restrict__ p, 
     }
 }
 
-template <int HS, int VS>
+// WIN (a decode region): the groups of 8 pixels are aligned in image coordinates and only the region's pixels are
+// computed and stored (pixel (w.ox, w.oy) at bgr); the planes hold the window (w.px, w.py: luma plane origin, w.cx, w.cy:
+// chroma). Without WIN the whole image, its own planes (w is not read).
+template <int HS, int VS, bool WIN>
 __global__ void __launch_bounds__(256)
-k_upcolor(const uint8_t *__restrict__ py, const uint8_t *__restrict__ pcb, const uint8_t *__restrict__ pcr, Geom g,
+k_upcolor(const uint8_t *__restrict__ py, const uint8_t *__restrict__ pcb, const uint8_t *__restrict__ pcr, Geom g, DecWin w,
           uint8_t *__restrict__ bgr, size_t step, int rlo, int rhi) {   // rlo / rhi: first / last chroma row the vertical filter may read
     const int gx = blockIdx.x * blockDim.x + threadIdx.x;  // group of 8 pixels
-    const int y = blockIdx.y;
-    const int x0 = gx * 8;
-    if (x0 >= g.W) return;
-    const size_t ys = (size_t)g.mcux * 8 * HS, cs = (size_t)g.mcux * 8;
+    const int ox = WIN ? w.ox : 0, xe = WIN ? w.ox + w.ow : g.W;
+    const int y = (WIN ? w.oy : 0) + blockIdx.y;
+    const int x0 = ((ox >> 3) + gx) * 8;
+    if (x0 >= xe) return;
+    const size_t ys = WIN ? (size_t)w.ys : (size_t)g.mcux * 8 * HS, cs = WIN ? (size_t)w.cs : (size_t)g.mcux * 8;
+    const int px = WIN ? w.px : 0, cx = WIN ? w.cx : 0, cy = WIN ? w.cy : 0;
     const int dw = g.dw[1];
-    uint8_t *dst = bgr + (size_t)y * step + (size_t)x0 * 3;
+    const uint8_t *yrow = py + (size_t)(y - (WIN ? w.py : 0)) * ys;   // luma column x at yrow[x - px]
+    uint8_t *dst = bgr + (size_t)blockIdx.y * step + (size_t)x0 * 3 - (size_t)ox * 3;
     uint8_t o[24];
-    // interior groups (all neighbours of all eight pixels exist, 8-byte aligned destination): vector loads and stores
-    if (x0 >= 8 && x0 + 16 <= g.W && (reinterpret_cast<uintptr_t>(dst) & 7) == 0) {
-        const uint2 yw = *reinterpret_cast<const uint2 *>(py + (size_t)y * ys + x0);
+    // interior groups (all neighbours of all eight pixels exist, all eight in the region, 8-byte aligned destination):
+    // vector loads and stores
+    if (x0 >= 8 && x0 + 16 <= g.W && x0 >= ox && x0 + 8 <= xe && (reinterpret_cast<uintptr_t>(dst) & 7) == 0) {
+        const uint2 yw = *reinterpret_cast<const uint2 *>(yrow + (x0 - px));
         int cbv[8], crv[8];
         uint32_t o32[6];
-        chroma8_interior<HS, VS>(pcb, cs, rlo, rhi, x0, y, cbv);
-        chroma8_interior<HS, VS>(pcr, cs, rlo, rhi, x0, y, crv);
+        chroma8_interior<HS, VS>(pcb, cs, cx, cy, rlo, rhi, x0, y, cbv);
+        chroma8_interior<HS, VS>(pcr, cs, cx, cy, rlo, rhi, x0, y, crv);
         // jdcolor.c ycc_rgb_convert with the tables written out: r = y + ((91881 (cr - 128) + 32768) >> 16) etc. Here y sits
         // at bit 16 of the accumulator, the -128 and the rounding are one constant per channel, the sum is clamped to
         // [0, 255.99..] and the result is byte 2 of the word: same integers, a third fewer instructions per pixel.
@@ -1140,10 +1230,11 @@ k_upcolor(const uint8_t *__restrict__ py, const uint8_t *__restrict__ pcb, const
     }
 #pragma unroll
     for (int i = 0; i < 8; i++) {
-        const int x = min(x0 + i, g.W - 1);
-        const int Y = py[(size_t)y * ys + x];
-        const int cb = chroma_at<HS, VS>(pcb, cs, dw, rlo, rhi, x, y) - 128;
-        const int cr = chroma_at<HS, VS>(pcr, cs, dw, rlo, rhi, x, y) - 128;
+        // (a region: its own pixels only, so every sample read lies in the window)
+        const int x = WIN ? min(max(x0 + i, ox), xe - 1) : min(x0 + i, g.W - 1);
+        const int Y = yrow[x - px];
+        const int cb = chroma_at<HS, VS>(pcb, cs, cx, cy, dw, rlo, rhi, x, y) - 128;
+        const int cr = chroma_at<HS, VS>(pcr, cs, cx, cy, dw, rlo, rhi, x, y) - 128;
         const int r = Y + ((91881 * cr + 32768) >> 16);
         const int b = Y + ((116130 * cb + 32768) >> 16);
         const int gg = Y + ((-22554 * cb - 46802 * cr + 32768) >> 16);
@@ -1151,8 +1242,7 @@ k_upcolor(const uint8_t *__restrict__ py, const uint8_t *__restrict__ pcb, const
         o[3 * i + 1] = (uint8_t)min(255, max(0, gg));
         o[3 * i + 2] = (uint8_t)min(255, max(0, r));
     }
-    const int nv = min(8, g.W - x0);
-    for (int j = 0; j < nv * 3; j++) dst[j] = o[j];
+    for (int j = max(0, ox - x0) * 3; j < min(8, xe - x0) * 3; j++) dst[j] = o[j];
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -1178,9 +1268,13 @@ static cudaError_t dec_attr() {
     if (e != cudaSuccess) return e;
     e = cudaFuncSetAttribute(k_dec_sync<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecShared));
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_dec_write<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecWriteShared));
+    e = cudaFuncSetAttribute(k_dec_write<false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecWriteShared));
     if (e != cudaSuccess) return e;
-    e = cudaFuncSetAttribute(k_dec_write<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecWriteShared));
+    e = cudaFuncSetAttribute(k_dec_write<true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecWriteShared));
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(k_dec_write<false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecWriteShared));
+    if (e != cudaSuccess) return e;
+    e = cudaFuncSetAttribute(k_dec_write<true, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(DecWriteShared));
     if (e != cudaSuccess) return e;
     done.fetch_or(bit, std::memory_order_release);
     return cudaSuccess;
@@ -1214,14 +1308,32 @@ cudaError_t launch_dec_sync_long(const uint8_t *u, const uint64_t *u_len, const 
 
 cudaError_t launch_dec_write(const uint8_t *u, const uint64_t *u_len, const void *tb, const uint64_t *st_out,
                              const uint32_t *blk_start, int bpm, int hv, int16_t *coef, int16_t *dcarr, uint32_t nblocks,
-                             uint32_t *err, size_t nsub_max, const uint32_t *bnd, const uint32_t *nmark, cudaStream_t s) {
+                             uint32_t *err, size_t nsub_max, const uint32_t *bnd, const uint32_t *nmark, const Geom &g,
+                             const DecWin *win, cudaStream_t s) {
     cudaError_t e = dec_attr();
     if (e != cudaSuccess) return e;
     const unsigned grid = (unsigned)((nsub_max + DEC_THREADS - 1) / DEC_THREADS);
-    if (bnd) k_dec_write<true><<<grid, DEC_THREADS, sizeof(DecWriteShared), s>>>(u, u_len, (const DecTables *)tb, st_out, blk_start, bpm,
-                                                                              hv, coef, dcarr, nblocks, err, bnd, nmark);
-    else k_dec_write<false><<<grid, DEC_THREADS, sizeof(DecWriteShared), s>>>(u, u_len, (const DecTables *)tb, st_out, blk_start, bpm,
-                                                                           hv, coef, dcarr, nblocks, err, nullptr, nullptr);
+    const size_t sm = sizeof(DecWriteShared);
+    const DecTables *t = (const DecTables *)tb;
+    if (win) {
+        const DecWin &w = *win;
+        if (bnd) k_dec_write<true, true><<<grid, DEC_THREADS, sm, s>>>(u, u_len, t, st_out, blk_start, bpm, hv, coef, dcarr, nblocks, err,
+                                                                        bnd, nmark, g.mcux, w.m0, w.mx0, w.mx1, w.my0);
+        else k_dec_write<false, true><<<grid, DEC_THREADS, sm, s>>>(u, u_len, t, st_out, blk_start, bpm, hv, coef, dcarr, nblocks, err,
+                                                                     nullptr, nullptr, g.mcux, w.m0, w.mx0, w.mx1, w.my0);
+    } else if (bnd) {
+        k_dec_write<true, false><<<grid, DEC_THREADS, sm, s>>>(u, u_len, t, st_out, blk_start, bpm, hv, coef, dcarr, nblocks, err, bnd, nmark,
+                                                                0, 0, 0, 0, 0);
+    } else {
+        k_dec_write<false, false><<<grid, DEC_THREADS, sm, s>>>(u, u_len, t, st_out, blk_start, bpm, hv, coef, dcarr, nblocks, err, nullptr,
+                                                                 nullptr, 0, 0, 0, 0, 0);
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_dec_range(const uint8_t *u, const uint64_t *u_len, const uint32_t *bnd, const uint32_t *nmark, uint32_t j0,
+                             uint32_t j1, uint8_t *dst, uint64_t *dst_len, uint32_t *dst_bnd, uint32_t *dst_nmark, cudaStream_t s) {
+    k_dec_range<<<148 * 2, 256, 0, s>>>(u, u_len, bnd, nmark, j0, j1, reinterpret_cast<uint32_t *>(dst), dst_len, dst_bnd, dst_nmark);
     return cudaGetLastError();
 }
 
@@ -1231,16 +1343,16 @@ cudaError_t launch_scan_u32(const uint32_t *in, uint32_t *out, size_t n, uint64_
     return cudaGetLastError();
 }
 
-cudaError_t launch_dc_scan(int16_t *coef, const Geom &g, int ncomp, uint64_t *desc, uint32_t *ticket, size_t desc_stride,
+cudaError_t launch_dc_scan(int16_t *coef, const Geom &g, size_t nmcu, int ncomp, uint64_t *desc, uint32_t *ticket, size_t desc_stride,
                            uint32_t *err, cudaStream_t s) {
     dim3 grid(148 * 2, ncomp);
-    k_dc_scan<<<grid, 256, 0, s>>>(coef, g.bpm, g.hs * g.vs, (size_t)g.mcux * g.mcuy, desc, ticket, desc_stride, err);
+    k_dc_scan<<<grid, 256, 0, s>>>(coef, g.bpm, g.hs * g.vs, nmcu, desc, ticket, desc_stride, err);
     return cudaGetLastError();
 }
 
-template <bool GRAY>
-static cudaError_t idct_launch(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *py, uint8_t *pcb,
-                               uint8_t *pcr, int rst_mcus, size_t out_step, cudaStream_t s) {
+template <bool GRAY, bool WIN>
+static cudaError_t idct_launch(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecWin &w, const void *tb, uint8_t *py,
+                               uint8_t *pcb, uint8_t *pcr, int rst_mcus, size_t out_step, cudaStream_t s) {
     // the dynamic shared-memory attribute is per device: one bit per device ordinal
     static std::atomic<uint64_t> attr_done{0};
     int dev = 0;
@@ -1248,41 +1360,48 @@ static cudaError_t idct_launch(const int16_t *coef, const int16_t *dcarr, const 
     if (e != cudaSuccess) return e;
     const uint64_t bit = 1ull << (dev & 63);
     if (!(attr_done.load(std::memory_order_acquire) & bit)) {
-        e = cudaFuncSetAttribute(k_idct<GRAY>, cudaFuncAttributeMaxDynamicSharedMemorySize, IDCT_SMEM);
+        e = cudaFuncSetAttribute(k_idct<GRAY, WIN>, cudaFuncAttributeMaxDynamicSharedMemorySize, IDCT_SMEM);
         if (e != cudaSuccess) return e;
         attr_done.fetch_or(bit, std::memory_order_release);
     }
-    const int ntile = (g.nblocks + IDCT_TILE - 1) / IDCT_TILE;
-    k_idct<GRAY><<<std::max(1, std::min(ntile, 148 * 2)), 256, IDCT_SMEM, s>>>(coef, dcarr, g, (const DecTables *)tb, py, pcb, pcr,
+    const int ntile = ((w.my1 - w.my0) * (w.mx1 - w.mx0) * g.bpm + IDCT_TILE - 1) / IDCT_TILE;
+    k_idct<GRAY, WIN><<<std::max(1, std::min(ntile, 148 * 2)), 256, IDCT_SMEM, s>>>(coef, dcarr, g, w, (const DecTables *)tb, py, pcb, pcr,
                                                                                rst_mcus, out_step);
     return cudaGetLastError();
 }
 
-cudaError_t launch_idct(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *py, uint8_t *pcb,
-                        uint8_t *pcr, int rst_mcus, cudaStream_t s) {
-    return idct_launch<false>(coef, dcarr, g, tb, py, pcb, pcr, rst_mcus, 0, s);
+cudaError_t launch_idct(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecWin *w, const void *tb, uint8_t *py,
+                        uint8_t *pcb, uint8_t *pcr, int rst_mcus, cudaStream_t s) {
+    const int whole[4] = {0, 0, 0, 0};
+    if (w && !w->whole) return idct_launch<false, true>(coef, dcarr, g, *w, tb, py, pcb, pcr, rst_mcus, 0, s);
+    return idct_launch<false, false>(coef, dcarr, g, dec_window(g, 1, whole), tb, py, pcb, pcr, rst_mcus, 0, s);
 }
 
-cudaError_t launch_idct_gray(const int16_t *coef, const int16_t *dcarr, const Geom &g, const void *tb, uint8_t *gray, size_t step,
-                             int rst_mcus, cudaStream_t s) {
-    return idct_launch<true>(coef, dcarr, g, tb, gray, nullptr, nullptr, rst_mcus, step, s);
+cudaError_t launch_idct_gray(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecWin &w, const void *tb, uint8_t *gray,
+                             size_t step, int rst_mcus, cudaStream_t s) {
+    if (!w.whole) return idct_launch<true, true>(coef, dcarr, g, w, tb, gray, nullptr, nullptr, rst_mcus, step, s);
+    return idct_launch<true, false>(coef, dcarr, g, w, tb, gray, nullptr, nullptr, rst_mcus, step, s);
 }
 
 template <int HS, int VS>
-static cudaError_t upcolor_one(const uint8_t *py, const uint8_t *pcb, const uint8_t *pcr, const Geom &g, uint8_t *bgr,
+static cudaError_t upcolor_one(const uint8_t *py, const uint8_t *pcb, const uint8_t *pcr, const Geom &g, const DecWin &w, uint8_t *bgr,
                                size_t step, int halo_top, int halo_bottom, cudaStream_t s) {
-    dim3 grid(((g.W + 7) / 8 + 255) / 256, g.H);
-    k_upcolor<HS, VS><<<grid, 256, 0, s>>>(py, pcb, pcr, g, bgr, step, halo_top ? -1 : 0, halo_bottom ? g.dh[1] : g.dh[1] - 1);
+    dim3 grid((((w.ox + w.ow + 7) / 8 - w.ox / 8) + 255) / 256, w.oh);
+    const int rlo = halo_top ? -1 : 0, rhi = halo_bottom ? g.dh[1] : g.dh[1] - 1;
+    if (w.whole) k_upcolor<HS, VS, false><<<grid, 256, 0, s>>>(py, pcb, pcr, g, w, bgr, step, rlo, rhi);
+    else k_upcolor<HS, VS, true><<<grid, 256, 0, s>>>(py, pcb, pcr, g, w, bgr, step, rlo, rhi);
     return cudaGetLastError();
 }
 
-cudaError_t launch_upcolor(const uint8_t *py, const uint8_t *pcb, const uint8_t *pcr, const Geom &g, uint8_t *bgr, size_t step,
-                           cudaStream_t s, int halo_top, int halo_bottom) {
-    if (g.hs == 1 && g.vs == 1) return upcolor_one<1, 1>(py, pcb, pcr, g, bgr, step, halo_top, halo_bottom, s);
-    if (g.hs == 2 && g.vs == 1) return upcolor_one<2, 1>(py, pcb, pcr, g, bgr, step, halo_top, halo_bottom, s);
-    if (g.hs == 1 && g.vs == 2) return upcolor_one<1, 2>(py, pcb, pcr, g, bgr, step, halo_top, halo_bottom, s);
-    if (g.hs == 2 && g.vs == 2) return upcolor_one<2, 2>(py, pcb, pcr, g, bgr, step, halo_top, halo_bottom, s);
-    if (g.hs == 4 && g.vs == 1) return upcolor_one<4, 1>(py, pcb, pcr, g, bgr, step, halo_top, halo_bottom, s);
+cudaError_t launch_upcolor(const uint8_t *py, const uint8_t *pcb, const uint8_t *pcr, const Geom &g, const DecWin *win, uint8_t *bgr,
+                           size_t step, cudaStream_t s, int halo_top, int halo_bottom) {
+    const int whole[4] = {0, 0, 0, 0};
+    const DecWin w = win ? *win : dec_window(g, 1, whole);
+    if (g.hs == 1 && g.vs == 1) return upcolor_one<1, 1>(py, pcb, pcr, g, w, bgr, step, halo_top, halo_bottom, s);
+    if (g.hs == 2 && g.vs == 1) return upcolor_one<2, 1>(py, pcb, pcr, g, w, bgr, step, halo_top, halo_bottom, s);
+    if (g.hs == 1 && g.vs == 2) return upcolor_one<1, 2>(py, pcb, pcr, g, w, bgr, step, halo_top, halo_bottom, s);
+    if (g.hs == 2 && g.vs == 2) return upcolor_one<2, 2>(py, pcb, pcr, g, w, bgr, step, halo_top, halo_bottom, s);
+    if (g.hs == 4 && g.vs == 1) return upcolor_one<4, 1>(py, pcb, pcr, g, w, bgr, step, halo_top, halo_bottom, s);
     return cudaErrorInvalidValue;
 }
 

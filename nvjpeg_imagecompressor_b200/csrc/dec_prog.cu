@@ -337,7 +337,7 @@ k_prog_apply(const uint64_t *__restrict__ cm, const uint64_t *__restrict__ corr,
 
 int dec_progressive(const uint8_t *jpg, size_t len, const JpegInfo &info, const Geom &g, int16_t *d_coef, void *d_tb,
                     uint8_t *d_planes, uint8_t *d_bgr, size_t step, bool gray_out, cudaStream_t s, uint64_t *launches,
-                    char *err, size_t errlen, int scale) {
+                    char *err, size_t errlen, int scale, const DecWin &w) {
     int rc = B2J_OK;
     uint8_t *d_all = nullptr, *d_file = nullptr, *d_u = nullptr;
     ProgScanDev *d_sc = nullptr;
@@ -417,7 +417,7 @@ int dec_progressive(const uint8_t *jpg, size_t len, const JpegInfo &info, const 
         memcpy(htb->q, info.qt, sizeof(htb->q));
         PCK(cudaMemcpyAsync(d_tb, htb, dec_tables_size(), cudaMemcpyHostToDevice, s));
         // the blocks hold their own DCs (dcarr NULL)
-        PCK(dec_back_end(d_coef, nullptr, g, d_tb, d_planes, d_bgr, step, gray_out, scale, 0, s, nullptr, nullptr, launches));
+        PCK(dec_back_end(d_coef, nullptr, g, w, d_tb, d_planes, d_bgr, step, gray_out, scale, 0, s, nullptr, nullptr, launches));
     }
     PCK(cudaStreamSynchronize(s));   // the host vectors and the temporary buffers go away below
 done:

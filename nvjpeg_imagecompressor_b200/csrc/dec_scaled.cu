@@ -129,16 +129,18 @@ __device__ __forceinline__ void store_plane(uint8_t *dst, size_t stride, const u
     }
 }
 
-// One thread per block, persistent CTAs; every warp takes 32 consecutive blocks at a time and loads the coefficients of
-// those that need them (output size above 1) with coalesced 16-byte loads into its own bank-swizzled shared slice.
-// g: the file's block layout; v: the scaled view (dec_scale_setup): output size v.W x v.H, Y plane pitch
-// v.mcux * 8 * v.hs, chroma pitch v.mcux * 8.
-// S / SC: output size of a luma / chroma block. GRAY: luma only, straight into the caller's pitched image, clipped at
-// v.W / v.H. REP (SC = 1 only): 1 = every chroma sample stored twice side by side, 2 = twice one above the other (the
-// plain replication libjpeg does for 4:2:2 / 4:4:0 at 1/8, where its fancy filters are off).
+// One thread per block, persistent CTAs; every warp takes 32 consecutive blocks of the window at a time (k_idct's walk:
+// the blocks of the MCUs w.mx0 .. w.mx1 of the rows w.my0 .. w.my1) and loads the coefficients of those that need them
+// (output size above 1) with coalesced 16-byte loads into its own bank-swizzled shared slice.
+// g: the file's block layout; w: the window (dec_window): planes of pitch w.ys / w.cs whose sample (0, 0) is view sample
+// (w.px, w.py) / chroma sample (w.cx, w.cy).
+// S / SC: output size of a luma / chroma block. GRAY: luma only, straight into the caller's pitched image, clipped to
+// the region (pixel (w.ox, w.oy) at py). REP (SC = 1 only): 1 = every chroma sample stored twice side by side, 2 =
+// twice one above the other (the plain replication libjpeg does for 4:2:2 / 4:4:0 at 1/8, where its fancy filters are
+// off).
 template <int S, int SC, bool GRAY, int REP>
 __global__ void __launch_bounds__(SC_THREADS)
-k_idct_scaled(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom g, Geom v, const DecTables *__restrict__ tb,
+k_idct_scaled(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcarr, Geom g, DecWin w, const DecTables *__restrict__ tb,
               uint8_t *__restrict__ py, uint8_t *__restrict__ pcb, uint8_t *__restrict__ pcr, int rst_mcus, size_t out_step) {
     constexpr bool LOAD = S > 1 || (!GRAY && SC > 1);   // some block needs more than its DC
     __shared__ __align__(16) uint4 s_c[LOAD ? SC_THREADS * 8 : 1];
@@ -147,35 +149,37 @@ k_idct_scaled(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcar
     if (tid < 128) s_q[tid >> 6][tid & 63] = (int)tb->q[tid >> 6][tid & 63];
     __syncthreads();
     const int hv = GRAY ? g.hs * g.vs : g.bpm - 2;   // luma blocks per MCU (a colour file on a gray context keeps its chroma)
-    const size_t ys = (size_t)v.mcux * 8 * v.hs, cs = (size_t)v.mcux * 8;
+    const size_t ys = (size_t)w.ys, cs = (size_t)w.cs;
+    const int wbpr = (w.mx1 - w.mx0) * g.bpm, rowb = g.mcux * g.bpm;   // blocks per window row / per image row
+    const int nwb = (w.my1 - w.my0) * wbpr;
+    const int cbase = (w.my0 * g.mcux + w.mx0 - w.m0) * g.bpm;
     uint4 *sw = s_c + (LOAD ? warp * 32 * 8 : 0);
     const uint4 *coef4 = reinterpret_cast<const uint4 *>(coef);
-    // the block needs its coefficients (not only its DC): a luma block if S > 1, a chroma block if SC > 1
-    auto wants = [&](int b) {
-        const int bn = b % g.bpm;
-        return bn < hv ? S > 1 : (!GRAY && SC > 1);
-    };
-    for (int base = (blockIdx.x * (SC_THREADS / 32) + warp) * 32; base < g.nblocks; base += gridDim.x * SC_THREADS) {
+    for (int base = (blockIdx.x * (SC_THREADS / 32) + warp) * 32; base < nwb; base += gridDim.x * SC_THREADS) {
+        const int wb = base + lane, r = wb / wbpr, ro = wb - r * wbpr, mm = ro / g.bpm, bn = ro - mm * g.bpm;
+        const int b = cbase + r * rowb + ro;   // coefficient block
+        // the block needs its coefficients (not only its DC): a luma block if S > 1, a chroma block if SC > 1
+        const bool want = wb < nwb && (bn < hv ? S > 1 : (!GRAY && SC > 1));
         if (LOAD) {
             __syncwarp();   // the slice's previous blocks are done
 #pragma unroll
             for (int i = 0; i < 8; i++) {
-                const int k = i * 32 + lane, bl = k >> 3, c = k & 7, b = base + bl;
-                if (b < g.nblocks && wants(b)) sw[bl * 8 + (c ^ (bl & 7))] = __ldg(coef4 + (size_t)b * 8 + c);
+                const int k = i * 32 + lane, bl = k >> 3, c = k & 7;
+                const int bb = __shfl_sync(0xffffffffu, b, bl);
+                if (__shfl_sync(0xffffffffu, want, bl)) sw[bl * 8 + (c ^ (bl & 7))] = __ldg(coef4 + (size_t)bb * 8 + c);
             }
             __syncwarp();
         }
-        const int b = base + lane;
-        if (b >= g.nblocks) continue;
-        const int m = b / g.bpm, bn = b - m * g.bpm;
+        if (wb >= nwb) continue;
         if (GRAY && bn >= hv) continue;
-        const int my = m / g.mcux, mx = m - my * g.mcux;
+        const int my = w.my0 + r, mx = w.mx0 + mm, m = my * g.mcux + mx;
         const bool isY = bn < hv;
         // the un-differenced DC, as k_idct takes it: k_dc_scan's running sum from the start of the block's restart
-        // interval, or (dcarr == NULL: progressive files) the coefficient array's own DC
+        // interval (the sum starts at block 0, the first block of MCU w.m0), or (dcarr == NULL: progressive files) the
+        // coefficient array's own DC
         int dcv = dcarr ? (int)dcarr[b] : (int)coef[(size_t)b * 64];
-        if (dcarr && rst_mcus > 0 && m >= rst_mcus) {
-            const int pm = (m / rst_mcus) * rst_mcus - 1;   // last MCU of the previous interval
+        if (dcarr && rst_mcus > 0 && (m / rst_mcus) * rst_mcus > w.m0) {
+            const int pm = (m / rst_mcus) * rst_mcus - 1 - w.m0;   // last MCU of the previous interval
             dcv = (int16_t)(dcv - (int)dcarr[pm * g.bpm + (isY ? hv - 1 : bn)]);
         }
         const int *q = s_q[isY ? 0 : 1];
@@ -185,42 +189,48 @@ k_idct_scaled(const int16_t *__restrict__ coef, const int16_t *__restrict__ dcar
             block_samples<S>(sc, lane & 7, q, dcv, o);
             const int by = bn / g.hs, bx = bn - by * g.hs;
             const int gy0 = (my * g.vs + by) * S, gx0 = (mx * g.hs + bx) * S;
-            if (GRAY) {
-                const int nr = min(S, v.H - gy0), ncol = min(S, v.W - gx0);
-                uint8_t *dst = py + (size_t)gy0 * out_step + gx0;
-                for (int r = 0; r < nr; r++)
-                    for (int c = 0; c < ncol; c++) dst[(size_t)r * out_step + c] = o[r * S + c];
+            if (GRAY) {   // relative to the region
+                const int ry = gy0 - w.oy, rx = gx0 - w.ox;
+                const int r0 = max(0, -ry), r1 = min(S, w.oh - ry), c0 = max(0, -rx), c1 = min(S, w.ow - rx);
+#pragma unroll
+                for (int rr = 0; rr < S; rr++) {   // unrolled with predicates: o stays in registers
+#pragma unroll
+                    for (int c = 0; c < S; c++)
+                        if (rr >= r0 && rr < r1 && c >= c0 && c < c1) py[(size_t)(ry + rr) * out_step + (rx + c)] = o[rr * S + c];
+                }
             } else {
-                store_plane<S>(py + (size_t)gy0 * ys + gx0, ys, o);
+                store_plane<S>(py + (size_t)(gy0 - w.py) * ys + (gx0 - w.px), ys, o);
             }
         } else if (!GRAY) {
             block_samples<SC>(sc, lane & 7, q, dcv, o);
             uint8_t *pl = bn == hv ? pcb : pcr;
             if (REP == 1) {
-                pl[(size_t)my * cs + 2 * mx] = o[0];
-                pl[(size_t)my * cs + 2 * mx + 1] = o[0];
+                uint8_t *d = pl + (size_t)(my - w.cy) * cs + (2 * mx - w.cx);
+                d[0] = o[0];
+                d[1] = o[0];
             } else if (REP == 2) {
-                pl[(size_t)(2 * my) * cs + mx] = o[0];
-                pl[(size_t)(2 * my + 1) * cs + mx] = o[0];
+                uint8_t *d = pl + (size_t)(2 * my - w.cy) * cs + (mx - w.cx);
+                d[0] = o[0];
+                d[cs] = o[0];
             } else {
-                store_plane<SC>(pl + (size_t)my * SC * cs + (size_t)mx * SC, cs, o);
+                store_plane<SC>(pl + (size_t)(my * SC - w.cy) * cs + (size_t)(mx * SC - w.cx), cs, o);
             }
         }
     }
 }
 
 template <int S, int SC, bool GRAY, int REP>
-static cudaError_t scaled_one(const int16_t *coef, const int16_t *dcarr, const Geom &g, const Geom &v, const void *tb, uint8_t *py,
+static cudaError_t scaled_one(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecWin &v, const void *tb, uint8_t *py,
                               uint8_t *pcb, uint8_t *pcr, int rst_mcus, size_t out_step, cudaStream_t s) {
-    const int nwarps = (g.nblocks + 31) / 32;
+    const int nwarps = ((v.my1 - v.my0) * (v.mx1 - v.mx0) * g.bpm + 31) / 32;
     const int grid = std::max(1, std::min((nwarps + SC_THREADS / 32 - 1) / (SC_THREADS / 32), 148 * 4));
     k_idct_scaled<S, SC, GRAY, REP><<<grid, SC_THREADS, 0, s>>>(coef, dcarr, g, v, (const DecTables *)tb, py, pcb, pcr, rst_mcus, out_step);
     return cudaGetLastError();
 }
 
-cudaError_t launch_idct_scaled(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecScale &sc, const void *tb,
-                               uint8_t *py, uint8_t *pcb, uint8_t *pcr, bool gray, size_t out_step, int rst_mcus, cudaStream_t s) {
-    const Geom &v = sc.view;
+cudaError_t launch_idct_scaled(const int16_t *coef, const int16_t *dcarr, const Geom &g, const DecScale &sc, const DecWin &v,
+                               const void *tb, uint8_t *py, uint8_t *pcb, uint8_t *pcr, bool gray, size_t out_step, int rst_mcus,
+                               cudaStream_t s) {
     if (gray) {
         if (sc.S == 4) return scaled_one<4, 4, true, 0>(coef, dcarr, g, v, tb, py, nullptr, nullptr, rst_mcus, out_step, s);
         if (sc.S == 2) return scaled_one<2, 2, true, 0>(coef, dcarr, g, v, tb, py, nullptr, nullptr, rst_mcus, out_step, s);

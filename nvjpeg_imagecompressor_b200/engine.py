@@ -133,6 +133,15 @@ class Engine:
         decode_device / decode_scan_device write and report the reduced size ceil(W / denom) x ceil(H / denom)."""
         self._ck(self._L.b2j_set_decode_scale(self._h, int(denom)))
 
+    def set_decode_region(self, x, y=None, w=None, h=None):
+        """Decode only columns x .. x + w - 1 and rows y .. y + h - 1 of the output (after the decode scale): decode
+        returns and decode_device / decode_scan_device write and report that (h, w) rectangle of what they would return
+        without it. set_decode_region(None) (or 0, 0, 0, 0) is the whole image. A region outside a file's output size
+        makes its decode fail before anything is written."""
+        if x is None:
+            x = y = w = h = 0
+        self._ck(self._L.b2j_set_decode_region(self._h, int(x), int(y), int(w), int(h)))
+
     # ---------------------------------------------------------------- device API (pointers from torch tensors)
     def decode_scan_device(self, hdr, d_scan_ptr, scan_len, d_bgr_ptr, step, height_override=0):
         """Baseline JPEG with its scan bytes already in device memory (hdr: host bytes SOI .. SOS header) -> (W, H)."""
